@@ -4,7 +4,7 @@ bench.py -- headline benchmark of the wav -> x-vector hot path (BASELINE.json: "
 B200; MFCC GB/s vs HBM peak").
 
     python bench.py --gpus N --steps K --warmup W [--impl reference]
-                    [--workload wav2xvec|frontend|tdnn|plda] [--no-stages] [--no-cpu-baseline]
+                    [--workload wav2xvec|frontend|tdnn|plda] [--no-stages] [--no-cpu-baseline] [--dump-outputs DIR]
 
 Default workload (N = 1 and under torchrun): the BASELINE config 4 shard -- full wav2xvec (fused MFCC -> VAD mask +
 compaction -> CMVN(300) -> SITW TDNN on the tcgen05 stack -> statistics -> LDA / length-norm) on 1024 gated-noise
@@ -29,6 +29,10 @@ One JSON line is printed by rank 0 (DESIGN.md section 6 explains every field):
                            sub-block against the float64 oracle
 
 `--workload X` makes one of the stages the headline line with the same schema.
+
+`--dump-outputs DIR` writes what the last timed step of the headline workload returned, as DIR/<name>.npy: `xvectors`
+(wav2xvec), `features` (frontend, CMVN output), `embeddings` (tdnn), `scores` and `transformed_test` (plda).  The inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 
 `--impl reference` times the CPU port with all host threads on a bounded sample of the same workload (rank 0 only); it
 is the only other place allowed to execute oracle/.
@@ -409,6 +413,7 @@ class Harness:
             dist.init_process_group("nccl", device_id=self.dev)
         self.args = args
         self.flush_buf = None
+        self.last_output = None
 
     def barrier(self):
         if self.world > 1:
@@ -428,7 +433,8 @@ class Harness:
 
     def timed(self, step, steps, warmup, flush=False, inner=None):
         """W warm-up steps, then K steps bracketed by barrier + synchronize; returns (ms total [max over
-        ranks], launches, clocks, mean ms of the `inner` event pairs recorded by step())."""
+        ranks], launches, clocks, mean ms of the `inner` event pairs recorded by step()).  What the last timed
+        step returned is left in `self.last_output`."""
         import kaldi_tflite_b200 as ktf
         torch = self.torch
         for _ in range(max(warmup, 3)):
@@ -444,8 +450,9 @@ class Harness:
             evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
             for s in range(steps):
                 self.flush_l2()
+                self.last_output = None                       # freed before the next step, as a caller would
                 evs[s][0].record()
-                step(pairs)
+                self.last_output = step(pairs)
                 evs[s][1].record()
             self.barrier()
             ms = sum(a.elapsed_time(b) for a, b in evs)
@@ -453,7 +460,8 @@ class Harness:
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
             for s in range(steps):
-                step(pairs)
+                self.last_output = None
+                self.last_output = step(pairs)
             e1.record()
             self.barrier()
             ms = e0.elapsed_time(e1)
@@ -467,7 +475,29 @@ def ev_pair(torch):
     return torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
 
 
-def stage_tdnn(h, steps, warmup):
+DUMP_BYTES = 60 << 20                  # under 64 MB (10^6 bytes each) with the .npy headers
+
+
+def host_outputs(arrays, seed=0):
+    """{name: tensor} -> {name: float32 / float64 host array} for --dump-outputs.  Every array gets an equal share of
+    DUMP_BYTES; a larger one keeps a sample of its leading-axis rows drawn with a fixed seed (sorted), so that two
+    builds run with the same arguments dump the same elements."""
+    import torch
+    out = {}
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.dtype != torch.float64:
+            t = t.float()
+        row_bytes = t[0].numel() * t.element_size() if t.dim() > 1 else t.element_size()
+        keep = max(1, DUMP_BYTES // len(arrays) // row_bytes)
+        if t.shape[0] > keep:
+            rows = np.sort(np.random.default_rng(seed).choice(t.shape[0], size=keep, replace=False))
+            t = t[torch.from_numpy(rows).to(t.device)]
+        out[name] = t.cpu().numpy()
+    return out
+
+
+def stage_tdnn(h, steps, warmup, dump=False):
     import kaldi_tflite_b200 as ktf
     torch = h.torch
     mdl = ktf.models.SequentialFromConfig(sitw_nnet_cfg(), None, "cmvn2xvec", precision="bf16", seed=0)
@@ -477,8 +507,9 @@ def stage_tdnn(h, steps, warmup):
     offs = torch.arange(B + 1, device=h.dev, dtype=torch.int64) * Tn
 
     def step(pairs):
-        mdl.forward_ragged(feats, offs)
+        return mdl.forward_ragged(feats, offs)[0]
     ms, launches, clocks, _ = h.timed(step, steps, warmup, flush=True)
+    outputs = host_outputs({"embeddings": h.last_output}) if dump else None
     flops = (TDNN_FLOP_PER_FRAME * B * Tn + TDNN_FLOP_PER_UTT * B) * steps
     host_in = torch.empty((B * Tn, 30), dtype=torch.float32, pin_memory=True).copy_(feats)
     host_out = torch.empty((B, 512), dtype=torch.float32, pin_memory=True)
@@ -488,7 +519,7 @@ def stage_tdnn(h, steps, warmup):
         host_out.copy_(y, non_blocking=True)
     ms_e2e, _, _, _ = h.timed(e2e, steps, 2)
     return {"ms": ms, "steps": steps, "launches": launches, "clocks": clocks, "units": B * 3.0 * h.world * steps,
-            "flops": flops, "ms_e2e": ms_e2e, "h2d": B * Tn * 30 * 4, "d2h": B * 512 * 4}
+            "flops": flops, "ms_e2e": ms_e2e, "h2d": B * Tn * 30 * 4, "d2h": B * 512 * 4, "outputs": outputs}
 
 
 def h2d_ceiling(h, mbytes=256, reps=6):
@@ -517,7 +548,7 @@ def h2d_ceiling(h, mbytes=256, reps=6):
     return gbs, gbs, gbs
 
 
-def stage_wav2xvec(h, steps, warmup, batch=BATCH):
+def stage_wav2xvec(h, steps, warmup, batch=BATCH, dump=False):
     import kaldi_tflite_b200 as ktf
     torch = h.torch
     # default precision of the public API: bf16 operands on the tcgen05 stack
@@ -554,8 +585,9 @@ def stage_wav2xvec(h, steps, warmup, batch=BATCH):
             emb, _ = ext.xvec.forward_ragged(normed, voffs)
             b.record()
         pairs.append((a, b))
-        ext.backend(emb)
+        return ext.backend(emb)
     ms, launches, clocks, tdnn_ms = h.timed(step, steps, warmup)
+    outputs = host_outputs({"xvectors": h.last_output}) if dump else None
     host_in = torch.empty((batch, UTT_SAMPLES), dtype=torch.float32, pin_memory=True).copy_(wav)
     host_out = torch.empty((batch, 128), dtype=torch.float32, pin_memory=True)
 
@@ -578,7 +610,8 @@ def stage_wav2xvec(h, steps, warmup, batch=BATCH):
             "flops": TDNN_FLOP_PER_FRAME * kept + TDNN_FLOP_PER_UTT * batch, "vad_keep": kept / (batch * FRAMES),
             "ms_e2e": ms_e2e, "h2d": batch * UTT_SAMPLES * 4, "d2h": batch * 128 * 4,
             "h2d_ceiling": {"per_rank_min_gbs": ceil_min, "aggregate_gbs": ceil_sum,
-                            "how": "plain pinned cudaMemcpyAsync loop, 256 MB x 6, all ranks at once"}}
+                            "how": "plain pinned cudaMemcpyAsync loop, 256 MB x 6, all ranks at once"},
+            "outputs": outputs}
 
 
 def plda_parity(layer, x_test_rows, x_enroll_rows, got_block):
@@ -597,7 +630,7 @@ def plda_parity(layer, x_test_rows, x_enroll_rows, got_block):
     return worst
 
 
-def stage_plda(h, steps, warmup, n=50000):
+def stage_plda(h, steps, warmup, n=50000, dump=False):
     import kaldi_tflite_b200 as ktf
     from kaldi_tflite_b200 import parallel
     torch = h.torch
@@ -620,8 +653,10 @@ def stage_plda(h, steps, warmup, n=50000):
     def step(pairs):
         # transforms + the only collective (ONE asynchronous NCCL all-gather of the transformed test vectors, 25.6 MB in
         # total; the local rows are scored underneath it) + the score GEMMs of the other ranks' rows
-        parallel.plda_score_sharded(layer, x_test, x_enroll, test_counts=counts, out=scores)
+        return parallel.plda_score_sharded(layer, x_test, x_enroll, test_counts=counts, out=scores)
     ms, launches, clocks, _ = h.timed(step, steps, warmup)
+    # taken now: the checks below write into the same score buffer
+    outputs = host_outputs(dict(zip(("scores", "transformed_test"), h.last_output))) if dump else None
 
     # ---- in-run parity: sampled rows x sampled columns of THIS rank's block against the float64 oracle
     sc, u_all_chk = parallel.plda_score_sharded(layer, x_test, x_enroll, test_counts=counts, out=scores)
@@ -703,10 +738,10 @@ def stage_plda(h, steps, warmup, n=50000):
             "score_ms": score_ms, "score_bytes": float(n) * (hi - lo) * 4, "flops": 2.0 * n * (hi - lo) * PLDA_DIM,
             "allgather_ms": gather_ms, "allgather_bytes": n * PLDA_DIM * 4, "parity_max_rel": parity, "n": n,
             "score16_ms": score16_ms, "top1_ms": top1_ms,
-            "ms_e2e": ms_e2e, "h2d": 2 * (hi - lo) * PLDA_DIM * 4, "d2h": n * 4}
+            "ms_e2e": ms_e2e, "h2d": 2 * (hi - lo) * PLDA_DIM * 4, "d2h": n * 4, "outputs": outputs}
 
 
-def stage_frontend(h, steps, warmup):
+def stage_frontend(h, steps, warmup, dump=False):
     import kaldi_tflite_b200 as ktf
     torch = h.torch
     g = torch.Generator(device=h.dev).manual_seed(1234 + h.rank)
@@ -725,8 +760,9 @@ def stage_frontend(h, steps, warmup):
         feats, _ = fe.forward(wav)                           # the fused front-end kernel (one launch)
         b.record()
         pairs.append((a, b))
-        cmvn(feats)
+        return cmvn(feats)
     ms, launches, clocks, k_ms = h.timed(step, steps, warmup)
+    outputs = host_outputs({"features": h.last_output}) if dump else None
     host_in = torch.empty((BATCH, UTT_SAMPLES), dtype=torch.float32, pin_memory=True).copy_(wav)
     host_out = torch.empty((BATCH, FRAMES, NUM_CEPS), dtype=torch.float32, pin_memory=True)
 
@@ -758,7 +794,7 @@ def stage_frontend(h, steps, warmup):
             "pcm16": {"ms": ms_pcm, "kernel_ms": k_ms_pcm, "ms_e2e": ms_e2e_pcm, "h2d": BATCH * UTT_SAMPLES * 2,
                       "algo_bytes": BATCH * (UTT_SAMPLES * 2 + FRAMES * NUM_CEPS * 4)},
             "units": BATCH * UTT_SECONDS * h.world * steps, "kernel_ms": k_ms,
-            "ms_e2e": ms_e2e, "h2d": BATCH * UTT_SAMPLES * 4, "d2h": BATCH * FRAMES * NUM_CEPS * 4}
+            "ms_e2e": ms_e2e, "h2d": BATCH * UTT_SAMPLES * 4, "d2h": BATCH * FRAMES * NUM_CEPS * 4, "outputs": outputs}
 
 
 def measured_traffic(kernel_key):
@@ -854,8 +890,12 @@ def run_ours(args):
     h = Harness(args)
     pk = peaks()
     w = args.workload
-    r = STAGES[w](h, args.steps, args.warmup)
+    r = STAGES[w](h, args.steps, args.warmup, dump=args.dump_outputs is not None)
     line = None
+    if h.rank == 0 and args.dump_outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in r["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
     if h.rank == 0:
         e2e_s = r["ms_e2e"] * 1e-3 / args.steps
         line = {
@@ -938,7 +978,14 @@ def main():
     ap.add_argument("--workload", default=DEFAULT_WORKLOAD, choices=sorted(STAGES))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-stages", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the headline workload computed (rank 0) as DIR/<name>.npy, "
+                         "float32 / float64, at most 64 MB in all (larger outputs: a fixed, seeded sample of rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path (--impl ours)")
     _claim_stdout()
     if args.impl == "reference":
         run_reference(args)

@@ -191,6 +191,32 @@ def test_bench_reference_arm_prints_one_json_line():
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
 
 
+def test_bench_output_dump_is_bounded_and_seeded():
+    # bench.py --dump-outputs: float32 / float64 host arrays, at most 64 MB in all; a larger output keeps the same
+    # seeded, sorted sample of rows on every run
+    import importlib.util
+    import subprocess
+    import sys
+    import torch
+    spec = importlib.util.spec_from_file_location("ktf_bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    big = torch.arange(3000, dtype=torch.float32)[:, None].expand(3000, 8192).contiguous()     # 98 MB, row r holds r
+    small = torch.rand(7, 3, dtype=torch.float64)
+    a = bench.host_outputs({"big": big, "small": small, "half": torch.ones(4, 2, dtype=torch.bfloat16)})
+    b = bench.host_outputs({"big": big, "small": small, "half": torch.ones(4, 2, dtype=torch.bfloat16)})
+    assert sum(x.nbytes for x in a.values()) <= bench.DUMP_BYTES
+    assert a["big"].dtype == np.float32 and a["half"].dtype == np.float32 and a["small"].dtype == np.float64
+    assert np.array_equal(a["small"], small.numpy()) and np.array_equal(a["half"], np.ones((4, 2), np.float32))
+    rows = a["big"][:, 0]
+    assert 0 < len(rows) < 3000 and np.all(np.diff(rows) > 0)
+    assert np.array_equal(a["big"], big.numpy()[rows.astype(np.int64)]) and np.array_equal(a["big"], b["big"])
+    for bad in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *bad], capture_output=True, text=True,
+                           timeout=120)
+        assert p.returncode == 2 and not p.stdout, (bad, p.stderr)
+
+
 def test_committed_traffic_summary_feeds_the_bench_roofline():
     """bench.py takes roofline.traffic (DRAM bytes per launch of the dominant kernel) from profiles/r02_traffic.json, which
     scripts/summarize_profiles.py writes from the ncu --set full captures: the file must carry the three kernels the
