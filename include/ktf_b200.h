@@ -278,7 +278,13 @@ int ktf_affine_forward(const ktf_affine* a, const float* x_dev, const int64_t* i
  * stats_after_layer = index of the layer whose output is pooled over time (-1: no pooling);
  * layers after it must have context [0].  The pooled layer runs with its operands swapped and
  * accumulates the per-utterance sum / sum of squares in its epilogue (fp32), so its activation is
- * never stored.  The stack borrows the layer handles and owns a grow-only device workspace:
+ * never stored; the sums are centred on the BatchNorm moving mean of each unit (-offset / scale), so a unit
+ * whose post-ReLU values sit far above zero keeps its pooled std (no E[r^2] - E[r]^2 cancellation in fp32).
+ * Empty utterances (offsets_dev[b] == offsets_dev[b+1]) are allowed: one produces no per-frame rows, a pooled
+ * row of NaN (the mean over zero frames, as the reference's reduce_mean) that later layers compute from, and
+ * leaves the other utterances' results unchanged; nothing outside the caller's rows of feats_dev is read.
+ * The same holds for a KTF_PREC_BF16 ktf_affine_forward.
+ * The stack borrows the layer handles and owns a grow-only device workspace:
  * forward calls on ONE stack handle must be issued on one stream at a time. */
 typedef struct ktf_tdnn_stack ktf_tdnn_stack;
 int ktf_tdnn_stack_create(ktf_affine* const* layers, int32_t num_layers, int32_t stats_after_layer,

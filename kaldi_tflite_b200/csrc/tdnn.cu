@@ -233,7 +233,7 @@ int ktf_affine_create(const ktf_affine_cfg* cfg, const float* weights_host, cons
     if ((rc = ktf::upload(&a->d_offset, bn_offset_host, U)) != KTF_OK) return fail(rc);
   }
   if (cfg->precision == KTF_PREC_BF16) {
-    if ((rc = ktf::affine_tc_prepare(a, weights_host)) != KTF_OK) return fail(rc);
+    if ((rc = ktf::affine_tc_prepare(a, weights_host, bn_scale_host, bn_offset_host)) != KTF_OK) return fail(rc);
   }
   *out = a;
   return KTF_OK;

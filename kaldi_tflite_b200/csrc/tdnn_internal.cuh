@@ -13,7 +13,7 @@ struct ktf_affine {
 };
 
 namespace ktf {
-int affine_tc_prepare(ktf_affine* a, const float* weights_host);
+int affine_tc_prepare(ktf_affine* a, const float* weights_host, const float* bn_scale_host, const float* bn_offset_host);
 void affine_tc_release(ktf_affine* a);
 int affine_tc_forward(const ktf_affine* a, const float* x_dev, const int64_t* in_offsets_dev,
                       const int64_t* out_offsets_dev, int64_t batch, int64_t total_in_rows,

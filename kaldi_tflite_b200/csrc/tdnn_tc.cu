@@ -65,6 +65,7 @@ enum { kModeBf16 = 0, kModeF32 = 1, kModeStats = 2 };
 // rowmap flags
 constexpr int kRowStore = 1, kRowFirst = 2, kRowLast = 4;
 constexpr int kRowFlagMask = 7;      // bits above hold splice bookkeeping (build_padded_kernel)
+constexpr int kRowEmpty = 8;         // halo row of an empty utterance: the splices write zeros and read nothing
 
 struct TcArgs {
   int num_taps;
@@ -84,7 +85,8 @@ struct TcArgs {
   int relu;
   void* out;                // bf16 or fp32, row-major
   long long out_ld;
-  float* sums;              // STATS: (batch, 2, m_rows) raw sum / sum of squares of relu(acc + bias)
+  float* sums;              // STATS: (batch, 2, m_rows) sum / sum of squares of relu(acc + bias) - shift
+  const float* shift;       // STATS: per unit centre of the sums (TcLayer::d_shift), or nullptr = 0
   const void* act_base;     // activation matrix (the operand that streams from HBM), for the L2 prefetch
   long long act_ld_bytes;   // its row pitch and row count
   long long act_rows;
@@ -727,7 +729,10 @@ tdnn_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         }
         const bool unit_ok = row < m_rows;
         const float b = (unit_ok && a.bias) ? a.bias[row] : 0.0f;
-        const float relu_lo = a.relu ? 0.0f : -3.402823466e+38f;
+        // the sums are of r - c (TcLayer::d_shift), computed as max(acc + (b - c), lo - c): no instruction per frame
+        const float ctr = (unit_ok && a.shift) ? a.shift[row] : 0.0f;
+        const float bc = b - ctr;
+        const float relu_lo = a.relu ? -ctr : -3.402823466e+38f;
         asm volatile("bar.sync 1, 256;\n" ::: "memory");
         mbar_wait(&tfull_bar[acc], acc_phase);
         tc_fence_after();
@@ -753,7 +758,7 @@ tdnn_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             if (first != cur) { flush(); cur = first; s = 0.0f; s2 = 0.0f; }
 #pragma unroll
             for (int i = 0; i < 32; ++i) {
-              const float t = fmaxf(__uint_as_float(r[c & 1][i]) + b, relu_lo);
+              const float t = fmaxf(__uint_as_float(r[c & 1][i]) + bc, relu_lo);
               s += t;
               s2 = fmaf(t, t, s2);
             }
@@ -763,7 +768,7 @@ tdnn_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
               const int u = sc[i];
               if (u >= 0) {
                 if (u != cur) { flush(); cur = u; s = 0.0f; s2 = 0.0f; }
-                const float t = fmaxf(__uint_as_float(r[c & 1][i]) + b, relu_lo);
+                const float t = fmaxf(__uint_as_float(r[c & 1][i]) + bc, relu_lo);
                 s += t;
                 s2 = fmaf(t, t, s2);
               }
@@ -1276,11 +1281,16 @@ __global__ void build_padded_kernel(const long long* __restrict__ offs, long lon
       if (t == T - 1) f |= kRowLast;
     }
     // bits 8..11 / 12..15: frames available before / after the (clamped) frame, saturated at 15; bits 16..23: 8 + the
-    // displacement of the clamped frame (halo rows replicate the edge frames) -- used by splice_rows_kernel
-    const long long tc = min(max(t, 0LL), T - 1);
-    f |= (int)min(tc, 15LL) << 8;
-    f |= (int)min(T - 1 - tc, 15LL) << 12;
-    f |= (int)(tc - t + 8) << 16;
+    // displacement of the clamped frame (halo rows replicate the edge frames) -- used by splice_rows_kernel.  An empty
+    // utterance (T = 0) has no frame to clamp to: its 2 kHalo halo rows carry kRowEmpty and no displacement.
+    if (T > 0) {
+      const long long tc = min(max(t, 0LL), T - 1);
+      f |= (int)min(tc, 15LL) << 8;
+      f |= (int)min(T - 1 - tc, 15LL) << 12;
+      f |= (int)(tc - t + 8) << 16;
+    } else {
+      f = kRowEmpty | (8 << 16);
+    }
     rowmap[p0 + i] = f;
     rowseg[p0 + i] = real ? (int)b : -1 - (int)b;
   }
@@ -1319,7 +1329,7 @@ __global__ void splice_kernel(const TIn* __restrict__ x, int D, long long x_ld, 
     for (int i = 0; i < 8; ++i) {
       const int c = c0 + i;
       float f = 0.0f;
-      if (c < cols) {
+      if (c < cols && T > 0) {                     // an empty utterance has no frame to clamp to: zero rows
         const int k = c / D, d = c - k * D;
         const long long tt = min(max(t + s_ctx[k], 0LL), T - 1);
         f = (float)x[(base + tt) * x_ld + d];
@@ -1353,7 +1363,10 @@ splice_rows_kernel(const float* __restrict__ x, int D, const int* __restrict__ r
     const long long srow = p - (long long)kHalo * (2 * b + 1) + delta;   // source row of the (clamped) frame
     const bool inside = (ctx0 >= -lo) && (ctx0 + K - 1 <= hi);
     float f[8];
-    if (inside) {
+    if (m & kRowEmpty) {                           // halo row of an empty utterance: nothing to read
+#pragma unroll
+      for (int i = 0; i < 8; ++i) f[i] = 0.0f;
+    } else if (inside) {
       const float* src = x + (srow + ctx0) * D + c0;
       if (c0 + 8 <= cols) {
         const float2* s2 = reinterpret_cast<const float2*>(src);   // D even, c0 % 8 == 0: 8-byte aligned
@@ -1631,23 +1644,27 @@ size_t prepass_smem_bytes(int tc, int window, int dim) {
   return (a + y + blk) * sizeof(float) + (size_t)(tc + 2 * kHalo + window) * sizeof(long long);
 }
 
-// (batch, 2, U) raw sums of r = relu(acc + bias) over the frames of each utterance -> mean || std of
-// y = scale * r + offset (batchnorm.py:81-88 folded in algebraically; stats_pooling.py:228-240):
-//   mean_y = scale * mean_r + offset,  var_y = scale^2 * (E[r^2] - mean_r^2),  std = sqrt(relu(var_y) + eps)
+// (batch, 2, U) sums of d = r - c, r = relu(acc + bias), c = shift (TcLayer::d_shift, 0 if null), over the frames of each
+// utterance -> mean || std of y = scale * r + offset (batchnorm.py:81-88 folded in algebraically;
+// stats_pooling.py:228-240):
+//   mean_y = scale * mean_d + (scale * c + offset),  var_y = scale^2 * (E[d^2] - mean_d^2),  std = sqrt(relu(var_y) + eps)
+// (scale * c + offset is 0 up to rounding).  An empty utterance pools to NaN, the mean over zero frames.
 __global__ void stats_finalize_tc_kernel(const float* __restrict__ sums, const long long* __restrict__ offs, int U,
                                          const float* __restrict__ scale, const float* __restrict__ offset,
-                                         int include_std, float eps, __nv_bfloat16* __restrict__ out_bf16,
+                                         const float* __restrict__ shift, int include_std, float eps,
+                                         __nv_bfloat16* __restrict__ out_bf16,
                                          float* __restrict__ out_f32, long long out_ld) {
   const int u = blockIdx.y * blockDim.x + threadIdx.x;
   if (u >= U) return;
   const long long b = blockIdx.x;
   const float n = (float)(offs[b + 1] - offs[b]);
-  const float mr = sums[(b * 2 + 0) * U + u] / n;
-  const float vr = sums[(b * 2 + 1) * U + u] / n - __fmul_rn(mr, mr);
+  const float md = sums[(b * 2 + 0) * U + u] / n;
+  const float vr = sums[(b * 2 + 1) * U + u] / n - __fmul_rn(md, md);
   const float sc = scale ? scale[u] : 1.0f;
   const float of = offset ? offset[u] : 0.0f;
-  const float mean = fmaf(sc, mr, of);
-  const float sd = sqrtf(fmaxf(sc * sc * vr, 0.0f) + eps);
+  float mean = fmaf(sc, md, fmaf(sc, shift ? shift[u] : 0.0f, of));
+  float sd = sqrtf(fmaxf(sc * sc * vr, 0.0f) + eps);
+  if (!(n > 0.0f)) mean = sd = __int_as_float(0x7fc00000);   // (fmaxf would turn a NaN variance into sqrt(eps))
   if (out_bf16) {
     out_bf16[b * out_ld + u] = __float2bfloat16_rn(mean);
     if (include_std) out_bf16[b * out_ld + U + u] = __float2bfloat16_rn(sd);
@@ -1682,6 +1699,12 @@ struct TcLayer {
   long long w_ld = 0;               // bf16 weight row stride (elements)
   __nv_bfloat16* d_w = nullptr;     // (U, w_ld)
   int* d_ctx = nullptr;
+  // Centre of the pooled sums, per unit: c = -offset / scale, the moving mean BatchNorm subtracts from
+  // r = relu(acc + bias) (nullptr without BatchNorm).  The STATS epilogue accumulates r - c and the finaliser adds c
+  // back: r can sit far from zero (mean / std of 200 is possible for a unit BatchNorm re-centres), and E[r^2] - E[r]^2
+  // formed from fp32 sums of r itself cancels -- 9e-3 relative error in the pooled std at mean / std = 200 over 300
+  // frames.  Centred, the sums are of the size of the std.
+  float* d_shift = nullptr;
   CUtensorMap tmW_n;                // weights as the B operand (box BK x BN)
   CUtensorMap tmW_m;                // weights as the A operand (box BK x BM), STATS mode
   ktf::Workspace ws;                // scratch of the stand-alone layer call
@@ -1787,6 +1810,7 @@ void release_layer(TcLayer* L) {
   if (!L) return;
   cudaFree(L->d_w);
   cudaFree(L->d_ctx);
+  cudaFree(L->d_shift);
   L->ws.release();
 }
 
@@ -2004,6 +2028,7 @@ int run_layer_stats(const TcLayer& L, const ktf_affine* a, const __nv_bfloat16* 
   args.reverse = reverse;
   args.rowseg = rowseg;
   args.bias = a->d_bias;
+  args.shift = L.d_shift;       // the sums are centred on the BatchNorm moving mean
   args.relu = a->cfg.activation == KTF_ACT_RELU;
   args.sums = sums;
   return launch_gemm<kModeStats>(L.tmW_m, tmX, args, st);
@@ -2017,11 +2042,18 @@ unsigned blocks_for(long long items, int threads) {
 
 namespace ktf {
 
-int affine_tc_prepare(ktf_affine* a, const float* weights_host) {
+int affine_tc_prepare(ktf_affine* a, const float* weights_host, const float* bn_scale_host,
+                      const float* bn_offset_host) {
   int rc = check_arch();
   if (rc != KTF_OK) return rc;
   TcLayer* L = new TcLayer();
   rc = prepare_layer(L, a->cfg, weights_host);
+  if (rc == KTF_OK && bn_scale_host && bn_offset_host) {
+    std::vector<float> c(a->cfg.out_dim);
+    for (int u = 0; u < a->cfg.out_dim; ++u)
+      c[u] = bn_scale_host[u] != 0.0f ? -bn_offset_host[u] / bn_scale_host[u] : 0.0f;
+    rc = ktf::upload(&L->d_shift, c.data(), c.size());
+  }
   if (rc != KTF_OK) {
     release_layer(L);
     delete L;
@@ -2354,8 +2386,9 @@ static int stack_forward_impl(ktf_tdnn_stack* s, const float* feats_dev, const i
       if ((rc = run_layer_stats(L, a, A, a_ld, a_cols, prow, rowseg, sums, spliced, st, i & 1, prow_dev)) != KTF_OK)
         return rc;
       dim3 grid((unsigned)batch, (unsigned)((L.U + 127) / 128));
-      stats_finalize_tc_kernel<<<grid, 128, 0, st>>>(sums, offs, L.U, a->d_scale, a->d_offset, s->include_std,
-                                                     s->stats_eps, last ? nullptr : pooled, last ? out_dev : nullptr,
+      stats_finalize_tc_kernel<<<grid, 128, 0, st>>>(sums, offs, L.U, a->d_scale, a->d_offset, L.d_shift,
+                                                     s->include_std, s->stats_eps, last ? nullptr : pooled,
+                                                     last ? out_dev : nullptr,
                                                      last ? (long long)pooled_dim : p_ld);
       KTF_LAUNCH_OK();
       cur = pooled;
