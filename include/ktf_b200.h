@@ -93,7 +93,7 @@ enum { KTF_OUT_MFCC = 0, KTF_OUT_FBANK = 1, KTF_OUT_WINDOWED = 2 };
 typedef struct {
   int32_t frame_width;      /* samples gathered per frame = 2*(frame_size/2) (framing.py:107-109) */
   int32_t frame_shift;      /* samples between frame starts; == frame_width for pre-framed input */
-  int32_t fft_length;       /* next power of two >= frame_width (filterbank.py:133-136,156) */
+  int32_t fft_length;       /* next power of two >= frame_width (filterbank.py:133-136,156): 256 .. 4096 */
   int32_t num_mels;         /* columns of mel_bank */
   int32_t num_ceps;         /* columns of dct (<= num_mels); ignored unless KTF_OUT_MFCC */
   int32_t output;           /* KTF_OUT_* */
@@ -155,7 +155,8 @@ int ktf_frontend_forward_ragged(const ktf_frontend* fe, const float* wav_dev, in
  *   sample_format  KTF_SAMPLE_F32: float32 samples in int16 scale (the reference's input convention,
  *                  models/kaldi/xvector_extractor.py:90-91); KTF_SAMPLE_S16: raw int16 PCM as stored in a wav file --
  *                  replaces the loaders' int16 -> float32 step (testdata/feats/feats.py:31-34) and halves the bytes
- *                  that cross PCIe and HBM.  int16 needs the fused 400-sample / 512-point MFCC / fbank kernel.
+ *                  that cross PCIe and HBM.  int16 needs the fused 400-sample / 512-point MFCC / fbank kernel
+ *                  or fft_length 1024..4096 (every output kind, dithered or not).
  *   snip_edges     1: frames as in framing.py:231-239 (no padding).  0: Kaldi's default snip-edges=false -- the
  *                  utterance is mirror-padded on both sides INSIDE the kernel (index reflection while staging), which
  *                  replaces kaldi_numpy.PadWaveform (kaldi_numpy/frame_extraction.py:54-89) on the host;

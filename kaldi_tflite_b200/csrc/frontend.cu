@@ -27,62 +27,13 @@
 #include <vector>
 
 #include "common.cuh"
-#include "twiddles64.h"
 
 #include "frontend_internal.cuh"
 
 using namespace ktf_fe;
+using namespace ktf_fe::radix2;
 
 namespace {
-
-__device__ __forceinline__ float2 cadd(float2 a, float2 b) { return make_float2(a.x + b.x, a.y + b.y); }
-__device__ __forceinline__ float2 csub(float2 a, float2 b) { return make_float2(a.x - b.x, a.y - b.y); }
-__device__ __forceinline__ float2 cmul(float2 a, float2 b) {
-  return make_float2(fmaf(a.x, b.x, -a.y * b.y), fmaf(a.x, b.y, a.y * b.x));
-}
-__device__ __forceinline__ float cnorm(float2 a) { return fmaf(a.x, a.x, a.y * a.y); }
-
-constexpr __host__ __device__ int brev(int v, int bits) {
-  int r = 0;
-  for (int i = 0; i < bits; ++i) r |= ((v >> i) & 1) << (bits - 1 - i);
-  return r;
-}
-constexpr __host__ __device__ int ilog2(int n) { return n <= 1 ? 0 : 1 + ilog2(n / 2); }
-
-// In-register decimation-in-frequency radix-2 FFT of x[OFF .. OFF+N); output bit-reversed.
-// All indices and twiddles are compile-time constants once unrolled.
-template <int N, int OFF, int TOT>
-__device__ __forceinline__ void fft_dif(float2 (&x)[TOT]) {
-  if constexpr (N >= 2) {
-    constexpr int H = N / 2;
-#pragma unroll
-    for (int i = 0; i < H; ++i) {
-      const float2 a = x[OFF + i];
-      const float2 b = x[OFF + i + H];
-      x[OFF + i] = cadd(a, b);
-      const float2 d = csub(a, b);
-      float2 r;
-      if (i == 0) {
-        r = d;
-      } else if (4 * i == N) {          // W = -i
-        r = make_float2(d.y, -d.x);
-      } else if (8 * i == N) {          // W = (1 - i)/sqrt2
-        const float c = 0.70710678118654752440f;
-        r = make_float2((d.x + d.y) * c, (d.y - d.x) * c);
-      } else if (8 * i == 3 * N) {      // W = (-1 - i)/sqrt2
-        const float c = 0.70710678118654752440f;
-        r = make_float2((d.y - d.x) * c, -(d.x + d.y) * c);
-      } else {
-        const float wr = KTF_COS64[i * (64 / N)];
-        const float wi = -KTF_SIN64[i * (64 / N)];
-        r = make_float2(fmaf(d.x, wr, -d.y * wi), fmaf(d.x, wi, d.y * wr));
-      }
-      x[OFF + i + H] = r;
-    }
-    fft_dif<H, OFF, TOT>(x);
-    fft_dif<H, OFF + H, TOT>(x);
-  }
-}
 
 template <int R>
 struct Geo {
@@ -510,6 +461,7 @@ int launch(const ktf_frontend* fe, FrontendArgs& a, cudaStream_t st) {
 }
 
 int dispatch(const ktf_frontend* fe, FrontendArgs& a, cudaStream_t st) {
+  if (fe->d_wide != nullptr) return wide_launch(fe, a, st);
   if (fe->d_r16 != nullptr) return r16_launch(fe, a, st);
   const int W = fe->cfg.frame_width;
   const bool even_shift = (fe->cfg.frame_shift & 1) == 0;
@@ -568,8 +520,10 @@ int ktf_frontend_create(const ktf_frontend_cfg* cfg, const float* window_host,
   const int W = cfg->frame_width, N = cfg->fft_length;
   KTF_CHECK_ARG(W > 0 && cfg->frame_shift > 0, "frame_width and frame_shift must be > 0");
   KTF_CHECK_ARG(N >= W && (N & (N - 1)) == 0, "fft_length must be a power of two >= frame_width");
-  KTF_CHECK_ARG(N == 256 || N == 512,
-                "fft_length %d not supported by the fused front-end (supported: 256, 512)", N);
+  KTF_CHECK_ARG(N <= 4096, "fft_length %d (frame_width %d) is too long for the fused front-end: the maximum is 4096 "
+                "(frame_width <= 4096)", N, W);
+  KTF_CHECK_ARG(N == 256 || N == 512 || N == 1024 || N == 2048 || N == 4096,
+                "fft_length %d not supported by the fused front-end (supported: 256, 512, 1024, 2048, 4096)", N);
   KTF_CHECK_ARG(cfg->frame_shift <= 2 * N, "frame_shift %d too large", cfg->frame_shift);
   KTF_CHECK_ARG(cfg->output >= KTF_OUT_MFCC && cfg->output <= KTF_OUT_WINDOWED, "bad output kind");
   const bool need_mel = cfg->output != KTF_OUT_WINDOWED;
@@ -594,6 +548,12 @@ int ktf_frontend_create(const ktf_frontend_cfg* cfg, const float* window_host,
 
   int rc = KTF_OK;
   auto fail = [&](int code) { ktf_frontend_destroy(fe); return code; };
+
+  if (N > 512) {   // 1024..4096 points: the one-frame-per-warp kernel of frontend_wide.cu, with its own tables
+    if ((rc = wide_build(fe, window_host, mel_bank_host, dct_host, lifter_host)) != KTF_OK) return fail(rc);
+    *out = fe;
+    return KTF_OK;
+  }
 
   if ((rc = ktf::upload(&fe->d_window, window_host, (size_t)W)) != KTF_OK) return fail(rc);
 
@@ -668,6 +628,7 @@ void ktf_frontend_destroy(ktf_frontend* fe) {
   cudaFree(fe->d_dct);
   cudaFree(fe->d_lifter);
   cudaFree(fe->d_r16);
+  cudaFree(fe->d_wide);
   delete fe;
 }
 
@@ -691,8 +652,9 @@ int set_ingest(const ktf_frontend* fe, FrontendArgs& a, const void* wav_dev, int
   KTF_CHECK_ARG(sample_format == KTF_SAMPLE_F32 || sample_format == KTF_SAMPLE_S16, "unknown sample_format %d",
                 sample_format);
   if (sample_format == KTF_SAMPLE_S16) {
-    KTF_CHECK_ARG(fe->d_r16 != nullptr,
-                  "int16 input is implemented by the fused 400-sample / 512-point MFCC / fbank kernel only");
+    KTF_CHECK_ARG(fe->d_r16 != nullptr || fe->d_wide != nullptr,
+                  "int16 input is implemented by the fused 400-sample / 512-point MFCC / fbank kernel and by the "
+                  "1024- to 4096-point kernel only");
     a.wav16 = static_cast<const short*>(wav_dev);
   } else {
     a.wav = static_cast<const float*>(wav_dev);

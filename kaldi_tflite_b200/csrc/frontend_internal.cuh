@@ -1,8 +1,10 @@
 // Internals shared by the front-end translation units (frontend.cu: generic radix-2 kernel and the
-// C-ABI; frontend_r16.cu: the 16 x 16 fast path for 512-point FFTs).
+// C-ABI; frontend_r16.cu: the 16 x 16 fast path for 512-point FFTs; frontend_wide.cu: one frame per warp for
+// 1024- to 4096-point FFTs).
 #pragma once
 
 #include "common.cuh"
+#include "twiddles64.h"
 
 namespace ktf_fe {
 
@@ -49,7 +51,67 @@ struct FrontendArgs {
   // 16 x 16 fast path (frontend_r16.cu): one blob laid out like the CTA's table region
   const float* r16_blob;
   int r16_blob_floats, r16_nf, r16_melw_floats;
+  // wide kernel (frontend_wide.cu): one blob laid out like the CTA's table region, and the per-warp region size
+  const float* wide_blob;
+  int wide_blob_floats, wide_warp_floats;
+  int wide_off_tw, wide_off_ustart, wide_off_units, wide_off_fslot, wide_off_melw, wide_off_dct, wide_off_lifter;
+  int wide_lm_floats;
 };
+
+// Complex helpers and the in-register radix-2 FFT shared by the generic kernel (frontend.cu) and the wide kernel
+// (frontend_wide.cu).
+namespace radix2 {
+
+__device__ __forceinline__ float2 cadd(float2 a, float2 b) { return make_float2(a.x + b.x, a.y + b.y); }
+__device__ __forceinline__ float2 csub(float2 a, float2 b) { return make_float2(a.x - b.x, a.y - b.y); }
+__device__ __forceinline__ float2 cmul(float2 a, float2 b) {
+  return make_float2(fmaf(a.x, b.x, -a.y * b.y), fmaf(a.x, b.y, a.y * b.x));
+}
+__device__ __forceinline__ float cnorm(float2 a) { return fmaf(a.x, a.x, a.y * a.y); }
+
+constexpr __host__ __device__ int brev(int v, int bits) {
+  int r = 0;
+  for (int i = 0; i < bits; ++i) r |= ((v >> i) & 1) << (bits - 1 - i);
+  return r;
+}
+constexpr __host__ __device__ int ilog2(int n) { return n <= 1 ? 0 : 1 + ilog2(n / 2); }
+
+// In-register decimation-in-frequency radix-2 FFT of x[OFF .. OFF+N); output bit-reversed.
+// All indices and twiddles are compile-time constants once unrolled.
+template <int N, int OFF, int TOT>
+__device__ __forceinline__ void fft_dif(float2 (&x)[TOT]) {
+  if constexpr (N >= 2) {
+    constexpr int H = N / 2;
+#pragma unroll
+    for (int i = 0; i < H; ++i) {
+      const float2 a = x[OFF + i];
+      const float2 b = x[OFF + i + H];
+      x[OFF + i] = cadd(a, b);
+      const float2 d = csub(a, b);
+      float2 r;
+      if (i == 0) {
+        r = d;
+      } else if (4 * i == N) {          // W = -i
+        r = make_float2(d.y, -d.x);
+      } else if (8 * i == N) {          // W = (1 - i)/sqrt2
+        const float c = 0.70710678118654752440f;
+        r = make_float2((d.x + d.y) * c, (d.y - d.x) * c);
+      } else if (8 * i == 3 * N) {      // W = (-1 - i)/sqrt2
+        const float c = 0.70710678118654752440f;
+        r = make_float2((d.y - d.x) * c, -(d.x + d.y) * c);
+      } else {
+        const float wr = KTF_COS64[i * (64 / N)];
+        const float wi = -KTF_SIN64[i * (64 / N)];
+        r = make_float2(fmaf(d.x, wr, -d.y * wi), fmaf(d.x, wi, d.y * wr));
+      }
+      x[OFF + i + H] = r;
+    }
+    fft_dif<H, OFF, TOT>(x);
+    fft_dif<H, OFF + H, TOT>(x);
+  }
+}
+
+}  // namespace radix2
 
 __device__ __forceinline__ float group_sum8(float v) {
   v += __shfl_xor_sync(0xffffffffu, v, 1);
@@ -232,6 +294,11 @@ struct ktf_frontend {
   // 16 x 16 fast path (frontend_r16.cu); null when the configuration is not eligible
   float* d_r16 = nullptr;
   int r16_blob_floats = 0, r16_nf = 0, r16_melw_floats = 0, r16_dct_sym = 0;
+  // wide kernel (frontend_wide.cu, fft_length 1024..4096); null for shorter FFTs
+  float* d_wide = nullptr;
+  int wide_blob_floats = 0, wide_warp_floats = 0, wide_warps = 0, wide_lm_floats = 0;
+  int wide_off_tw = 0, wide_off_ustart = 0, wide_off_units = 0, wide_off_fslot = 0, wide_off_melw = 0,
+      wide_off_dct = 0, wide_off_lifter = 0;
 };
 
 namespace ktf_fe {
@@ -240,4 +307,9 @@ namespace ktf_fe {
 int r16_build(ktf_frontend* fe, const float* window_host, const float* mel_bank_host, const float* dct_host,
               const float* lifter_host);
 int r16_launch(const ktf_frontend* fe, FrontendArgs& a, cudaStream_t st);
+// Builds the wide kernel's tables (fft_length 1024, 2048 or 4096) and picks its CTA size; fails with KTF_EINVAL when
+// even a one-warp CTA would need more than 227 KB of shared memory.
+int wide_build(ktf_frontend* fe, const float* window_host, const float* mel_bank_host, const float* dct_host,
+               const float* lifter_host);
+int wide_launch(const ktf_frontend* fe, FrontendArgs& a, cudaStream_t st);
 }  // namespace ktf_fe

@@ -242,6 +242,7 @@ class _Frontend:
         self.out_dim = N.lib().ktf_frontend_out_dim(self.handle)
         self.want_energy = bool(cfg.output == N.KTF_OUT_WINDOWED and cfg.use_energy)
         self.dither = float(cfg.dither)
+        self.wide = cfg.fft_length > 512      # 1024..4096 points: a kernel that reads int16 PCM in every mode
 
     def __del__(self):
         try:
@@ -254,8 +255,9 @@ class _Frontend:
         return int(N.lib().ktf_frontend_num_frames_ex(self.handle, n, int(bool(snip_edges))))
 
     def _ingest(self, wav):
-        # the dithering (generic) kernel takes float32 samples: raw PCM is widened first (dither != 0 only)
-        if self.dither != 0.0 and wav.dtype == torch.int16:
+        # the dithering 256 / 512-point (generic) kernel takes float32 samples: raw PCM is widened first (dither != 0
+        # only); the 1024..4096-point kernel converts int16 itself, dithered or not
+        if self.dither != 0.0 and wav.dtype == torch.int16 and not self.wide:
             return wav.to(torch.float32)
         return wav
 
