@@ -308,10 +308,17 @@ int ktf_tdnn_stack_forward(ktf_tdnn_stack* s, const float* feats_dev, const int6
  *               feats_dev already holds the compacted rows
  *   offsets_dev compacted frame offsets (batch + 1, device); total_rows >= offsets_dev[batch] (upper bound)
  *   max_frames  any upper bound on the longest compacted utterance (sizes the grid)
- * Requires a first layer with consecutive contexts; other CMVN modes: ktf_cmvn_forward + ktf_tdnn_stack_forward. */
+ * Requires a first layer with consecutive contexts and a tile that fits (ktf_tdnn_stack_vad_prepass_fits); other CMVN
+ * modes: ktf_cmvn_forward + ktf_tdnn_stack_forward. */
 int ktf_tdnn_stack_forward_vad(ktf_tdnn_stack* s, const float* feats_dev, const int64_t* index_dev,
                                const int64_t* offsets_dev, int64_t batch, int64_t total_rows, int64_t max_frames,
                                int32_t cmvn_window, float* out_dev, void* stream);
+
+/* 1 when ktf_tdnn_stack_forward_vad accepts (cmvn_window, max_frames): a first layer with consecutive contexts within
+ * +-4, and a pre-pass tile of 32..256 frames whose rows (tile + window + 8 halo frames) fit in shared memory.  With 30-dim
+ * features windows up to 800 fit; with 80-dim features up to 262.  0 otherwise: run ktf_vad_compact with the gather,
+ * ktf_cmvn_forward and ktf_tdnn_stack_forward instead. */
+int32_t ktf_tdnn_stack_vad_prepass_fits(const ktf_tdnn_stack* s, int32_t cmvn_window, int64_t max_frames);
 
 /* Element-wise helpers for callers that use ReLU / BatchNorm as stand-alone layers. */
 int ktf_relu_forward(const float* x_dev, int64_t n, float* y_dev, void* stream);

@@ -91,6 +91,7 @@ _SIGNATURES = {
     "ktf_tdnn_stack_out_dim": (c_int32, [_P]),
     "ktf_tdnn_stack_forward": (c_int32, [_P, _P, _P, c_int64, c_int64, _P, _P]),
     "ktf_tdnn_stack_forward_vad": (c_int32, [_P, _P, _P, _P, c_int64, c_int64, c_int64, c_int32, _P, _P]),
+    "ktf_tdnn_stack_vad_prepass_fits": (c_int32, [_P, c_int32, c_int64]),
     "ktf_relu_forward": (c_int32, [_P, c_int64, _P, _P]),
     "ktf_scale_offset_forward": (c_int32, [_P, c_int64, c_int32, _P, _P, _P, _P]),
     "ktf_stats_finalize": (c_int32, [_P, _P, c_int64, c_int32, c_int32, c_float, c_int32, _P, _P]),

@@ -1490,7 +1490,8 @@ gather_cmvn_splice_kernel(const float* __restrict__ feats, int dim, const long l
   float* sx = spre;                                                             // [R][dim] staged rows
   float* sy = spre + (((size_t)max_rows * dim + 3) & ~(size_t)3);               // [e1 - e0][dim] normalised rows (+ 8 pad)
   float* bsum = sy + (((size_t)(tc + 2 * kHalo) * dim + 8 + 3) & ~(size_t)3);   // [nblk][dim] sums of 32-row blocks
-  long long* srow = reinterpret_cast<long long*>(bsum + (size_t)(max_rows / kPreBlk + 2) * dim + (dim & 1));   // [R]
+  // [R] source rows, 8-byte aligned: the block sums are rounded up to an even float count
+  long long* srow = reinterpret_cast<long long*>(bsum + (((size_t)(max_rows / kPreBlk + 2) * dim + 1) & ~(size_t)1));
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
   // ---- 1. stage (gather): source rows first (independent loads, one latency), then the copies ----------------
@@ -1640,8 +1641,26 @@ gather_cmvn_splice_kernel(const float* __restrict__ feats, int dim, const long l
 size_t prepass_smem_bytes(int tc, int window, int dim) {
   const size_t a = (((size_t)(tc + 2 * kHalo + window) * dim + 3) & ~(size_t)3);
   const size_t y = (((size_t)(tc + 2 * kHalo) * dim + 8 + 3) & ~(size_t)3);
-  const size_t blk = (size_t)((tc + 2 * kHalo + window) / kPreBlk + 2) * dim + (dim & 1);
+  const size_t blk = ((size_t)((tc + 2 * kHalo + window) / kPreBlk + 2) * dim + 1) & ~(size_t)1;
   return (a + y + blk) * sizeof(float) + (size_t)(tc + 2 * kHalo + window) * sizeof(long long);
+}
+
+// Frames per CTA of the pre-pass: the largest even tc <= 256 (KTF_PREPASS_TC) and >= 32 whose CTA fits 113 KB of shared
+// memory, balanced over the longest utterance (998 frames -> 4 x 250) with at most 65535 CTAs per utterance.  A wide
+// window or feature dimension takes a smaller tile (D 30: window <= 372 at tc 256, <= 800 at tc 32).  False when even
+// tc = 32 does not fit (D 80 at window 300): the caller then runs the separate gather -> CMVN -> splice kernels.
+bool prepass_tile(long long max_frames, int window, int dim, int* tc_out, long long* gys_out) {
+  static const int tc_target = getenv("KTF_PREPASS_TC") ? std::max(atoi(getenv("KTF_PREPASS_TC")), 32) : 256;
+  for (int target = tc_target & ~1; target >= 32; target -= 2) {
+    const long long gys = (max_frames + target - 1) / target;
+    const int tc = (int)((((max_frames + gys - 1) / gys) + 1) & ~1LL);
+    if (gys <= 65535 && prepass_smem_bytes(tc, window, dim) <= 113 * 1024) {
+      *tc_out = tc;
+      *gys_out = gys;
+      return true;
+    }
+  }
+  return false;
 }
 
 // (batch, 2, U) sums of d = r - c, r = relu(acc + bias), c = shift (TcLayer::d_shift, 0 if null), over the frames of each
@@ -2351,12 +2370,12 @@ static int stack_forward_impl(ktf_tdnn_stack* s, const float* feats_dev, const i
       const unsigned grid = blocks_for(prow * (ld >> 3), 256);
       if (i == 0 && pre != nullptr) {
         // VAD gather + sliding CMVN + splice in one pass (the rows never exist as a gathered / normalised fp32 matrix)
-        static const int tc_target = getenv("KTF_PREPASS_TC") ? std::max(atoi(getenv("KTF_PREPASS_TC")), 32) : 256;
-        const long long gys = (pre->max_frames + tc_target - 1) / tc_target;
-        const int tc = (int)((((pre->max_frames + gys - 1) / gys) + 1) & ~1LL);
-        const size_t smem = prepass_smem_bytes(tc, pre->cmvn_window, L.D);
-        KTF_CHECK_ARG(smem <= 113 * 1024 && gys <= 65535, "CMVN window %d x dim %d does not fit the fused pre-pass",
+        int tc = 0;
+        long long gys = 0;
+        KTF_CHECK_ARG(prepass_tile(pre->max_frames, pre->cmvn_window, L.D, &tc, &gys),
+                      "CMVN window %d x dim %d does not fit the fused pre-pass (see ktf_tdnn_stack_vad_prepass_fits)",
                       pre->cmvn_window, L.D);
+        const size_t smem = prepass_smem_bytes(tc, pre->cmvn_window, L.D);
         static unsigned long long attr_set = 0;
         if (ktf::first_use_on_device(&attr_set))
           KTF_CUDA(cudaFuncSetAttribute(gather_cmvn_splice_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 113 * 1024));
@@ -2417,6 +2436,15 @@ static int stack_forward_impl(ktf_tdnn_stack* s, const float* feats_dev, const i
   return KTF_OK;
 }
 
+// The pre-pass emits the first layer's splice: its contexts must be consecutive and within the +-kHalo padding.
+static bool prepass_contexts_ok(const ktf_tdnn_stack* s) {
+  const TcLayer& L0 = *static_cast<const TcLayer*>(s->layers[0]->tc);
+  bool ok = true;
+  for (int k = 1; k < L0.K; ++k) ok = ok && (L0.ctx[k] == L0.ctx[0] + k);
+  for (int k = 0; k < L0.K; ++k) ok = ok && L0.ctx[k] >= -kHalo && L0.ctx[k] <= kHalo;
+  return ok;
+}
+
 extern "C" {
 
 int ktf_tdnn_stack_forward(ktf_tdnn_stack* s, const float* feats_dev, const int64_t* offsets_dev,
@@ -2430,13 +2458,17 @@ int ktf_tdnn_stack_forward_vad(ktf_tdnn_stack* s, const float* feats_dev, const 
                                int32_t cmvn_window, float* out_dev, void* stream) {
   KTF_CHECK_ARG(s && feats_dev && offsets_dev && out_dev, "ktf_tdnn_stack_forward_vad: null argument");
   KTF_CHECK_ARG(cmvn_window > 0 && max_frames > 0, "`window` and `min_window` must be > 0");
-  const TcLayer& L0 = *static_cast<const TcLayer*>(s->layers[0]->tc);
-  bool ok = true;
-  for (int k = 1; k < L0.K; ++k) ok = ok && (L0.ctx[k] == L0.ctx[0] + k);
-  for (int k = 0; k < L0.K; ++k) ok = ok && L0.ctx[k] >= -kHalo && L0.ctx[k] <= kHalo;
-  KTF_CHECK_ARG(ok, "the fused VAD / CMVN pre-pass needs a first layer with consecutive contexts within +-%d", kHalo);
+  KTF_CHECK_ARG(prepass_contexts_ok(s),
+                "the fused VAD / CMVN pre-pass needs a first layer with consecutive contexts within +-%d", kHalo);
   StackPre pre{(const long long*)index_dev, (long long)max_frames, cmvn_window};
   return stack_forward_impl(s, feats_dev, offsets_dev, batch, total_rows, out_dev, &pre, (cudaStream_t)stream);
+}
+
+int32_t ktf_tdnn_stack_vad_prepass_fits(const ktf_tdnn_stack* s, int32_t cmvn_window, int64_t max_frames) {
+  if (!s || cmvn_window <= 0 || max_frames <= 0 || !prepass_contexts_ok(s)) return 0;
+  int tc = 0;
+  long long gys = 0;
+  return prepass_tile(max_frames, cmvn_window, static_cast<const TcLayer*>(s->layers[0]->tc)->D, &tc, &gys) ? 1 : 0;
 }
 
 }  // extern "C"

@@ -132,10 +132,15 @@ class _Stack:
                                                T.stream_ptr()))
         return out
 
-    def can_fuse_vad_cmvn(self):
-        """First layer with consecutive contexts: the VAD gather + CMVN + splice pre-pass applies."""
+    def can_fuse_vad_cmvn(self, cmvn_window=None, max_frames=None):
+        """First layer with consecutive contexts: the VAD gather + CMVN + splice pre-pass applies.  Given the CMVN window
+        and the longest utterance, also whether the pre-pass tile fits in shared memory (ktf_tdnn_stack_vad_prepass_fits)."""
         ctx = self.affines[0].context
-        return all(c == ctx[0] + k for k, c in enumerate(ctx)) and max(abs(c) for c in ctx) <= 4
+        if not (all(c == ctx[0] + k for k, c in enumerate(ctx)) and max(abs(c) for c in ctx) <= 4):
+            return False
+        if cmvn_window is None:
+            return True
+        return bool(N.lib().ktf_tdnn_stack_vad_prepass_fits(self.handle, int(cmvn_window), int(max_frames)))
 
     def forward_vad(self, feats2d, index, offsets, max_frames, cmvn_window):
         """Un-normalised features + VAD index list + compacted offsets -> stack output (ktf_tdnn_stack_forward_vad)."""

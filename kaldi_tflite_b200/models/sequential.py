@@ -143,10 +143,13 @@ class Sequential:
             self._plan_version = self._weights_version()
             self._stack = self._try_stack(self._plan)       # None unless every layer runs on the tcgen05 engine
 
-    def fused_vad_cmvn_stack(self, feat_dim):
-        """The tcgen05 stack if it can take un-normalised features + a VAD index list directly (fused pre-pass)."""
+    def fused_vad_cmvn_stack(self, feat_dim, cmvn_window=None, max_frames=None):
+        """The tcgen05 stack if it can take un-normalised features + a VAD index list directly (fused pre-pass).  With
+        `cmvn_window` and `max_frames` (an upper bound on the longest utterance), only if the pre-pass fits them."""
         self._ensure_plan(feat_dim)
-        return self._stack if (self._stack is not None and self._stack.can_fuse_vad_cmvn()) else None
+        if self._stack is None or not self._stack.can_fuse_vad_cmvn(cmvn_window, max_frames):
+            return None
+        return self._stack
 
     def forward_ragged(self, x2d, offsets):
         """x2d CUDA (rows, D); utterance b = rows offsets[b]..offsets[b+1].  Returns (y2d, offsets)."""

@@ -108,14 +108,15 @@ class XvectorExtractor:
     def embed(self, feats, offsets, max_frames=None):
         mask = self.vad.mask_ragged(feats, offsets)
         stack = None
+        mf = feats.shape[0] if max_frames is None else max_frames
         if self.fusePrepass and self.cmvn.padding == "SAME" and not self.cmvn.normVar:
-            stack = self.xvec.fused_vad_cmvn_stack(feats.shape[-1])
+            # None when the window is too wide for the pre-pass tile: the separate kernels below take any window
+            stack = self.xvec.fused_vad_cmvn_stack(feats.shape[-1], self.cmvn.N, mf)
         if stack is not None and stack.pools:
             # tcgen05 stack: gather -> CMVN -> splice is ONE pre-pass kernel in front of the GEMMs; the kept rows are
             # never written as a gathered / normalised fp32 matrix
             _, voffs, index = self.vad.compact_ragged(feats, mask, offsets, gather=False)
             self._voffs = voffs                # examined only when the result leaves as a host array (see __call__)
-            mf = feats.shape[0] if max_frames is None else max_frames
             emb = stack.forward_vad(feats, index, voffs, mf, self.cmvn.N)
             return emb, mask, voffs
         # `voiced` keeps the upper-bound row count; the kept-row count stays on the device (voffs[-1])
