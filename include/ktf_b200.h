@@ -395,6 +395,26 @@ int ktf_plda_score_ex(const ktf_plda* p, const void* u_test_dev, int64_t n_test,
 int ktf_plda_score_top1(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,
                         int64_t n_enroll, float* best_score_dev, int64_t* best_index_dev, void* stream);
 
+/* k best trials per test vector (the top-k form of ktf_plda_score_top1), 1 <= k <= KTF_PLDA_TOPK_MAX:
+ * scores_dev / index_dev are (n_test, k) row-major; row i holds the k largest entries of row i of the score matrix
+ * ktf_plda_score would write -- the same fp32-equivalent values, bit for bit -- and their enrolled columns, sorted by
+ * score, descending; on equal scores the lower column comes first (a stable descending sort of the row).  When
+ * k > n_enroll, entries n_enroll .. k-1 are (-inf, -1); n_enroll == 0 gives (-inf, -1) everywhere.  The matrix is never
+ * written.  Needs a float32 handle (the tcgen05 score GEMM) and n_enroll < 2^32; k outside 1 .. KTF_PLDA_TOPK_MAX is
+ * KTF_EINVAL.  No host synchronisation: the scratch (partial lists of every row) lives in the handle's grow-only
+ * workspace, so once it has grown for a shape the call can be captured in a CUDA graph.  As every call that uses that
+ * workspace, calls on one handle must not run concurrently on different streams. */
+#define KTF_PLDA_TOPK_MAX 32
+int ktf_plda_score_topk(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,
+                        int64_t n_enroll, int32_t k, float* scores_dev, int64_t* index_dev, void* stream);
+/* Merge of per-row top-k lists, e.g. of enrolled shards scored on different GPUs (indexes offset to the global
+ * numbering): scores_in_dev / index_in_dev are (num_lists, n_rows, k_in); entries with index < 0 are skipped, lists need
+ * not be sorted.  Output (n_rows, k), 1 <= k <= KTF_PLDA_TOPK_MAX: the k best candidates of every row with the ordering
+ * and padding of ktf_plda_score_topk (score descending, lower index first on equal scores, (-inf, -1) past the last
+ * candidate). */
+int ktf_topk_merge(const float* scores_in_dev, const int64_t* index_in_dev, int32_t num_lists, int64_t n_rows,
+                   int32_t k_in, int32_t k, float* scores_dev, int64_t* index_dev, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -19,6 +19,7 @@ KTF_PREC_F32, KTF_PREC_BF16 = 0, 1
 KTF_ACT_NONE, KTF_ACT_RELU = 0, 1
 KTF_SCORES_NATIVE, KTF_SCORES_BF16 = 0, 1
 KTF_MAX_CONTEXT = 16
+KTF_PLDA_TOPK_MAX = 32
 KTF_NCCL_UNIQUE_ID_BYTES = 128
 KTF_EINVAL, KTF_ECUDA, KTF_ENOMEM = -1, -2, -3
 
@@ -106,6 +107,8 @@ _SIGNATURES = {
     "ktf_plda_score": (c_int32, [_P, _P, c_int64, _P, c_int64, _P, c_int64, _P]),
     "ktf_plda_score_ex": (c_int32, [_P, _P, c_int64, _P, c_int64, _P, c_int64, c_int32, _P]),
     "ktf_plda_score_top1": (c_int32, [_P, _P, c_int64, _P, c_int64, _P, _P, _P]),
+    "ktf_plda_score_topk": (c_int32, [_P, _P, c_int64, _P, c_int64, c_int32, _P, _P, _P]),
+    "ktf_topk_merge": (c_int32, [_P, _P, c_int32, c_int64, c_int32, c_int32, _P, _P, _P]),
 }
 
 _lib = None

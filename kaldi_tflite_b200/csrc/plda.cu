@@ -151,9 +151,86 @@ __global__ void plda_top1_decode_kernel(const unsigned long long* __restrict__ k
   index[i] = key ? (long long)(0xffffffffu - (unsigned)(key & 0xffffffffull)) : -1;
 }
 
-// top1_score / top1_index non-null: no score matrix, the best enrolled column of every test row instead.
-int score_tc(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, void* scores, int64_t ld,
-             int scores_bf16, cudaStream_t st, float* top1_score = nullptr, long long* top1_index = nullptr) {
+// Candidate of a top-k merge: larger score first (top1_key's order-preserving bits), then the lower index, then the
+// lower position in the input (c < 0: none).
+struct MergeCand {
+  unsigned u;
+  long long idx;
+  int c;
+};
+__device__ __forceinline__ bool merge_before(const MergeCand& a, const MergeCand& b) {
+  if (a.c < 0) return false;
+  if (b.c < 0) return true;
+  if (a.u != b.u) return a.u > b.u;
+  if (a.idx != b.idx) return a.idx < b.idx;
+  return a.c < b.c;
+}
+
+// One warp per row: the k best of the row's num_lists x k_in (score, index) candidates (index < 0: none), best first,
+// ties to the lower index, padded with (-inf, -1).  A lane holds the best of its candidates (positions lane, lane + 32,
+// ...); each round the warp takes the best of the lanes' and only the lane that gave it looks for its next one.
+__global__ void topk_merge_kernel(const float* __restrict__ s_in, const long long* __restrict__ i_in, int num_lists,
+                                  long long n_rows, int k_in, int k, float* __restrict__ s_out,
+                                  long long* __restrict__ i_out) {
+  const long long row = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (row >= n_rows) return;
+  const int lane = threadIdx.x & 31;
+  const int n_cand = num_lists * k_in;
+  auto next_after = [&](const MergeCand& prev) {   // my best candidate that comes after prev (prev.c < 0: no bound)
+    MergeCand b{0u, 0, -1};
+    for (int c = lane; c < n_cand; c += 32) {
+      const long long off = ((long long)(c / k_in) * n_rows + row) * k_in + c % k_in;
+      const long long idx = i_in[off];
+      if (idx < 0) continue;
+      const unsigned bits = __float_as_uint(s_in[off]);
+      const MergeCand x{(bits & 0x80000000u) ? ~bits : (bits | 0x80000000u), idx, c};
+      if ((prev.c < 0 || merge_before(prev, x)) && merge_before(x, b)) b = x;
+    }
+    return b;
+  };
+  MergeCand mine = next_after(MergeCand{0u, 0, -1});
+  float out_s = -INFINITY;
+  long long out_i = -1;
+  for (int i = 0; i < k; ++i) {
+    MergeCand w = mine;
+    for (int o = 16; o > 0; o >>= 1) {
+      const MergeCand x{__shfl_xor_sync(0xffffffffu, w.u, o), __shfl_xor_sync(0xffffffffu, w.idx, o),
+                        __shfl_xor_sync(0xffffffffu, w.c, o)};
+      if (merge_before(x, w)) w = x;
+    }
+    if (w.c < 0) break;                            // warp-uniform: fewer than k candidates
+    if (lane == i) {
+      out_s = __uint_as_float((w.u & 0x80000000u) ? (w.u & 0x7fffffffu) : ~w.u);
+      out_i = w.idx;
+    }
+    if (mine.c == w.c) mine = next_after(w);
+  }
+  if (lane < k) {
+    s_out[row * k + lane] = out_s;
+    i_out[row * k + lane] = out_i;
+  }
+}
+
+int topk_merge(const float* s_in, const long long* i_in, int num_lists, long long n_rows, int k_in, int k, float* s_out,
+               long long* i_out, cudaStream_t st) {
+  if (n_rows <= 0) return KTF_OK;
+  topk_merge_kernel<<<(unsigned)((n_rows + 7) / 8), 256, 0, st>>>(s_in, i_in, num_lists, n_rows, k_in, k, s_out, i_out);
+  KTF_LAUNCH_OK();
+  return KTF_OK;
+}
+
+// Operands of the tensor-core score GEMM, in the handle's workspace: the fp16 hi/lo splits of both sides (K = 3 dim) and
+// A_i / B_j, followed by `extra` bytes of the caller's.
+struct TcOperands {
+  const __half* A;
+  const __half* B;
+  const float* Ai;
+  const float* Bj;
+  char* extra;
+};
+
+int tc_operands(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, size_t extra,
+                cudaStream_t st, TcOperands* o) {
   const int dim = p->dim;
   const long long K = 3LL * dim;
   ktf::Carver cv;
@@ -161,7 +238,7 @@ int score_tc(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, in
   const size_t o_b = cv.take((size_t)ne * K * sizeof(__half));
   const size_t o_ai = cv.take((size_t)nt * sizeof(float));
   const size_t o_bj = cv.take((size_t)ne * sizeof(float));
-  const size_t o_key = cv.take(top1_score ? (size_t)nt * sizeof(unsigned long long) : 0);
+  const size_t o_extra = cv.take(extra);
   int rc = p->ws.ensure(cv.off);
   if (rc != KTF_OK) return rc;
   char* base = static_cast<char*>(p->ws.ptr);
@@ -181,14 +258,45 @@ int score_tc(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, in
   KTF_LAUNCH_OK();
   plda_split_kernel<<<blocks(ne * dim), 256, 0, st>>>(ue, ne, dim, nullptr, 1, Bs);
   KTF_LAUNCH_OK();
+  *o = TcOperands{As, Bs, Ai, Bj, base + o_extra};
+  return KTF_OK;
+}
+
+// top1_score / top1_index non-null: no score matrix, the best enrolled column of every test row instead.
+int score_tc(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, void* scores, int64_t ld,
+             int scores_bf16, cudaStream_t st, float* top1_score = nullptr, long long* top1_index = nullptr) {
+  const long long K = 3LL * p->dim;
+  TcOperands o;
+  int rc = tc_operands(p, ut, nt, ue, ne, top1_score ? (size_t)nt * sizeof(unsigned long long) : 0, st, &o);
+  if (rc != KTF_OK) return rc;
   if (top1_score == nullptr)
-    return ktf::tc_gemm_nt(As, nt, K, Bs, ne, K, K, /*fp16=*/1, Ai, Bj, scores, ld, scores_bf16, st);
-  unsigned long long* keys = reinterpret_cast<unsigned long long*>(base + o_key);
+    return ktf::tc_gemm_nt(o.A, nt, K, o.B, ne, K, K, /*fp16=*/1, o.Ai, o.Bj, scores, ld, scores_bf16, st);
+  unsigned long long* keys = reinterpret_cast<unsigned long long*>(o.extra);
   KTF_CUDA(cudaMemsetAsync(keys, 0, (size_t)nt * sizeof(unsigned long long), st));
-  if ((rc = ktf::tc_gemm_nt(As, nt, K, Bs, ne, K, K, /*fp16=*/1, Ai, Bj, nullptr, ne, 0, st, keys)) != KTF_OK) return rc;
+  if ((rc = ktf::tc_gemm_nt(o.A, nt, K, o.B, ne, K, K, /*fp16=*/1, o.Ai, o.Bj, nullptr, ne, 0, st, keys)) != KTF_OK)
+    return rc;
   plda_top1_decode_kernel<<<(unsigned)((nt + 255) / 256), 256, 0, st>>>(keys, nt, top1_score, top1_index);
   KTF_LAUNCH_OK();
   return KTF_OK;
+}
+
+// The k best enrolled columns of every test row: the score GEMM leaves partial lists (one per n-range and column quarter
+// of a row) in the workspace, topk_merge reduces them to (nt, k).
+int score_tc_topk(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, int k, float* score,
+                  long long* index, cudaStream_t st) {
+  const long long K = 3LL * p->dim;
+  const int lists = ktf::tc_topk_lists(nt, ne, K);
+  if (lists == 0) return topk_merge(nullptr, nullptr, 0, nt, k, k, score, index, st);   // no enrolled vector
+  const size_t n_part = (size_t)lists * nt * k;
+  const size_t s_bytes = (n_part * sizeof(float) + 255) & ~(size_t)255;
+  TcOperands o;
+  int rc = tc_operands(p, ut, nt, ue, ne, s_bytes + n_part * sizeof(long long), st, &o);
+  if (rc != KTF_OK) return rc;
+  float* part_s = reinterpret_cast<float*>(o.extra);
+  long long* part_i = reinterpret_cast<long long*>(o.extra + s_bytes);
+  if ((rc = ktf::tc_gemm_topk(o.A, nt, K, o.B, ne, K, K, /*fp16=*/1, o.Ai, o.Bj, k, part_s, part_i, st)) != KTF_OK)
+    return rc;
+  return topk_merge(part_s, part_i, lists, nt, k, k, score, index, st);
 }
 
 template <typename T>
@@ -347,6 +455,33 @@ int ktf_plda_score_top1(const ktf_plda* p, const void* u_test_dev, int64_t n_tes
   if (n_test <= 0) return KTF_OK;
   return score_tc(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, nullptr, n_enroll, 0,
                   (cudaStream_t)stream, best_score_dev, (long long*)best_index_dev);
+}
+
+int ktf_plda_score_topk(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,
+                        int64_t n_enroll, int32_t k, float* scores_dev, int64_t* index_dev, void* stream) {
+  KTF_CHECK_ARG(p, "ktf_plda_score_topk: null handle");
+  KTF_CHECK_ARG(k >= 1 && k <= KTF_PLDA_TOPK_MAX, "ktf_plda_score_topk: k = %d, must be 1 .. %d (KTF_PLDA_TOPK_MAX)", k,
+                KTF_PLDA_TOPK_MAX);
+  KTF_CHECK_ARG(p->use_tc, "ktf_plda_score_topk needs a float32 PLDA handle on an sm_100 device");
+  KTF_CHECK_ARG(n_enroll >= 0 && n_enroll < (1LL << 32), "ktf_plda_score_topk: n_enroll must be in 0 .. 2^32 - 1");
+  if (n_test <= 0) return KTF_OK;
+  KTF_CHECK_ARG(u_test_dev && scores_dev && index_dev && (u_enroll_dev || n_enroll == 0),
+                "ktf_plda_score_topk: null argument");
+  return score_tc_topk(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, k, scores_dev,
+                       (long long*)index_dev, (cudaStream_t)stream);
+}
+
+int ktf_topk_merge(const float* scores_in_dev, const int64_t* index_in_dev, int32_t num_lists, int64_t n_rows,
+                   int32_t k_in, int32_t k, float* scores_dev, int64_t* index_dev, void* stream) {
+  KTF_CHECK_ARG(k >= 1 && k <= KTF_PLDA_TOPK_MAX, "ktf_topk_merge: k = %d, must be 1 .. %d (KTF_PLDA_TOPK_MAX)", k,
+                KTF_PLDA_TOPK_MAX);
+  KTF_CHECK_ARG(num_lists >= 0 && k_in >= 1 && (long long)num_lists * k_in < (1LL << 31),
+                "ktf_topk_merge: bad num_lists / k_in");
+  if (n_rows <= 0) return KTF_OK;
+  KTF_CHECK_ARG(scores_dev && index_dev && (num_lists == 0 || (scores_in_dev && index_in_dev)),
+                "ktf_topk_merge: null argument");
+  return topk_merge(scores_in_dev, (const long long*)index_in_dev, num_lists, n_rows, k_in, k, scores_dev,
+                    (long long*)index_dev, (cudaStream_t)stream);
 }
 
 int ktf_plda_score(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,

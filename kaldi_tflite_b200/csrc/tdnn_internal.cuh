@@ -29,4 +29,11 @@ int stats_sums_f32(const float* y_dev, const int64_t* offsets_dev, int64_t batch
 int tc_gemm_nt(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
                int fp16, const float* row_add, const float* col_add, void* C, long long ldc, int c_bf16,
                cudaStream_t st, unsigned long long* row_best = nullptr);
+// The same GEMM reduced to the k (1..32) largest entries of every row, nothing else stored: partial lists
+// (num_lists, m, k) of fp32 values and columns, unordered, (-inf, -1) where a list has fewer than k entries; every column
+// is in exactly one list.  num_lists = tc_topk_lists(m, n, K) (0 when m or n is 0).
+int tc_topk_lists(long long m, long long n, long long K);
+int tc_gemm_topk(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
+                 int fp16, const float* row_add, const float* col_add, int k, float* part_score, long long* part_index,
+                 cudaStream_t st);
 }  // namespace ktf

@@ -61,6 +61,10 @@ static_assert((kStages * kStageBytes) % 512 == 0 && (32 * kStgPitch) % 512 == 0,
               "staging buffers are TMA-store sources with the 64-byte swizzle: 512-byte aligned");
 
 enum { kModeBf16 = 0, kModeF32 = 1, kModeStats = 2 };
+// Pair kernel, per-row top-k (nothing stored, see TcArgs::topk_k): lists of up to 8, 16 or 32 entries per thread.  The
+// capacity is part of the mode because it sets the shared-memory layout and with it the number of ring stages.
+enum { kModeTopk8 = 3, kModeTopk16 = 4, kModeTopk32 = 5 };
+constexpr int topk_cap(int mode) { return mode >= kModeTopk8 ? 8 << (mode - kModeTopk8) : 0; }
 
 // rowmap flags
 constexpr int kRowStore = 1, kRowFirst = 2, kRowLast = 4;
@@ -105,6 +109,14 @@ struct TcArgs {
   long long* trace;         // development (KTF_TC_TRACE=file): clock64 of cluster 0's tile phases, 4 slots per tile
   unsigned long long* row_best;   // pair kernel, optional: instead of storing C, keep the best entry of every row as an
                                   // atomically maximised key (order-preserving float bits << 32 | ~column), see top1_key
+  // pair kernel, top-k modes: the tile walk is a sequence of units (one 256-row block x topk_unit_tiles consecutive
+  // n-tiles); every (row, column quarter) thread keeps the topk_k best entries of its columns over the unit and writes
+  // them, unordered, as one partial list: topk_score / topk_index (num_lists, m_rows, topk_k), list = split * EW / 4 +
+  // column quarter, (-inf, -1) for empty entries
+  int topk_k;
+  int topk_unit_tiles;
+  float* topk_score;
+  long long* topk_index;
 };
 
 __device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
@@ -390,6 +402,10 @@ __device__ __forceinline__ unsigned long long top1_key(float v, int col) {
   const unsigned b = __float_as_uint(v);
   const unsigned u = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
   return ((unsigned long long)u << 32) | (unsigned long long)(0xffffffffu - (unsigned)col);
+}
+__device__ __forceinline__ float top1_key_value(unsigned long long key) {
+  const unsigned u = (unsigned)(key >> 32);
+  return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
 }
 constexpr int kBoxRow = 128;                         // bytes per staged row of a box
 constexpr int kBoxBytes = 32 * kBoxRow;
@@ -882,6 +898,23 @@ template <int EW> struct PairCfg {
   static constexpr int kSmem = kStages * kPairStageBytes + 1024 + 256 + kVecBytes + kStgBytes;
 };
 static_assert(PairCfg<8>::kSmem <= 226 * 1024 && PairCfg<16>::kSmem <= 226 * 1024, "pair kernel shared memory");
+// Top-k modes store nothing: no staging boxes, only the bias of the per-warp vectors.  What they hold instead: per thread
+// a list of CAP 64-bit keys (interleaved by thread, so any per-lane entry index is bank-conflict free) and per warp a
+// 16 x 32 float scratch through which a lane walks its candidates of half a chunk.  The ring gets what is left, at most
+// the 5 stages of the storing modes.  EW = 8: CAP 8 / 16 / 32 -> 16 / 32 / 64 KB of lists, 5 / 5 / 4 stages;
+// EW = 16: 32 / 64 / 128 KB, 4 / 3 / 1 stages.
+template <int EW, int CAP> struct TopkCfg {
+  static constexpr int kCols = BN / (EW / 4);
+  static constexpr int kVecBytes = EW * kCols * 4;
+  static constexpr int kScratchBytes = EW * 16 * 32 * 4;
+  static constexpr int kListBytes = EW * 32 * CAP * 8;
+  static constexpr int kFixed = 1024 + 256 + kVecBytes + kScratchBytes + kListBytes;
+  static constexpr int kStages = std::min(5, (226 * 1024 - kFixed) / kPairStageBytes);
+  static constexpr int kSmem = kStages * kPairStageBytes + kFixed;
+};
+static_assert(TopkCfg<8, 32>::kStages == 4 && TopkCfg<16, 32>::kStages >= 1, "top-k pair kernel shared memory");
+template <int MODE, int EW>
+constexpr int pair_smem() { return topk_cap(MODE) ? TopkCfg<EW, topk_cap(MODE) ? topk_cap(MODE) : 8>::kSmem : PairCfg<EW>::kSmem; }
 
 __device__ __forceinline__ unsigned cluster_ctarank() {
   unsigned r;
@@ -936,14 +969,19 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                     const __grid_constant__ CUtensorMap tmC, const TcArgs a) {
   static_assert(MODE != kModeStats, "the pair kernel covers the row-storing modes");
   using Cfg = PairCfg<EW>;
-  constexpr int kPairStages = Cfg::kStages;
+  constexpr int kCap = topk_cap(MODE);
+  constexpr bool kTopk = kCap > 0;
+  using TCfg = TopkCfg<EW, kTopk ? kCap : 8>;
+  constexpr int kPairStages = kTopk ? TCfg::kStages : Cfg::kStages;
   constexpr int kPCols = Cfg::kCols, kPChunks = Cfg::kChunks;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   unsigned char* sA = smem;
   unsigned char* sB = smem + kPairStages * kPairABytes;
   unsigned char* s_stg = smem + kPairStages * kPairStageBytes;          // [EW] boxes of 32 rows x 128 bytes (1024-byte aligned)
-  unsigned long long* bars = reinterpret_cast<unsigned long long*>(s_stg + Cfg::kStgBytes);
+  // (top-k: [EW] candidate scratches, then the lists)
+  unsigned long long* bars =
+      reinterpret_cast<unsigned long long*>(s_stg + (kTopk ? TCfg::kScratchBytes + TCfg::kListBytes : Cfg::kStgBytes));
   unsigned long long* full_bar = bars;                        // [kPairStages]   (used in the leader)
   unsigned long long* empty_bar = bars + kPairStages;         // [kPairStages]
   unsigned long long* tfull_bar = bars + 2 * kPairStages;     // [kAccStages]
@@ -962,9 +1000,23 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   const int n_tiles = (int)((n_rows + BN - 1) / BN);
   const long long total_tiles = m_tiles * n_tiles;
   const int num_kb = a.num_taps * a.kblocks_per_tap;
-  const long long t_begin = cluster_id, t_end = total_tiles, t_step = num_clusters;   // this cluster's tiles
+  // top-k: the cluster runs units cluster_id, cluster_id + num_clusters, ... whole; unit u = split * m_tiles + row block
+  // (split-major: the clusters running at the same time sweep the same range of B).  Every unit has unit_tiles n-tiles;
+  // those of the last split past the matrix only load zeros (out-of-bounds boxes) and hold no candidates.
+  const unsigned unit_tiles = kTopk ? (unsigned)a.topk_unit_tiles : 1u;
+  const long long topk_units = kTopk ? m_tiles * (((long long)n_tiles + unit_tiles - 1) / unit_tiles) : 0;
+  const long long topk_mine = cluster_id < topk_units ? (topk_units - 1 - cluster_id) / num_clusters + 1 : 0;
+  const long long t_begin = kTopk ? 0 : cluster_id;                                    // this cluster's tiles
+  const long long t_end = kTopk ? topk_mine * unit_tiles : total_tiles, t_step = kTopk ? 1 : num_clusters;
+  auto topk_unit = [&](long long tile_) { return (unsigned)cluster_id + ((unsigned)tile_ / unit_tiles) * (unsigned)num_clusters; };
   auto coords = [&](long long tile_, long long& mt_, int& nt_) {
-    tile_coords<MODE>(tile_, m_tiles, n_tiles, a.reverse, a.group_m, mt_, nt_);
+    if constexpr (kTopk) {
+      const unsigned u = topk_unit(tile_), s = u / (unsigned)m_tiles;
+      mt_ = u - s * (unsigned)m_tiles;
+      nt_ = (int)(s * unit_tiles + (unsigned)tile_ % unit_tiles);
+    } else {
+      tile_coords<MODE>(tile_, m_tiles, n_tiles, a.reverse, a.group_m, mt_, nt_);
+    }
   };
 
   if (threadIdx.x == 0) {
@@ -1075,7 +1127,32 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     // Per-column vectors of the warp's 128 columns live in a region PRIVATE to the warp (no CTA-wide barrier when the
     // n-tile changes -- in PLDA scoring it changes on every tile): lane l owns columns 4l .. 4l+3, the next tile's values
     // are loaded into registers one tile ahead.
-    float* wv = s_vec + (warp - 2) * (3 * kPCols);
+    float* wv = s_vec + (warp - 2) * ((kTopk ? 1 : 3) * kPCols);
+    // top-k: this thread's list (entry i at s_list[i * kNT + et]: interleaved by thread), its fill, the entry holding its
+    // smallest key and that key's value, the bar every later candidate has to pass (-inf while the list is not full)
+    constexpr int kNT = EW * 32;
+    const int et = threadIdx.x - 64;
+    unsigned long long* s_list = reinterpret_cast<unsigned long long*>(s_stg + TCfg::kScratchBytes);
+    float* scratch = reinterpret_cast<float*>(s_stg) + (warp - 2) * (16 * 32);
+    int tk_cnt = 0, tk_min = 0;
+    float tk_bar = -INFINITY;
+    auto topk_insert = [&](float x, int col) {
+      const int k = a.topk_k;
+      const unsigned long long key = top1_key(x, col);
+      if (tk_cnt < k) {
+        s_list[tk_cnt * kNT + et] = key;
+        if (++tk_cnt < k) return;
+      } else {
+        s_list[tk_min * kNT + et] = key;
+      }
+      unsigned long long lo = ~0ull;
+#pragma unroll 4
+      for (int i = 0; i < k; ++i) {
+        const unsigned long long e = s_list[i * kNT + et];
+        if (e < lo) { lo = e; tk_min = i; }
+      }
+      tk_bar = top1_key_value(lo);
+    };
     constexpr int kVW = kPCols / 32;           // columns per lane: 4 (EW = 8) or 2 (EW = 16)
     int wv_nt = -1, pre_nt = -1;
     float pre_b[kVW], pre_s[kVW], pre_o[kVW];
@@ -1116,6 +1193,10 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       const long long row = row0 + quarter * 32 + lane;
       const unsigned taddr0 =
           tmem_base + ((unsigned)(quarter * 32) << 16) + (unsigned)(acc * BN) + (unsigned)(colq * kPCols);
+      if (kTopk && (unsigned)tile % unit_tiles == 0) {   // a new unit: empty lists
+        tk_cnt = 0;
+        tk_bar = -INFINITY;
+      }
 
       if (wv_nt != nt) {
         if (pre_nt != nt) prefetch_vec(nt);
@@ -1175,6 +1256,42 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         tmem_ld_wait(r[c % kRB]);
         if (kRB == 2 && c + 1 < kPChunks) tmem_ld32_issue(taddr0 + (unsigned)((c + 1) * 32), r[(c + 1) % kRB]);
         const int col0 = col_base + colq * kPCols + c * 32;
+        if constexpr (kTopk) {
+          // the add-only form of the epilogue as below; a value enters the list only if it beats the list's smallest
+          // entry (ties lose: every listed column is lower).  A lane with candidates in half a chunk parks the half in its
+          // column of the warp's scratch and walks them there, so the warp pays for its busiest lane, not for every
+          // column some lane wants to insert.
+          const float4* b4 = reinterpret_cast<const float4*>(wv + c * 32);
+#pragma unroll
+          for (int h = 0; h < 2; ++h) {
+            float v[16];
+            unsigned cand = 0;
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+              const float4 bb = b4[4 * h + q];
+              v[4 * q + 0] = (__uint_as_float(r[c % kRB][16 * h + 4 * q + 0]) + bb.x) + radd;
+              v[4 * q + 1] = (__uint_as_float(r[c % kRB][16 * h + 4 * q + 1]) + bb.y) + radd;
+              v[4 * q + 2] = (__uint_as_float(r[c % kRB][16 * h + 4 * q + 2]) + bb.z) + radd;
+              v[4 * q + 3] = (__uint_as_float(r[c % kRB][16 * h + 4 * q + 3]) + bb.w) + radd;
+            }
+#pragma unroll
+            for (int j = 0; j < 16; ++j)
+              if (col0 + 16 * h + j < n_cols && v[j] > tk_bar) cand |= 1u << j;
+            if (cand != 0) {
+#pragma unroll
+              for (int j = 0; j < 16; ++j) scratch[j * 32 + lane] = v[j];
+              while (cand != 0) {
+                const int j = __ffs(cand) - 1;
+                cand &= cand - 1;
+                const float x = scratch[j * 32 + lane];
+                if (x > tk_bar) topk_insert(x, col0 + 16 * h + j);
+              }
+            }
+          }
+          __syncwarp();                          // converged again before the next .sync.aligned TMEM load / wait
+          if (kRB == 1 && c + 1 < kPChunks) tmem_ld32_issue(taddr0 + (unsigned)((c + 1) * 32), r[0]);
+          continue;
+        }
         if (a.row_best != nullptr) {
           // compact output: nothing is stored, the row keeps its best entry -- the add-only form of the epilogue, columns
           // in ascending order and a strict comparison, so the lowest column wins a tie
@@ -1240,6 +1357,17 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         else mbar_arrive_cluster(acc ? tempty_leader1 : tempty_leader0);
         if (a.trace != nullptr && cluster_id == 0 && rank == 0 && warp == 2 && it < 512)
           a.trace[4 * it + 3] = clock64();                                                         // warp 2 drained its part
+      }
+      if (kTopk && (unsigned)tile % unit_tiles == unit_tiles - 1 && row < m_rows) {   // end of the unit: partial list out
+        const int k = a.topk_k;
+        const long long list = (long long)(topk_unit(tile) / (unsigned)m_tiles) * (EW / 4) + colq;
+        float* os = a.topk_score + (list * m_rows + row) * k;
+        long long* oi = a.topk_index + (list * m_rows + row) * k;
+        for (int i = 0; i < k; ++i) {
+          const unsigned long long key = i < tk_cnt ? s_list[i * kNT + et] : 0ull;
+          os[i] = i < tk_cnt ? top1_key_value(key) : -INFINITY;
+          oi[i] = i < tk_cnt ? (long long)(0xffffffffu - (unsigned)(key & 0xffffffffull)) : -1LL;
+        }
       }
     }
     if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;\n" ::: "memory");   // smem outlives the last boxes
@@ -1908,7 +2036,7 @@ int launch_gemm_pair(const CUtensorMap& tmA, const CUtensorMap& tmB_half, const 
 
 template <int MODE, int EW>
 int launch_gemm_pair_ew(const CUtensorMap& tmA, const CUtensorMap& tmB_half, const TcArgs& args_in, cudaStream_t st) {
-  constexpr int kSmemPair = PairCfg<EW>::kSmem;
+  constexpr int kSmemPair = pair_smem<MODE, EW>();
   constexpr int kPairThreads = PairCfg<EW>::kThreads;
   TcArgs args = args_in;
   if (args.row_add != nullptr && (args.scale != nullptr || args.offset != nullptr)) return KTF_EINVAL;
@@ -1923,8 +2051,11 @@ int launch_gemm_pair_ew(const CUtensorMap& tmA, const CUtensorMap& tmB_half, con
   static unsigned long long attr_done = 0;
   if (ktf::first_use_on_device(&attr_done))
     KTF_CUDA(cudaFuncSetAttribute(tdnn_tc_pair_kernel<MODE, EW>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemPair));
-  const long long tiles = ((args.m_rows + 2 * BM - 1) / (2 * BM)) * ((args.n_rows + BN - 1) / BN);
+  long long tiles = ((args.m_rows + 2 * BM - 1) / (2 * BM)) * ((args.n_rows + BN - 1) / BN);
   if (tiles <= 0) return KTF_OK;
+  if (topk_cap(MODE))   // work units, not tiles, are what the clusters share out
+    tiles = ((args.m_rows + 2 * BM - 1) / (2 * BM)) *
+            (((args.n_rows + BN - 1) / BN + args.topk_unit_tiles - 1) / args.topk_unit_tiles);
   static int dbg = -1;
   if (dbg < 0) {
     const char* e = getenv("KTF_TC_DEBUG");
@@ -2211,6 +2342,84 @@ int tc_gemm_nt(const void* A, long long m, long long lda, const void* B, long lo
     return c_bf16 ? launch_gemm_pair<kModeBf16>(tmA, tmBh, args, st) : launch_gemm_pair<kModeF32>(tmA, tmBh, args, st);
   }
   return c_bf16 ? launch_gemm<kModeBf16>(tmA, tmB, args, st) : launch_gemm<kModeF32>(tmA, tmB, args, st);
+}
+
+}  // namespace ktf
+
+namespace {
+
+// Work units of the top-k walk: how many n-ranges (splits) a 256-row block is cut into.  Few splits keep the lists
+// long-lived (a list fills up once per unit, and every unit writes one partial list per row and column quarter); enough
+// of them give the clusters balanced waves.  Chosen by the modelled time: waves x (tiles per unit + one tile for filling
+// and writing out the lists).  50 000 x 50 000: 196 row blocks x 3 splits of 66 n-tiles = 588 units, 7.9 waves of 74.
+struct TopkPlan {
+  int ew;             // epilogue warps per CTA
+  int unit_tiles;     // n-tiles per unit
+  int splits;
+};
+
+TopkPlan topk_plan(long long m, long long n, long long K) {
+  TopkPlan pl{pair_epi_warps((int)((K + BK - 1) / BK)), 1, 0};
+  const long long m_tiles = (m + 2 * BM - 1) / (2 * BM), n_tiles = (n + BN - 1) / BN;
+  const long long clusters = std::max(1, ktf::num_sms() / 2);
+  double best = 0.0;
+  for (long long s = 1; s <= std::min<long long>(n_tiles, 16); ++s) {
+    const long long len = (n_tiles + s - 1) / s, splits = (n_tiles + len - 1) / len;
+    if (splits != s) continue;                     // the same cut as a smaller s
+    const double cost = (double)((m_tiles * splits + clusters - 1) / clusters) * (double)(len + 1);
+    if (pl.splits == 0 || cost < best) {
+      best = cost;
+      pl.unit_tiles = (int)len;
+      pl.splits = (int)splits;
+    }
+  }
+  return pl;
+}
+
+}  // namespace
+
+namespace ktf {
+
+int tc_topk_lists(long long m, long long n, long long K) {
+  if (m <= 0 || n <= 0) return 0;
+  const TopkPlan pl = topk_plan(m, n, K);
+  return pl.splits * (pl.ew / 4);
+}
+
+int tc_gemm_topk(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
+                 int fp16, const float* row_add, const float* col_add, int k, float* part_score, long long* part_index,
+                 cudaStream_t st) {
+  int rc = check_arch();
+  if (rc != KTF_OK) return rc;
+  if (m <= 0 || n <= 0) return KTF_OK;
+  if (k < 1 || k > 32) {
+    ktf::set_error("tc_gemm_topk: k = %d outside 1..32", k);
+    return KTF_EINVAL;
+  }
+  CUtensorMap tmA, tmBh;
+  if ((rc = encode_map(&tmA, A, (unsigned long long)K, (unsigned long long)m, (unsigned long long)lda, BK, BM)) != KTF_OK)
+    return rc;
+  if ((rc = encode_map(&tmBh, B, (unsigned long long)K, (unsigned long long)n, (unsigned long long)ldb, BK, BN / 2)) != KTF_OK)
+    return rc;
+  const TopkPlan pl = topk_plan(m, n, K);
+  TcArgs args{};
+  args.num_taps = 1;
+  args.kblocks_per_tap = (int)((K + BK - 1) / BK);
+  args.fp16 = fp16;
+  args.m_rows = m;
+  args.n_rows = n;
+  args.bias = col_add;
+  args.row_add = row_add;
+  args.topk_k = k;
+  args.topk_unit_tiles = pl.unit_tiles;
+  args.topk_score = part_score;
+  args.topk_index = part_index;
+#define KTF_TOPK_LAUNCH(MODE_)                                                         \
+  (pl.ew == 16 ? launch_gemm_pair_ew<MODE_, 16>(tmA, tmBh, args, st)                   \
+               : launch_gemm_pair_ew<MODE_, 8>(tmA, tmBh, args, st))
+  rc = k <= 8 ? KTF_TOPK_LAUNCH(kModeTopk8) : k <= 16 ? KTF_TOPK_LAUNCH(kModeTopk16) : KTF_TOPK_LAUNCH(kModeTopk32);
+#undef KTF_TOPK_LAUNCH
+  return rc;
 }
 
 }  // namespace ktf

@@ -143,6 +143,23 @@ class PLDA(Layer):
                                             T.ptr(best), T.ptr(index), T.stream_ptr()))
         return best, index
 
+    def bestMatches(self, u_test, u_enroll=None, *, k, num_examples=1.0):
+        """The k best enrolled vectors per test vector, 1 <= k <= 32: (scores (n_test, k) float32, indexes (n_test, k)
+        int64), row i = the k largest entries of row i of `logLikelihoodRatio` (same arithmetic, bit for bit) and their
+        columns, best first, the lower index first on equal scores -- the first k of a stable descending sort of the row
+        -- without writing the (n_test, n_enroll) matrix (float32 layers only).  Past the last enrolled vector the
+        entries are (-inf, -1).  `u_enroll=None` scores the set against itself."""
+        if self.paramDtype != np.float32:
+            raise ValueError("bestMatches needs a float32 PLDA layer")
+        k = int(k)
+        u_enroll = u_test if u_enroll is None else u_enroll
+        nt, ne = u_test.shape[0], u_enroll.shape[0]
+        scores = torch.empty((nt, max(k, 0)), device=u_test.device, dtype=torch.float32)
+        index = torch.empty((nt, max(k, 0)), device=u_test.device, dtype=torch.int64)
+        N.check(N.lib().ktf_plda_score_topk(self.handle_for(num_examples), T.ptr(u_test), nt, T.ptr(u_enroll), ne, k,
+                                            T.ptr(scores), T.ptr(index), T.stream_ptr()))
+        return scores, index
+
     def call(self, inputs):
         x = T.as_device(inputs)
         self._maybe_build(x.shape)

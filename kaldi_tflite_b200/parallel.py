@@ -12,6 +12,7 @@ Multi-GPU plumbing: one process per GPU (torchrun), torch.distributed for rendez
 import torch
 import torch.distributed as dist
 
+from . import _native
 from . import _tensor as T
 
 
@@ -150,6 +151,45 @@ def plda_score_sharded(plda, x_test_local, x_enroll_local, test_counts=None, out
         works[r].wait()                       # the compute stream waits for block r only
         plda.logLikelihoodRatio(u_all[offs[r]:offs[r + 1]], u_enroll_local, out=scores[offs[r]:offs[r + 1]])
     return scores, u_all
+
+
+def plda_best_matches_sharded(plda, x_test_local, x_enroll_local, k, test_counts=None):
+    """
+    Sharded k-best trial search: `PLDA.bestMatches` of ALL test vectors against ALL enrolled vectors, where each rank
+    holds a slice of both (raw, (n, dim) float32).  The transformed test vectors are all-gathered
+    (`exchange_test_vectors`), the enrolled ones stay where they are: every rank finds the k best of its own enrolled
+    shard for every test row, with indexes offset to the global enrolled numbering (shards in rank order), the ranks
+    exchange these (n_test, k) lists once, and `ktf_topk_merge` reduces them on every rank.  Returns (scores, indexes),
+    (n_test, k) each, test rows ordered by rank -- equal to `bestMatches` on the whole set.
+    """
+    rank, w = world()
+    u_test_local = plda.transformVector(x_test_local.contiguous())
+    if w == 1:
+        return plda.bestMatches(u_test_local, plda.transformVector(x_enroll_local.contiguous()), k=k)
+    u_all, offs, works = exchange_test_vectors(u_test_local, test_counts)
+    u_enroll_local = plda.transformVector(x_enroll_local.contiguous())
+    n = torch.tensor([u_enroll_local.shape[0]], device=u_enroll_local.device, dtype=torch.int64)
+    sizes = [torch.zeros_like(n) for _ in range(w)]
+    dist.all_gather(sizes, n)
+    e_off = sum(int(s.item()) for s in sizes[:rank])
+    for wk in works:
+        if wk is not None:
+            wk.wait()
+    scores, index = plda.bestMatches(u_all, u_enroll_local, k=k)
+    index = torch.where(index >= 0, index + e_off, index)
+    # one exchange: the score bits ride in the int64 tensor next to the indexes
+    local = torch.cat([scores.view(torch.int32).to(torch.int64), index], dim=1)
+    lists = [torch.empty_like(local) for _ in range(w)]
+    dist.all_gather(lists, local)
+    lists = torch.stack(lists)                                     # (w, n_test, 2k)
+    s_in = lists[:, :, :k].to(torch.int32).view(torch.float32).contiguous()
+    i_in = lists[:, :, k:].contiguous()
+    n_test = u_all.shape[0]
+    out_s = torch.empty((n_test, k), device=u_all.device, dtype=torch.float32)
+    out_i = torch.empty((n_test, k), device=u_all.device, dtype=torch.int64)
+    _native.check(_native.lib().ktf_topk_merge(T.ptr(s_in), T.ptr(i_in), w, n_test, k, k, T.ptr(out_s), T.ptr(out_i),
+                                               T.stream_ptr()))
+    return out_s, out_i
 
 
 def stream_batches(fn, host_in, chunk, host_out=None, depth=3):
