@@ -607,7 +607,7 @@ int ktf_frontend_create(const ktf_frontend_cfg* cfg, const float* window_host,
     if ((rc = ktf::upload(&fe->d_dct, dp.data(), dp.size())) != KTF_OK) return fail(rc);
     if ((rc = ktf::upload(&fe->d_lifter, lf.data(), lf.size())) != KTF_OK) return fail(rc);
   }
-  if (getenv("KTF_FRONTEND_GENERIC") == nullptr && cfg->dither == 0.0f &&   // dither: generic kernel (it draws the noise)
+  if (cfg->dither == 0.0f &&   // dither: generic kernel (it draws the noise)
       (rc = r16_build(fe, window_host, mel_bank_host, dct_host, lifter_host)) != KTF_OK) return fail(rc);
   fe->smem_bytes = (R == 32) ? smem_for<32>(fe) : smem_for<16>(fe);
   if (fe->smem_bytes > 227 * 1024) {

@@ -15,8 +15,8 @@
 //     replicas the next layer's taps need and skips the halo rows of its own tile;
 //   * two kernels share the helpers.  tdnn_tc_pair_kernel (row-storing layers, PLDA scoring): clusters of two CTAs
 //     compute 256 x 256 tiles with cta_group::2 (each CTA owns 128 rows and loads half of B), 8 or 16 epilogue warps,
-//     a 5- or 4-stage ring of 32 KB k-blocks, rows leave as 32-row x 128-byte TMA store boxes.  tdnn_tc_kernel
-//     (single CTA, M128 x N256 x K16, 4-stage ring of 48 KB): the STATS layer, and every launch under KTF_TC_PAIR=0;
+//     a 5- or 4-stage ring of 32 KB k-blocks, rows leave as 32-row x 128-byte TMA store boxes.  tdnn_tc_stats_kernel
+//     (single CTA, M128 x N256 x K16, 4-stage ring of 48 KB): the STATS layer;
 //   * warp roles: warp 0 = TMA producer, warp 1 = MMA issuer (one elected lane) + TMEM allocator, the others = epilogue
 //     (a thread owns one accumulator row: TMEM load -> per-column vectors -> staging -> boxed / per-row store);
 //   * 2 accumulator stages of 256 TMEM columns between MMA and epilogue, persistent CTAs (one per SM);
@@ -51,16 +51,11 @@ constexpr int kEpiChunks = kEpiCols / 32;            // 32-column TMEM loads per
 constexpr int kABytes = BM * BK * 2;                 // 16 KB
 constexpr int kBBytes = BN * BK * 2;                 // 32 KB
 constexpr int kStageBytes = kABytes + kBBytes;
-constexpr int kVecBytes = kAccStages * 3 * BN * 4;   // epilogue vectors (bias / scale / offset)
 constexpr int kSegBytes = kAccStages * BN * 4;       // STATS: utterance id of every frame of the tile
-constexpr int kRowSeg = 64;                          // bytes of one output row written by one group of lanes
-constexpr int kStgPitch = kRowSeg + 16;              // staged row pitch: payload + 16 B (bank spread)
-constexpr int kStgBytes = kEpiWarps * 32 * kStgPitch;  // per-warp 32-row transpose buffers for coalesced stores
-constexpr int kSmemTc = kStages * kStageBytes + 1024 /*align*/ + 256 /*barriers*/ + kVecBytes + kSegBytes + kStgBytes;
-static_assert((kStages * kStageBytes) % 512 == 0 && (32 * kStgPitch) % 512 == 0,
-              "staging buffers are TMA-store sources with the 64-byte swizzle: 512-byte aligned");
+constexpr int kSmemTc = kStages * kStageBytes + 1024 /*align*/ + 256 /*barriers*/ + kSegBytes;
+constexpr int kStgPitch = 64 + 16;                   // staged row pitch of the ragged store: 16 floats + 16 B (bank spread)
 
-enum { kModeBf16 = 0, kModeF32 = 1, kModeStats = 2 };
+enum { kModeBf16 = 0, kModeF32 = 1 };                // pair kernel: rows stored as bf16 / fp32
 // Pair kernel, per-row top-k (nothing stored, see TcArgs::topk_k): lists of up to 8, 16 or 32 entries per thread.  The
 // capacity is part of the mode because it sets the shared-memory layout and with it the number of ring stages.
 enum { kModeTopk8 = 3, kModeTopk16 = 4, kModeTopk32 = 5 };
@@ -76,7 +71,7 @@ struct TcArgs {
   int ctx[KTF_MAX_CONTEXT];
   int kblocks_per_tap;      // ceil(D / 64)
   int tap_cols;             // column distance between taps in the weight matrix (= D)
-  int shift_b;              // 0: taps shift the A rows (activations are A); 1: taps shift the B rows (STATS)
+  int pad0;                 // unused: keeps the fields below 16-byte aligned (the kernels load them in pairs, LDCU.128)
   int fp16;                 // operand format: 0 = bf16, 1 = fp16
   long long m_rows;         // rows of the A operand (output rows; STATS: units)
   long long n_rows;         // rows of the B operand (output columns; STATS: frames)
@@ -95,15 +90,15 @@ struct TcArgs {
   long long act_ld_bytes;   // its row pitch and row count
   long long act_rows;
   const long long* rows_dev;  // optional: the ACTUAL number of activation rows, read on the device (m_rows, or n_rows
-                              // when shift_b); the host value is then only an upper bound (VAD-compacted batches: no
+                              // for STATS); the host value is then only an upper bound (VAD-compacted batches: no
                               // host round trip for the kept-row count)
   int group_m;              // > 1: grouped tile walk (see tile_coords)
-  int tma_store;            // rows are written with TMA tensor stores (tmC is valid; see store_chunk)
+  int tma_store;            // rows are written with TMA tensor stores (tmC is valid; see store_box)
   int l2_stream_out;        // the output is a pure stream much larger than L2 while the operands are re-read by every
-                            // tile (PLDA scoring: 10 GB of scores against 76 MB of vectors): operand loads carry an
-                            // evict-last L2 policy and the boxed stores evict-first, so the stream does not push the
-                            // operands out to HBM (measured without: 3.4-4.3 GB of DRAM reads for 76 MB of inputs)
-  int reverse;              // walk the tiles from the last row block to the first (see launch_gemm)
+                            // tile (PLDA scoring: 10 GB of scores against 76 MB of vectors): the boxed stores carry
+                            // an evict-first L2 policy, so the stream does not push the operands out to HBM (measured
+                            // without: 3.4-4.3 GB of DRAM reads for 76 MB of inputs)
+  int reverse;              // walk the tiles from the last row block to the first (the stack's serpentine order)
   int debug;                // development knobs (KTF_TC_DEBUG): 1 = skip global stores, 2 = skip the epilogue math,
                             // 4 = stage the boxes but never issue their stores
   long long* trace;         // development (KTF_TC_TRACE=file): clock64 of cluster 0's tile phases, 4 slots per tile
@@ -158,19 +153,6 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m
       : "memory");
 }
 
-__device__ __forceinline__ void tma_load_2d_hint(void* smem_dst, const CUtensorMap* map, unsigned long long* bar,
-                                                 int c0, int c1, unsigned long long policy) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4}], "
-      "[%2], %5;\n" ::"r"(smem_u32(smem_dst)),
-      "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "l"(policy)
-      : "memory");
-}
-__device__ __forceinline__ unsigned long long l2_policy_evict_last() {
-  unsigned long long p;
-  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;\n" : "=l"(p));
-  return p;
-}
 __device__ __forceinline__ unsigned long long l2_policy_evict_first() {
   unsigned long long p;
   asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;\n" : "=l"(p));
@@ -185,7 +167,7 @@ __device__ __forceinline__ void bulk_prefetch_l2(const void* p, unsigned bytes) 
 }
 
 // TMA tensor store of one staged box (smem -> global) as a bulk async-group; the staging buffer may be rewritten once
-// tma_store_wait_read() has returned (the group has finished READING shared memory).
+// cp.async.bulk.wait_group.read has returned (the group has finished READING shared memory).
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, const void* smem_src, int c0, int c1) {
   asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];\n"
                "cp.async.bulk.commit_group;\n" ::"l"(map), "r"(smem_u32(smem_src)), "r"(c0), "r"(c1)
@@ -196,9 +178,6 @@ __device__ __forceinline__ void tma_store_2d_hint(const CUtensorMap* map, const 
   asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group.L2::cache_hint [%0, {%2, %3}], [%1], %4;\n"
                "cp.async.bulk.commit_group;\n" ::"l"(map), "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "l"(policy)
                : "memory");
-}
-__device__ __forceinline__ void tma_store_wait_read() {
-  asm volatile("cp.async.bulk.wait_group.read 0;\n" ::: "memory");
 }
 // generic-proxy writes to shared memory (the staging STS) -> visible to the async proxy (TMA)
 __device__ __forceinline__ void fence_proxy_async_smem() {
@@ -261,131 +240,8 @@ __device__ __forceinline__ unsigned pack_bf16x2(float lo, float hi) {
   return *reinterpret_cast<unsigned*>(&h);
 }
 
-// One 32-column chunk of a warp's 32 accumulator rows: y = scale * max(acc + bias, relu_lo) + offset (+ radd).
-// A thread owns one ROW of the accumulator (TMEM lane), so storing straight from registers would make every
-// warp-wide store touch 32 different rows with 16 bytes each (32 partial sectors per instruction -- measured
-// as the bottleneck of the K <= 512 layers).  The chunk is therefore transposed through a per-warp staging
-// buffer in kRowSeg-byte row segments (32 bf16 / 16 fp32 columns): lanes write their own row, then 4
-// consecutive lanes read back one row segment, so a warp store covers 8 rows x 64 contiguous bytes (16 full
-// sectors).
-// Rows flagged first / last also write their kHalo replicas; rows without kRowStore are skipped.
-// VEC = false (ragged right edge, unaligned output): fp32 staging, bounds-checked scalar stores.
-// VEC staging layout: row r of the 32 x 64-byte block starts at 64 r and its 16-byte piece g sits at position
-// g ^ ((r >> 1) & 3): the eight lanes of a quarter-warp hit 32 different banks both when lanes write their own row
-// (STS.128, rows 8q .. 8q+7) and when four consecutive lanes read back one row (LDS.128, rows 2q', 2q'+1).
-// `plain` (warp-uniform): every one of the warp's 32 rows is a plain kRowStore row -- no per-row flag traffic.
-template <bool OUT_BF16, bool VEC>
-__device__ __forceinline__ void store_chunk(const unsigned (&r)[32], const float* vb, float relu_lo, float radd,
-                                            unsigned char* stg, int lane, int flags, bool plain, unsigned char* out0,
-                                            long long ld_bytes, int cols_left, const CUtensorMap* tmC, int tma_col,
-                                            int tma_row, bool& tma_pending, unsigned long long store_policy) {
-  const float4* b4 = reinterpret_cast<const float4*>(vb);
-  const float4* s4 = reinterpret_cast<const float4*>(vb + BN);
-  const float4* o4 = reinterpret_cast<const float4*>(vb + 2 * BN);
-  constexpr bool kPacked = OUT_BF16 && VEC;        // staged as bf16 or as fp32
-  constexpr int kCols = kRowSeg / (kPacked ? 2 : 4);   // columns per staged row segment
-  constexpr int kPieces = kRowSeg / 16;            // 16-byte pieces per row segment
-  constexpr int kEs = OUT_BF16 ? 2 : 4;
-  constexpr int kPitch = VEC ? kRowSeg : kStgPitch;
-  constexpr int kGroups = kCols / 8;               // groups of 8 columns per pass
-  const int wsw = (lane >> 1) & 3;                 // swizzle of my own row (VEC): the 64-byte TMA swizzle pattern
-  // `plain` VEC blocks (all 32 rows stored, no halo replicas) leave through a TMA tensor store of the staged box:
-  // no read-back, no per-lane global stores.  tmC == nullptr: st.global path.
-  const bool tma = VEC && plain && tmC != nullptr;
-#pragma unroll
-  for (int pass = 0; pass < 32 / kCols; ++pass) {
-    uint4* mine = reinterpret_cast<uint4*>(stg + lane * kPitch);
-    uint4 val[kPacked ? kGroups : 2 * kGroups];    // the math first: it covers the wait for the previous box
-#pragma unroll
-    for (int g = 0; g < kGroups; ++g) {            // 8 columns per group
-      const int c8 = pass * kGroups + g;           // which group of 8 columns of the chunk
-      float x[8];
-#pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        const float4 bb = b4[2 * c8 + h], ss = s4[2 * c8 + h], oo = o4[2 * c8 + h];
-        x[4 * h + 0] = fmaf(fmaxf(__uint_as_float(r[8 * c8 + 4 * h + 0]) + bb.x, relu_lo), ss.x, oo.x);
-        x[4 * h + 1] = fmaf(fmaxf(__uint_as_float(r[8 * c8 + 4 * h + 1]) + bb.y, relu_lo), ss.y, oo.y);
-        x[4 * h + 2] = fmaf(fmaxf(__uint_as_float(r[8 * c8 + 4 * h + 2]) + bb.z, relu_lo), ss.z, oo.z);
-        x[4 * h + 3] = fmaf(fmaxf(__uint_as_float(r[8 * c8 + 4 * h + 3]) + bb.w, relu_lo), ss.w, oo.w);
-      }
-      if (kPacked) {
-        val[g] = make_uint4(pack_bf16x2(x[0] + radd, x[1] + radd), pack_bf16x2(x[2] + radd, x[3] + radd),
-                            pack_bf16x2(x[4] + radd, x[5] + radd), pack_bf16x2(x[6] + radd, x[7] + radd));
-      } else {
-        val[2 * g] = make_uint4(__float_as_uint(x[0] + radd), __float_as_uint(x[1] + radd),
-                                __float_as_uint(x[2] + radd), __float_as_uint(x[3] + radd));
-        val[2 * g + 1] = make_uint4(__float_as_uint(x[4] + radd), __float_as_uint(x[5] + radd),
-                                    __float_as_uint(x[6] + radd), __float_as_uint(x[7] + radd));
-      }
-    }
-    if (tma_pending) {                             // warp-uniform: the previous box still reads the staging buffer
-      if (lane == 0) tma_store_wait_read();
-      __syncwarp();
-      tma_pending = false;
-    }
-#pragma unroll
-    for (int g = 0; g < kGroups; ++g) {
-      if (kPacked) {
-        mine[g ^ wsw] = val[g];
-      } else {
-        const int sw = VEC ? wsw : 0;
-        mine[(2 * g) ^ sw] = val[2 * g];
-        mine[(2 * g + 1) ^ sw] = val[2 * g + 1];
-      }
-    }
-    if (tma) {
-      fence_proxy_async_smem();
-      __syncwarp();
-      if (lane == 0) {
-        if (store_policy != 0ull) tma_store_2d_hint(tmC, stg, tma_col + pass * kCols, tma_row, store_policy);
-        else tma_store_2d(tmC, stg, tma_col + pass * kCols, tma_row);
-      }
-      tma_pending = true;
-      continue;
-    }
-    __syncwarp();
-    if (VEC) {
-#pragma unroll
-      for (int j = 0; j < kPieces; ++j) {
-        const int q = j * 32 + lane, rr = q / kPieces, part = q % kPieces;
-        const uint4 v = *reinterpret_cast<const uint4*>(stg + rr * kRowSeg + ((part ^ ((rr >> 1) & 3)) * 16));
-        unsigned char* dst = out0 + rr * ld_bytes + pass * kRowSeg + part * 16;
-        if (plain) {
-          *reinterpret_cast<uint4*>(dst) = v;
-          continue;
-        }
-        const int f = __shfl_sync(0xffffffffu, flags, rr);
-        if (f & kRowStore) {
-          *reinterpret_cast<uint4*>(dst) = v;
-          if (f & (kRowFirst | kRowLast)) {
-            const int lo = (f & kRowFirst) ? kHalo : 0, hi = (f & kRowLast) ? kHalo : 0;
-#pragma unroll 1
-            for (int h = -lo; h <= hi; ++h)
-              if (h != 0) *reinterpret_cast<uint4*>(dst + h * ld_bytes) = v;
-          }
-        }
-      }
-    } else {
-#pragma unroll 1
-      for (int k = lane; k < 32 * kCols; k += 32) {
-        const int rr = k / kCols, col = k % kCols;
-        const float v = *reinterpret_cast<const float*>(stg + rr * kStgPitch + col * 4);
-        const int f = __shfl_sync(0xffffffffu, flags, rr);
-        if ((f & kRowStore) && pass * kCols + col < cols_left) {
-          const int lo = (f & kRowFirst) ? kHalo : 0, hi = (f & kRowLast) ? kHalo : 0;
-          unsigned char* dst = out0 + rr * ld_bytes + (long long)(pass * kCols + col) * kEs;
-#pragma unroll 1
-          for (int h = -lo; h <= hi; ++h) {
-            if (OUT_BF16) *reinterpret_cast<__nv_bfloat16*>(dst + h * ld_bytes) = __float2bfloat16_rn(v);
-            else *reinterpret_cast<float*>(dst + h * ld_bytes) = v;
-          }
-        }
-      }
-    }
-    __syncwarp();
-  }
-}
-
+// A thread owns one ROW of the accumulator (TMEM lane), so storing straight from registers would make every warp-wide
+// store touch 32 different rows with 16 bytes each (measured as the bottleneck of the K <= 512 layers): rows are staged.
 // Pair-kernel chunk store through 128-byte-wide staging boxes (32 rows x 128 bytes, the 128-byte TMA swizzle): a 32-column
 // chunk of fp32 rows fills a box, a chunk of bf16 rows fills half of one (HALF = chunk & 1) and the box leaves after the
 // second half -- one boxed store per 4 KB instead of one per 2 KB, i.e. half the fence / elect / issue sequences per tile.
@@ -535,9 +391,8 @@ __device__ __forceinline__ void store_chunk_ragged(const unsigned (&r)[32], cons
   }
 }
 
-// Tile walk: row-storing modes go n-fastest (the n-tiles of one row block run on neighbouring CTAs and
-// share the activation rows through L2); STATS goes m-fastest (the unit tiles of one frame block).
-template <int MODE>
+// Tile walk of the row-storing modes: n-fastest (the n-tiles of one row block run on neighbouring CTAs and share the
+// activation rows through L2).
 __device__ __forceinline__ void tile_coords(long long tile64, long long m_tiles64, int n_tiles, int reverse, int group_m,
                                             long long& mt, int& nt) {
   // tile counts fit 32 bits (2^31 tiles of 128 x 256 outputs is 10^14 elements): 32-bit divisions, not 64-bit ones --
@@ -545,11 +400,7 @@ __device__ __forceinline__ void tile_coords(long long tile64, long long m_tiles6
   const unsigned m_tiles = (unsigned)m_tiles64, nt_n = (unsigned)n_tiles;
   unsigned tile = (unsigned)tile64;
   if (reverse) tile = m_tiles * nt_n - 1u - tile;
-  if (MODE == kModeStats) {
-    const unsigned q = tile / m_tiles;
-    mt = tile - q * m_tiles;
-    nt = (int)q;
-  } else if (group_m > 1) {
+  if (group_m > 1) {
     // grouped walk for wide outputs (PLDA: 196 n-tiles): the 148 CTAs of a wave cover group_m row blocks x ~148 /
     // group_m column blocks, so a wave re-uses its B tiles group_m times while they are hot and the whole B operand is
     // swept once per group_m row blocks instead of once per row block (it has to survive in L2 against the output stream)
@@ -566,37 +417,43 @@ __device__ __forceinline__ void tile_coords(long long tile64, long long m_tiles6
   }
 }
 
-template <int MODE>
+// The layer that feeds StatsPooling, on single-CTA M128 x N256 tiles with the operands swapped: A = weights (M = units),
+// B = activations (N = frames), the taps shift the B rows.
 __global__ void __launch_bounds__(kThreadsTc, 1)
-tdnn_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-               const __grid_constant__ CUtensorMap tmC, const TcArgs a) {
+tdnn_tc_stats_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const TcArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   // 1024-byte alignment for the 128B swizzle; offsetting the __shared__ array (instead of rounding a generic
   // pointer) keeps the address space visible to the compiler, so the epilogue reads are LDS, not generic LD.
   unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   unsigned char* sA = smem;
   unsigned char* sB = smem + kStages * kABytes;
-  unsigned char* s_stg = smem + kStages * kStageBytes;   // [kEpiWarps][32][kStgPitch], 512-byte aligned (TMA store source)
-  unsigned long long* bars = reinterpret_cast<unsigned long long*>(smem + kStages * kStageBytes + kStgBytes);
+  unsigned long long* bars = reinterpret_cast<unsigned long long*>(smem + kStages * kStageBytes);
   unsigned long long* full_bar = bars;                       // [kStages]
   unsigned long long* empty_bar = bars + kStages;            // [kStages]
   unsigned long long* tfull_bar = bars + 2 * kStages;        // [kAccStages]
   unsigned long long* tempty_bar = tfull_bar + kAccStages;   // [kAccStages]
   unsigned* tmem_slot = reinterpret_cast<unsigned*>(tempty_bar + kAccStages);
-  float* s_vec = reinterpret_cast<float*>(smem + kStages * kStageBytes + kStgBytes + 256);  // [kAccStages][3][BN]
-  int* s_seg = reinterpret_cast<int*>(smem + kStages * kStageBytes + kStgBytes + 256 + kVecBytes);  // [kAccStages][BN]
+  int* s_seg = reinterpret_cast<int*>(smem + kStages * kStageBytes + 256);  // [kAccStages][BN]
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  long long m_rows = a.m_rows, n_rows = a.n_rows;
-  if (a.rows_dev != nullptr) {
-    const long long actual = *a.rows_dev;
-    if (a.shift_b) n_rows = min(n_rows, actual); else m_rows = min(m_rows, actual);
-  }
-  const long long act_rows = a.rows_dev != nullptr ? (a.shift_b ? n_rows : m_rows) : a.act_rows;
+  const long long m_rows = a.m_rows;
+  long long n_rows = a.n_rows;
+  if (a.rows_dev != nullptr) n_rows = min(n_rows, *a.rows_dev);
+  const long long act_rows = a.rows_dev != nullptr ? n_rows : a.act_rows;
   const long long m_tiles = (m_rows + BM - 1) / BM;
   const int n_tiles = (int)((n_rows + BN - 1) / BN);
   const long long total_tiles = m_tiles * n_tiles;
   const int num_kb = a.num_taps * a.kblocks_per_tap;
+  // tile walk: m-fastest (the unit tiles of one frame block run on neighbouring CTAs and share its rows through L2),
+  // 32-bit divisions as in tile_coords
+  auto coords = [&](long long tile_, long long& mt_, int& nt_) {
+    const unsigned mt_n = (unsigned)m_tiles;
+    unsigned t = (unsigned)tile_;
+    if (a.reverse) t = mt_n * (unsigned)n_tiles - 1u - t;
+    const unsigned q = t / mt_n;
+    mt_ = t - q * mt_n;
+    nt_ = (int)q;
+  };
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < kStages; ++s) {
@@ -624,25 +481,20 @@ tdnn_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     if (lane == 0) {
       asm volatile("prefetch.tensormap [%0];\n" ::"l"(&tmA) : "memory");
       asm volatile("prefetch.tensormap [%0];\n" ::"l"(&tmB) : "memory");
-      if (a.tma_store) asm volatile("prefetch.tensormap [%0];\n" ::"l"(&tmC) : "memory");
       int stage = 0;
       unsigned phase = 0;
-      const unsigned long long keep = a.l2_stream_out ? l2_policy_evict_last() : 0ull;
       for (long long tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
         long long mt;
         int nt;
-        tile_coords<MODE>(tile, m_tiles, n_tiles, a.reverse, a.group_m, mt, nt);
+        coords(tile, mt, nt);
         const int m0 = (int)(mt * BM), n0 = nt * BN;
         if (a.act_base != nullptr && tile + gridDim.x < total_tiles) {
           long long mt2;
           int nt2;
-          tile_coords<MODE>(tile + gridDim.x, m_tiles, n_tiles, a.reverse, a.group_m, mt2, nt2);
-          // one CTA per activation row block issues the prefetch (the block is shared by the n- / m-tiles)
-          const bool mine = a.shift_b ? (mt2 == 0) : (nt2 == 0);
-          if (mine) {
-            const long long span = a.shift_b ? BN : BM;
-            long long r0 = (a.shift_b ? (long long)nt2 * BN : mt2 * BM) - kHalo;
-            long long r1 = r0 + span + 2 * kHalo;
+          coords(tile + gridDim.x, mt2, nt2);
+          if (mt2 == 0) {   // one CTA per frame block issues the prefetch (the block is shared by the unit tiles)
+            long long r0 = (long long)nt2 * BN - kHalo;
+            long long r1 = r0 + BN + 2 * kHalo;
             r0 = r0 < 0 ? 0 : r0;
             r1 = r1 > act_rows ? act_rows : r1;
             if (r1 > r0)
@@ -656,16 +508,8 @@ tdnn_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           const int wcol = tap * a.tap_cols + d0;          // column in the weight matrix
           mbar_wait(&empty_bar[stage], phase ^ 1);
           mbar_expect_tx(&full_bar[stage], kStageBytes);
-          if (a.shift_b) {
-            tma_load_2d(sA + stage * kABytes, &tmA, &full_bar[stage], wcol, m0);
-            tma_load_2d(sB + stage * kBBytes, &tmB, &full_bar[stage], d0, n0 + a.ctx[tap]);
-          } else if (keep != 0ull) {
-            tma_load_2d_hint(sA + stage * kABytes, &tmA, &full_bar[stage], d0, m0 + a.ctx[tap], keep);
-            tma_load_2d_hint(sB + stage * kBBytes, &tmB, &full_bar[stage], wcol, n0, keep);
-          } else {
-            tma_load_2d(sA + stage * kABytes, &tmA, &full_bar[stage], d0, m0 + a.ctx[tap]);
-            tma_load_2d(sB + stage * kBBytes, &tmB, &full_bar[stage], wcol, n0);
-          }
+          tma_load_2d(sA + stage * kABytes, &tmA, &full_bar[stage], wcol, m0);
+          tma_load_2d(sB + stage * kBBytes, &tmB, &full_bar[stage], d0, n0 + a.ctx[tap]);
           if (++stage == kStages) { stage = 0; phase ^= 1; }
         }
       }
@@ -708,27 +552,11 @@ tdnn_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     const int quarter = warp & 3;             // TMEM lane quarter this warp may access
     const int colq = (warp - 2) >> 2;         // which kEpiCols of the tile's 256 columns
     const int et = threadIdx.x - 64;          // 0..255
-    int staged_nt0 = -1, staged_nt1 = -1;     // n-tile whose epilogue vectors sit in s_vec[0] / s_vec[1]
-    bool tma_pending = false;                 // a TMA store of this warp may still be reading its staging buffer
-    const unsigned long long store_policy = a.l2_stream_out ? l2_policy_evict_first() : 0ull;
-    const CUtensorMap* tmc = a.tma_store ? &tmC : nullptr;
-    float pre_b = 0.0f, pre_s = 1.0f, pre_o = 0.0f;   // column (nt * BN + et) of bias / scale / offset, prefetched
-    int pre_nt = -1;
-    auto prefetch_vec = [&](int nt_) {
-      if (MODE != kModeStats && et < BN) {
-        const int col = nt_ * BN + et;
-        const bool ok = col < n_rows;
-        pre_b = (ok && a.bias) ? a.bias[col] : 0.0f;
-        pre_s = (ok && a.scale) ? a.scale[col] : 1.0f;
-        pre_o = (ok && a.offset) ? a.offset[col] : 0.0f;
-      }
-      pre_nt = nt_;
-    };
     int it = 0;
     for (long long tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++it) {
       long long mt;
       int nt;
-      tile_coords<MODE>(tile, m_tiles, n_tiles, a.reverse, a.group_m, mt, nt);
+      coords(tile, mt, nt);
       const int col_base = nt * BN;
       const int acc = it & 1;
       const unsigned acc_phase = (unsigned)(it >> 1) & 1u;
@@ -736,131 +564,65 @@ tdnn_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       const unsigned taddr0 =
           tmem_base + ((unsigned)(quarter * 32) << 16) + (unsigned)(acc * BN) + (unsigned)(colq * kEpiCols);
 
-      if (MODE == kModeStats) {
-        // ---- per-unit running sums over the frames of the tile (stats_pooling.py:228-240) ----
-        int* seg = s_seg + acc * BN;
-        if (et < BN) {
-          const long long fr = (long long)col_base + et;
-          seg[et] = (fr < n_rows) ? a.rowseg[fr] : -1;
-        }
-        const bool unit_ok = row < m_rows;
-        const float b = (unit_ok && a.bias) ? a.bias[row] : 0.0f;
-        // the sums are of r - c (TcLayer::d_shift), computed as max(acc + (b - c), lo - c): no instruction per frame
-        const float ctr = (unit_ok && a.shift) ? a.shift[row] : 0.0f;
-        const float bc = b - ctr;
-        const float relu_lo = a.relu ? -ctr : -3.402823466e+38f;
-        asm volatile("bar.sync 1, 256;\n" ::: "memory");
-        mbar_wait(&tfull_bar[acc], acc_phase);
-        tc_fence_after();
+      // ---- per-unit running sums over the frames of the tile (stats_pooling.py:228-240) ----
+      int* seg = s_seg + acc * BN;
+      if (et < BN) {
+        const long long fr = (long long)col_base + et;
+        seg[et] = (fr < n_rows) ? a.rowseg[fr] : -1;
+      }
+      const bool unit_ok = row < m_rows;
+      const float b = (unit_ok && a.bias) ? a.bias[row] : 0.0f;
+      // the sums are of r - c (TcLayer::d_shift), computed as max(acc + (b - c), lo - c): no instruction per frame
+      const float ctr = (unit_ok && a.shift) ? a.shift[row] : 0.0f;
+      const float bc = b - ctr;
+      const float relu_lo = a.relu ? -ctr : -3.402823466e+38f;
+      asm volatile("bar.sync 1, 256;\n" ::: "memory");
+      mbar_wait(&tfull_bar[acc], acc_phase);
+      tc_fence_after();
 
-        const int* sg = seg + colq * kEpiCols;
-        float s = 0.0f, s2 = 0.0f;
-        int cur = -1;
-        auto flush = [&]() {
-          if (cur >= 0 && unit_ok) {
-            atomicAdd(a.sums + ((long long)cur * 2 + 0) * m_rows + row, s);
-            atomicAdd(a.sums + ((long long)cur * 2 + 1) * m_rows + row, s2);
+      const int* sg = seg + colq * kEpiCols;
+      float s = 0.0f, s2 = 0.0f;
+      int cur = -1;
+      auto flush = [&]() {
+        if (cur >= 0 && unit_ok) {
+          atomicAdd(a.sums + ((long long)cur * 2 + 0) * m_rows + row, s);
+          atomicAdd(a.sums + ((long long)cur * 2 + 1) * m_rows + row, s2);
+        }
+      };
+      unsigned r[2][32];
+      tmem_ld32_issue(taddr0, r[0]);
+#pragma unroll
+      for (int c = 0; c < kEpiChunks; ++c) {
+        tmem_ld_wait(r[c & 1]);
+        if (c + 1 < kEpiChunks) tmem_ld32_issue(taddr0 + (unsigned)((c + 1) * 32), r[(c + 1) & 1]);
+        const int* sc = sg + c * 32;
+        const int first = sc[0], last = sc[31];
+        if (first == last && first >= 0) {   // warp-uniform: the whole chunk lies inside one utterance
+          if (first != cur) { flush(); cur = first; s = 0.0f; s2 = 0.0f; }
+#pragma unroll
+          for (int i = 0; i < 32; ++i) {
+            const float t = fmaxf(__uint_as_float(r[c & 1][i]) + bc, relu_lo);
+            s += t;
+            s2 = fmaf(t, t, s2);
           }
-        };
-        unsigned r[2][32];
-        tmem_ld32_issue(taddr0, r[0]);
+        } else {                             // utterance boundary / halo rows inside the chunk
 #pragma unroll
-        for (int c = 0; c < kEpiChunks; ++c) {
-          tmem_ld_wait(r[c & 1]);
-          if (c + 1 < kEpiChunks) tmem_ld32_issue(taddr0 + (unsigned)((c + 1) * 32), r[(c + 1) & 1]);
-          const int* sc = sg + c * 32;
-          const int first = sc[0], last = sc[31];
-          if (first == last && first >= 0) {   // warp-uniform: the whole chunk lies inside one utterance
-            if (first != cur) { flush(); cur = first; s = 0.0f; s2 = 0.0f; }
-#pragma unroll
-            for (int i = 0; i < 32; ++i) {
+          for (int i = 0; i < 32; ++i) {
+            const int u = sc[i];
+            if (u >= 0) {
+              if (u != cur) { flush(); cur = u; s = 0.0f; s2 = 0.0f; }
               const float t = fmaxf(__uint_as_float(r[c & 1][i]) + bc, relu_lo);
               s += t;
               s2 = fmaf(t, t, s2);
             }
-          } else {                             // utterance boundary / halo rows inside the chunk
-#pragma unroll
-            for (int i = 0; i < 32; ++i) {
-              const int u = sc[i];
-              if (u >= 0) {
-                if (u != cur) { flush(); cur = u; s = 0.0f; s2 = 0.0f; }
-                const float t = fmaxf(__uint_as_float(r[c & 1][i]) + bc, relu_lo);
-                s += t;
-                s2 = fmaf(t, t, s2);
-              }
-            }
           }
-        }
-        flush();
-      } else {
-        // ---- bias / ReLU / BatchNorm per column, rows stored as bf16 or fp32 ----
-        float* vb = s_vec + acc * 3 * BN;
-        // The per-column vectors of an n-tile are staged once per accumulator stage and reused while the
-        // CTA keeps drawing the same n-tile (always, when gridDim.x is a multiple of n_tiles).
-        const int have_nt = acc ? staged_nt1 : staged_nt0;
-        if (have_nt != nt) {                                 // uniform over all epilogue threads
-          if (pre_nt != nt) prefetch_vec(nt);                 // normally issued one tile earlier (see below)
-          asm volatile("bar.sync 1, 256;\n" ::: "memory");    // every warp is done reading the old vectors
-          if (et < BN) {
-            vb[et] = pre_b;
-            vb[BN + et] = pre_s;
-            vb[2 * BN + et] = pre_o;
-          }
-          asm volatile("bar.sync 1, 256;\n" ::: "memory");
-          if (acc) staged_nt1 = nt; else staged_nt0 = nt;
-        }
-        {
-          // the next tile's per-column vectors: global loads issued now, consumed after this tile's stores
-          const long long next = tile + gridDim.x;
-          if (next < total_tiles) {
-            long long mt2;
-            int nt2;
-            tile_coords<MODE>(next, m_tiles, n_tiles, a.reverse, a.group_m, mt2, nt2);
-            const int have2 = acc ? staged_nt0 : staged_nt1;   // the next tile uses the other accumulator stage
-            if (have2 != nt2 && pre_nt != nt2) prefetch_vec(nt2);
-          }
-        }
-        int flags = 0;
-        if (row < m_rows) flags = a.rowmap ? a.rowmap[row] : kRowStore;
-        if (a.debug & 1) flags = 0;
-        const bool plain = __all_sync(0xffffffffu, (flags & kRowFlagMask) == kRowStore);
-        float radd = 0.0f;
-        if (a.row_add != nullptr && row < m_rows) radd = a.row_add[row];
-        mbar_wait(&tfull_bar[acc], acc_phase);
-        tc_fence_after();
-
-        const int n_cols = (int)n_rows;
-        constexpr bool kBf16 = (MODE == kModeBf16);
-        constexpr int kEs = kBf16 ? 2 : 4;                   // output element size
-        const long long ld_bytes = a.out_ld * kEs;
-        unsigned char* owarp = reinterpret_cast<unsigned char*>(a.out) + (mt * BM + quarter * 32) * ld_bytes;
-        unsigned char* stg = s_stg + (warp - 2) * (32 * kStgPitch);
-        const bool vec_ok = ((reinterpret_cast<unsigned long long>(a.out) | (unsigned long long)ld_bytes) & 15ull) == 0;
-        const float relu_lo = a.relu ? 0.0f : -3.402823466e+38f;
-        unsigned r[2][32];                                // TMEM loads run one chunk ahead of the math / stores
-        tmem_ld32_issue(taddr0, r[0]);
-#pragma unroll
-        for (int c = 0; c < kEpiChunks; ++c) {
-          tmem_ld_wait(r[c & 1]);
-          if (c + 1 < kEpiChunks) tmem_ld32_issue(taddr0 + (unsigned)((c + 1) * 32), r[(c + 1) & 1]);
-          const int cc = colq * kEpiCols + c * 32;        // column offset inside the tile
-          const int col0 = col_base + cc;
-          if (col0 >= n_cols || (a.debug & 2)) continue;  // warp-uniform
-          unsigned char* out0 = owarp + (long long)col0 * kEs;
-          const int trow = (int)(mt * BM) + quarter * 32;
-          if (vec_ok && col0 + 32 <= n_cols)
-            store_chunk<kBf16, true>(r[c & 1], vb + cc, relu_lo, radd, stg, lane, flags, plain, out0, ld_bytes, 32, tmc,
-                                     col0, trow, tma_pending, store_policy);
-          else
-            store_chunk<kBf16, false>(r[c & 1], vb + cc, relu_lo, radd, stg, lane, flags, false, out0, ld_bytes,
-                                      n_cols - col0, nullptr, 0, 0, tma_pending, 0ull);
         }
       }
+      flush();
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&tempty_bar[acc]);
     }
-    if (tma_pending && lane == 0) tma_store_wait_read();   // shared memory must outlive the last box
   }
 
   tc_fence_before();
@@ -967,7 +729,6 @@ template <int MODE, int EW>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(PairCfg<EW>::kThreads, 1)
 tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                     const __grid_constant__ CUtensorMap tmC, const TcArgs a) {
-  static_assert(MODE != kModeStats, "the pair kernel covers the row-storing modes");
   using Cfg = PairCfg<EW>;
   constexpr int kCap = topk_cap(MODE);
   constexpr bool kTopk = kCap > 0;
@@ -1015,7 +776,7 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       mt_ = u - s * (unsigned)m_tiles;
       nt_ = (int)(s * unit_tiles + (unsigned)tile_ % unit_tiles);
     } else {
-      tile_coords<MODE>(tile_, m_tiles, n_tiles, a.reverse, a.group_m, mt_, nt_);
+      tile_coords(tile_, m_tiles, n_tiles, a.reverse, a.group_m, mt_, nt_);
     }
   };
 
@@ -1852,8 +1613,8 @@ struct TcLayer {
   // formed from fp32 sums of r itself cancels -- 9e-3 relative error in the pooled std at mean / std = 200 over 300
   // frames.  Centred, the sums are of the size of the std.
   float* d_shift = nullptr;
-  CUtensorMap tmW_n;                // weights as the B operand (box BK x BN)
-  CUtensorMap tmW_m;                // weights as the A operand (box BK x BM), STATS mode
+  CUtensorMap tmW_m;                // weights, box BK x BM: the pair kernel's B operand (each CTA loads 128 of a tile's
+                                    // 256 columns) and the stats kernel's A operand
   ktf::Workspace ws;                // scratch of the stand-alone layer call
 };
 
@@ -1900,21 +1661,20 @@ int encode_map(CUtensorMap* map, const void* base, unsigned long long inner, uns
 }
 
 // Output map for the TMA-store epilogue: row-major (rows, cols) matrix of 2-byte (bf16) or 4-byte (fp32) elements, boxes
-// of 32 rows x 64 bytes with the 64-byte swizzle (the layout store_chunk stages) or 32 rows x 128 bytes with the 128-byte
-// swizzle (store_box, pair kernel).  Returns false when the matrix cannot
+// of 32 rows x 128 bytes with the 128-byte swizzle (the layout store_box stages).  Returns false when the matrix cannot
 // be described (unaligned base / pitch): the epilogue then keeps its st.global path.
 bool encode_map_out(CUtensorMap* map, const void* base, int elem_bytes, unsigned long long cols, unsigned long long rows,
-                    unsigned long long ld_elems, int row_bytes = kRowSeg) {
+                    unsigned long long ld_elems) {
   EncodeTiledFn fn = encode_tiled_fn();
   if (fn == nullptr || base == nullptr || rows == 0 || cols == 0) return false;
   if ((reinterpret_cast<unsigned long long>(base) & 15ull) != 0 || ((ld_elems * elem_bytes) & 15ull) != 0) return false;
   cuuint64_t dims[2] = {cols, rows};
   cuuint64_t strides[1] = {ld_elems * elem_bytes};
-  cuuint32_t box[2] = {(cuuint32_t)(row_bytes / elem_bytes), 32};
+  cuuint32_t box[2] = {(cuuint32_t)(kBoxRow / elem_bytes), 32};
   cuuint32_t estr[2] = {1, 1};
   const CUresult r = fn(map, elem_bytes == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2,
                         const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        row_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
+                        CU_TENSOR_MAP_SWIZZLE_128B,
                         CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return r == CUDA_SUCCESS;
 }
@@ -1946,9 +1706,6 @@ int prepare_layer(TcLayer* L, const ktf_affine_cfg& c, const float* w_host) {
   int rc;
   if ((rc = ktf::upload(&L->d_w, wb.data(), wb.size())) != KTF_OK) return rc;
   if ((rc = ktf::upload(&L->d_ctx, L->ctx, (size_t)KTF_MAX_CONTEXT)) != KTF_OK) return rc;
-  if ((rc = encode_map(&L->tmW_n, L->d_w, (unsigned long long)cols, (unsigned long long)c.out_dim,
-                       (unsigned long long)L->w_ld, BK, BN)) != KTF_OK)
-    return rc;
   return encode_map(&L->tmW_m, L->d_w, (unsigned long long)cols, (unsigned long long)c.out_dim,
                     (unsigned long long)L->w_ld, BK, BM);
 }
@@ -1961,54 +1718,20 @@ void release_layer(TcLayer* L) {
   L->ws.release();
 }
 
-int tma_store_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("KTF_TC_TMA_STORE");     // development knob: 0 = st.global epilogue
-    on = e ? atoi(e) : 1;
-  }
-  return on;
-}
-
-template <int MODE>
-int launch_gemm(const CUtensorMap& tmA, const CUtensorMap& tmB, const TcArgs& args_in, cudaStream_t st) {
-  TcArgs args = args_in;
-  CUtensorMap tmC = tmA;                                // placeholder when the epilogue does not use it
-  args.tma_store = 0;
-  if (MODE != kModeStats && tma_store_enabled() && args.out != nullptr) {
-    const int es = (MODE == kModeBf16) ? 2 : 4;
-    if (encode_map_out(&tmC, args.out, es, (unsigned long long)args.n_rows, (unsigned long long)args.m_rows,
-                       (unsigned long long)args.out_ld))
-      args.tma_store = 1;
-  }
+int launch_gemm_stats(const CUtensorMap& tmA, const CUtensorMap& tmB, const TcArgs& args, cudaStream_t st) {
   static unsigned long long attr_done = 0;              // per device (function attributes are per context)
   if (ktf::first_use_on_device(&attr_done))
-    KTF_CUDA(cudaFuncSetAttribute(tdnn_tc_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTc));
+    KTF_CUDA(cudaFuncSetAttribute(tdnn_tc_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTc));
   const long long tiles = ((args.m_rows + BM - 1) / BM) * ((args.n_rows + BN - 1) / BN);
   if (tiles <= 0) return KTF_OK;
-  static int dbg = -1;
-  if (dbg < 0) {
-    const char* e = getenv("KTF_TC_DEBUG");
-    dbg = e ? atoi(e) : 0;
-  }
-  args.debug = dbg;
   const unsigned grid = (unsigned)std::min<long long>(tiles, ktf::num_sms());
-  tdnn_tc_kernel<MODE><<<grid, kThreadsTc, kSmemTc, st>>>(tmA, tmB, tmC, args);
+  tdnn_tc_stats_kernel<<<grid, kThreadsTc, kSmemTc, st>>>(tmA, tmB, args);
   KTF_LAUNCH_OK();
   return KTF_OK;
 }
 
-int pair_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("KTF_TC_PAIR");     // development knob: 0 = single-CTA tiles for every launch
-    on = e ? atoi(e) : 1;
-  }
-  return on;
-}
-
 // CTA-pair launch of a row-storing mode.  tmB must be encoded with 128-row boxes (each CTA loads half of the tile's 256
-// columns); everything else as launch_gemm.
+// columns).
 // Epilogue warps per CTA of the pair kernel.  The per-tile trace (KTF_TC_TRACE) shows which side waits: with K <= 256
 // (tdnn1) the accumulator is ready long before the 16 epilogue warps are done -- epilogue-bound, 16 warps win (period 5.1 k
 // against 5.5 k clocks with 8); from K = 384 up the MMA thread waits for operands (tdnn4: 6.9 k of 7.5 k clocks per tile),
@@ -2042,10 +1765,10 @@ int launch_gemm_pair_ew(const CUtensorMap& tmA, const CUtensorMap& tmB_half, con
   if (args.row_add != nullptr && (args.scale != nullptr || args.offset != nullptr)) return KTF_EINVAL;
   CUtensorMap tmC = tmA;
   args.tma_store = 0;
-  if (tma_store_enabled() && args.out != nullptr) {
+  if (args.out != nullptr) {
     const int es = (MODE == kModeBf16) ? 2 : 4;
     if (encode_map_out(&tmC, args.out, es, (unsigned long long)args.n_rows, (unsigned long long)args.m_rows,
-                       (unsigned long long)args.out_ld, kBoxRow))
+                       (unsigned long long)args.out_ld))
       args.tma_store = 1;
   }
   static unsigned long long attr_done = 0;
@@ -2153,9 +1876,7 @@ int run_layer(const TcLayer& L, const ktf_affine* a, const __nv_bfloat16* A, lon
   args.relu = a->cfg.activation == KTF_ACT_RELU;
   args.out = out;
   args.out_ld = out_ld;
-  if (pair_enabled())   // CTA-pair tiles: each CTA loads 128 of the 256 weight rows of a tile (tmW_m has 128-row boxes)
-    return out_bf16 ? launch_gemm_pair<kModeBf16>(tmA, L.tmW_m, args, st) : launch_gemm_pair<kModeF32>(tmA, L.tmW_m, args, st);
-  return out_bf16 ? launch_gemm<kModeBf16>(tmA, L.tmW_n, args, st) : launch_gemm<kModeF32>(tmA, L.tmW_n, args, st);
+  return out_bf16 ? launch_gemm_pair<kModeBf16>(tmA, L.tmW_m, args, st) : launch_gemm_pair<kModeF32>(tmA, L.tmW_m, args, st);
 }
 
 // The layer that feeds StatsPooling: operands swapped (M = units, N = frames), epilogue accumulates
@@ -2168,7 +1889,6 @@ int run_layer_stats(const TcLayer& L, const ktf_affine* a, const __nv_bfloat16* 
   if (rc != KTF_OK) return rc;
   TcArgs args{};
   fill_taps(args, L, x_is_spliced, x_cols);
-  args.shift_b = 1;
   args.m_rows = L.U;
   args.n_rows = frames;
   args.act_base = X;
@@ -2181,7 +1901,7 @@ int run_layer_stats(const TcLayer& L, const ktf_affine* a, const __nv_bfloat16* 
   args.shift = L.d_shift;       // the sums are centred on the BatchNorm moving mean
   args.relu = a->cfg.activation == KTF_ACT_RELU;
   args.sums = sums;
-  return launch_gemm<kModeStats>(L.tmW_m, tmX, args, st);
+  return launch_gemm_stats(L.tmW_m, tmX, args, st);
 }
 
 unsigned blocks_for(long long items, int threads) {
@@ -2314,10 +2034,10 @@ int tc_gemm_nt(const void* A, long long m, long long lda, const void* B, long lo
                cudaStream_t st, unsigned long long* row_best) {
   int rc = check_arch();
   if (rc != KTF_OK) return rc;
-  CUtensorMap tmA, tmB;
+  CUtensorMap tmA, tmBh;   // B in 128-row boxes: each CTA of a pair loads half of the tile's 256 columns
   if ((rc = encode_map(&tmA, A, (unsigned long long)K, (unsigned long long)m, (unsigned long long)lda, BK, BM)) != KTF_OK)
     return rc;
-  if ((rc = encode_map(&tmB, B, (unsigned long long)K, (unsigned long long)n, (unsigned long long)ldb, BK, BN)) != KTF_OK)
+  if ((rc = encode_map(&tmBh, B, (unsigned long long)K, (unsigned long long)n, (unsigned long long)ldb, BK, BN / 2)) != KTF_OK)
     return rc;
   TcArgs args{};
   args.num_taps = 1;
@@ -2335,13 +2055,7 @@ int tc_gemm_nt(const void* A, long long m, long long lda, const void* B, long lo
   if (const char* e = getenv("KTF_TC_L2_HINTS")) args.l2_stream_out = atoi(e);
   args.group_m = (n + BN - 1) / BN > 8 ? 32 : 0;     // (measured at 50 000^2: 1 -> 2.77, 8 -> 2.61, 16 -> 2.54, 32 -> 2.47-2.51, 64 -> 2.65 ms)
   if (const char* e = getenv("KTF_TC_GROUP_M")) args.group_m = atoi(e);
-  if (pair_enabled() || row_best != nullptr) {    // (the best-entry epilogue exists in the pair kernel only)
-    CUtensorMap tmBh;
-    if ((rc = encode_map(&tmBh, B, (unsigned long long)K, (unsigned long long)n, (unsigned long long)ldb, BK, BN / 2)) != KTF_OK)
-      return rc;
-    return c_bf16 ? launch_gemm_pair<kModeBf16>(tmA, tmBh, args, st) : launch_gemm_pair<kModeF32>(tmA, tmBh, args, st);
-  }
-  return c_bf16 ? launch_gemm<kModeBf16>(tmA, tmB, args, st) : launch_gemm<kModeF32>(tmA, tmB, args, st);
+  return c_bf16 ? launch_gemm_pair<kModeBf16>(tmA, tmBh, args, st) : launch_gemm_pair<kModeF32>(tmA, tmBh, args, st);
 }
 
 }  // namespace ktf

@@ -11,7 +11,7 @@ ncu --set full --clock-control none --import-source on -k regex:frontend_r16 -s 
 ncu --set full --clock-control none --import-source on -k regex:cmvn_staged -s 3 -c 1 \
     -o gpurun_out/prof_cmvn_$TAG -f python scripts/quick_time.py 1024 > gpurun_out/ncu_cmvn_$TAG.log 2>&1
 cat gpurun_out/bench_$TAG.json
-ncu --set full --clock-control none -k regex:tdnn_tc_kernel -s 14 -c 7 \
+ncu --set full --clock-control none -k "regex:tdnn_tc_(pair|stats)_kernel" -s 14 -c 7 \
     -o gpurun_out/prof_tdnn_$TAG -f python bench.py --workload tdnn --steps 3 --warmup 1 --no-stages --no-cpu-baseline > gpurun_out/ncu_tdnn_$TAG.log 2>&1
 python bench.py --impl reference --steps 2 --warmup 1 > gpurun_out/bench_ref_$TAG.json 2> gpurun_out/bench_ref_$TAG.err
 python -c "import __graft_entry__ as g; g.smoke()" > gpurun_out/smoke_$TAG.log 2>&1; tail -2 gpurun_out/smoke_$TAG.log

@@ -112,7 +112,7 @@ def traffic(dst, *_):
             continue
         seen.add(key)
         per.append(k)
-    out["tdnn_stack"] = {"kernel": "gather_cmvn_splice_kernel + tdnn_tc_pair_kernel x5 + tdnn_tc_kernel<STATS> (one "
+    out["tdnn_stack"] = {"kernel": "gather_cmvn_splice_kernel + tdnn_tc_pair_kernel x5 + tdnn_tc_stats_kernel (one "
                                    "wav2xvec step)",
                          "dram_bytes_per_launch": sum(k["dram_bytes"] for k in per),
                          "gpu_time_us": sum(k["us"] for k in per), "per_kernel": per,
