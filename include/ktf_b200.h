@@ -415,6 +415,34 @@ int ktf_plda_score_topk(const ktf_plda* p, const void* u_test_dev, int64_t n_tes
 int ktf_topk_merge(const float* scores_in_dev, const int64_t* index_in_dev, int32_t num_lists, int64_t n_rows,
                    int32_t k_in, int32_t k, float* scores_dev, int64_t* index_dev, void* stream);
 
+/* Adaptive symmetric score normalisation (AS-norm1, Matejka et al., Interspeech 2017) in two steps.
+ *
+ * Cohort statistics: for each of the n vectors u_dev (n, dim), the mean (mean_dev[i]) and the population standard
+ * deviation (std_dev[i], ddof 0) of its top_n largest scores against the n_cohort cohort vectors, and optionally
+ * (nth_dev, nullable) the top_n-th largest score itself.  role KTF_COHORT_AS_TEST: the scores are row i of
+ * ktf_plda_score(p, u, cohort) -- the vector plays the test role, the cohort vectors are enrolled ones.
+ * KTF_COHORT_AS_ENROLLED: column i of ktf_plda_score(p, cohort, u) -- the vector keeps its enrolled role (and the
+ * handle's num_examples), the cohort vectors are test vectors.  The scores are bit-equal to those matrix entries and the
+ * selection is exact; the statistics are evaluated in float64 and rounded once, and each vector's depend on nothing
+ * but that vector and the cohort.  KTF_EINVAL unless 2 <= top_n <= n_cohort < 2^32; n == 0 is a no-op.  Needs a float32
+ * handle (the tcgen05 score GEMM).  The raw cohort scores go through the handle's grow-only workspace in row chunks of
+ * at most 64 MB; no host synchronisation, so once the workspace has grown for a shape the call can be captured in a
+ * CUDA graph.  Calls on one handle must not run concurrently on different streams.
+ *
+ * Normalised scores: scores_dev (n_test, ld) float32 with, for s = the ktf_plda_score entry (same arithmetic, bit for
+ * bit) and the statistics the caller passes (e.g. enrolment statistics computed once for many test batches),
+ *     scores[i, j] = 0.5 ((s - enroll_mean[j]) / enroll_std[j] + (s - test_mean[i]) / test_std[i])
+ * evaluated with the reciprocals of the deviations; a deviation of 0 gives the IEEE result of the division, not an
+ * error.  The normalisation happens in the score kernel's epilogue: the matrix is written once.  Needs a float32 handle;
+ * the workspace rules of ktf_plda_cohort_stats apply. */
+enum { KTF_COHORT_AS_TEST = 0, KTF_COHORT_AS_ENROLLED = 1 };
+int ktf_plda_cohort_stats(const ktf_plda* p, const void* u_dev, int64_t n, const void* u_cohort_dev, int64_t n_cohort,
+                          int64_t top_n, int32_t role, float* mean_dev, float* std_dev, float* nth_dev, void* stream);
+int ktf_plda_score_asnorm(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,
+                          int64_t n_enroll, const float* test_mean_dev, const float* test_std_dev,
+                          const float* enroll_mean_dev, const float* enroll_std_dev, float* scores_dev, int64_t ld,
+                          void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -220,7 +220,11 @@ int topk_merge(const float* s_in, const long long* i_in, int num_lists, long lon
 }
 
 // Operands of the tensor-core score GEMM, in the handle's workspace: the fp16 hi/lo splits of both sides (K = 3 dim) and
-// A_i / B_j, followed by `extra` bytes of the caller's.
+// A_i / B_j, followed by `extra` bytes of the caller's.  The GEMM's rows are normally the test vectors (c-scaled split,
+// A addend) and its columns the enrolled ones (plain split, B addend).  With `enrolled_rows` the roles swap sides: the
+// rows (ut) are enrolled vectors and get the plain split and the B addend, the columns (ue) play the test role.  The
+// cross term is symmetric and the three partial products meet the same K positions, so the accumulator is the transpose
+// of the normal one; Ai / Bj are then the row / column addends (B of the rows, A of the columns).
 struct TcOperands {
   const __half* A;
   const __half* B;
@@ -230,7 +234,7 @@ struct TcOperands {
 };
 
 int tc_operands(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, size_t extra,
-                cudaStream_t st, TcOperands* o) {
+                cudaStream_t st, TcOperands* o, bool enrolled_rows = false) {
   const int dim = p->dim;
   const long long K = 3LL * dim;
   ktf::Carver cv;
@@ -246,17 +250,24 @@ int tc_operands(const ktf_plda* p, const float* ut, int64_t nt, const float* ue,
   __half* Bs = reinterpret_cast<__half*>(base + o_b);
   float* Ai = reinterpret_cast<float*>(base + o_ai);
   float* Bj = reinterpret_cast<float*>(base + o_bj);
-  plda_quad_kernel<float><<<(unsigned)((nt + 7) / 8), 256, 0, st>>>(ut, nt, dim, (const float*)p->d_wa,
-                                                                    (float)p->logdet_term, Ai);
+  const float* wa = (const float*)p->d_wa;
+  const float* wb = (const float*)p->d_wb;
+  const float* c = (const float*)p->d_c;
+  const float ld = (float)p->logdet_term;
+  plda_quad_kernel<float><<<(unsigned)((nt + 7) / 8), 256, 0, st>>>(ut, nt, dim, enrolled_rows ? wb : wa,
+                                                                    enrolled_rows ? 0.0f : ld, Ai);
   KTF_LAUNCH_OK();
-  plda_quad_kernel<float><<<(unsigned)((ne + 7) / 8), 256, 0, st>>>(ue, ne, dim, (const float*)p->d_wb, 0.0f, Bj);
+  plda_quad_kernel<float><<<(unsigned)((ne + 7) / 8), 256, 0, st>>>(ue, ne, dim, enrolled_rows ? wa : wb,
+                                                                    enrolled_rows ? ld : 0.0f, Bj);
   KTF_LAUNCH_OK();
   auto blocks = [](long long items) {
     return (unsigned)std::min<long long>((items + 255) / 256, (long long)ktf::num_sms() * 16);
   };
-  plda_split_kernel<<<blocks(nt * dim), 256, 0, st>>>(ut, nt, dim, (const float*)p->d_c, 0, As);
+  plda_split_kernel<<<blocks(nt * dim), 256, 0, st>>>(ut, nt, dim, enrolled_rows ? nullptr : c, enrolled_rows ? 1 : 0,
+                                                      As);
   KTF_LAUNCH_OK();
-  plda_split_kernel<<<blocks(ne * dim), 256, 0, st>>>(ue, ne, dim, nullptr, 1, Bs);
+  plda_split_kernel<<<blocks(ne * dim), 256, 0, st>>>(ue, ne, dim, enrolled_rows ? c : nullptr, enrolled_rows ? 0 : 1,
+                                                      Bs);
   KTF_LAUNCH_OK();
   *o = TcOperands{As, Bs, Ai, Bj, base + o_extra};
   return KTF_OK;
@@ -297,6 +308,186 @@ int score_tc_topk(const ktf_plda* p, const float* ut, int64_t nt, const float* u
   if ((rc = ktf::tc_gemm_topk(o.A, nt, K, o.B, ne, K, K, /*fp16=*/1, o.Ai, o.Bj, k, part_s, part_i, st)) != KTF_OK)
     return rc;
   return topk_merge(part_s, part_i, lists, nt, k, k, score, index, st);
+}
+
+// ---- AS-norm: per-vector statistics of the top-N cohort scores, normalised score matrix ----
+constexpr int kSelThreads = 512;
+constexpr int kSelBins = 4096;                    // histogram bins of the first radix pass (12 bits); the others use 10
+constexpr long long kSelSmemRowMax = 48 * 1024;   // rows up to this long are held in shared memory as keys (208 KB)
+constexpr double kCohortChunkBytes = 64e6;        // raw cohort scores per chunk: written by the GEMM, read from L2
+
+__device__ __forceinline__ unsigned order_key(float v) {   // unsigned order = float order
+  const unsigned b = __float_as_uint(v);
+  return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+}
+__device__ __forceinline__ float key_value(unsigned k) {
+  return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
+}
+
+// One CTA per row of a chunk of raw cohort accumulators x (pitch ld).  The score is (x + first) + second: column addend
+// then row addend for the test role (B of the cohort vector, A of the test vector), row addend then column addend for
+// the enrolled role (B of the enrolled vector, A of the cohort vector) -- the association of the score GEMM's epilogue,
+// so every score is bit-equal to its logLikelihoodRatio entry.
+// Exact top_n-th largest score: radix select on order keys, three passes of 12 + 10 + 10 bits, each a shared-memory
+// histogram of the keys under the prefix found so far.  Mean and std of the top_n multiset in float64, relative to that
+// threshold t: the keys above it contribute x - t and (x - t)^2, the (top_n - count above) copies of t contribute 0.
+// Every thread sums its columns in index order and the CTA adds the threads' sums in a fixed tree, so the statistics
+// depend on the row alone (not on its batch-mates or the chunking).
+__global__ void __launch_bounds__(kSelThreads) cohort_select_kernel(const float* __restrict__ x, long long ld,
+                                                                    long long nc, const float* __restrict__ row_add,
+                                                                    const float* __restrict__ col_add, int row_first,
+                                                                    unsigned top_n, int in_smem, float* __restrict__ mean,
+                                                                    float* __restrict__ stdev, float* __restrict__ nth) {
+  extern __shared__ unsigned sel_smem[];
+  unsigned* hist = sel_smem;                  // [kSelBins]
+  unsigned* keys = sel_smem + kSelBins;       // [nc] when in_smem
+  __shared__ unsigned s_warp[kSelThreads / 32];
+  __shared__ double s_sum[kSelThreads / 32], s_sq[kSelThreads / 32];
+  __shared__ unsigned s_digit, s_need;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const long long row = blockIdx.x;
+  const float* xr = x + row * ld;
+  const float ra = row_add[row];
+  auto key_at = [&](long long c) {
+    return order_key(row_first ? (xr[c] + ra) + col_add[c] : (xr[c] + col_add[c]) + ra);
+  };
+  if (in_smem)
+    for (long long c = tid; c < nc; c += kSelThreads) keys[c] = key_at(c);
+  auto key = [&](long long c) { return in_smem ? keys[c] : key_at(c); };
+
+  unsigned prefix = 0, pmask = 0, need = top_n;   // need: rank of the target among the keys under the prefix
+  for (int pass = 0; pass < 3; ++pass) {
+    const int shift = pass == 0 ? 20 : (pass == 1 ? 10 : 0);
+    const unsigned nb = pass == 0 ? 4096u : 1024u, per = nb / kSelThreads;
+    for (unsigned b = tid; b < nb; b += kSelThreads) hist[b] = 0;
+    __syncthreads();                              // (first pass: the keys are in shared memory too)
+    for (long long c = tid; c < nc; c += kSelThreads) {
+      const unsigned k = key(c);
+      if ((k & pmask) == prefix) atomicAdd(&hist[(k >> shift) & (nb - 1)], 1u);
+    }
+    __syncthreads();
+    // the digit d with #(keys above d) < need <= #(keys at or above d); thread t owns bins [t per, (t + 1) per)
+    unsigned loc = 0;
+    for (unsigned i = 0; i < per; ++i) loc += hist[tid * per + i];
+    unsigned incl = loc;                          // sum over this and the higher lanes of the warp
+    for (int o = 1; o < 32; o <<= 1) {
+      const unsigned v = __shfl_down_sync(0xffffffffu, incl, o);
+      if (lane + o < 32) incl += v;
+    }
+    if (lane == 0) s_warp[warp] = incl;
+    __syncthreads();
+    unsigned above = incl - loc;
+    for (int w = warp + 1; w < kSelThreads / 32; ++w) above += s_warp[w];
+    if (above < need && need <= above + loc) {    // exactly one thread
+      unsigned acc = above;
+      for (int i = (int)per - 1; i >= 0; --i) {
+        const unsigned h = hist[tid * per + i];
+        if (need <= acc + h) {
+          s_digit = tid * per + (unsigned)i;
+          s_need = need - acc;
+          break;
+        }
+        acc += h;
+      }
+    }
+    __syncthreads();
+    prefix |= s_digit << shift;
+    pmask |= (nb - 1) << shift;
+    need = s_need;
+    __syncthreads();                              // hist / s_warp / s_digit are rewritten by the next pass
+  }
+  const double thr = (double)key_value(prefix);
+  double sum = 0.0, sq = 0.0;
+  for (long long c = tid; c < nc; c += kSelThreads) {
+    const unsigned k = key(c);
+    if (k > prefix) {
+      const double d = (double)key_value(k) - thr;
+      sum += d;
+      sq += d * d;
+    }
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    sum += __shfl_xor_sync(0xffffffffu, sum, o);
+    sq += __shfl_xor_sync(0xffffffffu, sq, o);
+  }
+  if (lane == 0) {
+    s_sum[warp] = sum;
+    s_sq[warp] = sq;
+  }
+  __syncthreads();
+  if (tid == 0) {
+    double S = 0.0, Q = 0.0;
+    for (int w = 0; w < kSelThreads / 32; ++w) {
+      S += s_sum[w];
+      Q += s_sq[w];
+    }
+    const double m = S / (double)top_n;
+    mean[row] = (float)(thr + m);
+    stdev[row] = (float)sqrt(fmax(Q / (double)top_n - m * m, 0.0));
+    if (nth != nullptr) nth[row] = (float)thr;
+  }
+}
+
+// Cohort statistics of n vectors: the raw score GEMM against the cohort runs in row chunks of at most
+// kCohortChunkBytes into the workspace, each chunk is selected while it is still in L2.
+int cohort_stats_tc(const ktf_plda* p, const float* u, int64_t n, const float* uc, int64_t nc, long long top_n,
+                    bool enrolled, float* mean, float* stdev, float* nth, cudaStream_t st) {
+  const long long K = 3LL * p->dim;
+  const long long ld = (nc + 3) / 4 * 4;          // 16-byte row pitch: the GEMM's boxed stores
+  long long chunk = std::max(1LL, (long long)(kCohortChunkBytes / (double)(ld * (long long)sizeof(float))));
+  if (chunk >= 256) chunk = chunk / 256 * 256;    // whole pair tiles
+  chunk = std::min<long long>(chunk, n);
+  TcOperands o;
+  int rc = tc_operands(p, u, n, uc, nc, (size_t)chunk * ld * sizeof(float), st, &o, enrolled);
+  if (rc != KTF_OK) return rc;
+  float* raw = reinterpret_cast<float*>(o.extra);
+  const int in_smem = nc <= kSelSmemRowMax;
+  const size_t smem = (size_t)(kSelBins + (in_smem ? nc : 0)) * sizeof(unsigned);
+  static unsigned long long attr_done = 0;
+  if (ktf::first_use_on_device(&attr_done))
+    KTF_CUDA(cudaFuncSetAttribute(cohort_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)((kSelBins + kSelSmemRowMax) * sizeof(unsigned))));
+  for (long long r0 = 0; r0 < n; r0 += chunk) {
+    const long long rows = std::min(chunk, (long long)n - r0);
+    if ((rc = ktf::tc_gemm_nt(o.A + r0 * K, rows, K, o.B, nc, K, K, /*fp16=*/1, nullptr, nullptr, raw, ld, 0, st)) !=
+        KTF_OK)
+      return rc;
+    cohort_select_kernel<<<(unsigned)rows, kSelThreads, smem, st>>>(raw, ld, nc, o.Ai + r0, o.Bj, enrolled ? 1 : 0,
+                                                                     (unsigned)top_n, in_smem, mean + r0, stdev + r0,
+                                                                     nth ? nth + r0 : nullptr);
+    KTF_LAUNCH_OK();
+  }
+  return KTF_OK;
+}
+
+// Per-row (A_i, 0.5 / sigma_t, mu_t, 0) and per-column 0.5 / sigma_e of the normalising epilogue (IEEE divisions: a
+// sigma of 0 gives inf, and the score the IEEE quotient; 0.5 / sigma is exactly half of 1 / sigma).
+__global__ void asnorm_prep_kernel(const float* __restrict__ Ai, const float* __restrict__ t_mean,
+                                   const float* __restrict__ t_std, long long nt, const float* __restrict__ e_std,
+                                   long long ne, float4* __restrict__ row, float* __restrict__ e_half_inv) {
+  const long long items = nt > ne ? nt : ne;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < items; i += (long long)gridDim.x * blockDim.x) {
+    if (i < nt) row[i] = make_float4(Ai[i], 0.5f / t_std[i], t_mean[i], 0.0f);
+    if (i < ne) e_half_inv[i] = 0.5f / e_std[i];
+  }
+}
+
+int score_tc_asnorm(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, const float* t_mean,
+                    const float* t_std, const float* e_mean, const float* e_std, float* scores, int64_t ld,
+                    cudaStream_t st) {
+  const long long K = 3LL * p->dim;
+  const size_t row_bytes = ((size_t)nt * sizeof(float4) + 255) & ~(size_t)255;
+  TcOperands o;
+  int rc = tc_operands(p, ut, nt, ue, ne, row_bytes + (size_t)ne * sizeof(float), st, &o);
+  if (rc != KTF_OK) return rc;
+  float4* row = reinterpret_cast<float4*>(o.extra);
+  float* e_half_inv = reinterpret_cast<float*>(o.extra + row_bytes);
+  const long long items = std::max<long long>(nt, ne);
+  asnorm_prep_kernel<<<(unsigned)std::min<long long>((items + 255) / 256, (long long)ktf::num_sms() * 16), 256, 0, st>>>(
+      o.Ai, t_mean, t_std, nt, e_std, ne, row, e_half_inv);
+  KTF_LAUNCH_OK();
+  return ktf::tc_gemm_asnorm(o.A, nt, K, o.B, ne, K, K, /*fp16=*/1, reinterpret_cast<const float*>(row), o.Bj,
+                             e_half_inv, e_mean, scores, ld, st);
 }
 
 template <typename T>
@@ -469,6 +660,36 @@ int ktf_plda_score_topk(const ktf_plda* p, const void* u_test_dev, int64_t n_tes
                 "ktf_plda_score_topk: null argument");
   return score_tc_topk(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, k, scores_dev,
                        (long long*)index_dev, (cudaStream_t)stream);
+}
+
+int ktf_plda_cohort_stats(const ktf_plda* p, const void* u_dev, int64_t n, const void* u_cohort_dev, int64_t n_cohort,
+                          int64_t top_n, int32_t role, float* mean_dev, float* std_dev, float* nth_dev, void* stream) {
+  KTF_CHECK_ARG(p, "ktf_plda_cohort_stats: null handle");
+  KTF_CHECK_ARG(role == KTF_COHORT_AS_TEST || role == KTF_COHORT_AS_ENROLLED,
+                "ktf_plda_cohort_stats: role must be KTF_COHORT_AS_TEST or KTF_COHORT_AS_ENROLLED");
+  KTF_CHECK_ARG(p->use_tc, "ktf_plda_cohort_stats needs a float32 PLDA handle on an sm_100 device");
+  KTF_CHECK_ARG(top_n >= 2 && top_n <= n_cohort && n_cohort < (1LL << 32),
+                "ktf_plda_cohort_stats: top_n = %lld, n_cohort = %lld: needs 2 <= top_n <= n_cohort < 2^32",
+                (long long)top_n, (long long)n_cohort);
+  if (n <= 0) return KTF_OK;
+  KTF_CHECK_ARG(u_dev && u_cohort_dev && mean_dev && std_dev, "ktf_plda_cohort_stats: null argument");
+  return cohort_stats_tc(p, (const float*)u_dev, n, (const float*)u_cohort_dev, n_cohort, top_n,
+                         role == KTF_COHORT_AS_ENROLLED, mean_dev, std_dev, nth_dev, (cudaStream_t)stream);
+}
+
+int ktf_plda_score_asnorm(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,
+                          int64_t n_enroll, const float* test_mean_dev, const float* test_std_dev,
+                          const float* enroll_mean_dev, const float* enroll_std_dev, float* scores_dev, int64_t ld,
+                          void* stream) {
+  KTF_CHECK_ARG(p, "ktf_plda_score_asnorm: null handle");
+  KTF_CHECK_ARG(p->use_tc, "ktf_plda_score_asnorm needs a float32 PLDA handle on an sm_100 device");
+  KTF_CHECK_ARG(ld >= n_enroll, "ld must be >= n_enroll");
+  if (n_test <= 0 || n_enroll <= 0) return KTF_OK;
+  KTF_CHECK_ARG(u_test_dev && u_enroll_dev && test_mean_dev && test_std_dev && enroll_mean_dev && enroll_std_dev &&
+                    scores_dev,
+                "ktf_plda_score_asnorm: null argument");
+  return score_tc_asnorm(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, test_mean_dev,
+                         test_std_dev, enroll_mean_dev, enroll_std_dev, scores_dev, ld, (cudaStream_t)stream);
 }
 
 int ktf_topk_merge(const float* scores_in_dev, const int64_t* index_in_dev, int32_t num_lists, int64_t n_rows,

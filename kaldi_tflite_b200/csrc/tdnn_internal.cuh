@@ -29,6 +29,12 @@ int stats_sums_f32(const float* y_dev, const int64_t* offsets_dev, int64_t batch
 int tc_gemm_nt(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
                int fp16, const float* row_add, const float* col_add, void* C, long long ldc, int c_bf16,
                cudaStream_t st, unsigned long long* row_best = nullptr);
+// The same GEMM with the score normalised in the epilogue (PLDA AS-norm): with s = (acc + col_add[j]) + A_i,
+// C[i, j] = (s - col_mean[j]) * col_half_inv[j] + (s - mu_t) * h_t, where row_norm holds one float4 (A_i, h_t, mu_t,
+// unused) per row and the h are 0.5 / sigma.  C fp32.
+int tc_gemm_asnorm(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
+                   int fp16, const float* row_norm, const float* col_add, const float* col_half_inv,
+                   const float* col_mean, float* C, long long ldc, cudaStream_t st);
 // The same GEMM reduced to the k (1..32) largest entries of every row, nothing else stored: partial lists
 // (num_lists, m, k) of fp32 values and columns, unordered, (-inf, -1) where a list has fewer than k entries; every column
 // is in exactly one list.  num_lists = tc_topk_lists(m, n, K) (0 when m or n is 0).

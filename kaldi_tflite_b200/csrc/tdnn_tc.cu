@@ -56,6 +56,9 @@ constexpr int kSmemTc = kStages * kStageBytes + 1024 /*align*/ + 256 /*barriers*
 constexpr int kStgPitch = 64 + 16;                   // staged row pitch of the ragged store: 16 floats + 16 B (bank spread)
 
 enum { kModeBf16 = 0, kModeF32 = 1 };                // pair kernel: rows stored as bf16 / fp32
+// Pair kernel, fp32 rows in the AS-norm form of PLDA scoring (kEpiNorm): TcArgs::row_add then points to one float4 per
+// row (A_i, 0.5 / sigma_t, mu_t, unused), bias / scale / offset are the per-column B_j, 0.5 / sigma_e and mu_e.
+enum { kModeNorm = 2 };
 // Pair kernel, per-row top-k (nothing stored, see TcArgs::topk_k): lists of up to 8, 16 or 32 entries per thread.  The
 // capacity is part of the mode because it sets the shared-memory layout and with it the number of ring stages.
 enum { kModeTopk8 = 3, kModeTopk16 = 4, kModeTopk32 = 5 };
@@ -80,7 +83,7 @@ struct TcArgs {
   const float* bias;        // per column (STATS: per unit = per row)
   const float* scale;
   const float* offset;
-  const float* row_add;     // F32 mode: per-row addend or nullptr
+  const float* row_add;     // F32 mode: per-row addend or nullptr (Norm mode: float4 per row, see kModeNorm)
   int relu;
   void* out;                // bf16 or fp32, row-major
   long long out_ld;
@@ -251,7 +254,17 @@ __device__ __forceinline__ unsigned pack_bf16x2(float lo, float hi) {
 //      kEpiLean  y = max(acc + bias, lo) + row addend           (no per-column scale / offset)
 //      kEpiAdd   y = (acc + bias) + row addend                  (PLDA scoring: nothing to clamp)
 // all three round like the general form with scale 1 / offset 0 / lo = -FLT_MAX, so every path gives the same fp32 value.
-constexpr int kEpiFull = 0, kEpiLean = 1, kEpiAdd = 2;
+//      kEpiNorm  y = asnorm(...)                                (PLDA AS-norm, kModeNorm only)
+constexpr int kEpiFull = 0, kEpiLean = 1, kEpiAdd = 2, kEpiNorm = 3;
+
+// Adaptive symmetric normalisation of one PLDA score: s = (acc + B_j) + A_i exactly as kEpiAdd forms it, then
+// 0.5 ((s - mu_e) / sigma_e + (s - mu_t) / sigma_t) with the half reciprocals h = 0.5 / sigma precomputed:
+// (s - mu_e) h_e + (s - mu_t) h_t.  Differences first (not s h - mu h): a score near a mean keeps its relative
+// precision.  Explicit roundings (no free contraction), so the boxed and the ragged store paths give the same bits.
+__device__ __forceinline__ float asnorm(float acc, float bj, float h_e, float mu_e, float ai, float h_t, float mu_t) {
+  const float s = (acc + bj) + ai;
+  return __fmaf_rn(__fsub_rn(s, mu_e), h_e, __fmul_rn(__fsub_rn(s, mu_t), h_t));
+}
 
 // Key of (value, column) whose unsigned order is: larger value first, then SMALLER column.  0 never occurs for a real value.
 __device__ __forceinline__ unsigned long long top1_key(float v, int col) {
@@ -270,7 +283,8 @@ template <bool OUT_BF16, int EPI, int VSTRIDE, int HALF>
 __device__ __forceinline__ void store_box(const unsigned (&r)[32], const float* vb, float relu_lo, float radd,
                                           unsigned char* stg, int lane, int flags, bool plain,
                                           unsigned char* out_box, long long ld_bytes, const CUtensorMap* tmC, int tma_col,
-                                          int tma_row, bool& tma_pending, unsigned long long store_policy, int dbg) {
+                                          int tma_row, bool& tma_pending, unsigned long long store_policy, int dbg,
+                                          float rh = 0.0f, float rmu = 0.0f) {
   const float4* b4 = reinterpret_cast<const float4*>(vb);
   const float4* s4 = reinterpret_cast<const float4*>(vb + VSTRIDE);
   const float4* o4 = reinterpret_cast<const float4*>(vb + 2 * VSTRIDE);
@@ -290,6 +304,12 @@ __device__ __forceinline__ void store_box(const unsigned (&r)[32], const float* 
         x[4 * h + 1] = (a1 + bb.y) + radd;
         x[4 * h + 2] = (a2 + bb.z) + radd;
         x[4 * h + 3] = (a3 + bb.w) + radd;
+      } else if (EPI == kEpiNorm) {
+        const float4 ss = s4[2 * c8 + h], oo = o4[2 * c8 + h];
+        x[4 * h + 0] = asnorm(a0, bb.x, ss.x, oo.x, radd, rh, rmu);
+        x[4 * h + 1] = asnorm(a1, bb.y, ss.y, oo.y, radd, rh, rmu);
+        x[4 * h + 2] = asnorm(a2, bb.z, ss.z, oo.z, radd, rh, rmu);
+        x[4 * h + 3] = asnorm(a3, bb.w, ss.w, oo.w, radd, rh, rmu);
       } else if (EPI == kEpiLean) {
         x[4 * h + 0] = fmaxf(a0 + bb.x, relu_lo) + radd;
         x[4 * h + 1] = fmaxf(a1 + bb.y, relu_lo) + radd;
@@ -355,10 +375,11 @@ __device__ __forceinline__ void store_box(const unsigned (&r)[32], const float* 
 
 // Ragged / unaligned chunk of the pair kernel (right edge of the matrix, output pitch not a multiple of 16 bytes): fp32
 // staging, bounds-checked scalar stores with the per-row flags.  Same arithmetic (and association) as store_box.
-template <bool OUT_BF16, int VSTRIDE>
+template <bool OUT_BF16, int VSTRIDE, bool NORM = false>
 __device__ __forceinline__ void store_chunk_ragged(const unsigned (&r)[32], const float* vb, bool lean, float relu_lo,
                                                    float radd, unsigned char* stg, int lane, int flags, unsigned char* out0,
-                                                   long long ld_bytes, int cols_left) {
+                                                   long long ld_bytes, int cols_left, float rh = 0.0f,
+                                                   float rmu = 0.0f) {
   constexpr int kCols = 16;                              // columns per pass (kStgPitch = 80 bytes holds 16 floats + pad)
   constexpr int kEs = OUT_BF16 ? 2 : 4;
 #pragma unroll      // (compile-time indices into r[]: a rolled loop would push the accumulator registers to local memory)
@@ -367,6 +388,10 @@ __device__ __forceinline__ void store_chunk_ragged(const unsigned (&r)[32], cons
 #pragma unroll
     for (int i = 0; i < kCols; ++i) {
       const int c = pass * kCols + i;
+      if (NORM) {
+        mine[i] = asnorm(__uint_as_float(r[c]), vb[c], vb[VSTRIDE + c], vb[2 * VSTRIDE + c], radd, rh, rmu);
+        continue;
+      }
       const float b = vb[c], sc = lean ? 1.0f : vb[VSTRIDE + c], of = lean ? 0.0f : vb[2 * VSTRIDE + c];
       const float t = fmaxf(__uint_as_float(r[c]) + b, relu_lo);
       mine[i] = (lean ? t : fmaf(t, sc, of)) + radd;
@@ -732,6 +757,7 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   using Cfg = PairCfg<EW>;
   constexpr int kCap = topk_cap(MODE);
   constexpr bool kTopk = kCap > 0;
+  constexpr bool kNorm = MODE == kModeNorm;
   using TCfg = TopkCfg<EW, kTopk ? kCap : 8>;
   constexpr int kPairStages = kTopk ? TCfg::kStages : Cfg::kStages;
   constexpr int kPCols = Cfg::kCols, kPChunks = Cfg::kChunks;
@@ -933,13 +959,22 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       pre_nt = nt_;
     };
     int nx_flags = 0;
-    float nx_radd = 0.0f;
-    auto load_row_meta = [&](long long row_, int& f_, float& ra_) {
+    float nx_radd = 0.0f, nx_rh = 0.0f, nx_rmu = 0.0f;   // (rh / rmu: Norm mode's 0.5 / sigma_t and mu_t)
+    auto load_row_meta = [&](long long row_, int& f_, float& ra_, float& rh_, float& rmu_) {
       f_ = 0;
       ra_ = 0.0f;
+      rh_ = 0.0f;
+      rmu_ = 0.0f;
       if (row_ < m_rows) {
         f_ = a.rowmap ? a.rowmap[row_] : kRowStore;
-        if (a.row_add != nullptr) ra_ = a.row_add[row_];
+        if constexpr (kNorm) {
+          const float4 q = reinterpret_cast<const float4*>(a.row_add)[row_];
+          ra_ = q.x;
+          rh_ = q.y;
+          rmu_ = q.z;
+        } else if (a.row_add != nullptr) {
+          ra_ = a.row_add[row_];
+        }
       }
     };
     int it = 0;
@@ -976,8 +1011,8 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       // this tile's row flags / row addend were requested one tile ahead (a global load in front of every tile was 9 % of
       // the stall samples); request the next tile's now
       int flags = nx_flags;
-      float radd = nx_radd;
-      if (it == 0) load_row_meta(row, flags, radd);
+      float radd = nx_radd, rh = nx_rh, rmu = nx_rmu;
+      if (it == 0) load_row_meta(row, flags, radd, rh, rmu);
       {
         const long long next = tile + t_step;
         if (next < t_end) {
@@ -985,7 +1020,7 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           int nt2;
           coords(next, mt2, nt2);
           if (nt2 != nt && pre_nt != nt2) prefetch_vec(nt2);
-          load_row_meta(mt2 * BM2 + (long long)rank * BM + quarter * 32 + lane, nx_flags, nx_radd);
+          load_row_meta(mt2 * BM2 + (long long)rank * BM + quarter * 32 + lane, nx_flags, nx_radd, nx_rh, nx_rmu);
         }
       }
       mbar_wait(&tfull_bar[acc], acc_phase);
@@ -1086,8 +1121,10 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           const float* wvc = wv + c * 32;
 #define KTF_STORE_BOX(EPI_, HALF_)                                                                                      \
   store_box<kBf16, EPI_, kPCols, HALF_>(r[c % kRB], wvc, relu_lo, radd, stg2, lane, flags, plain, out_box, ld_bytes, tmc, \
-                                        box_col0, trow, tma_pending, store_policy, a.debug)
-          if ((c & 1) == 0) {
+                                        box_col0, trow, tma_pending, store_policy, a.debug, rh, rmu)
+          if constexpr (kNorm) {
+            KTF_STORE_BOX(kEpiNorm, 0);          // (fp32 rows: every chunk is a whole box)
+          } else if ((c & 1) == 0) {
             if (epi == kEpiFull) KTF_STORE_BOX(kEpiFull, 0);
             else if (epi == kEpiAdd) KTF_STORE_BOX(kEpiAdd, 0);
             else KTF_STORE_BOX(kEpiLean, 0);
@@ -1105,8 +1142,8 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           }
           // (the warp's staging boxes serve as the fp32 staging of the ragged path)
           unsigned char* out0 = owarp + (long long)col0 * kEs;
-          store_chunk_ragged<kBf16, kPCols>(r[c % kRB], wv + c * 32, lean, relu_lo, radd, stg2, lane, flags, out0, ld_bytes,
-                                            n_cols - col0);
+          store_chunk_ragged<kBf16, kPCols, kNorm>(r[c % kRB], wv + c * 32, lean, relu_lo, radd, stg2, lane, flags, out0,
+                                                   ld_bytes, n_cols - col0, rh, rmu);
         }
         if (kRB == 1 && c + 1 < kPChunks) tmem_ld32_issue(taddr0 + (unsigned)((c + 1) * 32), r[0]);
       }
@@ -1762,7 +1799,7 @@ int launch_gemm_pair_ew(const CUtensorMap& tmA, const CUtensorMap& tmB_half, con
   constexpr int kSmemPair = pair_smem<MODE, EW>();
   constexpr int kPairThreads = PairCfg<EW>::kThreads;
   TcArgs args = args_in;
-  if (args.row_add != nullptr && (args.scale != nullptr || args.offset != nullptr)) return KTF_EINVAL;
+  if (MODE != kModeNorm && args.row_add != nullptr && (args.scale != nullptr || args.offset != nullptr)) return KTF_EINVAL;
   CUtensorMap tmC = tmA;
   args.tma_store = 0;
   if (args.out != nullptr) {
@@ -2029,15 +2066,16 @@ int affine_tc_forward(const ktf_affine* a, const float* x_dev, const int64_t* in
 
 // C[i, j] = sum_k A[i, k] * B[j, k] + row_add[i] + col_add[j], A (m, K) and B (n, K) row-major 16-bit
 // (bf16 or fp16), C fp32 with row stride ldc.  K and both leading dimensions must be multiples of 8.
-int tc_gemm_nt(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
-               int fp16, const float* row_add, const float* col_add, void* C, long long ldc, int c_bf16,
-               cudaStream_t st, unsigned long long* row_best) {
+// Operand maps and arguments of a row-storing NT GEMM on the pair kernel (tc_gemm_nt, tc_gemm_asnorm).
+static int nt_setup(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
+                    int fp16, const float* row_add, const float* col_add, void* C, long long ldc, int c_bf16,
+                    CUtensorMap* tmA, CUtensorMap* tmBh, TcArgs* out) {
   int rc = check_arch();
   if (rc != KTF_OK) return rc;
-  CUtensorMap tmA, tmBh;   // B in 128-row boxes: each CTA of a pair loads half of the tile's 256 columns
-  if ((rc = encode_map(&tmA, A, (unsigned long long)K, (unsigned long long)m, (unsigned long long)lda, BK, BM)) != KTF_OK)
+  // B in 128-row boxes: each CTA of a pair loads half of the tile's 256 columns
+  if ((rc = encode_map(tmA, A, (unsigned long long)K, (unsigned long long)m, (unsigned long long)lda, BK, BM)) != KTF_OK)
     return rc;
-  if ((rc = encode_map(&tmBh, B, (unsigned long long)K, (unsigned long long)n, (unsigned long long)ldb, BK, BN / 2)) != KTF_OK)
+  if ((rc = encode_map(tmBh, B, (unsigned long long)K, (unsigned long long)n, (unsigned long long)ldb, BK, BN / 2)) != KTF_OK)
     return rc;
   TcArgs args{};
   args.num_taps = 1;
@@ -2049,13 +2087,36 @@ int tc_gemm_nt(const void* A, long long m, long long lda, const void* B, long lo
   args.row_add = row_add;
   args.out = C;
   args.out_ld = ldc;
-  args.row_best = row_best;
   // streaming output (PLDA: the score matrix), operands re-read by every tile: see TcArgs::l2_stream_out
   args.l2_stream_out = ((double)m * (double)n * (c_bf16 ? 2.0 : 4.0) > 64e6) ? 1 : 0;
   if (const char* e = getenv("KTF_TC_L2_HINTS")) args.l2_stream_out = atoi(e);
   args.group_m = (n + BN - 1) / BN > 8 ? 32 : 0;     // (measured at 50 000^2: 1 -> 2.77, 8 -> 2.61, 16 -> 2.54, 32 -> 2.47-2.51, 64 -> 2.65 ms)
   if (const char* e = getenv("KTF_TC_GROUP_M")) args.group_m = atoi(e);
+  *out = args;
+  return KTF_OK;
+}
+
+int tc_gemm_nt(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
+               int fp16, const float* row_add, const float* col_add, void* C, long long ldc, int c_bf16,
+               cudaStream_t st, unsigned long long* row_best) {
+  CUtensorMap tmA, tmBh;
+  TcArgs args;
+  int rc = nt_setup(A, m, lda, B, n, ldb, K, fp16, row_add, col_add, C, ldc, c_bf16, &tmA, &tmBh, &args);
+  if (rc != KTF_OK) return rc;
+  args.row_best = row_best;
   return c_bf16 ? launch_gemm_pair<kModeBf16>(tmA, tmBh, args, st) : launch_gemm_pair<kModeF32>(tmA, tmBh, args, st);
+}
+
+int tc_gemm_asnorm(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
+                   int fp16, const float* row_norm, const float* col_add, const float* col_half_inv,
+                   const float* col_mean, float* C, long long ldc, cudaStream_t st) {
+  CUtensorMap tmA, tmBh;
+  TcArgs args;
+  int rc = nt_setup(A, m, lda, B, n, ldb, K, fp16, row_norm, col_add, C, ldc, 0, &tmA, &tmBh, &args);
+  if (rc != KTF_OK) return rc;
+  args.scale = col_half_inv;
+  args.offset = col_mean;
+  return launch_gemm_pair<kModeNorm>(tmA, tmBh, args, st);
 }
 
 }  // namespace ktf

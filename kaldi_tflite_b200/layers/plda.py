@@ -160,6 +160,58 @@ class PLDA(Layer):
                                             T.ptr(scores), T.ptr(index), T.stream_ptr()))
         return scores, index
 
+    def cohortStats(self, u, u_cohort, *, top_n, role="test", num_examples=1.0):
+        """AS-norm statistics of every vector of `u` against an imposter cohort: (mean (n,), std (n,)) float32, the
+        mean and population std (ddof 0) of its `top_n` largest cohort scores.  role="test": the scores are row i of
+        `logLikelihoodRatio(u, u_cohort)` (num_examples 1); role="enrolled": column i of
+        `logLikelihoodRatio(u_cohort, u, num_examples=num_examples)`.  The selection is exact (bit-equal scores) and
+        the statistics are evaluated in float64 and rounded once; a vector's statistics do not depend on the other
+        vectors of the call.  2 <= top_n <= len(u_cohort); float32 layers only."""
+        if self.paramDtype != np.float32:
+            raise ValueError("cohortStats needs a float32 PLDA layer")
+        if role not in ("test", "enrolled"):
+            raise ValueError(f"role must be 'test' or 'enrolled', got {role!r}")
+        n = u.shape[0]
+        mean = torch.empty((n,), device=u.device, dtype=torch.float32)
+        std = torch.empty((n,), device=u.device, dtype=torch.float32)
+        h = self.handle_for(1.0) if role == "test" else self.handle_for(num_examples)
+        N.check(N.lib().ktf_plda_cohort_stats(h, T.ptr(u), n, T.ptr(u_cohort), u_cohort.shape[0], int(top_n),
+                                              N.KTF_COHORT_AS_TEST if role == "test" else N.KTF_COHORT_AS_ENROLLED,
+                                              T.ptr(mean), T.ptr(std), None, T.stream_ptr()))
+        return mean, std
+
+    def asNorm(self, u_test, u_enroll=None, u_cohort=None, *, top_n=None, test_stats=None, enroll_stats=None,
+               num_examples=1.0, out=None):
+        """Adaptive symmetric normalisation (AS-norm1) of the `logLikelihoodRatio` matrix:
+        s'[i, j] = 0.5 ((s[i, j] - mu_e[j]) / sigma_e[j] + (s[i, j] - mu_t[i]) / sigma_t[i]), float32 (n_test, n_enroll),
+        normalised in the score kernel (the raw matrix is never written).  `test_stats` / `enroll_stats` are
+        (mean, std) pairs from `cohortStats`; whichever is not given is computed from `u_cohort` and `top_n`
+        (test role for u_test, enrolled role with `num_examples` for u_enroll).  `u_enroll=None` scores the set against
+        itself.  float32 layers only."""
+        if self.paramDtype != np.float32:
+            raise ValueError("asNorm needs a float32 PLDA layer")
+        u_enroll = u_test if u_enroll is None else u_enroll
+        nt, ne = u_test.shape[0], u_enroll.shape[0]
+        if (test_stats is None or enroll_stats is None) and (u_cohort is None or top_n is None):
+            raise ValueError("asNorm needs u_cohort and top_n for the statistics it is not given")
+        if test_stats is None:
+            test_stats = self.cohortStats(u_test, u_cohort, top_n=top_n, role="test")
+        if enroll_stats is None:
+            enroll_stats = self.cohortStats(u_enroll, u_cohort, top_n=top_n, role="enrolled", num_examples=num_examples)
+        stats = []
+        for (m, s), n, side in ((test_stats, nt, "test"), (enroll_stats, ne, "enroll")):
+            for t in (m, s):
+                if t.dtype != torch.float32 or t.shape != (n,) or not t.is_contiguous():
+                    raise ValueError(f"{side}_stats must be two contiguous float32 tensors of shape ({n},)")
+                stats.append(t)
+        if out is None:
+            out = torch.empty((nt, ne), device=u_test.device, dtype=torch.float32)
+        elif out.dtype != torch.float32 or tuple(out.shape) != (nt, ne) or out.stride(1) != 1:
+            raise ValueError(f"out must be a float32 ({nt}, {ne}) tensor with unit column stride")
+        N.check(N.lib().ktf_plda_score_asnorm(self.handle_for(num_examples), T.ptr(u_test), nt, T.ptr(u_enroll), ne,
+                                              *(T.ptr(t) for t in stats), T.ptr(out), out.stride(0), T.stream_ptr()))
+        return out
+
     def call(self, inputs):
         x = T.as_device(inputs)
         self._maybe_build(x.shape)

@@ -192,6 +192,36 @@ def plda_best_matches_sharded(plda, x_test_local, x_enroll_local, k, test_counts
     return out_s, out_i
 
 
+def plda_asnorm_sharded(plda, x_test_local, x_enroll_local, u_cohort, top_n, test_counts=None):
+    """
+    Sharded AS-norm trial scoring on the layout of `plda_score_sharded`: each rank holds a slice of the test and of the
+    enrolled x-vectors (raw, (n, dim) float32) and the whole transformed cohort `u_cohort`.  Every rank computes the
+    cohort statistics of its own test rows and of its own enrolled shard; the test statistics travel with the test
+    vectors in the one all-gather (two extra columns), so no rank recomputes another's.  Returns this rank's block
+    `PLDA.asNorm`[all tests, local enrolled] -- test rows ordered by rank, row pitch padded to 16 bytes -- plus the
+    gathered transformed test vectors.
+    """
+    rank, w = world()
+    u_test_local = plda.transformVector(x_test_local.contiguous())
+    t_mean, t_std = plda.cohortStats(u_test_local, u_cohort, top_n=top_n, role="test")
+    u_enroll_local = plda.transformVector(x_enroll_local.contiguous())
+    e_stats = plda.cohortStats(u_enroll_local, u_cohort, top_n=top_n, role="enrolled")
+    ne = u_enroll_local.shape[0]
+    if w == 1:
+        return plda.asNorm(u_test_local, u_enroll_local, test_stats=(t_mean, t_std), enroll_stats=e_stats), u_test_local
+    dim = u_test_local.shape[1]
+    packed = torch.cat([u_test_local, t_mean[:, None], t_std[:, None]], dim=1)
+    p_all, offs, works = exchange_test_vectors(packed, test_counts)
+    for wk in works:
+        if wk is not None:
+            wk.wait()
+    u_all = p_all[:, :dim].contiguous()
+    t_stats = (p_all[:, dim].contiguous(), p_all[:, dim + 1].contiguous())
+    # row pitch padded to 16 bytes: the score kernel's boxed (TMA) stores need an aligned pitch
+    out = torch.empty((offs[-1], (ne + 7) // 8 * 8), device=u_all.device, dtype=torch.float32)[:, :ne]
+    return plda.asNorm(u_all, u_enroll_local, test_stats=t_stats, enroll_stats=e_stats, out=out), u_all
+
+
 def stream_batches(fn, host_in, chunk, host_out=None, depth=3):
     """
     Runs `fn` (any layer / model call taking a CUDA tensor of utterances and returning a CUDA tensor with
