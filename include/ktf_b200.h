@@ -442,6 +442,24 @@ int ktf_plda_score_asnorm(const ktf_plda* p, const void* u_test_dev, int64_t n_t
                           int64_t n_enroll, const float* test_mean_dev, const float* test_std_dev,
                           const float* enroll_mean_dev, const float* enroll_std_dev, float* scores_dev, int64_t ld,
                           void* stream);
+/* ktf_plda_score_asnorm with a choice of output format: score_format KTF_SCORES_NATIVE is ktf_plda_score_asnorm
+ * (scores_dev float32); KTF_SCORES_BF16 writes the same float32 value rounded once to bfloat16 (scores_dev (n_test, ld)
+ * bfloat16: half the bytes of the matrix).  Any other format is KTF_EINVAL. */
+int ktf_plda_score_asnorm_ex(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,
+                             int64_t n_enroll, const float* test_mean_dev, const float* test_std_dev,
+                             const float* enroll_mean_dev, const float* enroll_std_dev, void* scores_dev, int64_t ld,
+                             int32_t score_format, void* stream);
+/* k best trials per test vector by normalised score: scores_dev / index_dev (n_test, k), row i = the first k entries of
+ * a stable descending sort of row i of the ktf_plda_score_asnorm matrix (the same values, bit for bit) and their
+ * enrolled columns, with NaN and -inf entries left out and the row padded with (-inf, -1).  A deviation of 0 can give
+ * all three of +inf, -inf and NaN: +inf entries are listed, the others never.  The matrix is never written.
+ * 1 <= k <= KTF_PLDA_TOPK_MAX, a float32 handle and n_enroll < 2^32, else KTF_EINVAL; n_enroll == 0 gives (-inf, -1)
+ * everywhere (the enrolled pointers may then be null).  No host synchronisation; the workspace rules of
+ * ktf_plda_score_topk apply. */
+int ktf_plda_score_asnorm_topk(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,
+                               int64_t n_enroll, const float* test_mean_dev, const float* test_std_dev,
+                               const float* enroll_mean_dev, const float* enroll_std_dev, int32_t k, float* scores_dev,
+                               int64_t* index_dev, void* stream);
 
 #ifdef __cplusplus
 }

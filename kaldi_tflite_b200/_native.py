@@ -112,6 +112,8 @@ _SIGNATURES = {
     "ktf_topk_merge": (c_int32, [_P, _P, c_int32, c_int64, c_int32, c_int32, _P, _P, _P]),
     "ktf_plda_cohort_stats": (c_int32, [_P, _P, c_int64, _P, c_int64, c_int64, c_int32, _P, _P, _P, _P]),
     "ktf_plda_score_asnorm": (c_int32, [_P, _P, c_int64, _P, c_int64, _P, _P, _P, _P, _P, c_int64, _P]),
+    "ktf_plda_score_asnorm_ex": (c_int32, [_P, _P, c_int64, _P, c_int64, _P, _P, _P, _P, _P, c_int64, c_int32, _P]),
+    "ktf_plda_score_asnorm_topk": (c_int32, [_P, _P, c_int64, _P, c_int64, _P, _P, _P, _P, c_int32, _P, _P, _P]),
 }
 
 _lib = None

@@ -291,25 +291,6 @@ int score_tc(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, in
   return KTF_OK;
 }
 
-// The k best enrolled columns of every test row: the score GEMM leaves partial lists (one per n-range and column quarter
-// of a row) in the workspace, topk_merge reduces them to (nt, k).
-int score_tc_topk(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, int k, float* score,
-                  long long* index, cudaStream_t st) {
-  const long long K = 3LL * p->dim;
-  const int lists = ktf::tc_topk_lists(nt, ne, K);
-  if (lists == 0) return topk_merge(nullptr, nullptr, 0, nt, k, k, score, index, st);   // no enrolled vector
-  const size_t n_part = (size_t)lists * nt * k;
-  const size_t s_bytes = (n_part * sizeof(float) + 255) & ~(size_t)255;
-  TcOperands o;
-  int rc = tc_operands(p, ut, nt, ue, ne, s_bytes + n_part * sizeof(long long), st, &o);
-  if (rc != KTF_OK) return rc;
-  float* part_s = reinterpret_cast<float*>(o.extra);
-  long long* part_i = reinterpret_cast<long long*>(o.extra + s_bytes);
-  if ((rc = ktf::tc_gemm_topk(o.A, nt, K, o.B, ne, K, K, /*fp16=*/1, o.Ai, o.Bj, k, part_s, part_i, st)) != KTF_OK)
-    return rc;
-  return topk_merge(part_s, part_i, lists, nt, k, k, score, index, st);
-}
-
 // ---- AS-norm: per-vector statistics of the top-N cohort scores, normalised score matrix ----
 constexpr int kSelThreads = 512;
 constexpr int kSelBins = 4096;                    // histogram bins of the first radix pass (12 bits); the others use 10
@@ -472,22 +453,80 @@ __global__ void asnorm_prep_kernel(const float* __restrict__ Ai, const float* __
   }
 }
 
-int score_tc_asnorm(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, const float* t_mean,
-                    const float* t_std, const float* e_mean, const float* e_std, float* scores, int64_t ld,
-                    cudaStream_t st) {
-  const long long K = 3LL * p->dim;
-  const size_t row_bytes = ((size_t)nt * sizeof(float4) + 255) & ~(size_t)255;
+// Statistics of the normalising epilogue: the caller's per-vector mean and std of both sides (device, float32).
+struct AsnormStats {
+  const float* t_mean;
+  const float* t_std;
+  const float* e_mean;
+  const float* e_std;
+};
+
+// Operands of the normalising score GEMM: those of tc_operands, then the per-row float4 and the per-column 0.5 / sigma_e
+// of asnorm_prep_kernel, then `extra` bytes of the caller's.
+struct AsnormOperands {
   TcOperands o;
-  int rc = tc_operands(p, ut, nt, ue, ne, row_bytes + (size_t)ne * sizeof(float), st, &o);
+  const float* row;          // (nt) float4
+  const float* e_half_inv;   // (ne)
+  char* extra;
+};
+
+int asnorm_operands(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, const AsnormStats& s,
+                    size_t extra, cudaStream_t st, AsnormOperands* a) {
+  const size_t row_bytes = ((size_t)nt * sizeof(float4) + 255) & ~(size_t)255;
+  const size_t col_bytes = ((size_t)ne * sizeof(float) + 255) & ~(size_t)255;
+  TcOperands o;
+  int rc = tc_operands(p, ut, nt, ue, ne, row_bytes + col_bytes + extra, st, &o);
   if (rc != KTF_OK) return rc;
   float4* row = reinterpret_cast<float4*>(o.extra);
   float* e_half_inv = reinterpret_cast<float*>(o.extra + row_bytes);
   const long long items = std::max<long long>(nt, ne);
   asnorm_prep_kernel<<<(unsigned)std::min<long long>((items + 255) / 256, (long long)ktf::num_sms() * 16), 256, 0, st>>>(
-      o.Ai, t_mean, t_std, nt, e_std, ne, row, e_half_inv);
+      o.Ai, s.t_mean, s.t_std, nt, s.e_std, ne, row, e_half_inv);
   KTF_LAUNCH_OK();
-  return ktf::tc_gemm_asnorm(o.A, nt, K, o.B, ne, K, K, /*fp16=*/1, reinterpret_cast<const float*>(row), o.Bj,
-                             e_half_inv, e_mean, scores, ld, st);
+  *a = AsnormOperands{o, reinterpret_cast<const float*>(row), e_half_inv, o.extra + row_bytes + col_bytes};
+  return KTF_OK;
+}
+
+int score_tc_asnorm(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, const AsnormStats& s,
+                    void* scores, int64_t ld, int scores_bf16, cudaStream_t st) {
+  const long long K = 3LL * p->dim;
+  AsnormOperands a;
+  int rc = asnorm_operands(p, ut, nt, ue, ne, s, 0, st, &a);
+  if (rc != KTF_OK) return rc;
+  return ktf::tc_gemm_asnorm(a.o.A, nt, K, a.o.B, ne, K, K, /*fp16=*/1, a.row, a.o.Bj, a.e_half_inv, s.e_mean, scores, ld,
+                             scores_bf16, st);
+}
+
+// The k best enrolled columns of every test row, of the raw scores or (norm != nullptr) of the AS-norm scores: the score
+// GEMM leaves partial lists (one per n-range and column quarter of a row) in the workspace, topk_merge reduces them to
+// (nt, k).
+int score_tc_topk(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, int k, float* score,
+                  long long* index, cudaStream_t st, const AsnormStats* norm = nullptr) {
+  const long long K = 3LL * p->dim;
+  const int lists = ktf::tc_topk_lists(nt, ne, K);
+  if (lists == 0) return topk_merge(nullptr, nullptr, 0, nt, k, k, score, index, st);   // no enrolled vector
+  const size_t n_part = (size_t)lists * nt * k;
+  const size_t s_bytes = (n_part * sizeof(float) + 255) & ~(size_t)255;
+  const size_t part_bytes = s_bytes + n_part * sizeof(long long);
+  int rc;
+  char* parts;
+  AsnormOperands a;
+  if (norm == nullptr) {
+    rc = tc_operands(p, ut, nt, ue, ne, part_bytes, st, &a.o);
+    parts = a.o.extra;
+  } else {
+    rc = asnorm_operands(p, ut, nt, ue, ne, *norm, part_bytes, st, &a);
+    parts = a.extra;
+  }
+  if (rc != KTF_OK) return rc;
+  float* part_s = reinterpret_cast<float*>(parts);
+  long long* part_i = reinterpret_cast<long long*>(parts + s_bytes);
+  const TcOperands& o = a.o;
+  rc = norm == nullptr ? ktf::tc_gemm_topk(o.A, nt, K, o.B, ne, K, K, /*fp16=*/1, o.Ai, o.Bj, k, part_s, part_i, st)
+                       : ktf::tc_gemm_asnorm_topk(o.A, nt, K, o.B, ne, K, K, /*fp16=*/1, a.row, o.Bj, a.e_half_inv,
+                                                  norm->e_mean, k, part_s, part_i, st);
+  if (rc != KTF_OK) return rc;
+  return topk_merge(part_s, part_i, lists, nt, k, k, score, index, st);
 }
 
 template <typename T>
@@ -681,6 +720,16 @@ int ktf_plda_score_asnorm(const ktf_plda* p, const void* u_test_dev, int64_t n_t
                           int64_t n_enroll, const float* test_mean_dev, const float* test_std_dev,
                           const float* enroll_mean_dev, const float* enroll_std_dev, float* scores_dev, int64_t ld,
                           void* stream) {
+  return ktf_plda_score_asnorm_ex(p, u_test_dev, n_test, u_enroll_dev, n_enroll, test_mean_dev, test_std_dev,
+                                  enroll_mean_dev, enroll_std_dev, scores_dev, ld, KTF_SCORES_NATIVE, stream);
+}
+
+int ktf_plda_score_asnorm_ex(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,
+                             int64_t n_enroll, const float* test_mean_dev, const float* test_std_dev,
+                             const float* enroll_mean_dev, const float* enroll_std_dev, void* scores_dev, int64_t ld,
+                             int32_t score_format, void* stream) {
+  KTF_CHECK_ARG(score_format == KTF_SCORES_NATIVE || score_format == KTF_SCORES_BF16,
+                "ktf_plda_score_asnorm: bad score_format %d", score_format);
   KTF_CHECK_ARG(p, "ktf_plda_score_asnorm: null handle");
   KTF_CHECK_ARG(p->use_tc, "ktf_plda_score_asnorm needs a float32 PLDA handle on an sm_100 device");
   KTF_CHECK_ARG(ld >= n_enroll, "ld must be >= n_enroll");
@@ -688,8 +737,27 @@ int ktf_plda_score_asnorm(const ktf_plda* p, const void* u_test_dev, int64_t n_t
   KTF_CHECK_ARG(u_test_dev && u_enroll_dev && test_mean_dev && test_std_dev && enroll_mean_dev && enroll_std_dev &&
                     scores_dev,
                 "ktf_plda_score_asnorm: null argument");
-  return score_tc_asnorm(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, test_mean_dev,
-                         test_std_dev, enroll_mean_dev, enroll_std_dev, scores_dev, ld, (cudaStream_t)stream);
+  return score_tc_asnorm(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll,
+                         AsnormStats{test_mean_dev, test_std_dev, enroll_mean_dev, enroll_std_dev}, scores_dev, ld,
+                         score_format == KTF_SCORES_BF16 ? 1 : 0, (cudaStream_t)stream);
+}
+
+int ktf_plda_score_asnorm_topk(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,
+                               int64_t n_enroll, const float* test_mean_dev, const float* test_std_dev,
+                               const float* enroll_mean_dev, const float* enroll_std_dev, int32_t k, float* scores_dev,
+                               int64_t* index_dev, void* stream) {
+  KTF_CHECK_ARG(k >= 1 && k <= KTF_PLDA_TOPK_MAX,
+                "ktf_plda_score_asnorm_topk: k = %d, must be 1 .. %d (KTF_PLDA_TOPK_MAX)", k, KTF_PLDA_TOPK_MAX);
+  KTF_CHECK_ARG(p, "ktf_plda_score_asnorm_topk: null handle");
+  KTF_CHECK_ARG(p->use_tc, "ktf_plda_score_asnorm_topk needs a float32 PLDA handle on an sm_100 device");
+  KTF_CHECK_ARG(n_enroll >= 0 && n_enroll < (1LL << 32), "ktf_plda_score_asnorm_topk: n_enroll must be in 0 .. 2^32 - 1");
+  if (n_test <= 0) return KTF_OK;
+  KTF_CHECK_ARG(u_test_dev && test_mean_dev && test_std_dev && scores_dev && index_dev &&
+                    (n_enroll == 0 || (u_enroll_dev && enroll_mean_dev && enroll_std_dev)),
+                "ktf_plda_score_asnorm_topk: null argument");
+  const AsnormStats s{test_mean_dev, test_std_dev, enroll_mean_dev, enroll_std_dev};
+  return score_tc_topk(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, k, scores_dev,
+                       (long long*)index_dev, (cudaStream_t)stream, &s);
 }
 
 int ktf_topk_merge(const float* scores_in_dev, const int64_t* index_in_dev, int32_t num_lists, int64_t n_rows,

@@ -31,10 +31,10 @@ int tc_gemm_nt(const void* A, long long m, long long lda, const void* B, long lo
                cudaStream_t st, unsigned long long* row_best = nullptr);
 // The same GEMM with the score normalised in the epilogue (PLDA AS-norm): with s = (acc + col_add[j]) + A_i,
 // C[i, j] = (s - col_mean[j]) * col_half_inv[j] + (s - mu_t) * h_t, where row_norm holds one float4 (A_i, h_t, mu_t,
-// unused) per row and the h are 0.5 / sigma.  C fp32.
+// unused) per row and the h are 0.5 / sigma.  C fp32, or (c_bf16 != 0) the fp32 value rounded once to bf16.
 int tc_gemm_asnorm(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
                    int fp16, const float* row_norm, const float* col_add, const float* col_half_inv,
-                   const float* col_mean, float* C, long long ldc, cudaStream_t st);
+                   const float* col_mean, void* C, long long ldc, int c_bf16, cudaStream_t st);
 // The same GEMM reduced to the k (1..32) largest entries of every row, nothing else stored: partial lists
 // (num_lists, m, k) of fp32 values and columns, unordered, (-inf, -1) where a list has fewer than k entries; every column
 // is in exactly one list.  num_lists = tc_topk_lists(m, n, K) (0 when m or n is 0).
@@ -42,4 +42,9 @@ int tc_topk_lists(long long m, long long n, long long K);
 int tc_gemm_topk(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
                  int fp16, const float* row_add, const float* col_add, int k, float* part_score, long long* part_index,
                  cudaStream_t st);
+// tc_gemm_topk over the normalised value of tc_gemm_asnorm (same partial lists, same num_lists): every listed value is
+// bit-equal to its tc_gemm_asnorm entry; NaN and -inf values are never listed.
+int tc_gemm_asnorm_topk(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
+                        int fp16, const float* row_norm, const float* col_add, const float* col_half_inv,
+                        const float* col_mean, int k, float* part_score, long long* part_index, cudaStream_t st);
 }  // namespace ktf

@@ -62,7 +62,23 @@ enum { kModeNorm = 2 };
 // Pair kernel, per-row top-k (nothing stored, see TcArgs::topk_k): lists of up to 8, 16 or 32 entries per thread.  The
 // capacity is part of the mode because it sets the shared-memory layout and with it the number of ring stages.
 enum { kModeTopk8 = 3, kModeTopk16 = 4, kModeTopk32 = 5 };
-constexpr int topk_cap(int mode) { return mode >= kModeTopk8 ? 8 << (mode - kModeTopk8) : 0; }
+// Pair kernel, the top-k walk of kModeTopk* over the AS-norm value of kModeNorm (row float4 and the three per-column
+// vectors as there): every listed value is bit-equal to its kModeNorm matrix entry.
+enum { kModeNormTopk8 = 6, kModeNormTopk16 = 7, kModeNormTopk32 = 8 };
+// Pair kernel, the AS-norm rows of kModeNorm rounded once to bf16 and stored as kModeBf16 stores its rows.
+enum { kModeNormBf16 = 9 };
+constexpr int kNumModes = 10;
+//                                   Bf16 F32 Norm Tk8 Tk16 Tk32 NTk8 NTk16 NTk32 NBf16
+constexpr int kModeTopkCap[kNumModes] = {0, 0, 0, 8, 16, 32, 8, 16, 32, 0};   // top-k list capacity, 0 = rows stored
+constexpr bool kModeIsNorm[kNumModes] = {0, 0, 1, 0, 0, 0, 1, 1, 1, 1};      // AS-norm value (kEpiNorm)
+constexpr bool kModeIsBf16[kNumModes] = {1, 0, 0, 0, 0, 0, 0, 0, 0, 1};      // rows stored as bf16
+// TcArgs::row_best is tested at run time (only tc_gemm_nt's fp32 form passes it).  The AS-norm modes after kModeTopk32
+// compile the test out: in kModeNormBf16 at 16 epilogue warps the dead path costs 8 bytes of spills.
+constexpr bool kModeRowBest[kNumModes] = {1, 1, 1, 1, 1, 1, 0, 0, 0, 0};
+constexpr int topk_cap(int mode) { return kModeTopkCap[mode]; }
+constexpr bool mode_norm(int mode) { return kModeIsNorm[mode]; }
+constexpr bool mode_bf16(int mode) { return kModeIsBf16[mode]; }
+constexpr bool mode_row_best(int mode) { return kModeRowBest[mode]; }
 
 // rowmap flags
 constexpr int kRowStore = 1, kRowFirst = 2, kRowLast = 4;
@@ -254,7 +270,7 @@ __device__ __forceinline__ unsigned pack_bf16x2(float lo, float hi) {
 //      kEpiLean  y = max(acc + bias, lo) + row addend           (no per-column scale / offset)
 //      kEpiAdd   y = (acc + bias) + row addend                  (PLDA scoring: nothing to clamp)
 // all three round like the general form with scale 1 / offset 0 / lo = -FLT_MAX, so every path gives the same fp32 value.
-//      kEpiNorm  y = asnorm(...)                                (PLDA AS-norm, kModeNorm only)
+//      kEpiNorm  y = asnorm(...)                                (PLDA AS-norm, mode_norm() modes only)
 constexpr int kEpiFull = 0, kEpiLean = 1, kEpiAdd = 2, kEpiNorm = 3;
 
 // Adaptive symmetric normalisation of one PLDA score: s = (acc + B_j) + A_i exactly as kEpiAdd forms it, then
@@ -685,23 +701,32 @@ template <int EW> struct PairCfg {
   static constexpr int kSmem = kStages * kPairStageBytes + 1024 + 256 + kVecBytes + kStgBytes;
 };
 static_assert(PairCfg<8>::kSmem <= 226 * 1024 && PairCfg<16>::kSmem <= 226 * 1024, "pair kernel shared memory");
-// Top-k modes store nothing: no staging boxes, only the bias of the per-warp vectors.  What they hold instead: per thread
-// a list of CAP 64-bit keys (interleaved by thread, so any per-lane entry index is bank-conflict free) and per warp a
-// 16 x 32 float scratch through which a lane walks its candidates of half a chunk.  The ring gets what is left, at most
-// the 5 stages of the storing modes.  EW = 8: CAP 8 / 16 / 32 -> 16 / 32 / 64 KB of lists, 5 / 5 / 4 stages;
-// EW = 16: 32 / 64 / 128 KB, 4 / 3 / 1 stages.
-template <int EW, int CAP> struct TopkCfg {
+// Top-k modes store nothing: no staging boxes, only the bias of the per-warp vectors (NV = 1; the AS-norm top-k modes
+// keep all three, NV = 3).  What they hold instead: per thread a list of CAP 64-bit keys (interleaved by thread, so any
+// per-lane entry index is bank-conflict free) and per warp a 16 x 32 float scratch through which a lane walks its
+// candidates of half a chunk.  The ring gets what is left, at most the 5 stages of the storing modes.  EW = 8: CAP 8 /
+// 16 / 32 -> 16 / 32 / 64 KB of lists, 5 / 5 / 4 stages; EW = 16: 32 / 64 / 128 KB, 4 / 3 / 1 stages -- with one vector
+// or three (the 8 KB more of NV = 3 fit in what the stage count leaves over).
+template <int EW, int CAP, int NV> struct TopkCfg {
   static constexpr int kCols = BN / (EW / 4);
-  static constexpr int kVecBytes = EW * kCols * 4;
+  static constexpr int kVecBytes = EW * NV * kCols * 4;
   static constexpr int kScratchBytes = EW * 16 * 32 * 4;
   static constexpr int kListBytes = EW * 32 * CAP * 8;
   static constexpr int kFixed = 1024 + 256 + kVecBytes + kScratchBytes + kListBytes;
   static constexpr int kStages = std::min(5, (226 * 1024 - kFixed) / kPairStageBytes);
   static constexpr int kSmem = kStages * kPairStageBytes + kFixed;
 };
-static_assert(TopkCfg<8, 32>::kStages == 4 && TopkCfg<16, 32>::kStages >= 1, "top-k pair kernel shared memory");
+static_assert(TopkCfg<8, 32, 1>::kStages == 4 && TopkCfg<16, 32, 1>::kStages >= 1, "top-k pair kernel shared memory");
+static_assert(TopkCfg<8, 8, 3>::kStages == 5 && TopkCfg<8, 16, 3>::kStages == 5 && TopkCfg<8, 32, 3>::kStages == 4 &&
+                  TopkCfg<16, 8, 3>::kStages == 4 && TopkCfg<16, 16, 3>::kStages == 3 &&
+                  TopkCfg<16, 32, 3>::kStages == 1,
+              "AS-norm top-k: the ring stages of the raw top-k modes");
+// per-column vectors a top-k mode keeps: the bias, or (AS-norm) bias, scale and offset
+constexpr int topk_vecs(int mode) { return mode_norm(mode) ? 3 : 1; }
 template <int MODE, int EW>
-constexpr int pair_smem() { return topk_cap(MODE) ? TopkCfg<EW, topk_cap(MODE) ? topk_cap(MODE) : 8>::kSmem : PairCfg<EW>::kSmem; }
+constexpr int pair_smem() {
+  return topk_cap(MODE) ? TopkCfg<EW, topk_cap(MODE) ? topk_cap(MODE) : 8, topk_vecs(MODE)>::kSmem : PairCfg<EW>::kSmem;
+}
 
 __device__ __forceinline__ unsigned cluster_ctarank() {
   unsigned r;
@@ -757,8 +782,9 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   using Cfg = PairCfg<EW>;
   constexpr int kCap = topk_cap(MODE);
   constexpr bool kTopk = kCap > 0;
-  constexpr bool kNorm = MODE == kModeNorm;
-  using TCfg = TopkCfg<EW, kTopk ? kCap : 8>;
+  constexpr bool kNorm = mode_norm(MODE);
+  constexpr int kTopkVecs = topk_vecs(MODE);
+  using TCfg = TopkCfg<EW, kTopk ? kCap : 8, kTopkVecs>;
   constexpr int kPairStages = kTopk ? TCfg::kStages : Cfg::kStages;
   constexpr int kPCols = Cfg::kCols, kPChunks = Cfg::kChunks;
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -914,7 +940,7 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     // Per-column vectors of the warp's 128 columns live in a region PRIVATE to the warp (no CTA-wide barrier when the
     // n-tile changes -- in PLDA scoring it changes on every tile): lane l owns columns 4l .. 4l+3, the next tile's values
     // are loaded into registers one tile ahead.
-    float* wv = s_vec + (warp - 2) * ((kTopk ? 1 : 3) * kPCols);
+    float* wv = s_vec + (warp - 2) * ((kTopk ? kTopkVecs : 3) * kPCols);
     // top-k: this thread's list (entry i at s_list[i * kNT + et]: interleaved by thread), its fill, the entry holding its
     // smallest key and that key's value, the bar every later candidate has to pass (-inf while the list is not full)
     constexpr int kNT = EW * 32;
@@ -1032,7 +1058,7 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       const bool plain = __all_sync(0xffffffffu, (flags & kRowFlagMask) == kRowStore);
 
       const int n_cols = (int)n_rows;
-      constexpr bool kBf16 = (MODE == kModeBf16);
+      constexpr bool kBf16 = mode_bf16(MODE);
       constexpr int kEs = kBf16 ? 2 : 4;
       const long long ld_bytes = a.out_ld * kEs;
       unsigned char* owarp = reinterpret_cast<unsigned char*>(a.out) + (row0 + quarter * 32) * ld_bytes;
@@ -1053,10 +1079,10 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         if (kRB == 2 && c + 1 < kPChunks) tmem_ld32_issue(taddr0 + (unsigned)((c + 1) * 32), r[(c + 1) % kRB]);
         const int col0 = col_base + colq * kPCols + c * 32;
         if constexpr (kTopk) {
-          // the add-only form of the epilogue as below; a value enters the list only if it beats the list's smallest
-          // entry (ties lose: every listed column is lower).  A lane with candidates in half a chunk parks the half in its
-          // column of the warp's scratch and walks them there, so the warp pays for its busiest lane, not for every
-          // column some lane wants to insert.
+          // the add-only form of the epilogue as below (AS-norm top-k: asnorm() as store_box forms it); a value enters
+          // the list only if it beats the list's smallest entry (ties lose: every listed column is lower; NaN and -inf
+          // never enter).  A lane with candidates in half a chunk parks the half in its column of the warp's scratch and
+          // walks them there, so the warp pays for its busiest lane, not for every column some lane wants to insert.
           const float4* b4 = reinterpret_cast<const float4*>(wv + c * 32);
 #pragma unroll
           for (int h = 0; h < 2; ++h) {
@@ -1065,6 +1091,15 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
               const float4 bb = b4[4 * h + q];
+              if constexpr (kNorm) {
+                const float4 ss = reinterpret_cast<const float4*>(wv + kPCols + c * 32)[4 * h + q];
+                const float4 oo = reinterpret_cast<const float4*>(wv + 2 * kPCols + c * 32)[4 * h + q];
+                v[4 * q + 0] = asnorm(__uint_as_float(r[c % kRB][16 * h + 4 * q + 0]), bb.x, ss.x, oo.x, radd, rh, rmu);
+                v[4 * q + 1] = asnorm(__uint_as_float(r[c % kRB][16 * h + 4 * q + 1]), bb.y, ss.y, oo.y, radd, rh, rmu);
+                v[4 * q + 2] = asnorm(__uint_as_float(r[c % kRB][16 * h + 4 * q + 2]), bb.z, ss.z, oo.z, radd, rh, rmu);
+                v[4 * q + 3] = asnorm(__uint_as_float(r[c % kRB][16 * h + 4 * q + 3]), bb.w, ss.w, oo.w, radd, rh, rmu);
+                continue;
+              }
               v[4 * q + 0] = (__uint_as_float(r[c % kRB][16 * h + 4 * q + 0]) + bb.x) + radd;
               v[4 * q + 1] = (__uint_as_float(r[c % kRB][16 * h + 4 * q + 1]) + bb.y) + radd;
               v[4 * q + 2] = (__uint_as_float(r[c % kRB][16 * h + 4 * q + 2]) + bb.z) + radd;
@@ -1088,7 +1123,7 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           if (kRB == 1 && c + 1 < kPChunks) tmem_ld32_issue(taddr0 + (unsigned)((c + 1) * 32), r[0]);
           continue;
         }
-        if (a.row_best != nullptr) {
+        if (mode_row_best(MODE) && a.row_best != nullptr) {
           // compact output: nothing is stored, the row keeps its best entry -- the add-only form of the epilogue, columns
           // in ascending order and a strict comparison, so the lowest column wins a tie
           const float4* b4 = reinterpret_cast<const float4*>(wv + c * 32);
@@ -1122,8 +1157,11 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 #define KTF_STORE_BOX(EPI_, HALF_)                                                                                      \
   store_box<kBf16, EPI_, kPCols, HALF_>(r[c % kRB], wvc, relu_lo, radd, stg2, lane, flags, plain, out_box, ld_bytes, tmc, \
                                         box_col0, trow, tma_pending, store_policy, a.debug, rh, rmu)
-          if constexpr (kNorm) {
+          if constexpr (kNorm && !kBf16) {
             KTF_STORE_BOX(kEpiNorm, 0);          // (fp32 rows: every chunk is a whole box)
+          } else if constexpr (kNorm) {
+            if ((c & 1) == 0) KTF_STORE_BOX(kEpiNorm, 0);
+            else KTF_STORE_BOX(kEpiNorm, 1);
           } else if ((c & 1) == 0) {
             if (epi == kEpiFull) KTF_STORE_BOX(kEpiFull, 0);
             else if (epi == kEpiAdd) KTF_STORE_BOX(kEpiAdd, 0);
@@ -1147,7 +1185,8 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         }
         if (kRB == 1 && c + 1 < kPChunks) tmem_ld32_issue(taddr0 + (unsigned)((c + 1) * 32), r[0]);
       }
-      if (a.row_best != nullptr && best_c >= 0 && row < m_rows) atomicMax(a.row_best + row, top1_key(best_v, best_c));
+      if (mode_row_best(MODE) && a.row_best != nullptr && best_c >= 0 && row < m_rows)
+        atomicMax(a.row_best + row, top1_key(best_v, best_c));
       tc_fence_before();
       __syncwarp();
       if (lane == 0) {
@@ -1799,11 +1838,11 @@ int launch_gemm_pair_ew(const CUtensorMap& tmA, const CUtensorMap& tmB_half, con
   constexpr int kSmemPair = pair_smem<MODE, EW>();
   constexpr int kPairThreads = PairCfg<EW>::kThreads;
   TcArgs args = args_in;
-  if (MODE != kModeNorm && args.row_add != nullptr && (args.scale != nullptr || args.offset != nullptr)) return KTF_EINVAL;
+  if (!mode_norm(MODE) && args.row_add != nullptr && (args.scale != nullptr || args.offset != nullptr)) return KTF_EINVAL;
   CUtensorMap tmC = tmA;
   args.tma_store = 0;
   if (args.out != nullptr) {
-    const int es = (MODE == kModeBf16) ? 2 : 4;
+    const int es = mode_bf16(MODE) ? 2 : 4;
     if (encode_map_out(&tmC, args.out, es, (unsigned long long)args.n_rows, (unsigned long long)args.m_rows,
                        (unsigned long long)args.out_ld))
       args.tma_store = 1;
@@ -2109,14 +2148,14 @@ int tc_gemm_nt(const void* A, long long m, long long lda, const void* B, long lo
 
 int tc_gemm_asnorm(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
                    int fp16, const float* row_norm, const float* col_add, const float* col_half_inv,
-                   const float* col_mean, float* C, long long ldc, cudaStream_t st) {
+                   const float* col_mean, void* C, long long ldc, int c_bf16, cudaStream_t st) {
   CUtensorMap tmA, tmBh;
   TcArgs args;
-  int rc = nt_setup(A, m, lda, B, n, ldb, K, fp16, row_norm, col_add, C, ldc, 0, &tmA, &tmBh, &args);
+  int rc = nt_setup(A, m, lda, B, n, ldb, K, fp16, row_norm, col_add, C, ldc, c_bf16, &tmA, &tmBh, &args);
   if (rc != KTF_OK) return rc;
   args.scale = col_half_inv;
   args.offset = col_mean;
-  return launch_gemm_pair<kModeNorm>(tmA, tmBh, args, st);
+  return c_bf16 ? launch_gemm_pair<kModeNormBf16>(tmA, tmBh, args, st) : launch_gemm_pair<kModeNorm>(tmA, tmBh, args, st);
 }
 
 }  // namespace ktf
@@ -2161,9 +2200,12 @@ int tc_topk_lists(long long m, long long n, long long K) {
   return pl.splits * (pl.ew / 4);
 }
 
-int tc_gemm_topk(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
-                 int fp16, const float* row_add, const float* col_add, int k, float* part_score, long long* part_index,
-                 cudaStream_t st) {
+// Operand maps, arguments and plan of a top-k GEMM (tc_gemm_topk, tc_gemm_asnorm_topk); KTF_OK with pl->splits = 0 when
+// there is nothing to do (m or n is 0).
+static int topk_setup(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
+                      int fp16, const float* row_add, const float* col_add, int k, float* part_score,
+                      long long* part_index, CUtensorMap* tmA, CUtensorMap* tmBh, TcArgs* out, TopkPlan* pl) {
+  *pl = TopkPlan{0, 0, 0};
   int rc = check_arch();
   if (rc != KTF_OK) return rc;
   if (m <= 0 || n <= 0) return KTF_OK;
@@ -2171,12 +2213,11 @@ int tc_gemm_topk(const void* A, long long m, long long lda, const void* B, long 
     ktf::set_error("tc_gemm_topk: k = %d outside 1..32", k);
     return KTF_EINVAL;
   }
-  CUtensorMap tmA, tmBh;
-  if ((rc = encode_map(&tmA, A, (unsigned long long)K, (unsigned long long)m, (unsigned long long)lda, BK, BM)) != KTF_OK)
+  if ((rc = encode_map(tmA, A, (unsigned long long)K, (unsigned long long)m, (unsigned long long)lda, BK, BM)) != KTF_OK)
     return rc;
-  if ((rc = encode_map(&tmBh, B, (unsigned long long)K, (unsigned long long)n, (unsigned long long)ldb, BK, BN / 2)) != KTF_OK)
+  if ((rc = encode_map(tmBh, B, (unsigned long long)K, (unsigned long long)n, (unsigned long long)ldb, BK, BN / 2)) != KTF_OK)
     return rc;
-  const TopkPlan pl = topk_plan(m, n, K);
+  *pl = topk_plan(m, n, K);
   TcArgs args{};
   args.num_taps = 1;
   args.kblocks_per_tap = (int)((K + BK - 1) / BK);
@@ -2186,16 +2227,44 @@ int tc_gemm_topk(const void* A, long long m, long long lda, const void* B, long 
   args.bias = col_add;
   args.row_add = row_add;
   args.topk_k = k;
-  args.topk_unit_tiles = pl.unit_tiles;
+  args.topk_unit_tiles = pl->unit_tiles;
   args.topk_score = part_score;
   args.topk_index = part_index;
+  *out = args;
+  return KTF_OK;
+}
+
+// the list capacity (8, 16, 32) and epilogue warp count of the plan pick the instantiation
 #define KTF_TOPK_LAUNCH(MODE_)                                                         \
   (pl.ew == 16 ? launch_gemm_pair_ew<MODE_, 16>(tmA, tmBh, args, st)                   \
                : launch_gemm_pair_ew<MODE_, 8>(tmA, tmBh, args, st))
-  rc = k <= 8 ? KTF_TOPK_LAUNCH(kModeTopk8) : k <= 16 ? KTF_TOPK_LAUNCH(kModeTopk16) : KTF_TOPK_LAUNCH(kModeTopk32);
-#undef KTF_TOPK_LAUNCH
-  return rc;
+
+int tc_gemm_topk(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
+                 int fp16, const float* row_add, const float* col_add, int k, float* part_score, long long* part_index,
+                 cudaStream_t st) {
+  CUtensorMap tmA, tmBh;
+  TcArgs args;
+  TopkPlan pl;
+  int rc = topk_setup(A, m, lda, B, n, ldb, K, fp16, row_add, col_add, k, part_score, part_index, &tmA, &tmBh, &args, &pl);
+  if (rc != KTF_OK || pl.splits == 0) return rc;
+  return k <= 8 ? KTF_TOPK_LAUNCH(kModeTopk8) : k <= 16 ? KTF_TOPK_LAUNCH(kModeTopk16) : KTF_TOPK_LAUNCH(kModeTopk32);
 }
+
+int tc_gemm_asnorm_topk(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
+                        int fp16, const float* row_norm, const float* col_add, const float* col_half_inv,
+                        const float* col_mean, int k, float* part_score, long long* part_index, cudaStream_t st) {
+  CUtensorMap tmA, tmBh;
+  TcArgs args;
+  TopkPlan pl;
+  int rc = topk_setup(A, m, lda, B, n, ldb, K, fp16, row_norm, col_add, k, part_score, part_index, &tmA, &tmBh, &args, &pl);
+  if (rc != KTF_OK || pl.splits == 0) return rc;
+  args.scale = col_half_inv;
+  args.offset = col_mean;
+  return k <= 8    ? KTF_TOPK_LAUNCH(kModeNormTopk8)
+         : k <= 16 ? KTF_TOPK_LAUNCH(kModeNormTopk16)
+                   : KTF_TOPK_LAUNCH(kModeNormTopk32);
+}
+#undef KTF_TOPK_LAUNCH
 
 }  // namespace ktf
 

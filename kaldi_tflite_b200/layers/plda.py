@@ -180,20 +180,13 @@ class PLDA(Layer):
                                               T.ptr(mean), T.ptr(std), None, T.stream_ptr()))
         return mean, std
 
-    def asNorm(self, u_test, u_enroll=None, u_cohort=None, *, top_n=None, test_stats=None, enroll_stats=None,
-               num_examples=1.0, out=None):
-        """Adaptive symmetric normalisation (AS-norm1) of the `logLikelihoodRatio` matrix:
-        s'[i, j] = 0.5 ((s[i, j] - mu_e[j]) / sigma_e[j] + (s[i, j] - mu_t[i]) / sigma_t[i]), float32 (n_test, n_enroll),
-        normalised in the score kernel (the raw matrix is never written).  `test_stats` / `enroll_stats` are
-        (mean, std) pairs from `cohortStats`; whichever is not given is computed from `u_cohort` and `top_n`
-        (test role for u_test, enrolled role with `num_examples` for u_enroll).  `u_enroll=None` scores the set against
-        itself.  float32 layers only."""
-        if self.paramDtype != np.float32:
-            raise ValueError("asNorm needs a float32 PLDA layer")
-        u_enroll = u_test if u_enroll is None else u_enroll
+    def _asNormStats(self, u_test, u_enroll, u_cohort, top_n, test_stats, enroll_stats, num_examples, caller):
+        """The four (mean, std) statistics tensors of an AS-norm call, test side first: those given, checked, and the
+        others computed from `u_cohort` and `top_n` (test role for u_test, enrolled role with `num_examples` for
+        u_enroll)."""
         nt, ne = u_test.shape[0], u_enroll.shape[0]
         if (test_stats is None or enroll_stats is None) and (u_cohort is None or top_n is None):
-            raise ValueError("asNorm needs u_cohort and top_n for the statistics it is not given")
+            raise ValueError(f"{caller} needs u_cohort and top_n for the statistics it is not given")
         if test_stats is None:
             test_stats = self.cohortStats(u_test, u_cohort, top_n=top_n, role="test")
         if enroll_stats is None:
@@ -204,13 +197,58 @@ class PLDA(Layer):
                 if t.dtype != torch.float32 or t.shape != (n,) or not t.is_contiguous():
                     raise ValueError(f"{side}_stats must be two contiguous float32 tensors of shape ({n},)")
                 stats.append(t)
+        return stats
+
+    def asNorm(self, u_test, u_enroll=None, u_cohort=None, *, top_n=None, test_stats=None, enroll_stats=None,
+               num_examples=1.0, out=None, score_dtype=None):
+        """Adaptive symmetric normalisation (AS-norm1) of the `logLikelihoodRatio` matrix:
+        s'[i, j] = 0.5 ((s[i, j] - mu_e[j]) / sigma_e[j] + (s[i, j] - mu_t[i]) / sigma_t[i]), float32 (n_test, n_enroll),
+        normalised in the score kernel (the raw matrix is never written).  `test_stats` / `enroll_stats` are
+        (mean, std) pairs from `cohortStats`; whichever is not given is computed from `u_cohort` and `top_n`
+        (test role for u_test, enrolled role with `num_examples` for u_enroll).  `u_enroll=None` scores the set against
+        itself.  `score_dtype=torch.bfloat16` (or a bfloat16 `out`) writes the same float32 value rounded once to
+        bfloat16: half the bytes of the matrix.  float32 layers only."""
+        if self.paramDtype != np.float32:
+            raise ValueError("asNorm needs a float32 PLDA layer")
+        compact = score_dtype is torch.bfloat16 or (out is not None and out.dtype is torch.bfloat16)
+        if score_dtype is not None and not compact and score_dtype != torch.float32:
+            raise ValueError("score_dtype must be torch.float32 or torch.bfloat16")
+        dtype = torch.bfloat16 if compact else torch.float32
+        u_enroll = u_test if u_enroll is None else u_enroll
+        nt, ne = u_test.shape[0], u_enroll.shape[0]
+        stats = self._asNormStats(u_test, u_enroll, u_cohort, top_n, test_stats, enroll_stats, num_examples, "asNorm")
         if out is None:
-            out = torch.empty((nt, ne), device=u_test.device, dtype=torch.float32)
-        elif out.dtype != torch.float32 or tuple(out.shape) != (nt, ne) or out.stride(1) != 1:
-            raise ValueError(f"out must be a float32 ({nt}, {ne}) tensor with unit column stride")
-        N.check(N.lib().ktf_plda_score_asnorm(self.handle_for(num_examples), T.ptr(u_test), nt, T.ptr(u_enroll), ne,
-                                              *(T.ptr(t) for t in stats), T.ptr(out), out.stride(0), T.stream_ptr()))
+            out = torch.empty((nt, ne), device=u_test.device, dtype=dtype)
+        elif out.dtype != dtype or tuple(out.shape) != (nt, ne) or out.stride(1) != 1:
+            raise ValueError(f"out must be a {dtype} ({nt}, {ne}) tensor with unit column stride")
+        N.check(N.lib().ktf_plda_score_asnorm_ex(self.handle_for(num_examples), T.ptr(u_test), nt, T.ptr(u_enroll), ne,
+                                                 *(T.ptr(t) for t in stats), T.ptr(out), out.stride(0),
+                                                 N.KTF_SCORES_BF16 if compact else N.KTF_SCORES_NATIVE, T.stream_ptr()))
         return out
+
+    def asNormBestMatches(self, u_test, u_enroll=None, u_cohort=None, *, k, top_n=None, test_stats=None,
+                          enroll_stats=None, num_examples=1.0):
+        """The k best enrolled vectors per test vector by AS-norm score, 1 <= k <= 32: (scores (n_test, k) float32,
+        indexes (n_test, k) int64), row i = the first k entries of a stable descending sort of row i of `asNorm` (same
+        statistics, same values bit for bit) and their columns, without writing the matrix.  NaN and -inf scores (a
+        deviation of 0 can give them) are never listed; past the last listed column the entries are (-inf, -1).  The
+        statistics are given or computed as in `asNorm`; `u_enroll=None` scores the set against itself.  float32 layers
+        only."""
+        if self.paramDtype != np.float32:
+            raise ValueError("asNormBestMatches needs a float32 PLDA layer")
+        k = int(k)
+        if not 1 <= k <= N.KTF_PLDA_TOPK_MAX:
+            raise ValueError(f"k = {k}, must be 1 .. {N.KTF_PLDA_TOPK_MAX}")
+        u_enroll = u_test if u_enroll is None else u_enroll
+        nt, ne = u_test.shape[0], u_enroll.shape[0]
+        stats = self._asNormStats(u_test, u_enroll, u_cohort, top_n, test_stats, enroll_stats, num_examples,
+                                  "asNormBestMatches")
+        scores = torch.empty((nt, k), device=u_test.device, dtype=torch.float32)
+        index = torch.empty((nt, k), device=u_test.device, dtype=torch.int64)
+        N.check(N.lib().ktf_plda_score_asnorm_topk(self.handle_for(num_examples), T.ptr(u_test), nt, T.ptr(u_enroll),
+                                                   ne, *(T.ptr(t) for t in stats), k, T.ptr(scores), T.ptr(index),
+                                                   T.stream_ptr()))
+        return scores, index
 
     def call(self, inputs):
         x = T.as_device(inputs)

@@ -162,20 +162,27 @@ def plda_best_matches_sharded(plda, x_test_local, x_enroll_local, k, test_counts
     exchange these (n_test, k) lists once, and `ktf_topk_merge` reduces them on every rank.  Returns (scores, indexes),
     (n_test, k) each, test rows ordered by rank -- equal to `bestMatches` on the whole set.
     """
-    rank, w = world()
+    _, w = world()
     u_test_local = plda.transformVector(x_test_local.contiguous())
     if w == 1:
         return plda.bestMatches(u_test_local, plda.transformVector(x_enroll_local.contiguous()), k=k)
     u_all, offs, works = exchange_test_vectors(u_test_local, test_counts)
     u_enroll_local = plda.transformVector(x_enroll_local.contiguous())
-    n = torch.tensor([u_enroll_local.shape[0]], device=u_enroll_local.device, dtype=torch.int64)
-    sizes = [torch.zeros_like(n) for _ in range(w)]
-    dist.all_gather(sizes, n)
-    e_off = sum(int(s.item()) for s in sizes[:rank])
     for wk in works:
         if wk is not None:
             wk.wait()
     scores, index = plda.bestMatches(u_all, u_enroll_local, k=k)
+    return _merge_shard_lists(scores, index, u_enroll_local.shape[0], k)
+
+
+def _merge_shard_lists(scores, index, n_enroll_local, k):
+    """The (n_test, k) lists every rank found in its own enrolled shard -> the lists of the whole enrolled set, on every
+    rank: indexes offset to the global enrolled numbering (shards in rank order), one exchange, `ktf_topk_merge`."""
+    rank, w = world()
+    n = torch.tensor([n_enroll_local], device=scores.device, dtype=torch.int64)
+    sizes = [torch.zeros_like(n) for _ in range(w)]
+    dist.all_gather(sizes, n)
+    e_off = sum(int(s.item()) for s in sizes[:rank])
     index = torch.where(index >= 0, index + e_off, index)
     # one exchange: the score bits ride in the int64 tensor next to the indexes
     local = torch.cat([scores.view(torch.int32).to(torch.int64), index], dim=1)
@@ -184,31 +191,26 @@ def plda_best_matches_sharded(plda, x_test_local, x_enroll_local, k, test_counts
     lists = torch.stack(lists)                                     # (w, n_test, 2k)
     s_in = lists[:, :, :k].to(torch.int32).view(torch.float32).contiguous()
     i_in = lists[:, :, k:].contiguous()
-    n_test = u_all.shape[0]
-    out_s = torch.empty((n_test, k), device=u_all.device, dtype=torch.float32)
-    out_i = torch.empty((n_test, k), device=u_all.device, dtype=torch.int64)
+    n_test = scores.shape[0]
+    out_s = torch.empty((n_test, k), device=scores.device, dtype=torch.float32)
+    out_i = torch.empty((n_test, k), device=scores.device, dtype=torch.int64)
     _native.check(_native.lib().ktf_topk_merge(T.ptr(s_in), T.ptr(i_in), w, n_test, k, k, T.ptr(out_s), T.ptr(out_i),
                                                T.stream_ptr()))
     return out_s, out_i
 
 
-def plda_asnorm_sharded(plda, x_test_local, x_enroll_local, u_cohort, top_n, test_counts=None):
-    """
-    Sharded AS-norm trial scoring on the layout of `plda_score_sharded`: each rank holds a slice of the test and of the
-    enrolled x-vectors (raw, (n, dim) float32) and the whole transformed cohort `u_cohort`.  Every rank computes the
-    cohort statistics of its own test rows and of its own enrolled shard; the test statistics travel with the test
-    vectors in the one all-gather (two extra columns), so no rank recomputes another's.  Returns this rank's block
-    `PLDA.asNorm`[all tests, local enrolled] -- test rows ordered by rank, row pitch padded to 16 bytes -- plus the
-    gathered transformed test vectors.
-    """
-    rank, w = world()
+def _asnorm_inputs_sharded(plda, x_test_local, x_enroll_local, u_cohort, top_n, test_counts):
+    """Transformed vectors and cohort statistics of the sharded AS-norm calls: ALL test vectors with their statistics,
+    this rank's enrolled shard with its statistics, and the test row offsets of the ranks.  Every rank computes the
+    statistics of its own test rows and enrolled shard; the test statistics travel with the test vectors in the one
+    all-gather (two extra columns), so no rank recomputes another's."""
+    _, w = world()
     u_test_local = plda.transformVector(x_test_local.contiguous())
     t_mean, t_std = plda.cohortStats(u_test_local, u_cohort, top_n=top_n, role="test")
     u_enroll_local = plda.transformVector(x_enroll_local.contiguous())
     e_stats = plda.cohortStats(u_enroll_local, u_cohort, top_n=top_n, role="enrolled")
-    ne = u_enroll_local.shape[0]
     if w == 1:
-        return plda.asNorm(u_test_local, u_enroll_local, test_stats=(t_mean, t_std), enroll_stats=e_stats), u_test_local
+        return u_test_local, (t_mean, t_std), u_enroll_local, e_stats, [0, u_test_local.shape[0]]
     dim = u_test_local.shape[1]
     packed = torch.cat([u_test_local, t_mean[:, None], t_std[:, None]], dim=1)
     p_all, offs, works = exchange_test_vectors(packed, test_counts)
@@ -217,9 +219,46 @@ def plda_asnorm_sharded(plda, x_test_local, x_enroll_local, u_cohort, top_n, tes
             wk.wait()
     u_all = p_all[:, :dim].contiguous()
     t_stats = (p_all[:, dim].contiguous(), p_all[:, dim + 1].contiguous())
-    # row pitch padded to 16 bytes: the score kernel's boxed (TMA) stores need an aligned pitch
-    out = torch.empty((offs[-1], (ne + 7) // 8 * 8), device=u_all.device, dtype=torch.float32)[:, :ne]
+    return u_all, t_stats, u_enroll_local, e_stats, offs
+
+
+def plda_asnorm_sharded(plda, x_test_local, x_enroll_local, u_cohort, top_n, test_counts=None, score_dtype=None):
+    """
+    Sharded AS-norm trial scoring on the layout of `plda_score_sharded`: each rank holds a slice of the test and of the
+    enrolled x-vectors (raw, (n, dim) float32) and the whole transformed cohort `u_cohort`.  Every rank computes the
+    cohort statistics of its own test rows and of its own enrolled shard; the test statistics travel with the test
+    vectors in the one all-gather (two extra columns), so no rank recomputes another's.  Returns this rank's block
+    `PLDA.asNorm`[all tests, local enrolled] -- test rows ordered by rank, row pitch padded to 16 bytes, float32 or
+    (`score_dtype=torch.bfloat16`) bfloat16 -- plus the gathered transformed test vectors.
+    """
+    _, w = world()
+    u_all, t_stats, u_enroll_local, e_stats, offs = _asnorm_inputs_sharded(plda, x_test_local, x_enroll_local,
+                                                                           u_cohort, top_n, test_counts)
+    if w == 1:
+        return plda.asNorm(u_all, u_enroll_local, test_stats=t_stats, enroll_stats=e_stats, score_dtype=score_dtype), u_all
+    ne = u_enroll_local.shape[0]
+    # row pitch padded to 16 bytes (8 elements: 32 B of float32, 16 B of bfloat16): the score kernel's boxed (TMA)
+    # stores need an aligned pitch
+    dtype = torch.bfloat16 if score_dtype is torch.bfloat16 else torch.float32
+    out = torch.empty((offs[-1], (ne + 7) // 8 * 8), device=u_all.device, dtype=dtype)[:, :ne]
     return plda.asNorm(u_all, u_enroll_local, test_stats=t_stats, enroll_stats=e_stats, out=out), u_all
+
+
+def plda_asnorm_best_matches_sharded(plda, x_test_local, x_enroll_local, u_cohort, top_n, k, test_counts=None):
+    """
+    Sharded k-best trial search by AS-norm score: `PLDA.asNormBestMatches` of ALL test vectors against ALL enrolled
+    vectors, on the layout of `plda_asnorm_sharded` (each rank holds a slice of the raw test and enrolled x-vectors and
+    the whole transformed cohort).  Every rank finds the normalised k best of its own enrolled shard for every test row;
+    the ranks then exchange and merge these lists as `plda_best_matches_sharded` does.  Returns (scores, indexes),
+    (n_test, k) each, test rows ordered by rank.
+    """
+    _, w = world()
+    u_all, t_stats, u_enroll_local, e_stats, _ = _asnorm_inputs_sharded(plda, x_test_local, x_enroll_local, u_cohort,
+                                                                        top_n, test_counts)
+    scores, index = plda.asNormBestMatches(u_all, u_enroll_local, k=k, test_stats=t_stats, enroll_stats=e_stats)
+    if w == 1:
+        return scores, index
+    return _merge_shard_lists(scores, index, u_enroll_local.shape[0], k)
 
 
 def stream_batches(fn, host_in, chunk, host_out=None, depth=3):
