@@ -415,6 +415,27 @@ int ktf_plda_score_topk(const ktf_plda* p, const void* u_test_dev, int64_t n_tes
 int ktf_topk_merge(const float* scores_in_dev, const int64_t* index_in_dev, int32_t num_lists, int64_t n_rows,
                    int32_t k_in, int32_t k, float* scores_dev, int64_t* index_dev, void* stream);
 
+/* ktf_plda_score_topk for 1 <= k <= KTF_PLDA_TOPK_LARGE_MAX (shortlists, recall@100, neighbour graphs): the same
+ * contract -- row i is the first k entries of a stable descending sort of row i of the ktf_plda_score matrix, bit for
+ * bit, (-inf, -1) past the last enrolled vector -- without the matrix in memory.  k <= KTF_PLDA_TOPK_MAX runs
+ * ktf_plda_score_topk's path.  Larger k writes the scores in row chunks of at most 128 MB into the handle's grow-only
+ * workspace and selects every chunk while it is in L2: one CTA per row finds the exact k-th largest score by radix
+ * select, emits the scores above it and the lowest columns equal to it, and sorts them.  k outside
+ * 1 .. KTF_PLDA_TOPK_LARGE_MAX is KTF_EINVAL; the handle and n_enroll rules of ktf_plda_score_topk apply.  No host
+ * synchronisation: once the workspace has grown for a shape the call can be captured in a CUDA graph; calls on one
+ * handle must not run concurrently on different streams. */
+#define KTF_PLDA_TOPK_LARGE_MAX 1024
+int ktf_plda_score_topk_large(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,
+                              int64_t n_enroll, int32_t k, float* scores_dev, int64_t* index_dev, void* stream);
+/* ktf_topk_merge for 1 <= k <= KTF_PLDA_TOPK_LARGE_MAX: row i of the output is the first k entries of a stable
+ * descending sort by score of the row's candidates taken list after list (entry j of list l is candidate l k_in + j),
+ * leaving out entries with index < 0 and NaN and -inf scores, padded with (-inf, -1).  On equal scores the earlier
+ * candidate comes first: the lower index when equal scores sit in index order, as in the lists ktf_plda_score_topk_large
+ * returns for enrolled shards taken in shard order.  KTF_EINVAL outside 1 .. KTF_PLDA_TOPK_LARGE_MAX or for
+ * num_lists k_in >= 2^31.  No workspace, no host synchronisation. */
+int ktf_topk_merge_large(const float* scores_in_dev, const int64_t* index_in_dev, int32_t num_lists, int64_t n_rows,
+                         int32_t k_in, int32_t k, float* scores_dev, int64_t* index_dev, void* stream);
+
 /* Adaptive symmetric score normalisation (AS-norm1, Matejka et al., Interspeech 2017) in two steps.
  *
  * Cohort statistics: for each of the n vectors u_dev (n, dim), the mean (mean_dev[i]) and the population standard
@@ -460,6 +481,15 @@ int ktf_plda_score_asnorm_topk(const ktf_plda* p, const void* u_test_dev, int64_
                                int64_t n_enroll, const float* test_mean_dev, const float* test_std_dev,
                                const float* enroll_mean_dev, const float* enroll_std_dev, int32_t k, float* scores_dev,
                                int64_t* index_dev, void* stream);
+/* ktf_plda_score_asnorm_topk for 1 <= k <= KTF_PLDA_TOPK_LARGE_MAX: the contract of ktf_plda_score_asnorm_topk (NaN and
+ * -inf never listed, +inf listed), on the path of ktf_plda_score_topk_large over the normalised score chunks.  k outside
+ * 1 .. KTF_PLDA_TOPK_LARGE_MAX is KTF_EINVAL; the workspace and synchronisation rules of ktf_plda_score_topk_large
+ * apply. */
+int ktf_plda_score_asnorm_topk_large(const ktf_plda* p, const void* u_test_dev, int64_t n_test,
+                                     const void* u_enroll_dev, int64_t n_enroll, const float* test_mean_dev,
+                                     const float* test_std_dev, const float* enroll_mean_dev,
+                                     const float* enroll_std_dev, int32_t k, float* scores_dev, int64_t* index_dev,
+                                     void* stream);
 
 #ifdef __cplusplus
 }

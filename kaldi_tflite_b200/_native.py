@@ -20,6 +20,7 @@ KTF_ACT_NONE, KTF_ACT_RELU = 0, 1
 KTF_SCORES_NATIVE, KTF_SCORES_BF16 = 0, 1
 KTF_MAX_CONTEXT = 16
 KTF_PLDA_TOPK_MAX = 32
+KTF_PLDA_TOPK_LARGE_MAX = 1024
 KTF_COHORT_AS_TEST, KTF_COHORT_AS_ENROLLED = 0, 1
 KTF_NCCL_UNIQUE_ID_BYTES = 128
 KTF_EINVAL, KTF_ECUDA, KTF_ENOMEM = -1, -2, -3
@@ -114,6 +115,9 @@ _SIGNATURES = {
     "ktf_plda_score_asnorm": (c_int32, [_P, _P, c_int64, _P, c_int64, _P, _P, _P, _P, _P, c_int64, _P]),
     "ktf_plda_score_asnorm_ex": (c_int32, [_P, _P, c_int64, _P, c_int64, _P, _P, _P, _P, _P, c_int64, c_int32, _P]),
     "ktf_plda_score_asnorm_topk": (c_int32, [_P, _P, c_int64, _P, c_int64, _P, _P, _P, _P, c_int32, _P, _P, _P]),
+    "ktf_plda_score_topk_large": (c_int32, [_P, _P, c_int64, _P, c_int64, c_int32, _P, _P, _P]),
+    "ktf_plda_score_asnorm_topk_large": (c_int32, [_P, _P, c_int64, _P, c_int64, _P, _P, _P, _P, c_int32, _P, _P, _P]),
+    "ktf_topk_merge_large": (c_int32, [_P, _P, c_int32, c_int64, c_int32, c_int32, _P, _P, _P]),
 }
 
 _lib = None

@@ -17,6 +17,7 @@
 // (64 FLOP per output byte), not by the tensor pipe (SURVEY.md 8d cfg5).  fp64 handles and
 // configurations whose operands could leave the fp16 range use exact SIMT tiles.
 #include <cuda_fp16.h>
+#include <assert.h>
 #include <math.h>
 
 #include <algorithm>
@@ -296,6 +297,9 @@ constexpr int kSelThreads = 512;
 constexpr int kSelBins = 4096;                    // histogram bins of the first radix pass (12 bits); the others use 10
 constexpr long long kSelSmemRowMax = 48 * 1024;   // rows up to this long are held in shared memory as keys (208 KB)
 constexpr double kCohortChunkBytes = 64e6;        // raw cohort scores per chunk: written by the GEMM, read from L2
+// Score chunk of the k > 32 top-k path: 512 rows at 50 000 columns.  Twice the cohort chunk halves the selection's
+// tail wave (256 -> 512 CTAs on 148 SMs); measured 15 % faster at 50 000 columns (DESIGN K5 (vi)).
+constexpr double kTopkChunkBytes = 128e6;
 
 __device__ __forceinline__ unsigned order_key(float v) {   // unsigned order = float order
   const unsigned b = __float_as_uint(v);
@@ -303,6 +307,90 @@ __device__ __forceinline__ unsigned order_key(float v) {   // unsigned order = f
 }
 __device__ __forceinline__ float key_value(unsigned k) {
   return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
+}
+
+// f(c, key(c)) for c = tid, tid + kSelThreads, ... < n in increasing c, with eight key loads in flight per thread (a
+// row that is not in shared memory is read from L2, and one dependent load per iteration would leave the CTA waiting).
+template <typename KeyFn, typename F>
+__device__ __forceinline__ void for_each_key(const KeyFn& key, long long n, const F& f) {
+  constexpr int kIlp = 8;
+  long long c = threadIdx.x;
+  for (; c + (kIlp - 1) * kSelThreads < n; c += kIlp * kSelThreads) {
+    unsigned k[kIlp];
+#pragma unroll
+    for (int u = 0; u < kIlp; ++u) k[u] = key(c + u * kSelThreads);
+#pragma unroll
+    for (int u = 0; u < kIlp; ++u) f(c + u * kSelThreads, k[u]);
+  }
+  for (; c < n; c += kSelThreads) f(c, key(c));
+}
+
+// Exact need-th largest of the keys key(c), c < n, of one row (need >= 1; key 0 is not counted -- order_key gives it
+// only to the NaN 0xffffffff): radix select, three passes of 12 + 10 + 10 bits, each a shared-memory histogram (hist:
+// kSelBins) of the keys under the prefix found so far.  Returns that key (thr), how many keys equal to it are among the
+// need largest (eq), how many there are (n_eq) and count = need; with fewer than need counted keys thr = eq = n_eq = 0
+// and count = the number of counted keys.  Called by all kSelThreads threads of the CTA.
+struct Selected {
+  unsigned thr, eq, n_eq, count;
+};
+template <typename KeyFn>
+__device__ Selected radix_select(KeyFn key, long long n, unsigned need, unsigned* hist) {
+  __shared__ unsigned s_warp[kSelThreads / 32];
+  __shared__ unsigned s_digit, s_need, s_neq;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const unsigned n_want = need;
+  unsigned prefix = 0, pmask = 0;   // need: rank of the target among the keys under the prefix
+  for (int pass = 0; pass < 3; ++pass) {
+    const int shift = pass == 0 ? 20 : (pass == 1 ? 10 : 0);
+    const unsigned nb = pass == 0 ? 4096u : 1024u, per = nb / kSelThreads;
+    for (unsigned b = tid; b < nb; b += kSelThreads) hist[b] = 0;
+    __syncthreads();                              // (first pass: the keys may be in shared memory too)
+    for_each_key(key, n, [&](long long, unsigned k) {
+      if (k != 0 && (k & pmask) == prefix) atomicAdd(&hist[(k >> shift) & (nb - 1)], 1u);
+    });
+    __syncthreads();
+    // the digit d with #(keys above d) < need <= #(keys at or above d); thread t owns bins [t per, (t + 1) per)
+    unsigned loc = 0;
+    for (unsigned i = 0; i < per; ++i) loc += hist[tid * per + i];
+    unsigned incl = loc;                          // sum over this and the higher lanes of the warp
+    for (int o = 1; o < 32; o <<= 1) {
+      const unsigned v = __shfl_down_sync(0xffffffffu, incl, o);
+      if (lane + o < 32) incl += v;
+    }
+    if (lane == 0) s_warp[warp] = incl;
+    __syncthreads();
+    unsigned above = incl - loc;
+    for (int w = warp + 1; w < kSelThreads / 32; ++w) above += s_warp[w];
+    if (pass == 0) {
+      unsigned total = 0;
+      for (int w = 0; w < kSelThreads / 32; ++w) total += s_warp[w];
+      if (total < need) {                         // CTA-uniform: every counted key is listed
+        __syncthreads();                          // hist / s_warp are rewritten by the caller or the next call
+        return Selected{0u, 0u, 0u, total};
+      }
+    }
+    if (above < need && need <= above + loc) {    // exactly one thread
+      unsigned acc = above;
+      for (int i = (int)per - 1; i >= 0; --i) {
+        const unsigned h = hist[tid * per + i];
+        if (need <= acc + h) {
+          s_digit = tid * per + (unsigned)i;
+          s_need = need - acc;
+          s_neq = h;
+          break;
+        }
+        acc += h;
+      }
+    }
+    __syncthreads();
+    prefix |= s_digit << shift;
+    pmask |= (nb - 1) << shift;
+    need = s_need;
+    const unsigned n_eq = s_neq;
+    __syncthreads();                              // hist / s_warp / s_digit are rewritten by the next pass
+    if (pass == 2) return Selected{prefix, need, n_eq, n_want};
+  }
+  return Selected{};
 }
 
 // One CTA per row of a chunk of raw cohort accumulators x (pitch ld).  The score is (x + first) + second: column addend
@@ -322,9 +410,7 @@ __global__ void __launch_bounds__(kSelThreads) cohort_select_kernel(const float*
   extern __shared__ unsigned sel_smem[];
   unsigned* hist = sel_smem;                  // [kSelBins]
   unsigned* keys = sel_smem + kSelBins;       // [nc] when in_smem
-  __shared__ unsigned s_warp[kSelThreads / 32];
   __shared__ double s_sum[kSelThreads / 32], s_sq[kSelThreads / 32];
-  __shared__ unsigned s_digit, s_need;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const long long row = blockIdx.x;
   const float* xr = x + row * ld;
@@ -336,47 +422,8 @@ __global__ void __launch_bounds__(kSelThreads) cohort_select_kernel(const float*
     for (long long c = tid; c < nc; c += kSelThreads) keys[c] = key_at(c);
   auto key = [&](long long c) { return in_smem ? keys[c] : key_at(c); };
 
-  unsigned prefix = 0, pmask = 0, need = top_n;   // need: rank of the target among the keys under the prefix
-  for (int pass = 0; pass < 3; ++pass) {
-    const int shift = pass == 0 ? 20 : (pass == 1 ? 10 : 0);
-    const unsigned nb = pass == 0 ? 4096u : 1024u, per = nb / kSelThreads;
-    for (unsigned b = tid; b < nb; b += kSelThreads) hist[b] = 0;
-    __syncthreads();                              // (first pass: the keys are in shared memory too)
-    for (long long c = tid; c < nc; c += kSelThreads) {
-      const unsigned k = key(c);
-      if ((k & pmask) == prefix) atomicAdd(&hist[(k >> shift) & (nb - 1)], 1u);
-    }
-    __syncthreads();
-    // the digit d with #(keys above d) < need <= #(keys at or above d); thread t owns bins [t per, (t + 1) per)
-    unsigned loc = 0;
-    for (unsigned i = 0; i < per; ++i) loc += hist[tid * per + i];
-    unsigned incl = loc;                          // sum over this and the higher lanes of the warp
-    for (int o = 1; o < 32; o <<= 1) {
-      const unsigned v = __shfl_down_sync(0xffffffffu, incl, o);
-      if (lane + o < 32) incl += v;
-    }
-    if (lane == 0) s_warp[warp] = incl;
-    __syncthreads();
-    unsigned above = incl - loc;
-    for (int w = warp + 1; w < kSelThreads / 32; ++w) above += s_warp[w];
-    if (above < need && need <= above + loc) {    // exactly one thread
-      unsigned acc = above;
-      for (int i = (int)per - 1; i >= 0; --i) {
-        const unsigned h = hist[tid * per + i];
-        if (need <= acc + h) {
-          s_digit = tid * per + (unsigned)i;
-          s_need = need - acc;
-          break;
-        }
-        acc += h;
-      }
-    }
-    __syncthreads();
-    prefix |= s_digit << shift;
-    pmask |= (nb - 1) << shift;
-    need = s_need;
-    __syncthreads();                              // hist / s_warp / s_digit are rewritten by the next pass
-  }
+  // top_n <= nc finite scores: the threshold always exists
+  const unsigned prefix = radix_select(key, nc, top_n, hist).thr;
   const double thr = (double)key_value(prefix);
   double sum = 0.0, sq = 0.0;
   for (long long c = tid; c < nc; c += kSelThreads) {
@@ -409,15 +456,20 @@ __global__ void __launch_bounds__(kSelThreads) cohort_select_kernel(const float*
   }
 }
 
+// Rows of a chunk of n rows of pitch ld floats: at most `bytes`, whole pair tiles when there are enough.
+long long chunk_rows(long long ld, long long n, double bytes) {
+  long long chunk = std::max(1LL, (long long)(bytes / (double)(ld * (long long)sizeof(float))));
+  if (chunk >= 256) chunk = chunk / 256 * 256;
+  return std::min<long long>(chunk, n);
+}
+
 // Cohort statistics of n vectors: the raw score GEMM against the cohort runs in row chunks of at most
 // kCohortChunkBytes into the workspace, each chunk is selected while it is still in L2.
 int cohort_stats_tc(const ktf_plda* p, const float* u, int64_t n, const float* uc, int64_t nc, long long top_n,
                     bool enrolled, float* mean, float* stdev, float* nth, cudaStream_t st) {
   const long long K = 3LL * p->dim;
   const long long ld = (nc + 3) / 4 * 4;          // 16-byte row pitch: the GEMM's boxed stores
-  long long chunk = std::max(1LL, (long long)(kCohortChunkBytes / (double)(ld * (long long)sizeof(float))));
-  if (chunk >= 256) chunk = chunk / 256 * 256;    // whole pair tiles
-  chunk = std::min<long long>(chunk, n);
+  const long long chunk = chunk_rows(ld, n, kCohortChunkBytes);
   TcOperands o;
   int rc = tc_operands(p, u, n, uc, nc, (size_t)chunk * ld * sizeof(float), st, &o, enrolled);
   if (rc != KTF_OK) return rc;
@@ -527,6 +579,201 @@ int score_tc_topk(const ktf_plda* p, const float* ut, int64_t nt, const float* u
                                                   norm->e_mean, k, part_s, part_i, st);
   if (rc != KTF_OK) return rc;
   return topk_merge(part_s, part_i, lists, nt, k, k, score, index, st);
+}
+
+// ---- the k best of a row for k up to KTF_PLDA_TOPK_LARGE_MAX: radix select, ordered emit, bitonic sort ----
+// Built with -DKTF_SELECT_CHECKS, topk_select_kernel asserts every shared-memory index and the global candidate it
+// reads and writes against the bounds the launch gives it (a bounds-checked build of the selection); otherwise the
+// checks compile to nothing.
+#ifdef KTF_SELECT_CHECKS
+#define KTF_SEL_CHECK(cond) assert(cond)
+#else
+#define KTF_SEL_CHECK(cond) ((void)0)
+#endif
+
+__device__ __forceinline__ unsigned listed_key(float v) {   // NaN and -inf are never listed: key 0
+  return (isnan(v) || v == -INFINITY) ? 0u : order_key(v);
+}
+
+// Candidates of a row of a score chunk (pitch ld): candidate c is column c.
+struct MatrixRows {
+  const float* x;
+  long long ld;
+  __device__ __forceinline__ unsigned key(long long row, long long c) const {
+    KTF_SEL_CHECK(row >= 0 && c >= 0 && c < ld);
+    return listed_key(x[row * ld + c]);
+  }
+  __device__ __forceinline__ long long index(long long, long long c) const { return c; }
+};
+
+// Candidates of a row of ktf_topk_merge_large's (num_lists, n_rows, k_in) lists: candidate c is entry c % k_in of list
+// c / k_in; an entry with index < 0 is none.
+struct ListRows {
+  const float* s;
+  const long long* i;
+  long long n_rows;
+  int k_in;
+  __device__ __forceinline__ long long at(long long row, long long c) const {
+    KTF_SEL_CHECK(row >= 0 && row < n_rows && c >= 0);
+    return (c / k_in * n_rows + row) * k_in + c % k_in;
+  }
+  __device__ __forceinline__ unsigned key(long long row, long long c) const {
+    const long long o = at(row, c);
+    return i[o] < 0 ? 0u : listed_key(s[o]);
+  }
+  __device__ __forceinline__ long long index(long long row, long long c) const { return i[at(row, c)]; }
+};
+
+// Sort entry of a listed candidate: the larger key first, then the lower candidate number (c < 2^32); 0 is none.
+__device__ __forceinline__ unsigned long long cand_entry(unsigned key, long long c) {
+  return ((unsigned long long)key << 32) | (0xffffffffu - (unsigned)c);
+}
+
+// One CTA per row (grid-stride): the k best of the row's n candidates -- the first k of a stable descending sort of
+// their values without NaN and -inf -- best first, padded with (-inf, -1).  radix_select finds the k-th largest key;
+// every key above it is emitted (shared-memory atomics: the order does not matter, the sort below fixes it), and so
+// are the keys equal to it when all of them are listed; otherwise the first `eq` equal keys in candidate order follow
+// (a CTA prefix count per tile of kSelThreads candidates, so equal keys are taken lowest candidate first whatever the
+// scheduling).  A bitonic sort of the <= k entries in shared memory puts them in order.  Keys are held in shared memory when in_smem (n <= kSelSmemRowMax), otherwise re-read (from L2) by
+// each pass.
+template <typename Rows>
+__global__ void __launch_bounds__(kSelThreads) topk_select_kernel(Rows rows, long long n_rows, long long n, int k,
+                                                                  int in_smem, float* __restrict__ s_out,
+                                                                  long long* __restrict__ i_out) {
+  extern __shared__ __align__(16) unsigned topk_smem[];
+  unsigned* hist = topk_smem;                                           // [kSelBins] during the select
+  unsigned long long* cand = reinterpret_cast<unsigned long long*>(topk_smem);   // [k] after it (8 KB <= 16 KB)
+  unsigned* keys = topk_smem + kSelBins;                                // [n] when in_smem
+  __shared__ unsigned s_above, s_warp_eq[kSelThreads / 32];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+#ifdef KTF_SELECT_CHECKS
+  unsigned smem_bytes;
+  asm("mov.u32 %0, %%dynamic_smem_size;" : "=r"(smem_bytes));
+  KTF_SEL_CHECK(blockDim.x == kSelThreads && k >= 1 && k <= KTF_PLDA_TOPK_LARGE_MAX &&
+                (!in_smem || n <= kSelSmemRowMax) &&
+                (kSelBins + (in_smem ? n : 0)) * sizeof(unsigned) <= smem_bytes &&
+                KTF_PLDA_TOPK_LARGE_MAX * sizeof(unsigned long long) <= kSelBins * sizeof(unsigned));
+#endif
+  for (long long row = blockIdx.x; row < n_rows; row += gridDim.x) {
+    auto row_key = [&](long long c) { return rows.key(row, c); };
+    if (in_smem) for_each_key(row_key, n, [&](long long c, unsigned kc) { keys[c] = kc; });
+    auto key = [&](long long c) {
+      KTF_SEL_CHECK(c >= 0 && c < n);
+      return in_smem ? keys[c] : rows.key(row, c);
+    };
+    const Selected sel = radix_select(key, n, (unsigned)k, hist);
+    const unsigned thr = sel.thr, eq = sel.eq, count = sel.count;
+    if (tid == 0) s_above = 0;
+    __syncthreads();
+    // every key equal to thr listed (no tie across rank k, or fewer than k keys): one unordered pass; otherwise the keys
+    // above thr unordered, then the first eq equal ones in candidate order
+    const bool all_eq = eq == sel.n_eq;
+    const unsigned lo = all_eq && thr != 0 ? thr : thr + 1;            // thr < 0xffffffff: NaN keys are 0
+    for_each_key(key, n, [&](long long c, unsigned kc) {
+      if (kc >= lo) {
+        const unsigned slot = atomicAdd(&s_above, 1u);
+        KTF_SEL_CHECK(slot < (all_eq ? count : count - eq));
+        cand[slot] = cand_entry(kc, c);
+      }
+    });
+    const unsigned n_above = count - eq;
+    unsigned taken = all_eq ? eq : 0u;                                  // equal keys seen so far (CTA-uniform)
+    for (long long c0 = 0; c0 < n && taken < eq; c0 += kSelThreads) {  // thr > 0 here: kc == thr means c < n
+      const long long c = c0 + tid;
+      const unsigned kc = c < n ? key(c) : 0u;
+      const unsigned ball = __ballot_sync(0xffffffffu, kc == thr);
+      if (lane == 0) s_warp_eq[warp] = __popc(ball);
+      __syncthreads();
+      unsigned before = taken + __popc(ball & ((1u << lane) - 1u)), tile = 0;
+      for (int w = 0; w < kSelThreads / 32; ++w) {
+        const unsigned v = s_warp_eq[w];
+        before += w < warp ? v : 0u;
+        tile += v;
+      }
+      if (kc == thr && before < eq) {
+        KTF_SEL_CHECK(n_above + before < count);
+        cand[n_above + before] = cand_entry(kc, c);
+      }
+      taken += tile;
+      __syncthreads();                                                  // s_warp_eq is rewritten by the next tile
+    }
+    unsigned P = 1;
+    while (P < count) P <<= 1;
+    KTF_SEL_CHECK(count <= (unsigned)k && P <= KTF_PLDA_TOPK_LARGE_MAX);
+    for (unsigned i = count + tid; i < P; i += kSelThreads) cand[i] = 0ull;
+    __syncthreads();
+    for (unsigned size = 2; size <= P; size <<= 1)
+      for (unsigned stride = size >> 1; stride > 0; stride >>= 1) {
+        for (unsigned i = tid; i < P / 2; i += kSelThreads) {
+          const unsigned lo = 2 * i - (i & (stride - 1)), hi = lo + stride;
+          KTF_SEL_CHECK(hi < P);
+          const unsigned long long a = cand[lo], b = cand[hi];
+          if ((a < b) == ((lo & size) == 0)) {                          // descending where lo & size == 0
+            cand[lo] = b;
+            cand[hi] = a;
+          }
+        }
+        __syncthreads();
+      }
+    for (int i = tid; i < k; i += kSelThreads) {
+      float s = -INFINITY;
+      long long idx = -1;
+      if ((unsigned)i < count) {
+        const unsigned long long e = cand[i];
+        KTF_SEL_CHECK(e != 0ull && (long long)(0xffffffffu - (unsigned)e) < n);
+        s = key_value((unsigned)(e >> 32));
+        idx = rows.index(row, (long long)(0xffffffffu - (unsigned)e));
+      }
+      s_out[row * k + i] = s;
+      i_out[row * k + i] = idx;
+    }
+    __syncthreads();                                                    // cand / keys are rewritten by the next row
+  }
+}
+
+template <typename Rows>
+int topk_select(const Rows& rows, long long n_rows, long long n, int k, float* s_out, long long* i_out, cudaStream_t st) {
+  if (n_rows <= 0) return KTF_OK;
+  const int in_smem = n <= kSelSmemRowMax;
+  const size_t smem = (size_t)(kSelBins + (in_smem ? n : 0)) * sizeof(unsigned);
+  static unsigned long long attr_done = 0;
+  if (ktf::first_use_on_device(&attr_done))
+    KTF_CUDA(cudaFuncSetAttribute(topk_select_kernel<Rows>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)((kSelBins + kSelSmemRowMax) * sizeof(unsigned))));
+  topk_select_kernel<Rows><<<(unsigned)std::min<long long>(n_rows, 1LL << 20), kSelThreads, smem, st>>>(
+      rows, n_rows, n, k, in_smem, s_out, i_out);
+  KTF_LAUNCH_OK();
+  return KTF_OK;
+}
+
+// score_tc_topk for 1 <= k <= KTF_PLDA_TOPK_LARGE_MAX.  k <= KTF_PLDA_TOPK_MAX keeps the GEMM's top-k epilogue (faster
+// there); larger k writes the raw (or, with norm, the AS-norm) scores in row chunks of at most kTopkChunkBytes into the
+// workspace -- the epilogue and operands of ktf_plda_score / ktf_plda_score_asnorm, so the values are bit-equal -- and
+// selects every chunk while it is still in L2.
+int score_tc_topk_large(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, int k, float* score,
+                        long long* index, cudaStream_t st, const AsnormStats* norm = nullptr) {
+  if (k <= KTF_PLDA_TOPK_MAX) return score_tc_topk(p, ut, nt, ue, ne, k, score, index, st, norm);
+  if (ne == 0) return topk_select(MatrixRows{nullptr, 0}, nt, 0, k, score, index, st);   // padding only
+  const long long K = 3LL * p->dim;
+  const long long ld = (ne + 3) / 4 * 4;          // 16-byte row pitch: the GEMM's boxed stores
+  const long long chunk = chunk_rows(ld, nt, kTopkChunkBytes);
+  const size_t chunk_bytes = (size_t)chunk * ld * sizeof(float);
+  AsnormOperands a;
+  const int rc0 = norm == nullptr ? tc_operands(p, ut, nt, ue, ne, chunk_bytes, st, &a.o)
+                                  : asnorm_operands(p, ut, nt, ue, ne, *norm, chunk_bytes, st, &a);
+  if (rc0 != KTF_OK) return rc0;
+  const TcOperands& o = a.o;
+  float* buf = reinterpret_cast<float*>(norm == nullptr ? o.extra : a.extra);
+  for (long long r0 = 0; r0 < nt; r0 += chunk) {
+    const long long rows = std::min(chunk, (long long)nt - r0);
+    int rc = norm == nullptr
+                 ? ktf::tc_gemm_nt(o.A + r0 * K, rows, K, o.B, ne, K, K, /*fp16=*/1, o.Ai + r0, o.Bj, buf, ld, 0, st)
+                 : ktf::tc_gemm_asnorm(o.A + r0 * K, rows, K, o.B, ne, K, K, /*fp16=*/1, a.row + 4 * r0, o.Bj,
+                                       a.e_half_inv, norm->e_mean, buf, ld, 0, st);
+    if (rc != KTF_OK) return rc;
+    if ((rc = topk_select(MatrixRows{buf, ld}, rows, ne, k, score + r0 * k, index + r0 * k, st)) != KTF_OK) return rc;
+  }
+  return KTF_OK;
 }
 
 template <typename T>
@@ -771,6 +1018,56 @@ int ktf_topk_merge(const float* scores_in_dev, const int64_t* index_in_dev, int3
                 "ktf_topk_merge: null argument");
   return topk_merge(scores_in_dev, (const long long*)index_in_dev, num_lists, n_rows, k_in, k, scores_dev,
                     (long long*)index_dev, (cudaStream_t)stream);
+}
+
+int ktf_plda_score_topk_large(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,
+                              int64_t n_enroll, int32_t k, float* scores_dev, int64_t* index_dev, void* stream) {
+  KTF_CHECK_ARG(k >= 1 && k <= KTF_PLDA_TOPK_LARGE_MAX,
+                "ktf_plda_score_topk_large: k = %d, must be 1 .. %d (KTF_PLDA_TOPK_LARGE_MAX)", k,
+                KTF_PLDA_TOPK_LARGE_MAX);
+  KTF_CHECK_ARG(p, "ktf_plda_score_topk_large: null handle");
+  KTF_CHECK_ARG(p->use_tc, "ktf_plda_score_topk_large needs a float32 PLDA handle on an sm_100 device");
+  KTF_CHECK_ARG(n_enroll >= 0 && n_enroll < (1LL << 32),
+                "ktf_plda_score_topk_large: n_enroll must be in 0 .. 2^32 - 1");
+  if (n_test <= 0) return KTF_OK;
+  KTF_CHECK_ARG(u_test_dev && scores_dev && index_dev && (u_enroll_dev || n_enroll == 0),
+                "ktf_plda_score_topk_large: null argument");
+  return score_tc_topk_large(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, k, scores_dev,
+                             (long long*)index_dev, (cudaStream_t)stream);
+}
+
+int ktf_plda_score_asnorm_topk_large(const ktf_plda* p, const void* u_test_dev, int64_t n_test,
+                                     const void* u_enroll_dev, int64_t n_enroll, const float* test_mean_dev,
+                                     const float* test_std_dev, const float* enroll_mean_dev,
+                                     const float* enroll_std_dev, int32_t k, float* scores_dev, int64_t* index_dev,
+                                     void* stream) {
+  KTF_CHECK_ARG(k >= 1 && k <= KTF_PLDA_TOPK_LARGE_MAX,
+                "ktf_plda_score_asnorm_topk_large: k = %d, must be 1 .. %d (KTF_PLDA_TOPK_LARGE_MAX)", k,
+                KTF_PLDA_TOPK_LARGE_MAX);
+  KTF_CHECK_ARG(p, "ktf_plda_score_asnorm_topk_large: null handle");
+  KTF_CHECK_ARG(p->use_tc, "ktf_plda_score_asnorm_topk_large needs a float32 PLDA handle on an sm_100 device");
+  KTF_CHECK_ARG(n_enroll >= 0 && n_enroll < (1LL << 32),
+                "ktf_plda_score_asnorm_topk_large: n_enroll must be in 0 .. 2^32 - 1");
+  if (n_test <= 0) return KTF_OK;
+  KTF_CHECK_ARG(u_test_dev && test_mean_dev && test_std_dev && scores_dev && index_dev &&
+                    (n_enroll == 0 || (u_enroll_dev && enroll_mean_dev && enroll_std_dev)),
+                "ktf_plda_score_asnorm_topk_large: null argument");
+  const AsnormStats s{test_mean_dev, test_std_dev, enroll_mean_dev, enroll_std_dev};
+  return score_tc_topk_large(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, k, scores_dev,
+                             (long long*)index_dev, (cudaStream_t)stream, &s);
+}
+
+int ktf_topk_merge_large(const float* scores_in_dev, const int64_t* index_in_dev, int32_t num_lists, int64_t n_rows,
+                         int32_t k_in, int32_t k, float* scores_dev, int64_t* index_dev, void* stream) {
+  KTF_CHECK_ARG(k >= 1 && k <= KTF_PLDA_TOPK_LARGE_MAX,
+                "ktf_topk_merge_large: k = %d, must be 1 .. %d (KTF_PLDA_TOPK_LARGE_MAX)", k, KTF_PLDA_TOPK_LARGE_MAX);
+  KTF_CHECK_ARG(num_lists >= 0 && k_in >= 1 && (long long)num_lists * k_in < (1LL << 31),
+                "ktf_topk_merge_large: bad num_lists / k_in");
+  if (n_rows <= 0) return KTF_OK;
+  KTF_CHECK_ARG(scores_dev && index_dev && (num_lists == 0 || (scores_in_dev && index_in_dev)),
+                "ktf_topk_merge_large: null argument");
+  return topk_select(ListRows{scores_in_dev, (const long long*)index_in_dev, n_rows, k_in}, n_rows,
+                     (long long)num_lists * k_in, k, scores_dev, (long long*)index_dev, (cudaStream_t)stream);
 }
 
 int ktf_plda_score(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,

@@ -160,6 +160,26 @@ class PLDA(Layer):
                                             T.ptr(scores), T.ptr(index), T.stream_ptr()))
         return scores, index
 
+    def bestMatchesLarge(self, u_test, u_enroll=None, *, k, num_examples=1.0):
+        """`bestMatches` for 1 <= k <= 1024 (shortlists, recall@100, neighbour graphs): (scores (n_test, k) float32,
+        indexes (n_test, k) int64), row i = the first k entries of a stable descending sort of row i of
+        `logLikelihoodRatio` (same values, bit for bit) and their columns, padded with (-inf, -1) past the last enrolled
+        vector, without the (n_test, n_enroll) matrix in memory: k <= 32 runs `bestMatches`, larger k scores row chunks
+        of at most 128 MB and selects each while it is in L2.  `u_enroll=None` scores the set against itself.  float32
+        layers only."""
+        if self.paramDtype != np.float32:
+            raise ValueError("bestMatchesLarge needs a float32 PLDA layer")
+        k = int(k)
+        if not 1 <= k <= N.KTF_PLDA_TOPK_LARGE_MAX:
+            raise ValueError(f"k = {k}, must be 1 .. {N.KTF_PLDA_TOPK_LARGE_MAX}")
+        u_enroll = u_test if u_enroll is None else u_enroll
+        nt, ne = u_test.shape[0], u_enroll.shape[0]
+        scores = torch.empty((nt, k), device=u_test.device, dtype=torch.float32)
+        index = torch.empty((nt, k), device=u_test.device, dtype=torch.int64)
+        N.check(N.lib().ktf_plda_score_topk_large(self.handle_for(num_examples), T.ptr(u_test), nt, T.ptr(u_enroll),
+                                                  ne, k, T.ptr(scores), T.ptr(index), T.stream_ptr()))
+        return scores, index
+
     def cohortStats(self, u, u_cohort, *, top_n, role="test", num_examples=1.0):
         """AS-norm statistics of every vector of `u` against an imposter cohort: (mean (n,), std (n,)) float32, the
         mean and population std (ddof 0) of its `top_n` largest cohort scores.  role="test": the scores are row i of
@@ -248,6 +268,30 @@ class PLDA(Layer):
         N.check(N.lib().ktf_plda_score_asnorm_topk(self.handle_for(num_examples), T.ptr(u_test), nt, T.ptr(u_enroll),
                                                    ne, *(T.ptr(t) for t in stats), k, T.ptr(scores), T.ptr(index),
                                                    T.stream_ptr()))
+        return scores, index
+
+    def asNormBestMatchesLarge(self, u_test, u_enroll=None, u_cohort=None, *, k, top_n=None, test_stats=None,
+                               enroll_stats=None, num_examples=1.0):
+        """`asNormBestMatches` for 1 <= k <= 1024: (scores (n_test, k) float32, indexes (n_test, k) int64), row i = the
+        first k entries of a stable descending sort of row i of `asNorm` (same statistics, same values bit for bit) and
+        their columns, NaN and -inf scores never listed (+inf is), padded with (-inf, -1), without the matrix in memory:
+        k <= 32 runs `asNormBestMatches`, larger k normalises row chunks of at most 128 MB and selects each while it is in
+        L2.  The statistics are given or computed as in `asNorm`; `u_enroll=None` scores the set against itself.  float32
+        layers only."""
+        if self.paramDtype != np.float32:
+            raise ValueError("asNormBestMatchesLarge needs a float32 PLDA layer")
+        k = int(k)
+        if not 1 <= k <= N.KTF_PLDA_TOPK_LARGE_MAX:
+            raise ValueError(f"k = {k}, must be 1 .. {N.KTF_PLDA_TOPK_LARGE_MAX}")
+        u_enroll = u_test if u_enroll is None else u_enroll
+        nt, ne = u_test.shape[0], u_enroll.shape[0]
+        stats = self._asNormStats(u_test, u_enroll, u_cohort, top_n, test_stats, enroll_stats, num_examples,
+                                  "asNormBestMatchesLarge")
+        scores = torch.empty((nt, k), device=u_test.device, dtype=torch.float32)
+        index = torch.empty((nt, k), device=u_test.device, dtype=torch.int64)
+        N.check(N.lib().ktf_plda_score_asnorm_topk_large(self.handle_for(num_examples), T.ptr(u_test), nt,
+                                                         T.ptr(u_enroll), ne, *(T.ptr(t) for t in stats), k,
+                                                         T.ptr(scores), T.ptr(index), T.stream_ptr()))
         return scores, index
 
     def call(self, inputs):

@@ -172,12 +172,33 @@ def plda_best_matches_sharded(plda, x_test_local, x_enroll_local, k, test_counts
         if wk is not None:
             wk.wait()
     scores, index = plda.bestMatches(u_all, u_enroll_local, k=k)
-    return _merge_shard_lists(scores, index, u_enroll_local.shape[0], k)
+    return _merge_shard_lists(scores, index, u_enroll_local.shape[0], k, _native.lib().ktf_topk_merge)
 
 
-def _merge_shard_lists(scores, index, n_enroll_local, k):
+def plda_best_matches_large_sharded(plda, x_test_local, x_enroll_local, k, test_counts=None):
+    """
+    `plda_best_matches_sharded` for 1 <= k <= 1024: `PLDA.bestMatchesLarge` of ALL test vectors against ALL enrolled
+    vectors on the same layout and exchange, with the lists merged by `ktf_topk_merge_large`.  The exchanged lists are
+    world_size x n_test x 2k int64 on every rank: 16 KB per test row and rank at k = 1024.  Returns (scores, indexes),
+    (n_test, k) each, test rows ordered by rank -- equal to `bestMatchesLarge` on the whole set.
+    """
+    _, w = world()
+    u_test_local = plda.transformVector(x_test_local.contiguous())
+    if w == 1:
+        return plda.bestMatchesLarge(u_test_local, plda.transformVector(x_enroll_local.contiguous()), k=k)
+    u_all, offs, works = exchange_test_vectors(u_test_local, test_counts)
+    u_enroll_local = plda.transformVector(x_enroll_local.contiguous())
+    for wk in works:
+        if wk is not None:
+            wk.wait()
+    scores, index = plda.bestMatchesLarge(u_all, u_enroll_local, k=k)
+    return _merge_shard_lists(scores, index, u_enroll_local.shape[0], k, _native.lib().ktf_topk_merge_large)
+
+
+def _merge_shard_lists(scores, index, n_enroll_local, k, merge):
     """The (n_test, k) lists every rank found in its own enrolled shard -> the lists of the whole enrolled set, on every
-    rank: indexes offset to the global enrolled numbering (shards in rank order), one exchange, `ktf_topk_merge`."""
+    rank: indexes offset to the global enrolled numbering (shards in rank order), one exchange, then `merge`
+    (`ktf_topk_merge` or `ktf_topk_merge_large`, whichever admits k)."""
     rank, w = world()
     n = torch.tensor([n_enroll_local], device=scores.device, dtype=torch.int64)
     sizes = [torch.zeros_like(n) for _ in range(w)]
@@ -194,8 +215,7 @@ def _merge_shard_lists(scores, index, n_enroll_local, k):
     n_test = scores.shape[0]
     out_s = torch.empty((n_test, k), device=scores.device, dtype=torch.float32)
     out_i = torch.empty((n_test, k), device=scores.device, dtype=torch.int64)
-    _native.check(_native.lib().ktf_topk_merge(T.ptr(s_in), T.ptr(i_in), w, n_test, k, k, T.ptr(out_s), T.ptr(out_i),
-                                               T.stream_ptr()))
+    _native.check(merge(T.ptr(s_in), T.ptr(i_in), w, n_test, k, k, T.ptr(out_s), T.ptr(out_i), T.stream_ptr()))
     return out_s, out_i
 
 
@@ -258,7 +278,23 @@ def plda_asnorm_best_matches_sharded(plda, x_test_local, x_enroll_local, u_cohor
     scores, index = plda.asNormBestMatches(u_all, u_enroll_local, k=k, test_stats=t_stats, enroll_stats=e_stats)
     if w == 1:
         return scores, index
-    return _merge_shard_lists(scores, index, u_enroll_local.shape[0], k)
+    return _merge_shard_lists(scores, index, u_enroll_local.shape[0], k, _native.lib().ktf_topk_merge)
+
+
+def plda_asnorm_best_matches_large_sharded(plda, x_test_local, x_enroll_local, u_cohort, top_n, k, test_counts=None):
+    """
+    `plda_asnorm_best_matches_sharded` for 1 <= k <= 1024: `PLDA.asNormBestMatchesLarge` of ALL test vectors against ALL
+    enrolled vectors on the same layout and exchange, with the lists merged by `ktf_topk_merge_large`.  The exchanged
+    lists are world_size x n_test x 2k int64 on every rank: 16 KB per test row and rank at k = 1024.  Returns (scores,
+    indexes), (n_test, k) each, test rows ordered by rank.
+    """
+    _, w = world()
+    u_all, t_stats, u_enroll_local, e_stats, _ = _asnorm_inputs_sharded(plda, x_test_local, x_enroll_local, u_cohort,
+                                                                        top_n, test_counts)
+    scores, index = plda.asNormBestMatchesLarge(u_all, u_enroll_local, k=k, test_stats=t_stats, enroll_stats=e_stats)
+    if w == 1:
+        return scores, index
+    return _merge_shard_lists(scores, index, u_enroll_local.shape[0], k, _native.lib().ktf_topk_merge_large)
 
 
 def stream_batches(fn, host_in, chunk, host_out=None, depth=3):
