@@ -140,7 +140,7 @@ __global__ void plda_split_kernel(const float* __restrict__ u, long long n, int 
   }
 }
 
-// Decodes the best-entry keys of tc_gemm_nt(row_best): score and column of every test row (-1: no enrolled vector).
+// Decodes the best-entry keys of tc_gemm_score(row_best): score and column of every test row (-1: no enrolled vector).
 __global__ void plda_top1_decode_kernel(const unsigned long long* __restrict__ keys, long long n,
                                         float* __restrict__ score, long long* __restrict__ index) {
   const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
@@ -216,78 +216,6 @@ int topk_merge(const float* s_in, const long long* i_in, int num_lists, long lon
                long long* i_out, cudaStream_t st) {
   if (n_rows <= 0) return KTF_OK;
   topk_merge_kernel<<<(unsigned)((n_rows + 7) / 8), 256, 0, st>>>(s_in, i_in, num_lists, n_rows, k_in, k, s_out, i_out);
-  KTF_LAUNCH_OK();
-  return KTF_OK;
-}
-
-// Operands of the tensor-core score GEMM, in the handle's workspace: the fp16 hi/lo splits of both sides (K = 3 dim) and
-// A_i / B_j, followed by `extra` bytes of the caller's.  The GEMM's rows are normally the test vectors (c-scaled split,
-// A addend) and its columns the enrolled ones (plain split, B addend).  With `enrolled_rows` the roles swap sides: the
-// rows (ut) are enrolled vectors and get the plain split and the B addend, the columns (ue) play the test role.  The
-// cross term is symmetric and the three partial products meet the same K positions, so the accumulator is the transpose
-// of the normal one; Ai / Bj are then the row / column addends (B of the rows, A of the columns).
-struct TcOperands {
-  const __half* A;
-  const __half* B;
-  const float* Ai;
-  const float* Bj;
-  char* extra;
-};
-
-int tc_operands(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, size_t extra,
-                cudaStream_t st, TcOperands* o, bool enrolled_rows = false) {
-  const int dim = p->dim;
-  const long long K = 3LL * dim;
-  ktf::Carver cv;
-  const size_t o_a = cv.take((size_t)nt * K * sizeof(__half));
-  const size_t o_b = cv.take((size_t)ne * K * sizeof(__half));
-  const size_t o_ai = cv.take((size_t)nt * sizeof(float));
-  const size_t o_bj = cv.take((size_t)ne * sizeof(float));
-  const size_t o_extra = cv.take(extra);
-  int rc = p->ws.ensure(cv.off);
-  if (rc != KTF_OK) return rc;
-  char* base = static_cast<char*>(p->ws.ptr);
-  __half* As = reinterpret_cast<__half*>(base + o_a);
-  __half* Bs = reinterpret_cast<__half*>(base + o_b);
-  float* Ai = reinterpret_cast<float*>(base + o_ai);
-  float* Bj = reinterpret_cast<float*>(base + o_bj);
-  const float* wa = (const float*)p->d_wa;
-  const float* wb = (const float*)p->d_wb;
-  const float* c = (const float*)p->d_c;
-  const float ld = (float)p->logdet_term;
-  plda_quad_kernel<float><<<(unsigned)((nt + 7) / 8), 256, 0, st>>>(ut, nt, dim, enrolled_rows ? wb : wa,
-                                                                    enrolled_rows ? 0.0f : ld, Ai);
-  KTF_LAUNCH_OK();
-  plda_quad_kernel<float><<<(unsigned)((ne + 7) / 8), 256, 0, st>>>(ue, ne, dim, enrolled_rows ? wa : wb,
-                                                                    enrolled_rows ? ld : 0.0f, Bj);
-  KTF_LAUNCH_OK();
-  auto blocks = [](long long items) {
-    return (unsigned)std::min<long long>((items + 255) / 256, (long long)ktf::num_sms() * 16);
-  };
-  plda_split_kernel<<<blocks(nt * dim), 256, 0, st>>>(ut, nt, dim, enrolled_rows ? nullptr : c, enrolled_rows ? 1 : 0,
-                                                      As);
-  KTF_LAUNCH_OK();
-  plda_split_kernel<<<blocks(ne * dim), 256, 0, st>>>(ue, ne, dim, enrolled_rows ? c : nullptr, enrolled_rows ? 0 : 1,
-                                                      Bs);
-  KTF_LAUNCH_OK();
-  *o = TcOperands{As, Bs, Ai, Bj, base + o_extra};
-  return KTF_OK;
-}
-
-// top1_score / top1_index non-null: no score matrix, the best enrolled column of every test row instead.
-int score_tc(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, void* scores, int64_t ld,
-             int scores_bf16, cudaStream_t st, float* top1_score = nullptr, long long* top1_index = nullptr) {
-  const long long K = 3LL * p->dim;
-  TcOperands o;
-  int rc = tc_operands(p, ut, nt, ue, ne, top1_score ? (size_t)nt * sizeof(unsigned long long) : 0, st, &o);
-  if (rc != KTF_OK) return rc;
-  if (top1_score == nullptr)
-    return ktf::tc_gemm_nt(o.A, nt, K, o.B, ne, K, K, /*fp16=*/1, o.Ai, o.Bj, scores, ld, scores_bf16, st);
-  unsigned long long* keys = reinterpret_cast<unsigned long long*>(o.extra);
-  KTF_CUDA(cudaMemsetAsync(keys, 0, (size_t)nt * sizeof(unsigned long long), st));
-  if ((rc = ktf::tc_gemm_nt(o.A, nt, K, o.B, ne, K, K, /*fp16=*/1, o.Ai, o.Bj, nullptr, ne, 0, st, keys)) != KTF_OK)
-    return rc;
-  plda_top1_decode_kernel<<<(unsigned)((nt + 255) / 256), 256, 0, st>>>(keys, nt, top1_score, top1_index);
   KTF_LAUNCH_OK();
   return KTF_OK;
 }
@@ -456,43 +384,6 @@ __global__ void __launch_bounds__(kSelThreads) cohort_select_kernel(const float*
   }
 }
 
-// Rows of a chunk of n rows of pitch ld floats: at most `bytes`, whole pair tiles when there are enough.
-long long chunk_rows(long long ld, long long n, double bytes) {
-  long long chunk = std::max(1LL, (long long)(bytes / (double)(ld * (long long)sizeof(float))));
-  if (chunk >= 256) chunk = chunk / 256 * 256;
-  return std::min<long long>(chunk, n);
-}
-
-// Cohort statistics of n vectors: the raw score GEMM against the cohort runs in row chunks of at most
-// kCohortChunkBytes into the workspace, each chunk is selected while it is still in L2.
-int cohort_stats_tc(const ktf_plda* p, const float* u, int64_t n, const float* uc, int64_t nc, long long top_n,
-                    bool enrolled, float* mean, float* stdev, float* nth, cudaStream_t st) {
-  const long long K = 3LL * p->dim;
-  const long long ld = (nc + 3) / 4 * 4;          // 16-byte row pitch: the GEMM's boxed stores
-  const long long chunk = chunk_rows(ld, n, kCohortChunkBytes);
-  TcOperands o;
-  int rc = tc_operands(p, u, n, uc, nc, (size_t)chunk * ld * sizeof(float), st, &o, enrolled);
-  if (rc != KTF_OK) return rc;
-  float* raw = reinterpret_cast<float*>(o.extra);
-  const int in_smem = nc <= kSelSmemRowMax;
-  const size_t smem = (size_t)(kSelBins + (in_smem ? nc : 0)) * sizeof(unsigned);
-  static unsigned long long attr_done = 0;
-  if (ktf::first_use_on_device(&attr_done))
-    KTF_CUDA(cudaFuncSetAttribute(cohort_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)((kSelBins + kSelSmemRowMax) * sizeof(unsigned))));
-  for (long long r0 = 0; r0 < n; r0 += chunk) {
-    const long long rows = std::min(chunk, (long long)n - r0);
-    if ((rc = ktf::tc_gemm_nt(o.A + r0 * K, rows, K, o.B, nc, K, K, /*fp16=*/1, nullptr, nullptr, raw, ld, 0, st)) !=
-        KTF_OK)
-      return rc;
-    cohort_select_kernel<<<(unsigned)rows, kSelThreads, smem, st>>>(raw, ld, nc, o.Ai + r0, o.Bj, enrolled ? 1 : 0,
-                                                                     (unsigned)top_n, in_smem, mean + r0, stdev + r0,
-                                                                     nth ? nth + r0 : nullptr);
-    KTF_LAUNCH_OK();
-  }
-  return KTF_OK;
-}
-
 // Per-row (A_i, 0.5 / sigma_t, mu_t, 0) and per-column 0.5 / sigma_e of the normalising epilogue (IEEE divisions: a
 // sigma of 0 gives inf, and the score the IEEE quotient; 0.5 / sigma is exactly half of 1 / sigma).
 __global__ void asnorm_prep_kernel(const float* __restrict__ Ai, const float* __restrict__ t_mean,
@@ -513,72 +404,118 @@ struct AsnormStats {
   const float* e_std;
 };
 
-// Operands of the normalising score GEMM: those of tc_operands, then the per-row float4 and the per-column 0.5 / sigma_e
-// of asnorm_prep_kernel, then `extra` bytes of the caller's.
-struct AsnormOperands {
-  TcOperands o;
-  const float* row;          // (nt) float4
-  const float* e_half_inv;   // (ne)
+// Operands of the tensor-core score GEMM, in the handle's workspace: the fp16 hi/lo splits of both sides (K = 3 dim) and
+// A_i / B_j; for AS-norm scores the per-row float4 and per-column 0.5 / sigma_e of asnorm_prep_kernel; then `extra`
+// bytes of the caller's.  The GEMM's rows are normally the test vectors (c-scaled split, A addend) and its columns the
+// enrolled ones (plain split, B addend).  With `enrolled_rows` (raw scores) the roles swap sides: the rows (ut) are
+// enrolled vectors and get the plain split and the B addend, the columns (ue) play the test role.  The cross term is
+// symmetric and the three partial products meet the same K positions, so the accumulator is the transpose of the normal
+// one; Ai / Bj are then the row / column addends (B of the rows, A of the columns).
+struct TcOperands {
+  const __half* A;
+  const __half* B;
+  long long K;
+  const float* Ai;
+  const float* Bj;
+  const float* row;          // the GEMM's per-row addend: Ai, or for AS-norm scores (nt) float4
+  const float* e_half_inv;   // AS-norm: (ne); otherwise null
+  const float* e_mean;       // AS-norm: the caller's; otherwise null
   char* extra;
+
+  // The score GEMM of rows [r0, r0 + rows) against n columns, rows output C (null for the other outputs).
+  ktf::TcScore gemm(long long r0, long long rows, long long n, const float* row_add, const float* col_add, void* C,
+                    long long ldc, int c_bf16 = 0) const {
+    return ktf::TcScore{A + r0 * K, rows, K, B, n, K, K, /*fp16=*/1,
+                        row_add == nullptr ? nullptr : row_add + (e_half_inv ? 4 : 1) * r0, col_add, e_half_inv, e_mean,
+                        C, ldc, c_bf16};
+  }
 };
 
-int asnorm_operands(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, const AsnormStats& s,
-                    size_t extra, cudaStream_t st, AsnormOperands* a) {
-  const size_t row_bytes = ((size_t)nt * sizeof(float4) + 255) & ~(size_t)255;
-  const size_t col_bytes = ((size_t)ne * sizeof(float) + 255) & ~(size_t)255;
-  TcOperands o;
-  int rc = tc_operands(p, ut, nt, ue, ne, row_bytes + col_bytes + extra, st, &o);
+int tc_operands(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, const AsnormStats* norm,
+                size_t extra, cudaStream_t st, TcOperands* o, bool enrolled_rows = false) {
+  const int dim = p->dim;
+  const long long K = 3LL * dim;
+  ktf::Carver cv;
+  const size_t o_a = cv.take((size_t)nt * K * sizeof(__half));
+  const size_t o_b = cv.take((size_t)ne * K * sizeof(__half));
+  const size_t o_ai = cv.take((size_t)nt * sizeof(float));
+  const size_t o_bj = cv.take((size_t)ne * sizeof(float));
+  const size_t o_row = cv.take(norm ? (size_t)nt * sizeof(float4) : 0);
+  const size_t o_half_inv = cv.take(norm ? (size_t)ne * sizeof(float) : 0);
+  const size_t o_extra = cv.take(extra);
+  int rc = p->ws.ensure(cv.off);
   if (rc != KTF_OK) return rc;
-  float4* row = reinterpret_cast<float4*>(o.extra);
-  float* e_half_inv = reinterpret_cast<float*>(o.extra + row_bytes);
-  const long long items = std::max<long long>(nt, ne);
-  asnorm_prep_kernel<<<(unsigned)std::min<long long>((items + 255) / 256, (long long)ktf::num_sms() * 16), 256, 0, st>>>(
-      o.Ai, s.t_mean, s.t_std, nt, s.e_std, ne, row, e_half_inv);
+  char* base = static_cast<char*>(p->ws.ptr);
+  __half* As = reinterpret_cast<__half*>(base + o_a);
+  __half* Bs = reinterpret_cast<__half*>(base + o_b);
+  float* Ai = reinterpret_cast<float*>(base + o_ai);
+  float* Bj = reinterpret_cast<float*>(base + o_bj);
+  const float* wa = (const float*)p->d_wa;
+  const float* wb = (const float*)p->d_wb;
+  const float* c = (const float*)p->d_c;
+  const float ld = (float)p->logdet_term;
+  plda_quad_kernel<float><<<(unsigned)((nt + 7) / 8), 256, 0, st>>>(ut, nt, dim, enrolled_rows ? wb : wa,
+                                                                    enrolled_rows ? 0.0f : ld, Ai);
   KTF_LAUNCH_OK();
-  *a = AsnormOperands{o, reinterpret_cast<const float*>(row), e_half_inv, o.extra + row_bytes + col_bytes};
+  plda_quad_kernel<float><<<(unsigned)((ne + 7) / 8), 256, 0, st>>>(ue, ne, dim, enrolled_rows ? wa : wb,
+                                                                    enrolled_rows ? ld : 0.0f, Bj);
+  KTF_LAUNCH_OK();
+  auto blocks = [](long long items) {
+    return (unsigned)std::min<long long>((items + 255) / 256, (long long)ktf::num_sms() * 16);
+  };
+  plda_split_kernel<<<blocks(nt * dim), 256, 0, st>>>(ut, nt, dim, enrolled_rows ? nullptr : c, enrolled_rows ? 1 : 0,
+                                                      As);
+  KTF_LAUNCH_OK();
+  plda_split_kernel<<<blocks(ne * dim), 256, 0, st>>>(ue, ne, dim, enrolled_rows ? c : nullptr, enrolled_rows ? 0 : 1,
+                                                      Bs);
+  KTF_LAUNCH_OK();
+  *o = TcOperands{As, Bs, K, Ai, Bj, Ai, nullptr, nullptr, base + o_extra};
+  if (norm != nullptr) {
+    float4* row = reinterpret_cast<float4*>(base + o_row);
+    float* e_half_inv = reinterpret_cast<float*>(base + o_half_inv);
+    asnorm_prep_kernel<<<blocks(std::max<long long>(nt, ne)), 256, 0, st>>>(Ai, norm->t_mean, norm->t_std, nt,
+                                                                           norm->e_std, ne, row, e_half_inv);
+    KTF_LAUNCH_OK();
+    o->row = reinterpret_cast<const float*>(row);
+    o->e_half_inv = e_half_inv;
+    o->e_mean = norm->e_mean;
+  }
   return KTF_OK;
 }
 
-int score_tc_asnorm(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, const AsnormStats& s,
-                    void* scores, int64_t ld, int scores_bf16, cudaStream_t st) {
-  const long long K = 3LL * p->dim;
-  AsnormOperands a;
-  int rc = asnorm_operands(p, ut, nt, ue, ne, s, 0, st, &a);
-  if (rc != KTF_OK) return rc;
-  return ktf::tc_gemm_asnorm(a.o.A, nt, K, a.o.B, ne, K, K, /*fp16=*/1, a.row, a.o.Bj, a.e_half_inv, s.e_mean, scores, ld,
-                             scores_bf16, st);
+// Rows of a chunk of n rows of pitch ld floats: at most `bytes`, whole pair tiles when there are enough.
+long long chunk_rows(long long ld, long long n, double bytes) {
+  long long chunk = std::max(1LL, (long long)(bytes / (double)(ld * (long long)sizeof(float))));
+  if (chunk >= 256) chunk = chunk / 256 * 256;
+  return std::min<long long>(chunk, n);
 }
 
-// The k best enrolled columns of every test row, of the raw scores or (norm != nullptr) of the AS-norm scores: the score
-// GEMM leaves partial lists (one per n-range and column quarter of a row) in the workspace, topk_merge reduces them to
-// (nt, k).
-int score_tc_topk(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, int k, float* score,
-                  long long* index, cudaStream_t st, const AsnormStats* norm = nullptr) {
+// Cohort statistics of n vectors: the raw score GEMM against the cohort runs in row chunks of at most
+// kCohortChunkBytes into the workspace, each chunk is selected while it is still in L2.
+int cohort_stats_tc(const ktf_plda* p, const float* u, int64_t n, const float* uc, int64_t nc, long long top_n,
+                    bool enrolled, float* mean, float* stdev, float* nth, cudaStream_t st) {
   const long long K = 3LL * p->dim;
-  const int lists = ktf::tc_topk_lists(nt, ne, K);
-  if (lists == 0) return topk_merge(nullptr, nullptr, 0, nt, k, k, score, index, st);   // no enrolled vector
-  const size_t n_part = (size_t)lists * nt * k;
-  const size_t s_bytes = (n_part * sizeof(float) + 255) & ~(size_t)255;
-  const size_t part_bytes = s_bytes + n_part * sizeof(long long);
-  int rc;
-  char* parts;
-  AsnormOperands a;
-  if (norm == nullptr) {
-    rc = tc_operands(p, ut, nt, ue, ne, part_bytes, st, &a.o);
-    parts = a.o.extra;
-  } else {
-    rc = asnorm_operands(p, ut, nt, ue, ne, *norm, part_bytes, st, &a);
-    parts = a.extra;
+  const long long ld = (nc + 3) / 4 * 4;          // 16-byte row pitch: the GEMM's boxed stores
+  const long long chunk = chunk_rows(ld, n, kCohortChunkBytes);
+  TcOperands o;
+  int rc = tc_operands(p, u, n, uc, nc, nullptr, (size_t)chunk * ld * sizeof(float), st, &o, enrolled);
+  if (rc != KTF_OK) return rc;
+  float* raw = reinterpret_cast<float*>(o.extra);
+  const int in_smem = nc <= kSelSmemRowMax;
+  const size_t smem = (size_t)(kSelBins + (in_smem ? nc : 0)) * sizeof(unsigned);
+  static unsigned long long attr_done = 0;
+  if (ktf::first_use_on_device(&attr_done))
+    KTF_CUDA(cudaFuncSetAttribute(cohort_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)((kSelBins + kSelSmemRowMax) * sizeof(unsigned))));
+  for (long long r0 = 0; r0 < n; r0 += chunk) {
+    const long long rows = std::min(chunk, (long long)n - r0);
+    if ((rc = ktf::tc_gemm_score(o.gemm(r0, rows, nc, nullptr, nullptr, raw, ld), st)) != KTF_OK) return rc;
+    cohort_select_kernel<<<(unsigned)rows, kSelThreads, smem, st>>>(raw, ld, nc, o.Ai + r0, o.Bj, enrolled ? 1 : 0,
+                                                                     (unsigned)top_n, in_smem, mean + r0, stdev + r0,
+                                                                     nth ? nth + r0 : nullptr);
+    KTF_LAUNCH_OK();
   }
-  if (rc != KTF_OK) return rc;
-  float* part_s = reinterpret_cast<float*>(parts);
-  long long* part_i = reinterpret_cast<long long*>(parts + s_bytes);
-  const TcOperands& o = a.o;
-  rc = norm == nullptr ? ktf::tc_gemm_topk(o.A, nt, K, o.B, ne, K, K, /*fp16=*/1, o.Ai, o.Bj, k, part_s, part_i, st)
-                       : ktf::tc_gemm_asnorm_topk(o.A, nt, K, o.B, ne, K, K, /*fp16=*/1, a.row, o.Bj, a.e_half_inv,
-                                                  norm->e_mean, k, part_s, part_i, st);
-  if (rc != KTF_OK) return rc;
-  return topk_merge(part_s, part_i, lists, nt, k, k, score, index, st);
+  return KTF_OK;
 }
 
 // ---- the k best of a row for k up to KTF_PLDA_TOPK_LARGE_MAX: radix select, ordered emit, bitonic sort ----
@@ -746,34 +683,97 @@ int topk_select(const Rows& rows, long long n_rows, long long n, int k, float* s
   return KTF_OK;
 }
 
-// score_tc_topk for 1 <= k <= KTF_PLDA_TOPK_LARGE_MAX.  k <= KTF_PLDA_TOPK_MAX keeps the GEMM's top-k epilogue (faster
-// there); larger k writes the raw (or, with norm, the AS-norm) scores in row chunks of at most kTopkChunkBytes into the
-// workspace -- the epilogue and operands of ktf_plda_score / ktf_plda_score_asnorm, so the values are bit-equal -- and
-// selects every chunk while it is still in L2.
-int score_tc_topk_large(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, int k, float* score,
-                        long long* index, cudaStream_t st, const AsnormStats* norm = nullptr) {
-  if (k <= KTF_PLDA_TOPK_MAX) return score_tc_topk(p, ut, nt, ue, ne, k, score, index, st, norm);
-  if (ne == 0) return topk_select(MatrixRows{nullptr, 0}, nt, 0, k, score, index, st);   // padding only
-  const long long K = 3LL * p->dim;
-  const long long ld = (ne + 3) / 4 * 4;          // 16-byte row pitch: the GEMM's boxed stores
-  const long long chunk = chunk_rows(ld, nt, kTopkChunkBytes);
-  const size_t chunk_bytes = (size_t)chunk * ld * sizeof(float);
-  AsnormOperands a;
-  const int rc0 = norm == nullptr ? tc_operands(p, ut, nt, ue, ne, chunk_bytes, st, &a.o)
-                                  : asnorm_operands(p, ut, nt, ue, ne, *norm, chunk_bytes, st, &a);
-  if (rc0 != KTF_OK) return rc0;
-  const TcOperands& o = a.o;
-  float* buf = reinterpret_cast<float*>(norm == nullptr ? o.extra : a.extra);
+// What a tensor-core score call writes: the score matrix (row pitch ld, fp32 or bf16), the best column of every test
+// row (top-1), or its k best columns (1 <= k <= KTF_PLDA_TOPK_LARGE_MAX) as (nt, k) scores and indexes, best first.
+struct ScoreOut {
+  enum Kind { kMatrix, kTop1, kTopk } kind;
+  void* scores;
+  long long* index;
+  int64_t ld;
+  int bf16;
+  int k;
+};
+
+// The raw scores of test rows ut against enrolled columns ue, or (norm != nullptr) their AS-norm scores, as `out` asks:
+// - the matrix: one GEMM;
+// - top-1: the GEMM keeps a best-entry key per row (row_best), plda_top1_decode_kernel decodes the keys;
+// - k <= KTF_PLDA_TOPK_MAX: the GEMM's top-k epilogue leaves partial lists (one per n-range and column quarter of a row)
+//   in the workspace, topk_merge reduces them to (nt, k);
+// - larger k: the GEMM writes the scores in row chunks of at most kTopkChunkBytes into the workspace -- the epilogue of
+//   the matrix, so the values are bit-equal -- and topk_select selects every chunk while it is still in L2.
+int score_tc(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, int64_t ne, const AsnormStats* norm,
+             const ScoreOut& out, cudaStream_t st) {
+  const int k = out.k;
+  float* score = static_cast<float*>(out.scores);
+  const bool top_small = out.kind == ScoreOut::kTopk && k <= KTF_PLDA_TOPK_MAX;
+  const bool top_large = out.kind == ScoreOut::kTopk && k > KTF_PLDA_TOPK_MAX;
+  int lists = 0;
+  long long ld = 0, chunk = 0;
+  size_t extra = 0, s_bytes = 0;
+  if (out.kind == ScoreOut::kTop1) extra = (size_t)nt * sizeof(unsigned long long);
+  if (top_small) {
+    lists = ktf::tc_topk_lists(nt, ne, 3LL * p->dim);
+    if (lists == 0) return topk_merge(nullptr, nullptr, 0, nt, k, k, score, out.index, st);   // no enrolled vector
+    const size_t n_part = (size_t)lists * nt * k;
+    s_bytes = (n_part * sizeof(float) + 255) & ~(size_t)255;
+    extra = s_bytes + n_part * sizeof(long long);
+  }
+  if (top_large) {
+    if (ne == 0) return topk_select(MatrixRows{nullptr, 0}, nt, 0, k, score, out.index, st);   // padding only
+    ld = (ne + 3) / 4 * 4;          // 16-byte row pitch: the GEMM's boxed stores
+    chunk = chunk_rows(ld, nt, kTopkChunkBytes);
+    extra = (size_t)chunk * ld * sizeof(float);
+  }
+  TcOperands o;
+  int rc = tc_operands(p, ut, nt, ue, ne, norm, extra, st, &o);
+  if (rc != KTF_OK) return rc;
+  if (out.kind == ScoreOut::kMatrix)
+    return ktf::tc_gemm_score(o.gemm(0, nt, ne, o.row, o.Bj, out.scores, out.ld, out.bf16), st);
+  if (out.kind == ScoreOut::kTop1) {
+    unsigned long long* keys = reinterpret_cast<unsigned long long*>(o.extra);
+    KTF_CUDA(cudaMemsetAsync(keys, 0, (size_t)nt * sizeof(unsigned long long), st));
+    ktf::TcScore g = o.gemm(0, nt, ne, o.row, o.Bj, nullptr, ne);
+    g.row_best = keys;
+    if ((rc = ktf::tc_gemm_score(g, st)) != KTF_OK) return rc;
+    plda_top1_decode_kernel<<<(unsigned)((nt + 255) / 256), 256, 0, st>>>(keys, nt, score, out.index);
+    KTF_LAUNCH_OK();
+    return KTF_OK;
+  }
+  if (top_small) {
+    float* part_s = reinterpret_cast<float*>(o.extra);
+    long long* part_i = reinterpret_cast<long long*>(o.extra + s_bytes);
+    ktf::TcScore g = o.gemm(0, nt, ne, o.row, o.Bj, nullptr, 0);
+    g.k = k;
+    g.part_score = part_s;
+    g.part_index = part_i;
+    if ((rc = ktf::tc_gemm_score(g, st)) != KTF_OK) return rc;
+    return topk_merge(part_s, part_i, lists, nt, k, k, score, out.index, st);
+  }
+  float* buf = reinterpret_cast<float*>(o.extra);
   for (long long r0 = 0; r0 < nt; r0 += chunk) {
     const long long rows = std::min(chunk, (long long)nt - r0);
-    int rc = norm == nullptr
-                 ? ktf::tc_gemm_nt(o.A + r0 * K, rows, K, o.B, ne, K, K, /*fp16=*/1, o.Ai + r0, o.Bj, buf, ld, 0, st)
-                 : ktf::tc_gemm_asnorm(o.A + r0 * K, rows, K, o.B, ne, K, K, /*fp16=*/1, a.row + 4 * r0, o.Bj,
-                                       a.e_half_inv, norm->e_mean, buf, ld, 0, st);
-    if (rc != KTF_OK) return rc;
-    if ((rc = topk_select(MatrixRows{buf, ld}, rows, ne, k, score + r0 * k, index + r0 * k, st)) != KTF_OK) return rc;
+    if ((rc = ktf::tc_gemm_score(o.gemm(r0, rows, ne, o.row, o.Bj, buf, ld), st)) != KTF_OK) return rc;
+    if ((rc = topk_select(MatrixRows{buf, ld}, rows, ne, k, score + r0 * k, out.index + r0 * k, st)) != KTF_OK) return rc;
   }
   return KTF_OK;
+}
+
+// Argument checks of the k-best entry points `fn`, one order for all: k (1 .. k_max, named k_max_name), the handle,
+// float32 / sm_100, n_enroll; n_test <= 0 is then a no-op, and the pointers are checked last.  Scores when they pass.
+int score_topk_checked(const char* fn, int k_max, const char* k_max_name, const ktf_plda* p, const void* u_test,
+                       int64_t n_test, const void* u_enroll, int64_t n_enroll, const AsnormStats* norm, int k,
+                       float* scores, int64_t* index, void* stream) {
+  KTF_CHECK_ARG(k >= 1 && k <= k_max, "%s: k = %d, must be 1 .. %d (%s)", fn, k, k_max, k_max_name);
+  KTF_CHECK_ARG(p, "%s: null handle", fn);
+  KTF_CHECK_ARG(p->use_tc, "%s needs a float32 PLDA handle on an sm_100 device", fn);
+  KTF_CHECK_ARG(n_enroll >= 0 && n_enroll < (1LL << 32), "%s: n_enroll must be in 0 .. 2^32 - 1", fn);
+  if (n_test <= 0) return KTF_OK;
+  KTF_CHECK_ARG(u_test && scores && index && (n_enroll == 0 || u_enroll) &&
+                    (norm == nullptr ||
+                     (norm->t_mean && norm->t_std && (n_enroll == 0 || (norm->e_mean && norm->e_std)))),
+                "%s: null argument", fn);
+  return score_tc(p, (const float*)u_test, n_test, (const float*)u_enroll, n_enroll, norm,
+                  ScoreOut{ScoreOut::kTopk, scores, (long long*)index, 0, 0, k}, (cudaStream_t)stream);
 }
 
 template <typename T>
@@ -918,8 +918,8 @@ int ktf_plda_score_ex(const ktf_plda* p, const void* u_test_dev, int64_t n_test,
   if (score_format == KTF_SCORES_BF16) {
     KTF_CHECK_ARG(p->use_tc, "KTF_SCORES_BF16 needs a float32 handle (the tcgen05 score GEMM)");
     if (n_test <= 0 || n_enroll <= 0) return KTF_OK;
-    return score_tc(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, scores_dev, ld, 1,
-                    (cudaStream_t)stream);
+    return score_tc(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, nullptr,
+                    ScoreOut{ScoreOut::kMatrix, scores_dev, nullptr, ld, 1, 0}, (cudaStream_t)stream);
   }
   return ktf_plda_score(p, u_test_dev, n_test, u_enroll_dev, n_enroll, scores_dev, ld, stream);
 }
@@ -930,22 +930,15 @@ int ktf_plda_score_top1(const ktf_plda* p, const void* u_test_dev, int64_t n_tes
   KTF_CHECK_ARG(p->use_tc, "ktf_plda_score_top1 needs a float32 PLDA handle on an sm_100 device");
   KTF_CHECK_ARG(n_enroll < (1LL << 32), "ktf_plda_score_top1: more than 2^32 enrolled vectors");
   if (n_test <= 0) return KTF_OK;
-  return score_tc(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, nullptr, n_enroll, 0,
-                  (cudaStream_t)stream, best_score_dev, (long long*)best_index_dev);
+  return score_tc(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, nullptr,
+                  ScoreOut{ScoreOut::kTop1, best_score_dev, (long long*)best_index_dev, n_enroll, 0, 1},
+                  (cudaStream_t)stream);
 }
 
 int ktf_plda_score_topk(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,
                         int64_t n_enroll, int32_t k, float* scores_dev, int64_t* index_dev, void* stream) {
-  KTF_CHECK_ARG(p, "ktf_plda_score_topk: null handle");
-  KTF_CHECK_ARG(k >= 1 && k <= KTF_PLDA_TOPK_MAX, "ktf_plda_score_topk: k = %d, must be 1 .. %d (KTF_PLDA_TOPK_MAX)", k,
-                KTF_PLDA_TOPK_MAX);
-  KTF_CHECK_ARG(p->use_tc, "ktf_plda_score_topk needs a float32 PLDA handle on an sm_100 device");
-  KTF_CHECK_ARG(n_enroll >= 0 && n_enroll < (1LL << 32), "ktf_plda_score_topk: n_enroll must be in 0 .. 2^32 - 1");
-  if (n_test <= 0) return KTF_OK;
-  KTF_CHECK_ARG(u_test_dev && scores_dev && index_dev && (u_enroll_dev || n_enroll == 0),
-                "ktf_plda_score_topk: null argument");
-  return score_tc_topk(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, k, scores_dev,
-                       (long long*)index_dev, (cudaStream_t)stream);
+  return score_topk_checked("ktf_plda_score_topk", KTF_PLDA_TOPK_MAX, "KTF_PLDA_TOPK_MAX", p, u_test_dev, n_test,
+                            u_enroll_dev, n_enroll, nullptr, k, scores_dev, index_dev, stream);
 }
 
 int ktf_plda_cohort_stats(const ktf_plda* p, const void* u_dev, int64_t n, const void* u_cohort_dev, int64_t n_cohort,
@@ -984,27 +977,19 @@ int ktf_plda_score_asnorm_ex(const ktf_plda* p, const void* u_test_dev, int64_t 
   KTF_CHECK_ARG(u_test_dev && u_enroll_dev && test_mean_dev && test_std_dev && enroll_mean_dev && enroll_std_dev &&
                     scores_dev,
                 "ktf_plda_score_asnorm: null argument");
-  return score_tc_asnorm(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll,
-                         AsnormStats{test_mean_dev, test_std_dev, enroll_mean_dev, enroll_std_dev}, scores_dev, ld,
-                         score_format == KTF_SCORES_BF16 ? 1 : 0, (cudaStream_t)stream);
+  const AsnormStats s{test_mean_dev, test_std_dev, enroll_mean_dev, enroll_std_dev};
+  return score_tc(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, &s,
+                  ScoreOut{ScoreOut::kMatrix, scores_dev, nullptr, ld, score_format == KTF_SCORES_BF16 ? 1 : 0, 0},
+                  (cudaStream_t)stream);
 }
 
 int ktf_plda_score_asnorm_topk(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,
                                int64_t n_enroll, const float* test_mean_dev, const float* test_std_dev,
                                const float* enroll_mean_dev, const float* enroll_std_dev, int32_t k, float* scores_dev,
                                int64_t* index_dev, void* stream) {
-  KTF_CHECK_ARG(k >= 1 && k <= KTF_PLDA_TOPK_MAX,
-                "ktf_plda_score_asnorm_topk: k = %d, must be 1 .. %d (KTF_PLDA_TOPK_MAX)", k, KTF_PLDA_TOPK_MAX);
-  KTF_CHECK_ARG(p, "ktf_plda_score_asnorm_topk: null handle");
-  KTF_CHECK_ARG(p->use_tc, "ktf_plda_score_asnorm_topk needs a float32 PLDA handle on an sm_100 device");
-  KTF_CHECK_ARG(n_enroll >= 0 && n_enroll < (1LL << 32), "ktf_plda_score_asnorm_topk: n_enroll must be in 0 .. 2^32 - 1");
-  if (n_test <= 0) return KTF_OK;
-  KTF_CHECK_ARG(u_test_dev && test_mean_dev && test_std_dev && scores_dev && index_dev &&
-                    (n_enroll == 0 || (u_enroll_dev && enroll_mean_dev && enroll_std_dev)),
-                "ktf_plda_score_asnorm_topk: null argument");
   const AsnormStats s{test_mean_dev, test_std_dev, enroll_mean_dev, enroll_std_dev};
-  return score_tc_topk(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, k, scores_dev,
-                       (long long*)index_dev, (cudaStream_t)stream, &s);
+  return score_topk_checked("ktf_plda_score_asnorm_topk", KTF_PLDA_TOPK_MAX, "KTF_PLDA_TOPK_MAX", p, u_test_dev, n_test,
+                            u_enroll_dev, n_enroll, &s, k, scores_dev, index_dev, stream);
 }
 
 int ktf_topk_merge(const float* scores_in_dev, const int64_t* index_in_dev, int32_t num_lists, int64_t n_rows,
@@ -1022,18 +1007,8 @@ int ktf_topk_merge(const float* scores_in_dev, const int64_t* index_in_dev, int3
 
 int ktf_plda_score_topk_large(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,
                               int64_t n_enroll, int32_t k, float* scores_dev, int64_t* index_dev, void* stream) {
-  KTF_CHECK_ARG(k >= 1 && k <= KTF_PLDA_TOPK_LARGE_MAX,
-                "ktf_plda_score_topk_large: k = %d, must be 1 .. %d (KTF_PLDA_TOPK_LARGE_MAX)", k,
-                KTF_PLDA_TOPK_LARGE_MAX);
-  KTF_CHECK_ARG(p, "ktf_plda_score_topk_large: null handle");
-  KTF_CHECK_ARG(p->use_tc, "ktf_plda_score_topk_large needs a float32 PLDA handle on an sm_100 device");
-  KTF_CHECK_ARG(n_enroll >= 0 && n_enroll < (1LL << 32),
-                "ktf_plda_score_topk_large: n_enroll must be in 0 .. 2^32 - 1");
-  if (n_test <= 0) return KTF_OK;
-  KTF_CHECK_ARG(u_test_dev && scores_dev && index_dev && (u_enroll_dev || n_enroll == 0),
-                "ktf_plda_score_topk_large: null argument");
-  return score_tc_topk_large(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, k, scores_dev,
-                             (long long*)index_dev, (cudaStream_t)stream);
+  return score_topk_checked("ktf_plda_score_topk_large", KTF_PLDA_TOPK_LARGE_MAX, "KTF_PLDA_TOPK_LARGE_MAX", p,
+                            u_test_dev, n_test, u_enroll_dev, n_enroll, nullptr, k, scores_dev, index_dev, stream);
 }
 
 int ktf_plda_score_asnorm_topk_large(const ktf_plda* p, const void* u_test_dev, int64_t n_test,
@@ -1041,20 +1016,9 @@ int ktf_plda_score_asnorm_topk_large(const ktf_plda* p, const void* u_test_dev, 
                                      const float* test_std_dev, const float* enroll_mean_dev,
                                      const float* enroll_std_dev, int32_t k, float* scores_dev, int64_t* index_dev,
                                      void* stream) {
-  KTF_CHECK_ARG(k >= 1 && k <= KTF_PLDA_TOPK_LARGE_MAX,
-                "ktf_plda_score_asnorm_topk_large: k = %d, must be 1 .. %d (KTF_PLDA_TOPK_LARGE_MAX)", k,
-                KTF_PLDA_TOPK_LARGE_MAX);
-  KTF_CHECK_ARG(p, "ktf_plda_score_asnorm_topk_large: null handle");
-  KTF_CHECK_ARG(p->use_tc, "ktf_plda_score_asnorm_topk_large needs a float32 PLDA handle on an sm_100 device");
-  KTF_CHECK_ARG(n_enroll >= 0 && n_enroll < (1LL << 32),
-                "ktf_plda_score_asnorm_topk_large: n_enroll must be in 0 .. 2^32 - 1");
-  if (n_test <= 0) return KTF_OK;
-  KTF_CHECK_ARG(u_test_dev && test_mean_dev && test_std_dev && scores_dev && index_dev &&
-                    (n_enroll == 0 || (u_enroll_dev && enroll_mean_dev && enroll_std_dev)),
-                "ktf_plda_score_asnorm_topk_large: null argument");
   const AsnormStats s{test_mean_dev, test_std_dev, enroll_mean_dev, enroll_std_dev};
-  return score_tc_topk_large(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, k, scores_dev,
-                             (long long*)index_dev, (cudaStream_t)stream, &s);
+  return score_topk_checked("ktf_plda_score_asnorm_topk_large", KTF_PLDA_TOPK_LARGE_MAX, "KTF_PLDA_TOPK_LARGE_MAX", p,
+                            u_test_dev, n_test, u_enroll_dev, n_enroll, &s, k, scores_dev, index_dev, stream);
 }
 
 int ktf_topk_merge_large(const float* scores_in_dev, const int64_t* index_in_dev, int32_t num_lists, int64_t n_rows,
@@ -1077,7 +1041,8 @@ int ktf_plda_score(const ktf_plda* p, const void* u_test_dev, int64_t n_test, co
   if (n_test <= 0 || n_enroll <= 0) return KTF_OK;
   cudaStream_t st = (cudaStream_t)stream;
   if (p->use_tc)
-    return score_tc(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, scores_dev, ld, 0, st);
+    return score_tc(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll, nullptr,
+                    ScoreOut{ScoreOut::kMatrix, scores_dev, nullptr, ld, 0, 0}, st);
   return p->dtype_bytes == 4
              ? score_impl<float>(p, (const float*)u_test_dev, n_test, (const float*)u_enroll_dev, n_enroll,
                                  (float*)scores_dev, ld, st)

@@ -21,30 +21,39 @@ int affine_tc_forward(const ktf_affine* a, const float* x_dev, const int64_t* in
 // per-utterance column sums / sums of squares of an fp32 (rows, dim) matrix -> (batch, 2, dim)
 int stats_sums_f32(const float* y_dev, const int64_t* offsets_dev, int64_t batch, int dim, float* sums_dev,
                    cudaStream_t st);
-// tcgen05 engine as a plain "NT" GEMM: C[i, j] = sum_k A[i, k] * B[j, k] + row_add[i] + col_add[j];
-// A (m, K), B (n, K) row-major 16-bit (bf16, or fp16 when fp16 != 0), C fp32 or (c_bf16 != 0) bf16, row stride ldc
-// elements.  With `row_best` (m zero-initialised 64-bit keys) nothing is stored (C may be null): every row keeps its best
-// entry as a key -- order-preserving float bits << 32 | (0xffffffff - column), maximised atomically; the lowest column
-// wins a tie.
-int tc_gemm_nt(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
-               int fp16, const float* row_add, const float* col_add, void* C, long long ldc, int c_bf16,
-               cudaStream_t st, unsigned long long* row_best = nullptr);
-// The same GEMM with the score normalised in the epilogue (PLDA AS-norm): with s = (acc + col_add[j]) + A_i,
-// C[i, j] = (s - col_mean[j]) * col_half_inv[j] + (s - mu_t) * h_t, where row_norm holds one float4 (A_i, h_t, mu_t,
-// unused) per row and the h are 0.5 / sigma.  C fp32, or (c_bf16 != 0) the fp32 value rounded once to bf16.
-int tc_gemm_asnorm(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
-                   int fp16, const float* row_norm, const float* col_add, const float* col_half_inv,
-                   const float* col_mean, void* C, long long ldc, int c_bf16, cudaStream_t st);
-// The same GEMM reduced to the k (1..32) largest entries of every row, nothing else stored: partial lists
-// (num_lists, m, k) of fp32 values and columns, unordered, (-inf, -1) where a list has fewer than k entries; every column
-// is in exactly one list.  num_lists = tc_topk_lists(m, n, K) (0 when m or n is 0).
+// One score GEMM on the tcgen05 engine: C[i, j] = sum_k A[i, k] * B[j, k] + row_add[i] + col_add[j] (the score s),
+// A (m, K) and B (n, K) row-major 16-bit (bf16, or fp16 when fp16 != 0), K and both leading dimensions multiples of 8.
+struct TcScore {
+  const void* A;
+  long long m, lda;
+  const void* B;
+  long long n, ldb;
+  long long K;
+  int fp16;
+  const float* row_add;
+  const float* col_add;
+  // Optional AS-norm part (PLDA): with s = (acc + col_add[j]) + A_i, the value is
+  // (s - col_mean[j]) * col_half_inv[j] + (s - mu_t) * h_t, where row_add then holds one float4 (A_i, h_t, mu_t, unused)
+  // per row and the h are 0.5 / sigma.  Absent when col_half_inv is null.
+  const float* col_half_inv;
+  const float* col_mean;
+  // Exactly one output:
+  // - rows: C fp32 or (c_bf16 != 0) the fp32 value rounded once to bf16, row stride ldc elements;
+  // - row_best (raw value only; m zero-initialised 64-bit keys, C may be null): every row keeps its best entry as a key
+  //   -- order-preserving float bits << 32 | (0xffffffff - column), maximised atomically; the lowest column wins a tie;
+  // - top-k (part_score non-null, 1 <= k <= 32): the k largest values of every row as partial lists (num_lists, m, k)
+  //   of fp32 values and columns, unordered, (-inf, -1) where a list has fewer than k entries; every column is in
+  //   exactly one list, num_lists = tc_topk_lists(m, n, K) (0 when m or n is 0).  AS-norm NaN and -inf values are
+  //   never listed.
+  // Every value is bit-equal whichever output carries it.
+  void* C;
+  long long ldc;
+  int c_bf16;
+  unsigned long long* row_best;
+  int k;
+  float* part_score;
+  long long* part_index;
+};
+int tc_gemm_score(const TcScore& s, cudaStream_t st);
 int tc_topk_lists(long long m, long long n, long long K);
-int tc_gemm_topk(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
-                 int fp16, const float* row_add, const float* col_add, int k, float* part_score, long long* part_index,
-                 cudaStream_t st);
-// tc_gemm_topk over the normalised value of tc_gemm_asnorm (same partial lists, same num_lists): every listed value is
-// bit-equal to its tc_gemm_asnorm entry; NaN and -inf values are never listed.
-int tc_gemm_asnorm_topk(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
-                        int fp16, const float* row_norm, const float* col_add, const float* col_half_inv,
-                        const float* col_mean, int k, float* part_score, long long* part_index, cudaStream_t st);
 }  // namespace ktf

@@ -72,7 +72,7 @@ constexpr int kNumModes = 10;
 constexpr int kModeTopkCap[kNumModes] = {0, 0, 0, 8, 16, 32, 8, 16, 32, 0};   // top-k list capacity, 0 = rows stored
 constexpr bool kModeIsNorm[kNumModes] = {0, 0, 1, 0, 0, 0, 1, 1, 1, 1};      // AS-norm value (kEpiNorm)
 constexpr bool kModeIsBf16[kNumModes] = {1, 0, 0, 0, 0, 0, 0, 0, 0, 1};      // rows stored as bf16
-// TcArgs::row_best is tested at run time (only tc_gemm_nt's fp32 form passes it).  The AS-norm modes after kModeTopk32
+// TcArgs::row_best is tested at run time (only tc_gemm_score's raw fp32 rows pass it).  The AS-norm modes after kModeTopk32
 // compile the test out: in kModeNormBf16 at 16 epilogue warps the dead path costs 8 bytes of spills.
 constexpr bool kModeRowBest[kNumModes] = {1, 1, 1, 1, 1, 1, 0, 0, 0, 0};
 constexpr int topk_cap(int mode) { return kModeTopkCap[mode]; }
@@ -2103,61 +2103,6 @@ int affine_tc_forward(const ktf_affine* a, const float* x_dev, const int64_t* in
   return KTF_OK;
 }
 
-// C[i, j] = sum_k A[i, k] * B[j, k] + row_add[i] + col_add[j], A (m, K) and B (n, K) row-major 16-bit
-// (bf16 or fp16), C fp32 with row stride ldc.  K and both leading dimensions must be multiples of 8.
-// Operand maps and arguments of a row-storing NT GEMM on the pair kernel (tc_gemm_nt, tc_gemm_asnorm).
-static int nt_setup(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
-                    int fp16, const float* row_add, const float* col_add, void* C, long long ldc, int c_bf16,
-                    CUtensorMap* tmA, CUtensorMap* tmBh, TcArgs* out) {
-  int rc = check_arch();
-  if (rc != KTF_OK) return rc;
-  // B in 128-row boxes: each CTA of a pair loads half of the tile's 256 columns
-  if ((rc = encode_map(tmA, A, (unsigned long long)K, (unsigned long long)m, (unsigned long long)lda, BK, BM)) != KTF_OK)
-    return rc;
-  if ((rc = encode_map(tmBh, B, (unsigned long long)K, (unsigned long long)n, (unsigned long long)ldb, BK, BN / 2)) != KTF_OK)
-    return rc;
-  TcArgs args{};
-  args.num_taps = 1;
-  args.kblocks_per_tap = (int)((K + BK - 1) / BK);
-  args.fp16 = fp16;
-  args.m_rows = m;
-  args.n_rows = n;
-  args.bias = col_add;
-  args.row_add = row_add;
-  args.out = C;
-  args.out_ld = ldc;
-  // streaming output (PLDA: the score matrix), operands re-read by every tile: see TcArgs::l2_stream_out
-  args.l2_stream_out = ((double)m * (double)n * (c_bf16 ? 2.0 : 4.0) > 64e6) ? 1 : 0;
-  if (const char* e = getenv("KTF_TC_L2_HINTS")) args.l2_stream_out = atoi(e);
-  args.group_m = (n + BN - 1) / BN > 8 ? 32 : 0;     // (measured at 50 000^2: 1 -> 2.77, 8 -> 2.61, 16 -> 2.54, 32 -> 2.47-2.51, 64 -> 2.65 ms)
-  if (const char* e = getenv("KTF_TC_GROUP_M")) args.group_m = atoi(e);
-  *out = args;
-  return KTF_OK;
-}
-
-int tc_gemm_nt(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
-               int fp16, const float* row_add, const float* col_add, void* C, long long ldc, int c_bf16,
-               cudaStream_t st, unsigned long long* row_best) {
-  CUtensorMap tmA, tmBh;
-  TcArgs args;
-  int rc = nt_setup(A, m, lda, B, n, ldb, K, fp16, row_add, col_add, C, ldc, c_bf16, &tmA, &tmBh, &args);
-  if (rc != KTF_OK) return rc;
-  args.row_best = row_best;
-  return c_bf16 ? launch_gemm_pair<kModeBf16>(tmA, tmBh, args, st) : launch_gemm_pair<kModeF32>(tmA, tmBh, args, st);
-}
-
-int tc_gemm_asnorm(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
-                   int fp16, const float* row_norm, const float* col_add, const float* col_half_inv,
-                   const float* col_mean, void* C, long long ldc, int c_bf16, cudaStream_t st) {
-  CUtensorMap tmA, tmBh;
-  TcArgs args;
-  int rc = nt_setup(A, m, lda, B, n, ldb, K, fp16, row_norm, col_add, C, ldc, c_bf16, &tmA, &tmBh, &args);
-  if (rc != KTF_OK) return rc;
-  args.scale = col_half_inv;
-  args.offset = col_mean;
-  return c_bf16 ? launch_gemm_pair<kModeNormBf16>(tmA, tmBh, args, st) : launch_gemm_pair<kModeNorm>(tmA, tmBh, args, st);
-}
-
 }  // namespace ktf
 
 namespace {
@@ -2190,6 +2135,24 @@ TopkPlan topk_plan(long long m, long long n, long long K) {
   return pl;
 }
 
+// The pair-kernel mode of a score: from its value (raw or AS-norm), its output (rows, row_best or top-k), the list
+// capacity k needs and the row format.  -1: no mode computes it (AS-norm with row_best, k outside 1..32).
+int score_mode(const ktf::TcScore& s) {
+  const bool norm = s.col_half_inv != nullptr;
+  if (s.part_score != nullptr) {
+    if (s.k < 1 || s.k > 32) return -1;
+    const int cap = s.k <= 8 ? 0 : s.k <= 16 ? 1 : 2;
+    return (norm ? kModeNormTopk8 : kModeTopk8) + cap;
+  }
+  if (norm) return s.row_best != nullptr ? -1 : s.c_bf16 ? kModeNormBf16 : kModeNorm;
+  return s.c_bf16 ? kModeBf16 : kModeF32;
+}
+
+template <int MODE>
+int launch_score(int ew, const CUtensorMap& tmA, const CUtensorMap& tmBh, const TcArgs& args, cudaStream_t st) {
+  return ew == 16 ? launch_gemm_pair_ew<MODE, 16>(tmA, tmBh, args, st) : launch_gemm_pair_ew<MODE, 8>(tmA, tmBh, args, st);
+}
+
 }  // namespace
 
 namespace ktf {
@@ -2200,71 +2163,68 @@ int tc_topk_lists(long long m, long long n, long long K) {
   return pl.splits * (pl.ew / 4);
 }
 
-// Operand maps, arguments and plan of a top-k GEMM (tc_gemm_topk, tc_gemm_asnorm_topk); KTF_OK with pl->splits = 0 when
-// there is nothing to do (m or n is 0).
-static int topk_setup(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
-                      int fp16, const float* row_add, const float* col_add, int k, float* part_score,
-                      long long* part_index, CUtensorMap* tmA, CUtensorMap* tmBh, TcArgs* out, TopkPlan* pl) {
-  *pl = TopkPlan{0, 0, 0};
+int tc_gemm_score(const TcScore& s, cudaStream_t st) {
   int rc = check_arch();
   if (rc != KTF_OK) return rc;
-  if (m <= 0 || n <= 0) return KTF_OK;
-  if (k < 1 || k > 32) {
-    ktf::set_error("tc_gemm_topk: k = %d outside 1..32", k);
+  const bool topk = s.part_score != nullptr;
+  if (topk && (s.m <= 0 || s.n <= 0)) return KTF_OK;
+  const int mode = score_mode(s);
+  if (mode < 0) {
+    ktf::set_error("tc_gemm_score: no pair-kernel mode for this score (AS-norm with row_best, or k = %d outside 1..32)",
+                   s.k);
     return KTF_EINVAL;
   }
-  if ((rc = encode_map(tmA, A, (unsigned long long)K, (unsigned long long)m, (unsigned long long)lda, BK, BM)) != KTF_OK)
+  CUtensorMap tmA, tmBh;
+  // B in 128-row boxes: each CTA of a pair loads half of the tile's 256 columns
+  if ((rc = encode_map(&tmA, s.A, (unsigned long long)s.K, (unsigned long long)s.m, (unsigned long long)s.lda, BK, BM)) !=
+      KTF_OK)
     return rc;
-  if ((rc = encode_map(tmBh, B, (unsigned long long)K, (unsigned long long)n, (unsigned long long)ldb, BK, BN / 2)) != KTF_OK)
+  if ((rc = encode_map(&tmBh, s.B, (unsigned long long)s.K, (unsigned long long)s.n, (unsigned long long)s.ldb, BK,
+                       BN / 2)) != KTF_OK)
     return rc;
-  *pl = topk_plan(m, n, K);
   TcArgs args{};
   args.num_taps = 1;
-  args.kblocks_per_tap = (int)((K + BK - 1) / BK);
-  args.fp16 = fp16;
-  args.m_rows = m;
-  args.n_rows = n;
-  args.bias = col_add;
-  args.row_add = row_add;
-  args.topk_k = k;
-  args.topk_unit_tiles = pl->unit_tiles;
-  args.topk_score = part_score;
-  args.topk_index = part_index;
-  *out = args;
-  return KTF_OK;
+  args.kblocks_per_tap = (int)((s.K + BK - 1) / BK);
+  args.fp16 = s.fp16;
+  args.m_rows = s.m;
+  args.n_rows = s.n;
+  args.bias = s.col_add;
+  args.row_add = s.row_add;
+  args.scale = s.col_half_inv;
+  args.offset = s.col_mean;
+  int ew;
+  if (topk) {
+    const TopkPlan pl = topk_plan(s.m, s.n, s.K);
+    ew = pl.ew;
+    args.topk_k = s.k;
+    args.topk_unit_tiles = pl.unit_tiles;
+    args.topk_score = s.part_score;
+    args.topk_index = s.part_index;
+  } else {
+    ew = pair_epi_warps(args.kblocks_per_tap);
+    args.out = s.C;
+    args.out_ld = s.ldc;
+    args.row_best = s.row_best;
+    // streaming output (PLDA: the score matrix), operands re-read by every tile: see TcArgs::l2_stream_out
+    args.l2_stream_out = ((double)s.m * (double)s.n * (s.c_bf16 ? 2.0 : 4.0) > 64e6) ? 1 : 0;
+    if (const char* e = getenv("KTF_TC_L2_HINTS")) args.l2_stream_out = atoi(e);
+    args.group_m = (s.n + BN - 1) / BN > 8 ? 32 : 0;     // (measured at 50 000^2: 1 -> 2.77, 8 -> 2.61, 16 -> 2.54, 32 -> 2.47-2.51, 64 -> 2.65 ms)
+    if (const char* e = getenv("KTF_TC_GROUP_M")) args.group_m = atoi(e);
+  }
+  switch (mode) {
+    case kModeBf16: return launch_score<kModeBf16>(ew, tmA, tmBh, args, st);
+    case kModeF32: return launch_score<kModeF32>(ew, tmA, tmBh, args, st);
+    case kModeNorm: return launch_score<kModeNorm>(ew, tmA, tmBh, args, st);
+    case kModeTopk8: return launch_score<kModeTopk8>(ew, tmA, tmBh, args, st);
+    case kModeTopk16: return launch_score<kModeTopk16>(ew, tmA, tmBh, args, st);
+    case kModeTopk32: return launch_score<kModeTopk32>(ew, tmA, tmBh, args, st);
+    case kModeNormTopk8: return launch_score<kModeNormTopk8>(ew, tmA, tmBh, args, st);
+    case kModeNormTopk16: return launch_score<kModeNormTopk16>(ew, tmA, tmBh, args, st);
+    case kModeNormTopk32: return launch_score<kModeNormTopk32>(ew, tmA, tmBh, args, st);
+    case kModeNormBf16: return launch_score<kModeNormBf16>(ew, tmA, tmBh, args, st);
+  }
+  return KTF_EINVAL;
 }
-
-// the list capacity (8, 16, 32) and epilogue warp count of the plan pick the instantiation
-#define KTF_TOPK_LAUNCH(MODE_)                                                         \
-  (pl.ew == 16 ? launch_gemm_pair_ew<MODE_, 16>(tmA, tmBh, args, st)                   \
-               : launch_gemm_pair_ew<MODE_, 8>(tmA, tmBh, args, st))
-
-int tc_gemm_topk(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
-                 int fp16, const float* row_add, const float* col_add, int k, float* part_score, long long* part_index,
-                 cudaStream_t st) {
-  CUtensorMap tmA, tmBh;
-  TcArgs args;
-  TopkPlan pl;
-  int rc = topk_setup(A, m, lda, B, n, ldb, K, fp16, row_add, col_add, k, part_score, part_index, &tmA, &tmBh, &args, &pl);
-  if (rc != KTF_OK || pl.splits == 0) return rc;
-  return k <= 8 ? KTF_TOPK_LAUNCH(kModeTopk8) : k <= 16 ? KTF_TOPK_LAUNCH(kModeTopk16) : KTF_TOPK_LAUNCH(kModeTopk32);
-}
-
-int tc_gemm_asnorm_topk(const void* A, long long m, long long lda, const void* B, long long n, long long ldb, long long K,
-                        int fp16, const float* row_norm, const float* col_add, const float* col_half_inv,
-                        const float* col_mean, int k, float* part_score, long long* part_index, cudaStream_t st) {
-  CUtensorMap tmA, tmBh;
-  TcArgs args;
-  TopkPlan pl;
-  int rc = topk_setup(A, m, lda, B, n, ldb, K, fp16, row_norm, col_add, k, part_score, part_index, &tmA, &tmBh, &args, &pl);
-  if (rc != KTF_OK || pl.splits == 0) return rc;
-  args.scale = col_half_inv;
-  args.offset = col_mean;
-  return k <= 8    ? KTF_TOPK_LAUNCH(kModeNormTopk8)
-         : k <= 16 ? KTF_TOPK_LAUNCH(kModeNormTopk16)
-                   : KTF_TOPK_LAUNCH(kModeNormTopk32);
-}
-#undef KTF_TOPK_LAUNCH
 
 }  // namespace ktf
 

@@ -98,6 +98,10 @@ class PLDA(Layer):
         except Exception:
             pass
 
+    def _need_float32(self, caller):
+        if self.paramDtype != np.float32:
+            raise ValueError(f"{caller} needs a float32 PLDA layer")
+
     @property
     def torchDtype(self):
         return torch.float64 if self.paramDtype == np.float64 else torch.float32
@@ -133,8 +137,7 @@ class PLDA(Layer):
         scores[i] = max_j LLR(test i | enrolled j) -- the entry of `logLikelihoodRatio` (plda.py:215-245), same
         arithmetic -- without writing the (n_test, n_enroll) matrix (SURVEY 8f rank 3, top-k = 1; float32 layers only).
         The lowest index wins a tie."""
-        if self.paramDtype != np.float32:
-            raise ValueError("bestMatch needs a float32 PLDA layer")
+        self._need_float32("bestMatch")
         u_enroll = u_test if u_enroll is None else u_enroll
         nt, ne = u_test.shape[0], u_enroll.shape[0]
         best = torch.empty((nt,), device=u_test.device, dtype=torch.float32)
@@ -149,16 +152,8 @@ class PLDA(Layer):
         columns, best first, the lower index first on equal scores -- the first k of a stable descending sort of the row
         -- without writing the (n_test, n_enroll) matrix (float32 layers only).  Past the last enrolled vector the
         entries are (-inf, -1).  `u_enroll=None` scores the set against itself."""
-        if self.paramDtype != np.float32:
-            raise ValueError("bestMatches needs a float32 PLDA layer")
-        k = int(k)
-        u_enroll = u_test if u_enroll is None else u_enroll
-        nt, ne = u_test.shape[0], u_enroll.shape[0]
-        scores = torch.empty((nt, max(k, 0)), device=u_test.device, dtype=torch.float32)
-        index = torch.empty((nt, max(k, 0)), device=u_test.device, dtype=torch.int64)
-        N.check(N.lib().ktf_plda_score_topk(self.handle_for(num_examples), T.ptr(u_test), nt, T.ptr(u_enroll), ne, k,
-                                            T.ptr(scores), T.ptr(index), T.stream_ptr()))
-        return scores, index
+        return self._bestMatches("bestMatches", N.lib().ktf_plda_score_topk, N.KTF_PLDA_TOPK_MAX, u_test, u_enroll, k,
+                                 None, num_examples)
 
     def bestMatchesLarge(self, u_test, u_enroll=None, *, k, num_examples=1.0):
         """`bestMatches` for 1 <= k <= 1024 (shortlists, recall@100, neighbour graphs): (scores (n_test, k) float32,
@@ -167,17 +162,25 @@ class PLDA(Layer):
         vector, without the (n_test, n_enroll) matrix in memory: k <= 32 runs `bestMatches`, larger k scores row chunks
         of at most 128 MB and selects each while it is in L2.  `u_enroll=None` scores the set against itself.  float32
         layers only."""
-        if self.paramDtype != np.float32:
-            raise ValueError("bestMatchesLarge needs a float32 PLDA layer")
+        return self._bestMatches("bestMatchesLarge", N.lib().ktf_plda_score_topk_large, N.KTF_PLDA_TOPK_LARGE_MAX,
+                                 u_test, u_enroll, k, None, num_examples)
+
+    def _bestMatches(self, caller, c_fn, k_max, u_test, u_enroll, k, stats, num_examples):
+        """The k best enrolled vectors per test vector from the native k-best call `c_fn` (1 <= k <= `k_max`): of the
+        raw scores, or with `stats` = (u_cohort, top_n, test_stats, enroll_stats) of the AS-norm scores, the statistics
+        resolved as in `asNorm`."""
+        self._need_float32(caller)
         k = int(k)
-        if not 1 <= k <= N.KTF_PLDA_TOPK_LARGE_MAX:
-            raise ValueError(f"k = {k}, must be 1 .. {N.KTF_PLDA_TOPK_LARGE_MAX}")
+        if not 1 <= k <= k_max:
+            raise ValueError(f"k = {k}, must be 1 .. {k_max}")
         u_enroll = u_test if u_enroll is None else u_enroll
         nt, ne = u_test.shape[0], u_enroll.shape[0]
+        if stats is not None:
+            stats = self._asNormStats(u_test, u_enroll, *stats, num_examples, caller)
         scores = torch.empty((nt, k), device=u_test.device, dtype=torch.float32)
         index = torch.empty((nt, k), device=u_test.device, dtype=torch.int64)
-        N.check(N.lib().ktf_plda_score_topk_large(self.handle_for(num_examples), T.ptr(u_test), nt, T.ptr(u_enroll),
-                                                  ne, k, T.ptr(scores), T.ptr(index), T.stream_ptr()))
+        N.check(c_fn(self.handle_for(num_examples), T.ptr(u_test), nt, T.ptr(u_enroll), ne,
+                     *(T.ptr(t) for t in (stats or ())), k, T.ptr(scores), T.ptr(index), T.stream_ptr()))
         return scores, index
 
     def cohortStats(self, u, u_cohort, *, top_n, role="test", num_examples=1.0):
@@ -187,8 +190,7 @@ class PLDA(Layer):
         `logLikelihoodRatio(u_cohort, u, num_examples=num_examples)`.  The selection is exact (bit-equal scores) and
         the statistics are evaluated in float64 and rounded once; a vector's statistics do not depend on the other
         vectors of the call.  2 <= top_n <= len(u_cohort); float32 layers only."""
-        if self.paramDtype != np.float32:
-            raise ValueError("cohortStats needs a float32 PLDA layer")
+        self._need_float32("cohortStats")
         if role not in ("test", "enrolled"):
             raise ValueError(f"role must be 'test' or 'enrolled', got {role!r}")
         n = u.shape[0]
@@ -228,8 +230,7 @@ class PLDA(Layer):
         (test role for u_test, enrolled role with `num_examples` for u_enroll).  `u_enroll=None` scores the set against
         itself.  `score_dtype=torch.bfloat16` (or a bfloat16 `out`) writes the same float32 value rounded once to
         bfloat16: half the bytes of the matrix.  float32 layers only."""
-        if self.paramDtype != np.float32:
-            raise ValueError("asNorm needs a float32 PLDA layer")
+        self._need_float32("asNorm")
         compact = score_dtype is torch.bfloat16 or (out is not None and out.dtype is torch.bfloat16)
         if score_dtype is not None and not compact and score_dtype != torch.float32:
             raise ValueError("score_dtype must be torch.float32 or torch.bfloat16")
@@ -254,21 +255,8 @@ class PLDA(Layer):
         deviation of 0 can give them) are never listed; past the last listed column the entries are (-inf, -1).  The
         statistics are given or computed as in `asNorm`; `u_enroll=None` scores the set against itself.  float32 layers
         only."""
-        if self.paramDtype != np.float32:
-            raise ValueError("asNormBestMatches needs a float32 PLDA layer")
-        k = int(k)
-        if not 1 <= k <= N.KTF_PLDA_TOPK_MAX:
-            raise ValueError(f"k = {k}, must be 1 .. {N.KTF_PLDA_TOPK_MAX}")
-        u_enroll = u_test if u_enroll is None else u_enroll
-        nt, ne = u_test.shape[0], u_enroll.shape[0]
-        stats = self._asNormStats(u_test, u_enroll, u_cohort, top_n, test_stats, enroll_stats, num_examples,
-                                  "asNormBestMatches")
-        scores = torch.empty((nt, k), device=u_test.device, dtype=torch.float32)
-        index = torch.empty((nt, k), device=u_test.device, dtype=torch.int64)
-        N.check(N.lib().ktf_plda_score_asnorm_topk(self.handle_for(num_examples), T.ptr(u_test), nt, T.ptr(u_enroll),
-                                                   ne, *(T.ptr(t) for t in stats), k, T.ptr(scores), T.ptr(index),
-                                                   T.stream_ptr()))
-        return scores, index
+        return self._bestMatches("asNormBestMatches", N.lib().ktf_plda_score_asnorm_topk, N.KTF_PLDA_TOPK_MAX, u_test,
+                                 u_enroll, k, (u_cohort, top_n, test_stats, enroll_stats), num_examples)
 
     def asNormBestMatchesLarge(self, u_test, u_enroll=None, u_cohort=None, *, k, top_n=None, test_stats=None,
                                enroll_stats=None, num_examples=1.0):
@@ -278,21 +266,9 @@ class PLDA(Layer):
         k <= 32 runs `asNormBestMatches`, larger k normalises row chunks of at most 128 MB and selects each while it is in
         L2.  The statistics are given or computed as in `asNorm`; `u_enroll=None` scores the set against itself.  float32
         layers only."""
-        if self.paramDtype != np.float32:
-            raise ValueError("asNormBestMatchesLarge needs a float32 PLDA layer")
-        k = int(k)
-        if not 1 <= k <= N.KTF_PLDA_TOPK_LARGE_MAX:
-            raise ValueError(f"k = {k}, must be 1 .. {N.KTF_PLDA_TOPK_LARGE_MAX}")
-        u_enroll = u_test if u_enroll is None else u_enroll
-        nt, ne = u_test.shape[0], u_enroll.shape[0]
-        stats = self._asNormStats(u_test, u_enroll, u_cohort, top_n, test_stats, enroll_stats, num_examples,
-                                  "asNormBestMatchesLarge")
-        scores = torch.empty((nt, k), device=u_test.device, dtype=torch.float32)
-        index = torch.empty((nt, k), device=u_test.device, dtype=torch.int64)
-        N.check(N.lib().ktf_plda_score_asnorm_topk_large(self.handle_for(num_examples), T.ptr(u_test), nt,
-                                                         T.ptr(u_enroll), ne, *(T.ptr(t) for t in stats), k,
-                                                         T.ptr(scores), T.ptr(index), T.stream_ptr()))
-        return scores, index
+        return self._bestMatches("asNormBestMatchesLarge", N.lib().ktf_plda_score_asnorm_topk_large,
+                                 N.KTF_PLDA_TOPK_LARGE_MAX, u_test, u_enroll, k, (u_cohort, top_n, test_stats,
+                                                                                  enroll_stats), num_examples)
 
     def call(self, inputs):
         x = T.as_device(inputs)

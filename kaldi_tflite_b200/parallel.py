@@ -130,11 +130,8 @@ def plda_score_sharded(plda, x_test_local, x_enroll_local, test_counts=None, out
         return plda.logLikelihoodRatio(u_test_local, u_enroll_local, out=out), u_test_local
     u_all, offs, works = exchange_test_vectors(u_test_local, test_counts)
     u_enroll_local = plda.transformVector(x_enroll_local.contiguous())
-    if out is None:
-        # row pitch padded to 16 bytes: the score kernel's boxed (TMA) stores need an aligned pitch
-        ne = u_enroll_local.shape[0]
-        out = torch.empty((offs[-1], (ne + 7) // 8 * 8), device=u_test_local.device, dtype=u_test_local.dtype)[:, :ne]
-    scores = out
+    scores = out if out is not None else _score_block(offs[-1], u_enroll_local.shape[0], u_test_local.dtype,
+                                                      u_test_local.device)
     if all(isinstance(wk, _Gathered) for wk in works):
         lo, hi = offs[rank], offs[rank + 1]
         if hi > lo:                           # local rows: no need to wait for anybody
@@ -153,6 +150,19 @@ def plda_score_sharded(plda, x_test_local, x_enroll_local, test_counts=None, out
     return scores, u_all
 
 
+def _score_block(n_test, n_enroll, dtype, device):
+    """An (n_test, n_enroll) score block whose row pitch is padded to 8 elements (32 B of float32, 16 B of bfloat16):
+    the score kernel's boxed (TMA) stores need a 16-byte aligned pitch."""
+    return torch.empty((n_test, (n_enroll + 7) // 8 * 8), device=device, dtype=dtype)[:, :n_enroll]
+
+
+def _wait_all(works):
+    """Makes the current stream wait for every block of an `exchange_test_vectors` exchange."""
+    for wk in works:
+        if wk is not None:
+            wk.wait()
+
+
 def plda_best_matches_sharded(plda, x_test_local, x_enroll_local, k, test_counts=None):
     """
     Sharded k-best trial search: `PLDA.bestMatches` of ALL test vectors against ALL enrolled vectors, where each rank
@@ -162,17 +172,7 @@ def plda_best_matches_sharded(plda, x_test_local, x_enroll_local, k, test_counts
     exchange these (n_test, k) lists once, and `ktf_topk_merge` reduces them on every rank.  Returns (scores, indexes),
     (n_test, k) each, test rows ordered by rank -- equal to `bestMatches` on the whole set.
     """
-    _, w = world()
-    u_test_local = plda.transformVector(x_test_local.contiguous())
-    if w == 1:
-        return plda.bestMatches(u_test_local, plda.transformVector(x_enroll_local.contiguous()), k=k)
-    u_all, offs, works = exchange_test_vectors(u_test_local, test_counts)
-    u_enroll_local = plda.transformVector(x_enroll_local.contiguous())
-    for wk in works:
-        if wk is not None:
-            wk.wait()
-    scores, index = plda.bestMatches(u_all, u_enroll_local, k=k)
-    return _merge_shard_lists(scores, index, u_enroll_local.shape[0], k, _native.lib().ktf_topk_merge)
+    return _best_matches_sharded(plda, x_test_local, x_enroll_local, k, test_counts, large=False)
 
 
 def plda_best_matches_large_sharded(plda, x_test_local, x_enroll_local, k, test_counts=None):
@@ -182,17 +182,34 @@ def plda_best_matches_large_sharded(plda, x_test_local, x_enroll_local, k, test_
     world_size x n_test x 2k int64 on every rank: 16 KB per test row and rank at k = 1024.  Returns (scores, indexes),
     (n_test, k) each, test rows ordered by rank -- equal to `bestMatchesLarge` on the whole set.
     """
+    return _best_matches_sharded(plda, x_test_local, x_enroll_local, k, test_counts, large=True)
+
+
+def _best_matches_sharded(plda, x_test_local, x_enroll_local, k, test_counts, *, large, asnorm=None):
+    """The sharded k-best search of the four public functions: every rank lists the k best of its own enrolled shard
+    for ALL test rows (`PLDA.bestMatches`, or with `large` `bestMatchesLarge`; with `asnorm` = (u_cohort, top_n) their
+    AS-norm forms), then `_merge_shard_lists` merges the ranks' lists (`ktf_topk_merge`, or with `large`
+    `ktf_topk_merge_large`)."""
     _, w = world()
-    u_test_local = plda.transformVector(x_test_local.contiguous())
+    if asnorm is None:
+        u_test_local = plda.transformVector(x_test_local.contiguous())
+        if w == 1:
+            u_all, u_enroll_local = u_test_local, plda.transformVector(x_enroll_local.contiguous())
+        else:
+            u_all, _, works = exchange_test_vectors(u_test_local, test_counts)
+            u_enroll_local = plda.transformVector(x_enroll_local.contiguous())
+            _wait_all(works)
+        best = plda.bestMatchesLarge if large else plda.bestMatches
+        scores, index = best(u_all, u_enroll_local, k=k)
+    else:
+        u_all, t_stats, u_enroll_local, e_stats, _ = _asnorm_inputs_sharded(plda, x_test_local, x_enroll_local,
+                                                                            *asnorm, test_counts)
+        best = plda.asNormBestMatchesLarge if large else plda.asNormBestMatches
+        scores, index = best(u_all, u_enroll_local, k=k, test_stats=t_stats, enroll_stats=e_stats)
     if w == 1:
-        return plda.bestMatchesLarge(u_test_local, plda.transformVector(x_enroll_local.contiguous()), k=k)
-    u_all, offs, works = exchange_test_vectors(u_test_local, test_counts)
-    u_enroll_local = plda.transformVector(x_enroll_local.contiguous())
-    for wk in works:
-        if wk is not None:
-            wk.wait()
-    scores, index = plda.bestMatchesLarge(u_all, u_enroll_local, k=k)
-    return _merge_shard_lists(scores, index, u_enroll_local.shape[0], k, _native.lib().ktf_topk_merge_large)
+        return scores, index
+    merge = _native.lib().ktf_topk_merge_large if large else _native.lib().ktf_topk_merge
+    return _merge_shard_lists(scores, index, u_enroll_local.shape[0], k, merge)
 
 
 def _merge_shard_lists(scores, index, n_enroll_local, k, merge):
@@ -234,9 +251,7 @@ def _asnorm_inputs_sharded(plda, x_test_local, x_enroll_local, u_cohort, top_n, 
     dim = u_test_local.shape[1]
     packed = torch.cat([u_test_local, t_mean[:, None], t_std[:, None]], dim=1)
     p_all, offs, works = exchange_test_vectors(packed, test_counts)
-    for wk in works:
-        if wk is not None:
-            wk.wait()
+    _wait_all(works)
     u_all = p_all[:, :dim].contiguous()
     t_stats = (p_all[:, dim].contiguous(), p_all[:, dim + 1].contiguous())
     return u_all, t_stats, u_enroll_local, e_stats, offs
@@ -256,11 +271,8 @@ def plda_asnorm_sharded(plda, x_test_local, x_enroll_local, u_cohort, top_n, tes
                                                                            u_cohort, top_n, test_counts)
     if w == 1:
         return plda.asNorm(u_all, u_enroll_local, test_stats=t_stats, enroll_stats=e_stats, score_dtype=score_dtype), u_all
-    ne = u_enroll_local.shape[0]
-    # row pitch padded to 16 bytes (8 elements: 32 B of float32, 16 B of bfloat16): the score kernel's boxed (TMA)
-    # stores need an aligned pitch
     dtype = torch.bfloat16 if score_dtype is torch.bfloat16 else torch.float32
-    out = torch.empty((offs[-1], (ne + 7) // 8 * 8), device=u_all.device, dtype=dtype)[:, :ne]
+    out = _score_block(offs[-1], u_enroll_local.shape[0], dtype, u_all.device)
     return plda.asNorm(u_all, u_enroll_local, test_stats=t_stats, enroll_stats=e_stats, out=out), u_all
 
 
@@ -272,13 +284,8 @@ def plda_asnorm_best_matches_sharded(plda, x_test_local, x_enroll_local, u_cohor
     the ranks then exchange and merge these lists as `plda_best_matches_sharded` does.  Returns (scores, indexes),
     (n_test, k) each, test rows ordered by rank.
     """
-    _, w = world()
-    u_all, t_stats, u_enroll_local, e_stats, _ = _asnorm_inputs_sharded(plda, x_test_local, x_enroll_local, u_cohort,
-                                                                        top_n, test_counts)
-    scores, index = plda.asNormBestMatches(u_all, u_enroll_local, k=k, test_stats=t_stats, enroll_stats=e_stats)
-    if w == 1:
-        return scores, index
-    return _merge_shard_lists(scores, index, u_enroll_local.shape[0], k, _native.lib().ktf_topk_merge)
+    return _best_matches_sharded(plda, x_test_local, x_enroll_local, k, test_counts, large=False,
+                                 asnorm=(u_cohort, top_n))
 
 
 def plda_asnorm_best_matches_large_sharded(plda, x_test_local, x_enroll_local, u_cohort, top_n, k, test_counts=None):
@@ -288,13 +295,8 @@ def plda_asnorm_best_matches_large_sharded(plda, x_test_local, x_enroll_local, u
     lists are world_size x n_test x 2k int64 on every rank: 16 KB per test row and rank at k = 1024.  Returns (scores,
     indexes), (n_test, k) each, test rows ordered by rank.
     """
-    _, w = world()
-    u_all, t_stats, u_enroll_local, e_stats, _ = _asnorm_inputs_sharded(plda, x_test_local, x_enroll_local, u_cohort,
-                                                                        top_n, test_counts)
-    scores, index = plda.asNormBestMatchesLarge(u_all, u_enroll_local, k=k, test_stats=t_stats, enroll_stats=e_stats)
-    if w == 1:
-        return scores, index
-    return _merge_shard_lists(scores, index, u_enroll_local.shape[0], k, _native.lib().ktf_topk_merge_large)
+    return _best_matches_sharded(plda, x_test_local, x_enroll_local, k, test_counts, large=True,
+                                 asnorm=(u_cohort, top_n))
 
 
 def stream_batches(fn, host_in, chunk, host_out=None, depth=3):

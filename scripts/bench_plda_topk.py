@@ -13,43 +13,11 @@ sort of the fp32 score matrix on a sample of rows.
 import argparse
 import json
 import os
-import subprocess
-import sys
 
 import numpy as np
 import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "tests"))
-
-import kaldi_tflite_b200 as ktf                     # noqa: E402
-from test_gpu_tdnn_plda import synthetic_plda       # noqa: E402
-
-DIM = 128
-
-
-def gpu_info():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"],
-                             capture_output=True, text=True, timeout=30).stdout.strip().splitlines()[0]
-        name, power = [s.strip() for s in out.split(",")]
-        return {"name": name, "power_limit": power}
-    except Exception as e:   # still record the torch device name
-        return {"name": torch.cuda.get_device_name(), "power_limit": f"unknown ({e})"}
-
-
-def time_ms(fn, steps, warmup):
-    for _ in range(warmup):
-        fn()
-    torch.cuda.synchronize()
-    t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    t0.record()
-    for _ in range(steps):
-        fn()
-    t1.record()
-    torch.cuda.synchronize()
-    return t0.elapsed_time(t1) / steps
+from plda_bench_common import DIM, ROOT, gpu_info, plda_setup, time_ms
 
 
 def main():
@@ -59,15 +27,8 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "plda_topk_bench.json"))
     args = ap.parse_args()
-    if not torch.cuda.is_available():
-        sys.exit("bench_plda_topk.py needs a CUDA device")
     n = args.n
-    mean, Tm, psi = synthetic_plda(DIM)
-    layer = ktf.layers.PLDA(DIM, mean, Tm, psi, dtype=np.float32, return_transformed=False)
-    g = torch.Generator(device="cuda").manual_seed(1234)
-    x = torch.randn((2 * n, DIM), generator=g, device="cuda")
-    u = layer.transformVector((x / x.norm(dim=1, keepdim=True) * DIM ** 0.5).contiguous())
-    ut, ue = u[:n].contiguous(), u[n:].contiguous()
+    layer, ut, ue, _ = plda_setup("bench_plda_topk.py", n)
     scores16 = torch.empty((n, n), device="cuda", dtype=torch.bfloat16)
 
     result = {"device": gpu_info(), "n_test": n, "n_enroll": n, "dim": DIM, "steps": args.steps, "warmup": args.warmup}

@@ -14,44 +14,12 @@ and checks every k against the stable sort of the float32 matrix on a sample of 
 import argparse
 import json
 import os
-import subprocess
-import sys
 
 import numpy as np
 import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "tests"))
-
-import kaldi_tflite_b200 as ktf                     # noqa: E402
-from test_gpu_tdnn_plda import synthetic_plda       # noqa: E402
-
-DIM = 128
+from plda_bench_common import DIM, ROOT, gpu_info, plda_setup, time_ms
 KS = (33, 64, 100, 256, 1024)
-
-
-def gpu_info():
-    try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"],
-                             capture_output=True, text=True, timeout=30).stdout.strip().splitlines()[0]
-        name, power = [s.strip() for s in out.split(",")]
-        return {"name": name, "power_limit": power}
-    except Exception as e:   # still record the torch device name
-        return {"name": torch.cuda.get_device_name(), "power_limit": f"unknown ({e})"}
-
-
-def time_ms(fn, steps, warmup):
-    for _ in range(warmup):
-        fn()
-    torch.cuda.synchronize()
-    t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    t0.record()
-    for _ in range(steps):
-        fn()
-    t1.record()
-    torch.cuda.synchronize()
-    return t0.elapsed_time(t1) / steps
 
 
 def main():
@@ -63,15 +31,8 @@ def main():
     ap.add_argument("--warmup", type=int, default=2)
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "plda_topk_large_bench.json"))
     args = ap.parse_args()
-    if not torch.cuda.is_available():
-        sys.exit("bench_plda_topk_large.py needs a CUDA device")
     n = args.n
-    mean, Tm, psi = synthetic_plda(DIM)
-    layer = ktf.layers.PLDA(DIM, mean, Tm, psi, dtype=np.float32, return_transformed=False)
-    g = torch.Generator(device="cuda").manual_seed(1234)
-    x = torch.randn((2 * n + args.cohort, DIM), generator=g, device="cuda")
-    u = layer.transformVector((x / x.norm(dim=1, keepdim=True) * DIM ** 0.5).contiguous())
-    ut, ue, uc = u[:n].contiguous(), u[n:2 * n].contiguous(), u[2 * n:].contiguous()
+    layer, ut, ue, uc = plda_setup("bench_plda_topk_large.py", n, args.cohort)
     ts = layer.cohortStats(ut, uc, top_n=args.top_n)
     es = layer.cohortStats(ue, uc, top_n=args.top_n, role="enrolled")
     st = (args.steps, args.warmup)

@@ -7,41 +7,25 @@ applied to the fp32 logLikelihoodRatio matrix and the returned statistics within
 """
 
 import ctypes
-import json
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
-from conftest import ROOT
 from oracle import ktf_oracle as O
+from plda_testlib import DIM, epilogue_warp_runs, ktf, plda_vectors, run_two_ranks  # noqa: F401
 from test_gpu_tdnn_plda import synthetic_plda
 
 pytestmark = pytest.mark.gpu
 
-DIM = 128
 NS = (1, 255, 257, 1037)
 TOP_NS = (2, 7, 100, 300, 1000)
 
 
 @pytest.fixture(scope="module")
-def ktf():
-    import kaldi_tflite_b200 as k
-    return k
-
-
-@pytest.fixture(scope="module")
 def setup(ktf):
     """A float32 layer, 1037 transformed test vectors and a 60 000-vector transformed cohort."""
-    import torch
-    mean, Tm, psi = synthetic_plda(DIM)
-    layer = ktf.layers.PLDA(DIM, mean, Tm, psi, dtype=np.float32, return_transformed=False)
-    g = torch.Generator(device="cuda").manual_seed(99)
-    x = torch.randn((1037 + 60000, DIM), generator=g, device="cuda")
-    u = layer.transformVector((x / x.norm(dim=1, keepdim=True) * DIM ** 0.5).contiguous())
-    return layer, u[:1037].contiguous(), u[1037:].contiguous()
+    layer, (ut, uc), _, _ = plda_vectors(ktf, (1037, 60000), 99, cuda_rng=True)
+    return layer, ut, uc
 
 
 def stats_with_nth(layer, u, uc, top_n, role, num_examples=1.0):
@@ -283,13 +267,6 @@ def test_cuda_graph_capture_and_replay(setup):
 
 
 _EW_CHILD = r"""
-import os, sys
-sys.path.insert(0, {root!r}); sys.path.insert(0, os.path.join({root!r}, "tests"))
-import numpy as np, torch
-import kaldi_tflite_b200 as ktf
-from test_gpu_tdnn_plda import synthetic_plda
-mean, Tm, psi = synthetic_plda(128)
-layer = ktf.layers.PLDA(128, mean, Tm, psi, dtype=np.float32, return_transformed=False)
 rng = np.random.default_rng(5)
 x = rng.standard_normal((1037 + 4099 + 5000, 128)).astype(np.float32)
 u = layer.transformVector(torch.from_numpy(x).cuda())
@@ -303,41 +280,19 @@ np.savez({path!r}, tm=ts[0].cpu().numpy(), ts=ts[1].cpu().numpy(), em=es[0].cpu(
 
 
 def test_independent_of_epilogue_warp_count(tmp_path):
-    res = {}
-    for ew in ("8", "16"):
-        path = str(tmp_path / f"ew{ew}.npz")
-        env = dict(os.environ, KTF_TC_PAIR_EPI_WARPS=ew)
-        p = subprocess.run([sys.executable, "-c", _EW_CHILD.format(root=ROOT, path=path)], env=env,
-                           stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=600)
-        assert p.returncode == 0, p.stdout
-        res[ew] = np.load(path)
+    res = epilogue_warp_runs(tmp_path, _EW_CHILD)
     for key in res["8"].files:
         assert np.array_equal(res["8"][key], res["16"][key]), key
 
 
-def _run_asnorm_shard_workers(tmp_path, backend):
-    worker = os.path.join(ROOT, "tests", "plda_asnorm_shard_worker.py")
-    port = 33600 + (os.getpid() % 2000) + (7 if backend == "nccl" else 0)
-    procs = []
-    for rank in range(2):
-        env = dict(os.environ, RANK=str(rank), WORLD_SIZE="2", MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-        procs.append(subprocess.Popen([sys.executable, worker, str(tmp_path), backend], env=env, stdout=subprocess.PIPE,
-                                      stderr=subprocess.STDOUT, text=True))
-    outs = [p.communicate(timeout=600)[0] for p in procs]
-    for rank, (p, o) in enumerate(zip(procs, outs)):
-        assert p.returncode == 0, f"rank {rank} failed:\n{o}"
-    for rank in range(2):
-        with open(os.path.join(str(tmp_path), f"asnorm_rank{rank}.json")) as f:
-            r = json.load(f)
-        assert r["ok"], r
-
-
 def test_sharded_two_ranks_gloo(tmp_path):
-    _run_asnorm_shard_workers(tmp_path, "gloo")
+    for r in run_two_ranks(tmp_path, "asnorm", "gloo"):
+        assert r["ok"], r
 
 
 def test_sharded_two_gpus_nccl(tmp_path):
     import torch
     if torch.cuda.device_count() < 2:
         pytest.skip("needs two GPUs")
-    _run_asnorm_shard_workers(tmp_path, "nccl")
+    for r in run_two_ranks(tmp_path, "asnorm", "nccl"):
+        assert r["ok"], r

@@ -11,21 +11,17 @@ The argument checks that need no device run everywhere; the rest is marked gpu.
 """
 
 import ctypes
-import json
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
-from conftest import ROOT
 from oracle import ktf_oracle as O
+from plda_testlib import DIM, check_equal, epilogue_warp_runs, expected_listed, ktf, listed_sort  # noqa: F401
+from plda_testlib import plda_vectors, run_two_ranks, stats
 from test_gpu_tdnn_plda import synthetic_plda
 
 gpu = pytest.mark.gpu
 
-DIM = 128
 KS = (1, 2, 7, 10, 16, 31, 32)
 
 
@@ -81,55 +77,10 @@ def test_python_argument_validation():
 # ---- on the GPU ----
 
 @pytest.fixture(scope="module")
-def ktf():
-    import kaldi_tflite_b200 as k
-    return k
-
-
-@pytest.fixture(scope="module")
 def setup(ktf):
     """A float32 layer, transformed vectors (1037 test, 4099 enrolled, a 2000-vector cohort) and the raw x-vectors."""
-    import torch
-    mean, Tm, psi = synthetic_plda(DIM)
-    layer = ktf.layers.PLDA(DIM, mean, Tm, psi, dtype=np.float32, return_transformed=False)
-    rng = np.random.default_rng(2025)
-    x = rng.standard_normal((1037 + 4099 + 2000, DIM))
-    x = (x / np.linalg.norm(x, axis=1, keepdims=True) * np.sqrt(DIM)).astype(np.float32)
-    u = layer.transformVector(torch.from_numpy(x).cuda())
-    return layer, u[:1037].contiguous(), u[1037:5136].contiguous(), u[5136:].contiguous()
-
-
-def expected(full, k):
-    """First k entries of a stable descending sort of every row without its NaN and -inf entries, padded with
-    (-inf, -1)."""
-    import torch
-    dropped = torch.isnan(full) | (full == float("-inf"))
-    s, i = torch.sort(full.masked_fill(dropped, float("-inf")), dim=1, descending=True, stable=True)
-    nt, ne = full.shape
-    m = min(k, ne)
-    want_s = torch.full((nt, k), float("-inf"), device=full.device, dtype=torch.float32)
-    want_i = torch.full((nt, k), -1, device=full.device, dtype=torch.int64)
-    want_s[:, :m] = s[:, :m]
-    want_i[:, :m] = i[:, :m]
-    kept = (~dropped).sum(dim=1, keepdim=True)
-    pad = torch.arange(k, device=full.device)[None, :] >= kept
-    want_s[pad] = float("-inf")
-    want_i[pad] = -1
-    return want_s, want_i
-
-
-def check_equal(got, want):
-    import torch
-    gs, gi = got
-    ws, wi = want
-    assert gs.dtype is torch.float32 and gi.dtype is torch.int64 and gs.shape == ws.shape and gi.shape == wi.shape
-    assert torch.equal(gi, wi), f"{int((gi != wi).sum())} of {gi.numel()} indexes differ"
-    assert torch.equal(gs, ws)
-
-
-def stats(layer, ut, ue, uc, top_n, num_examples=1.0):
-    return (layer.cohortStats(ut, uc, top_n=top_n),
-            layer.cohortStats(ue, uc, top_n=top_n, role="enrolled", num_examples=num_examples))
+    layer, (ut, ue, uc), _, _ = plda_vectors(ktf, (1037, 4099, 2000), 2025)
+    return layer, ut, ue, uc
 
 
 @gpu
@@ -142,10 +93,10 @@ def test_topk_equals_stable_sort_of_asnorm_matrix(setup, nt, ne, num_examples):
     full = layer.asNorm(ut[:nt], ue[:ne], test_stats=ts, enroll_stats=es, num_examples=num_examples)
     for k in KS:
         got = layer.asNormBestMatches(ut[:nt], ue[:ne], k=k, test_stats=ts, enroll_stats=es, num_examples=num_examples)
-        check_equal(got, expected(full, k))
+        check_equal(got, expected_listed(listed_sort(full), k))
     # statistics computed from the cohort inside the call
     got = layer.asNormBestMatches(ut[:nt], ue[:ne], uc, k=10, top_n=100, num_examples=num_examples)
-    check_equal(got, expected(full, 10))
+    check_equal(got, expected_listed(listed_sort(full), 10))
 
 
 @gpu
@@ -162,7 +113,7 @@ def test_topk_large(ktf, k):
     ts, es = stats(layer, ut, ue, uc, 300)
     got = layer.asNormBestMatches(ut, ue, k=k, test_stats=ts, enroll_stats=es)
     full = layer.asNorm(ut, ue, test_stats=ts, enroll_stats=es)
-    want = expected(full, k)
+    want = expected_listed(listed_sort(full), k)
     del full
     check_equal(got, want)
 
@@ -183,7 +134,8 @@ def test_ties_come_back_lowest_column_first(setup):
     row = full[0, cols]
     assert torch.equal(row, row[:1].expand(len(cols))), "copies of one vector must score equal"
     for k in (7, 16, 32):
-        check_equal(layer.asNormBestMatches(ut2, ue2, k=k, test_stats=ts, enroll_stats=es), expected(full, k))
+        check_equal(layer.asNormBestMatches(ut2, ue2, k=k, test_stats=ts, enroll_stats=es),
+                    expected_listed(listed_sort(full), k))
     s, i = layer.asNormBestMatches(ut2, ue2, k=32, test_stats=ts, enroll_stats=es)
     tied = [int(c) for c, v in zip(i[0].tolist(), s[0].tolist()) if v == float(row[0])]
     assert tied == cols
@@ -204,7 +156,7 @@ def test_sigma_zero_lists_plus_inf_only(setup):
     assert bool((full == float("inf")).any()) and bool((full == float("-inf")).any()) and bool(torch.isnan(full).any())
     for k in (1, 10, 32):
         s, i = layer.asNormBestMatches(ut[:nt], ue[:ne], k=k, test_stats=ts, enroll_stats=es)
-        check_equal((s, i), expected(full, k))
+        check_equal((s, i), expected_listed(listed_sort(full), k))
         assert not bool(torch.isnan(s).any()) and bool((s == float("inf")).any())
         listed = i >= 0
         assert not bool((s[listed] == float("-inf")).any())
@@ -218,7 +170,7 @@ def test_edges(setup, ktf):
     ts, es = stats(layer, ut[:40], ue[:5], uc, 100)
     # fewer enrolled vectors than k: (-inf, -1) after the last one
     s, i = layer.asNormBestMatches(ut[:40], ue[:5], k=9, test_stats=ts, enroll_stats=es)
-    check_equal((s, i), expected(layer.asNorm(ut[:40], ue[:5], test_stats=ts, enroll_stats=es), 9))
+    check_equal((s, i), expected_listed(listed_sort(layer.asNorm(ut[:40], ue[:5], test_stats=ts, enroll_stats=es)), 9))
     assert bool((i[:, 5:] == -1).all()) and bool((s[:, 5:] == float("-inf")).all())
     # no enrolled vector at all
     s, i = layer.asNormBestMatches(ut[:33], ue[:0], uc, k=4, top_n=100)
@@ -253,7 +205,8 @@ def test_edges(setup, ktf):
     ss = layer.cohortStats(ut, uc, top_n=100, role="enrolled", num_examples=3.0)
     st = layer.cohortStats(ut, uc, top_n=100)
     full = layer.asNorm(ut, test_stats=st, enroll_stats=ss, num_examples=3.0)
-    check_equal(layer.asNormBestMatches(ut, k=16, test_stats=st, enroll_stats=ss, num_examples=3.0), expected(full, 16))
+    check_equal(layer.asNormBestMatches(ut, k=16, test_stats=st, enroll_stats=ss, num_examples=3.0),
+                expected_listed(listed_sort(full), 16))
 
 
 @gpu
@@ -290,13 +243,6 @@ def test_against_float64_oracle(ktf):
 
 
 _EW_CHILD = r"""
-import os, sys
-sys.path.insert(0, {root!r}); sys.path.insert(0, os.path.join({root!r}, "tests"))
-import numpy as np, torch
-import kaldi_tflite_b200 as ktf
-from test_gpu_tdnn_plda import synthetic_plda
-mean, Tm, psi = synthetic_plda(128)
-layer = ktf.layers.PLDA(128, mean, Tm, psi, dtype=np.float32, return_transformed=False)
 rng = np.random.default_rng(6)
 x = rng.standard_normal((1037 + 4099 + 3000, 128)).astype(np.float32)
 u = layer.transformVector(torch.from_numpy(x).cuda())
@@ -312,14 +258,7 @@ np.savez({path!r}, **out)
 
 @gpu
 def test_independent_of_epilogue_warp_count(tmp_path):
-    res = {}
-    for ew in ("8", "16"):
-        path = str(tmp_path / f"ew{ew}.npz")
-        env = dict(os.environ, KTF_TC_PAIR_EPI_WARPS=ew)
-        p = subprocess.run([sys.executable, "-c", _EW_CHILD.format(root=ROOT, path=path)], env=env,
-                           stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=600)
-        assert p.returncode == 0, p.stdout
-        res[ew] = np.load(path)
+    res = epilogue_warp_runs(tmp_path, _EW_CHILD)
     for key in res["8"].files:
         assert np.array_equal(res["8"][key], res["16"][key]), key
 
@@ -376,26 +315,10 @@ def test_bf16_matrix_equals_rounded_float32(setup, ne):
         assert torch.equal(out.view(torch.int16), want.view(torch.int16)) and bool((buf[:, ne:] == 7.0).all())
 
 
-def _run_shard_workers(tmp_path, backend):
-    worker = os.path.join(ROOT, "tests", "plda_asnorm_topk_shard_worker.py")
-    port = 35700 + (os.getpid() % 2000) + (7 if backend == "nccl" else 0)
-    procs = []
-    for rank in range(2):
-        env = dict(os.environ, RANK=str(rank), WORLD_SIZE="2", MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-        procs.append(subprocess.Popen([sys.executable, worker, str(tmp_path), backend], env=env, stdout=subprocess.PIPE,
-                                      stderr=subprocess.STDOUT, text=True))
-    outs = [p.communicate(timeout=600)[0] for p in procs]
-    for rank, (p, o) in enumerate(zip(procs, outs)):
-        assert p.returncode == 0, f"rank {rank} failed:\n{o}"
-    for rank in range(2):
-        with open(os.path.join(str(tmp_path), f"asnorm_topk_rank{rank}.json")) as f:
-            r = json.load(f)
-        assert r["ok"], r
-
-
 @gpu
 def test_sharded_two_ranks_gloo(tmp_path):
-    _run_shard_workers(tmp_path, "gloo")
+    for r in run_two_ranks(tmp_path, "asnorm_topk", "gloo"):
+        assert r["ok"], r
 
 
 @gpu
@@ -403,4 +326,5 @@ def test_sharded_two_gpus_nccl(tmp_path):
     import torch
     if torch.cuda.device_count() < 2:
         pytest.skip("needs two GPUs")
-    _run_shard_workers(tmp_path, "nccl")
+    for r in run_two_ranks(tmp_path, "asnorm_topk", "nccl"):
+        assert r["ok"], r

@@ -5,63 +5,25 @@ stable descending sort of row i of the logLikelihoodRatio matrix, bit for bit, p
 """
 
 import ctypes
-import json
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
-from conftest import ROOT
 from oracle import ktf_oracle as O
+from plda_testlib import DIM, check_equal, epilogue_warp_runs, expected_sorted, ktf, plda_vectors  # noqa: F401
+from plda_testlib import run_two_ranks
 from test_gpu_tdnn_plda import synthetic_plda
 
 pytestmark = pytest.mark.gpu
 
-DIM = 128
 KS = (1, 2, 7, 10, 16, 31, 32)
-
-
-@pytest.fixture(scope="module")
-def ktf():
-    import kaldi_tflite_b200 as k
-    return k
 
 
 @pytest.fixture(scope="module")
 def setup(ktf):
     """A float32 layer and transformed vectors: 1037 test rows, 4099 enrolled rows."""
-    import torch
-    mean, Tm, psi = synthetic_plda(DIM)
-    layer = ktf.layers.PLDA(DIM, mean, Tm, psi, dtype=np.float32, return_transformed=False)
-    rng = np.random.default_rng(2024)
-    x = rng.standard_normal((1037 + 4099, DIM))
-    x = (x / np.linalg.norm(x, axis=1, keepdims=True) * np.sqrt(DIM)).astype(np.float32)
-    u = layer.transformVector(torch.from_numpy(x).cuda())
-    return layer, u[:1037].contiguous(), u[1037:].contiguous(), x, (mean, Tm, psi)
-
-
-def expected(full, k):
-    """First k entries of a stable descending sort of every row, padded with (-inf, -1)."""
-    import torch
-    s, i = torch.sort(full, dim=1, descending=True, stable=True)
-    nt, ne = full.shape
-    want_s = torch.full((nt, k), float("-inf"), device=full.device, dtype=torch.float32)
-    want_i = torch.full((nt, k), -1, device=full.device, dtype=torch.int64)
-    m = min(k, ne)
-    want_s[:, :m] = s[:, :m]
-    want_i[:, :m] = i[:, :m]
-    return want_s, want_i
-
-
-def check_equal(got, want):
-    import torch
-    gs, gi = got
-    ws, wi = want
-    assert gs.dtype is torch.float32 and gi.dtype is torch.int64 and gs.shape == ws.shape and gi.shape == wi.shape
-    assert torch.equal(gi, wi), f"{int((gi != wi).sum())} of {gi.numel()} indexes differ"
-    assert torch.equal(gs, ws)
+    layer, (ut, ue), x, params = plda_vectors(ktf, (1037, 4099), 2024)
+    return layer, ut, ue, x, params
 
 
 @pytest.mark.parametrize("nt", [1, 255, 257, 1037])
@@ -70,7 +32,7 @@ def test_topk_equals_stable_sort_of_score_matrix(setup, nt, ne):
     layer, ut, ue, _, _ = setup
     full = layer.logLikelihoodRatio(ut[:nt], ue[:ne])
     for k in KS:
-        check_equal(layer.bestMatches(ut[:nt], ue[:ne], k=k), expected(full, k))
+        check_equal(layer.bestMatches(ut[:nt], ue[:ne], k=k), expected_sorted(full, k))
 
 
 @pytest.mark.parametrize("k", [10, 32])
@@ -85,7 +47,7 @@ def test_topk_large_many_units_and_splits(ktf, k):
     ut, ue = u[:20000], u[20000:]
     got = layer.bestMatches(ut, ue, k=k)
     full = layer.logLikelihoodRatio(ut, ue)
-    want = expected(full, k)
+    want = expected_sorted(full, k)
     del full
     check_equal(got, want)
 
@@ -132,7 +94,7 @@ def test_ties_come_back_lowest_column_first(setup):
     assert torch.equal(row, row[:1].expand(len(cols))), "copies of one vector must score equal"
     for k in (7, 16, 32):
         got = layer.bestMatches(ut2, ue2, k=k)
-        check_equal(got, expected(full, k))
+        check_equal(got, expected_sorted(full, k))
     s, i = layer.bestMatches(ut2, ue2, k=32)
     tied = [int(c) for c, v in zip(i[0].tolist(), s[0].tolist()) if v == float(row[0])]
     assert tied == cols
@@ -144,7 +106,7 @@ def test_edges(setup, ktf):
     layer, ut, ue, _, _ = setup
     # fewer enrolled vectors than k: (-inf, -1) after the last one
     s, i = layer.bestMatches(ut[:40], ue[:5], k=9)
-    check_equal((s, i), expected(layer.logLikelihoodRatio(ut[:40], ue[:5]), 9))
+    check_equal((s, i), expected_sorted(layer.logLikelihoodRatio(ut[:40], ue[:5]), 9))
     assert bool((i[:, 5:] == -1).all()) and bool(torch.isinf(s[:, 5:]).all()) and float(s[:, 5:].max()) < 0
     # no enrolled vector at all
     s, i = layer.bestMatches(ut[:33], ue[:0], k=4)
@@ -168,13 +130,6 @@ def test_edges(setup, ktf):
 
 
 _EW_CHILD = r"""
-import os, sys
-sys.path.insert(0, {root!r}); sys.path.insert(0, os.path.join({root!r}, "tests"))
-import numpy as np, torch
-import kaldi_tflite_b200 as ktf
-from test_gpu_tdnn_plda import synthetic_plda
-mean, Tm, psi = synthetic_plda(128)
-layer = ktf.layers.PLDA(128, mean, Tm, psi, dtype=np.float32, return_transformed=False)
 rng = np.random.default_rng(5)
 x = rng.standard_normal((1037 + 4099, 128)).astype(np.float32)
 u = layer.transformVector(torch.from_numpy(x).cuda())
@@ -187,14 +142,7 @@ np.savez({path!r}, **out)
 
 
 def test_independent_of_epilogue_warp_count(tmp_path):
-    res = {}
-    for ew in ("8", "16"):
-        path = str(tmp_path / f"ew{ew}.npz")
-        env = dict(os.environ, KTF_TC_PAIR_EPI_WARPS=ew)
-        p = subprocess.run([sys.executable, "-c", _EW_CHILD.format(root=ROOT, path=path)], env=env,
-                           stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=600)
-        assert p.returncode == 0, p.stdout
-        res[ew] = np.load(path)
+    res = epilogue_warp_runs(tmp_path, _EW_CHILD)
     for key in res["8"].files:
         assert np.array_equal(res["8"][key], res["16"][key]), key
 
@@ -215,32 +163,17 @@ def test_cuda_graph_capture_and_replay(setup):
     check_equal((gs, gi), layer.bestMatches(ut[300:1000].contiguous(), ue[2000:3500].contiguous(), k=10))
 
 
-def _run_topk_shard_workers(tmp_path, backend):
-    worker = os.path.join(ROOT, "tests", "plda_topk_shard_worker.py")
-    port = 31500 + (os.getpid() % 2000) + (7 if backend == "nccl" else 0)
-    procs = []
-    for rank in range(2):
-        env = dict(os.environ, RANK=str(rank), WORLD_SIZE="2", MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-        procs.append(subprocess.Popen([sys.executable, worker, str(tmp_path), backend], env=env, stdout=subprocess.PIPE,
-                                      stderr=subprocess.STDOUT, text=True))
-    outs = [p.communicate(timeout=600)[0] for p in procs]
-    for rank, (p, o) in enumerate(zip(procs, outs)):
-        assert p.returncode == 0, f"rank {rank} failed:\n{o}"
-    for rank in range(2):
-        with open(os.path.join(str(tmp_path), f"topk_rank{rank}.json")) as f:
-            r = json.load(f)
-        assert r["ok"], r
-
-
 def test_sharded_two_ranks_gloo(tmp_path):
-    _run_topk_shard_workers(tmp_path, "gloo")
+    for r in run_two_ranks(tmp_path, "topk", "gloo"):
+        assert r["ok"], r
 
 
 def test_sharded_two_gpus_nccl(tmp_path):
     import torch
     if torch.cuda.device_count() < 2:
         pytest.skip("needs two GPUs")
-    _run_topk_shard_workers(tmp_path, "nccl")
+    for r in run_two_ranks(tmp_path, "topk", "nccl"):
+        assert r["ok"], r
 
 
 def _numpy_merge(s_in, i_in, k):

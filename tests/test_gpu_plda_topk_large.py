@@ -10,21 +10,17 @@ The argument checks that need no device run everywhere; the rest is marked gpu.
 """
 
 import ctypes
-import json
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
-from conftest import ROOT
 from oracle import ktf_oracle as O
+from plda_testlib import DIM, check_equal, expected_listed, ktf, listed_sort, plda_vectors  # noqa: F401
+from plda_testlib import run_two_ranks, stats
 from test_gpu_tdnn_plda import synthetic_plda
 
 gpu = pytest.mark.gpu
 
-DIM = 128
 KS = (33, 64, 100, 255, 256, 257, 1000, 1024)
 N_TEST, N_ENROLL, N_COHORT = 1037, 49153, 1500
 
@@ -77,61 +73,11 @@ def test_python_argument_validation():
 # ---- on the GPU ----
 
 @pytest.fixture(scope="module")
-def ktf():
-    import kaldi_tflite_b200 as k
-    return k
-
-
-@pytest.fixture(scope="module")
 def setup(ktf):
     """A float32 layer and transformed vectors: 1037 test, 49 153 enrolled (one past the shared-memory row limit), a
     1500-vector cohort."""
-    import torch
-    mean, Tm, psi = synthetic_plda(DIM)
-    layer = ktf.layers.PLDA(DIM, mean, Tm, psi, dtype=np.float32, return_transformed=False)
-    g = torch.Generator(device="cuda").manual_seed(2026)
-    x = torch.randn((N_TEST + N_ENROLL + N_COHORT, DIM), generator=g, device="cuda")
-    u = layer.transformVector((x / x.norm(dim=1, keepdim=True) * DIM ** 0.5).contiguous())
-    return (layer, u[:N_TEST].contiguous(), u[N_TEST:N_TEST + N_ENROLL].contiguous(),
-            u[N_TEST + N_ENROLL:].contiguous())
-
-
-def sorted_rows(full):
-    """Stable descending sort of every row with NaN and -inf entries moved last, and the number of listed entries."""
-    import torch
-    dropped = torch.isnan(full) | (full == float("-inf"))
-    s, i = torch.sort(full.masked_fill(dropped, float("-inf")), dim=1, descending=True, stable=True)
-    return s, i, (~dropped).sum(dim=1, keepdim=True)
-
-
-def expected(srt, k):
-    """First k of `sorted_rows`, padded with (-inf, -1) past the listed entries."""
-    import torch
-    s, i, kept = srt
-    nt, ne = s.shape
-    m = min(k, ne)
-    want_s = torch.full((nt, k), float("-inf"), device=s.device, dtype=torch.float32)
-    want_i = torch.full((nt, k), -1, device=s.device, dtype=torch.int64)
-    want_s[:, :m] = s[:, :m]
-    want_i[:, :m] = i[:, :m]
-    pad = torch.arange(k, device=s.device)[None, :] >= kept
-    want_s[pad] = float("-inf")
-    want_i[pad] = -1
-    return want_s, want_i
-
-
-def check_equal(got, want):
-    import torch
-    gs, gi = got
-    ws, wi = want
-    assert gs.dtype is torch.float32 and gi.dtype is torch.int64 and gs.shape == ws.shape and gi.shape == wi.shape
-    assert torch.equal(gi, wi), f"{int((gi != wi).sum())} of {gi.numel()} indexes differ"
-    assert torch.equal(gs, ws)
-
-
-def stats(layer, ut, ue, uc, top_n, num_examples=1.0):
-    return (layer.cohortStats(ut, uc, top_n=top_n),
-            layer.cohortStats(ue, uc, top_n=top_n, role="enrolled", num_examples=num_examples))
+    layer, (ut, ue, uc), _, _ = plda_vectors(ktf, (N_TEST, N_ENROLL, N_COHORT), 2026, cuda_rng=True)
+    return layer, ut, ue, uc
 
 
 def both_forms(layer, ut, ue, uc, num_examples=1.0, top_n=100):
@@ -151,13 +97,13 @@ def both_forms(layer, ut, ue, uc, num_examples=1.0, top_n=100):
 def test_equals_stable_sort_of_matrix(setup, nt, ne, num_examples):
     layer, ut, ue, uc = setup
     for name, full, run in both_forms(layer, ut[:nt], ue[:ne], uc, num_examples):
-        srt = sorted_rows(full)
+        srt = listed_sort(full)
         del full
         for k in KS:
-            check_equal(run(k), expected(srt, k))
+            check_equal(run(k), expected_listed(srt, k))
     # AS-norm statistics computed inside the call
     ts, es = stats(layer, ut[:nt], ue[:ne], uc, 100, num_examples)
-    want = expected(sorted_rows(layer.asNorm(ut[:nt], ue[:ne], test_stats=ts, enroll_stats=es,
+    want = expected_listed(listed_sort(layer.asNorm(ut[:nt], ue[:ne], test_stats=ts, enroll_stats=es,
                                              num_examples=num_examples)), 100)
     check_equal(layer.asNormBestMatchesLarge(ut[:nt], ue[:ne], uc, k=100, top_n=100, num_examples=num_examples), want)
 
@@ -178,10 +124,10 @@ def test_large_shapes(ktf):
         norm = layer.asNormBestMatchesLarge(ut, ue, k=k, test_stats=ts, enroll_stats=es)
         for r0 in range(0, 20000, 2000):
             rows = slice(r0, r0 + 2000)
-            want = expected(sorted_rows(layer.logLikelihoodRatio(ut[rows], ue)), k)
+            want = expected_listed(listed_sort(layer.logLikelihoodRatio(ut[rows], ue)), k)
             check_equal((raw[0][rows], raw[1][rows]), want)
             full = layer.asNorm(ut[rows], ue, test_stats=(ts[0][rows], ts[1][rows]), enroll_stats=es)
-            check_equal((norm[0][rows], norm[1][rows]), expected(sorted_rows(full), k))
+            check_equal((norm[0][rows], norm[1][rows]), expected_listed(listed_sort(full), k))
 
 
 @gpu
@@ -201,11 +147,11 @@ def test_ties_come_back_lowest_column_first(setup):
     for name, full, run in both_forms(layer, ut2, ue2, uc):
         tie = full[at][:, cols[:1]]
         assert torch.equal(full[at][:, cols], tie.expand(len(at), len(cols))), name
-        srt = sorted_rows(full)
+        srt = listed_sort(full)
         del full
         for k in (33, 256, 699, 700, 701, 1024):
             s, i = run(k)
-            check_equal((s, i), expected(srt, k))
+            check_equal((s, i), expected_listed(srt, k))
             for j, r in enumerate(at):
                 listed = i[r][s[r] == tie[j, 0]]
                 assert len(listed) > 0 and torch.equal(listed, cols[:len(listed)]), (name, k, r)
@@ -248,11 +194,11 @@ def test_ties_across_radix_digit_boundaries(setup, bit):
     ka, kb = _order_keys(va.reshape(1)), _order_keys(vb.reshape(1))
     assert bool(ka > kb) and bool((ka >> bit) != (kb >> bit))
     m = int((full[0] > va).sum())                              # rank of the first score of the upper group
-    srt = sorted_rows(full)
+    srt = listed_sort(full)
     ks = sorted({min(max(k, 33), 1024) for k in (m + 1, m + 100, m + 201, m + 202, m + 300, m + 402)})
     for k in ks:
         got = layer.bestMatchesLarge(ut2, ue2, k=k)
-        check_equal(got, expected(srt, k))
+        check_equal(got, expected_listed(srt, k))
         s0, i0 = got[0][0], got[1][0]
         for v in (va, vb):
             listed = i0[s0 == v]
@@ -294,17 +240,17 @@ def test_sigma_zero_lists_plus_inf_only(setup):
     ts, es = (ts[0], t_std), (es[0], e_std)
     full = layer.asNorm(ut[:nt], ue[:ne], test_stats=ts, enroll_stats=es)
     assert bool((full == float("inf")).any()) and bool((full == float("-inf")).any()) and bool(torch.isnan(full).any())
-    srt = sorted_rows(full)
+    srt = listed_sort(full)
     for k in (33, 100, 1024):
         s, i = layer.asNormBestMatchesLarge(ut[:nt], ue[:ne], k=k, test_stats=ts, enroll_stats=es)
-        check_equal((s, i), expected(srt, k))
+        check_equal((s, i), expected_listed(srt, k))
         assert not bool(torch.isnan(s).any()) and bool((s == float("inf")).any())
         assert not bool((s[i >= 0] == float("-inf")).any())
     flat = uc[:1].expand(200, DIM).contiguous()
     full = layer.asNorm(ut[:nt], ue[:ne], flat, top_n=100)
-    srt = sorted_rows(full)
+    srt = listed_sort(full)
     for k in (33, 1024):
-        check_equal(layer.asNormBestMatchesLarge(ut[:nt], ue[:ne], flat, k=k, top_n=100), expected(srt, k))
+        check_equal(layer.asNormBestMatchesLarge(ut[:nt], ue[:ne], flat, k=k, top_n=100), expected_listed(srt, k))
 
 
 @gpu
@@ -333,7 +279,7 @@ def test_edges(setup, ktf):
     # fewer enrolled vectors than k: (-inf, -1) after the last one
     for name, full, run in both_forms(layer, ut[:40], ue[:5], uc):
         s, i = run(100)
-        check_equal((s, i), expected(sorted_rows(full), 100))
+        check_equal((s, i), expected_listed(listed_sort(full), 100))
         assert bool((i[:, 5:] == -1).all()) and bool((s[:, 5:] == float("-inf")).all())
     # no enrolled vector at all
     for s, i in (layer.bestMatchesLarge(ut[:33], ue[:0], k=100),
@@ -374,9 +320,9 @@ def test_edges(setup, ktf):
     st = layer.cohortStats(ut, uc, top_n=100)
     ss = layer.cohortStats(ut, uc, top_n=100, role="enrolled", num_examples=3.0)
     check_equal(layer.bestMatchesLarge(ut, k=300, num_examples=3.0),
-                expected(sorted_rows(layer.logLikelihoodRatio(ut, num_examples=3.0)), 300))
+                expected_listed(listed_sort(layer.logLikelihoodRatio(ut, num_examples=3.0)), 300))
     check_equal(layer.asNormBestMatchesLarge(ut, k=300, test_stats=st, enroll_stats=ss, num_examples=3.0),
-                expected(sorted_rows(layer.asNorm(ut, test_stats=st, enroll_stats=ss, num_examples=3.0)), 300))
+                expected_listed(listed_sort(layer.asNorm(ut, test_stats=st, enroll_stats=ss, num_examples=3.0)), 300))
 
 
 @gpu
@@ -483,26 +429,10 @@ def test_topk_merge_large_against_numpy(ktf):
             assert np.array_equal(os_.cpu().numpy().view(np.uint32), ws.view(np.uint32)), (L, k_in, k)
 
 
-def _run_shard_workers(tmp_path, backend):
-    worker = os.path.join(ROOT, "tests", "plda_topk_large_shard_worker.py")
-    port = 36900 + (os.getpid() % 2000) + (7 if backend == "nccl" else 0)
-    procs = []
-    for rank in range(2):
-        env = dict(os.environ, RANK=str(rank), WORLD_SIZE="2", MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-        procs.append(subprocess.Popen([sys.executable, worker, str(tmp_path), backend], env=env, stdout=subprocess.PIPE,
-                                      stderr=subprocess.STDOUT, text=True))
-    outs = [p.communicate(timeout=600)[0] for p in procs]
-    for rank, (p, o) in enumerate(zip(procs, outs)):
-        assert p.returncode == 0, f"rank {rank} failed:\n{o}"
-    for rank in range(2):
-        with open(os.path.join(str(tmp_path), f"topk_large_rank{rank}.json")) as f:
-            r = json.load(f)
-        assert r["ok"], r
-
-
 @gpu
 def test_sharded_two_ranks_gloo(tmp_path):
-    _run_shard_workers(tmp_path, "gloo")
+    for r in run_two_ranks(tmp_path, "topk_large", "gloo"):
+        assert r["ok"], r
 
 
 @gpu
@@ -510,4 +440,5 @@ def test_sharded_two_gpus_nccl(tmp_path):
     import torch
     if torch.cuda.device_count() < 2:
         pytest.skip("needs two GPUs")
-    _run_shard_workers(tmp_path, "nccl")
+    for r in run_two_ranks(tmp_path, "topk_large", "nccl"):
+        assert r["ok"], r

@@ -27,6 +27,7 @@ import pytest
 from conftest import ROOT, golden_path, load_golden, read_wav_int16, rmse
 import helpers
 from oracle import ktf_oracle as O
+from plda_testlib import run_two_ranks
 from test_gpu_tdnn_plda import cosine, extractor_cfg, sitw_layers_for_oracle, synthetic_plda
 
 pytestmark = pytest.mark.gpu
@@ -407,27 +408,15 @@ def test_dither_in_kernel_is_per_framed_sample(ktf):
 # sharded PLDA, two ranks on one GPU
 # ------------------------------------------------------------------------------------------------
 
-def _run_shard_workers(tmp_path, extra=()):
-    worker = os.path.join(ROOT, "tests", "plda_shard_worker.py")
-    port = 29500 + (os.getpid() % 2000) + len(extra)
-    procs = []
-    for rank in range(2):
-        env = dict(os.environ, RANK=str(rank), WORLD_SIZE="2", MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
-        procs.append(subprocess.Popen([sys.executable, worker, str(tmp_path), *extra], env=env, stdout=subprocess.PIPE,
-                                      stderr=subprocess.STDOUT, text=True))
-    outs = [p.communicate(timeout=600)[0] for p in procs]
-    for rank, (p, o) in enumerate(zip(procs, outs)):
-        assert p.returncode == 0, f"rank {rank} failed:\n{o}"
-    for rank in range(2):
-        with open(os.path.join(str(tmp_path), f"rank{rank}.json")) as f:
-            r = json.load(f)
+def _check_llr_ranks(results):
+    for r in results:
         assert r["ok"], r
         assert r["max_rel"] <= 1e-3, r
         assert r["launches"] > 0
 
 
 def test_plda_sharded_two_ranks_vs_oracle(tmp_path):
-    _run_shard_workers(tmp_path)
+    _check_llr_ranks(run_two_ranks(tmp_path, "llr"))
 
 
 def test_plda_sharded_two_gpus_nccl_async_allgather(tmp_path):
@@ -436,8 +425,8 @@ def test_plda_sharded_two_gpus_nccl_async_allgather(tmp_path):
     import torch
     if torch.cuda.device_count() < 2:
         pytest.skip("needs two GPUs")
-    _run_shard_workers(tmp_path, ("nccl", "1500"))
-    _run_shard_workers(tmp_path, ("nccl", "1501"))
+    _check_llr_ranks(run_two_ranks(tmp_path, "llr", "nccl", "1500"))
+    _check_llr_ranks(run_two_ranks(tmp_path, "llr", "nccl", "1501"))
 
 
 def _run_cabi_workers(tmp_path, nranks):
