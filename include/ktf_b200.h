@@ -491,6 +491,44 @@ int ktf_plda_score_asnorm_topk_large(const ktf_plda* p, const void* u_test_dev, 
                                      const float* enroll_std_dev, int32_t k, float* scores_dev, int64_t* index_dev,
                                      void* stream);
 
+/* ------------------------------------------------------------------------------------
+ * Diarization back-end: Kaldi's ivector-plda-scoring-dense (without its per-recording PCA) and agglomerative-cluster for
+ * a batch of recordings.
+ * ---------------------------------------------------------------------------------- */
+/* Within-recording scores: group r is rows offsets_host[r] .. offsets_host[r + 1] of the transformed vectors u_dev
+ * (ktf_plda_transform output), and its n_r x n_r matrix S_r[i, j] = LLR(enrolled u_i | test u_j) -- Kaldi's dense
+ * scoring orientation, each value bit-equal to entry [j, i] of ktf_plda_score(p, u_r, u_r) -- is written to scores_dev
+ * at element sum_{q<r} n_q^2 with row pitch n_r (packed).  One tcgen05 score launch for the whole batch: every 256-row
+ * block computes only the column tiles of the groups its rows belong to.  Groups of 0 or 1 rows are allowed; a negative
+ * length, offsets_host[0] < 0, more than 2^31 - 1 rows, null pointers (with rows to score) or a handle other than float32
+ * on sm_100 is KTF_EINVAL.  No host synchronisation; the group table, tile list and operands live in the handle's
+ * grow-only workspace, so calls on one handle must not run concurrently on different streams. */
+int ktf_plda_score_within(const ktf_plda* p, const void* u_dev, const int64_t* offsets_host, int32_t num_groups,
+                          float* scores_dev, void* stream);
+
+/* Average-linkage agglomerative clustering, Kaldi's single-pass AgglomerativeClusterer, for every group of the packed
+ * score matrices scores_dev (the layout of ktf_plda_score_within: group r of n_r = offsets_host[r + 1] - offsets_host[r]
+ * points at element sum_{q<r} n_q^2, row pitch n_r; any square float32 matrices, e.g. read from Kaldi, work too):
+ * - cost(a, b) = -S[min(a, b)][max(a, b)] (only the upper triangle is read); points have ids 0 .. n-1 and the k-th
+ *   merge creates cluster id n + k;
+ * - W(a, b), the cost sum of two clusters, is the cost for two points; merging i and j into m gives every other active
+ *   cluster k W(k, m) = W(k, i) + W(k, j) (one float32 add); avg(k, m) = W(k, m) / (float)(size_k size_m) (int32
+ *   product, IEEE float32 division);
+ * - each step merges the active pair with the smallest (avg, lower id, higher id) among those with avg <= threshold (NaN
+ *   never; -0 and +0 are equal), and stops when none is left or the group has min_clusters clusters: 1, or
+ *   num_clusters_host[r] when that array is given, which also sets the threshold to FLT_MAX (Kaldi's reco2num_spk);
+ * - labels_dev (at offsets_host[r] - offsets_host[0]): the final clusters in increasing id order are labels 1 .. C_r;
+ * - merge_ids_dev (sum_r max(n_r - 1, 0), 2) int32 and merge_costs_dev (nullable, both or either): the merges in order as
+ *   (lower id, higher id, avg), then (-1, -1, NaN); cluster_counts_dev[r] = C_r.
+ * A thresholded run's merge list is therefore the prefix of the unthresholded run's list that ends before the first
+ * merge whose avg is above the threshold: one run serves a threshold sweep.  One CTA per group, the largest first.
+ * A group larger than KTF_AHC_MAX_POINTS, a negative length, a num_clusters entry < 1 or a null required pointer is
+ * KTF_EINVAL.  No host synchronisation (stream-ordered scratch of sum_r n_r^2 floats). */
+#define KTF_AHC_MAX_POINTS 16384
+int ktf_ahc_cluster(const float* scores_dev, const int64_t* offsets_host, int32_t num_groups, float threshold,
+                    const int32_t* num_clusters_host, int32_t* labels_dev, int32_t* merge_ids_dev,
+                    float* merge_costs_dev, int32_t* cluster_counts_dev, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

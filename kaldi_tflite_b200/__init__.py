@@ -7,8 +7,10 @@ wav -> x-vector hot path behind the reference's Python API.
                StatsPooling / PLDA
     ktf.models.XvectorExtractorFromConfig / XvectorExtractor / SequentialFromConfig
     ktf.io.KaldiNnet3Reader / KaldiPldaReader / ReadKaldiArray / KaldiObjReader
+    ktf.diarization.agglomerative_cluster
 """
 
+from . import diarization  # noqa: F401
 from . import io  # noqa: F401  (numpy only)
 from . import kaldi_numpy  # noqa: F401
 from . import layers  # noqa: F401

@@ -22,6 +22,7 @@ KTF_MAX_CONTEXT = 16
 KTF_PLDA_TOPK_MAX = 32
 KTF_PLDA_TOPK_LARGE_MAX = 1024
 KTF_COHORT_AS_TEST, KTF_COHORT_AS_ENROLLED = 0, 1
+KTF_AHC_MAX_POINTS = 16384
 KTF_NCCL_UNIQUE_ID_BYTES = 128
 KTF_EINVAL, KTF_ECUDA, KTF_ENOMEM = -1, -2, -3
 
@@ -118,6 +119,8 @@ _SIGNATURES = {
     "ktf_plda_score_topk_large": (c_int32, [_P, _P, c_int64, _P, c_int64, c_int32, _P, _P, _P]),
     "ktf_plda_score_asnorm_topk_large": (c_int32, [_P, _P, c_int64, _P, c_int64, _P, _P, _P, _P, c_int32, _P, _P, _P]),
     "ktf_topk_merge_large": (c_int32, [_P, _P, c_int32, c_int64, c_int32, c_int32, _P, _P, _P]),
+    "ktf_plda_score_within": (c_int32, [_P, _P, _P, c_int32, _P, _P]),
+    "ktf_ahc_cluster": (c_int32, [_P, _P, c_int32, c_float, _P, _P, _P, _P, _P, _P]),
 }
 
 _lib = None

@@ -758,6 +758,59 @@ int score_tc(const ktf_plda* p, const float* ut, int64_t nt, const float* ue, in
   return KTF_OK;
 }
 
+// Row i of a within-group score: the group g with offs[g] <= i < offs[g + 1] (offs relative to the first row; the last
+// such g skips empty groups), its columns and the packed position of entry (i, 0): base[g] + (i - offs[g]) n_g - offs[g],
+// so entry (i, j) lands at base[g] + (i - offs[g]) n_g + (j - offs[g]).
+__global__ void within_rows_kernel(const long long* __restrict__ offs, const long long* __restrict__ base, int num_groups,
+                                   long long n, ktf::WithinRow* __restrict__ rows) {
+  const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  int lo = 0, hi = num_groups - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (offs[mid] <= i) lo = mid;
+    else hi = mid - 1;
+  }
+  const long long c0 = offs[lo], c1 = offs[lo + 1];
+  rows[i] = ktf::WithinRow{base[lo] + (i - c0) * (c1 - c0) - c0, (int)c0, (int)c1};
+}
+
+// Within-group scores of the rows u (offsets relative to offsets[0]) in one pair-kernel launch: the GEMM's rows are the
+// enrolled side and its columns the test side (tc_operands' enrolled_rows), so row i of the accumulator is column i of
+// the normal one and (acc + B_i) + A_j keeps the association of the normal epilogue (acc + B_i) + A_j: every entry is
+// bit-equal to logLikelihoodRatio(u_g, u_g)[j, i].  The group table and the tile list are copied into the workspace with
+// one cudaMemcpyAsync from pageable memory, which returns once the host buffer has been staged (no device
+// synchronisation), so `host` may die at return.
+int score_within_tc(const ktf_plda* p, const float* u, const int64_t* offsets, int num_groups, float* scores,
+                    cudaStream_t st) {
+  const long long n = offsets[num_groups] - offsets[0];
+  const long long num_tiles = ktf::tc_within_tiles(offsets, num_groups, nullptr);
+  // host: offsets (G + 1), packed bases (G), then the tiles
+  std::vector<long long> host((size_t)(2 * num_groups + 1) + (size_t)num_tiles);
+  long long acc = 0;
+  for (int g = 0; g <= num_groups; ++g) host[g] = offsets[g] - offsets[0];
+  for (int g = 0; g < num_groups; ++g) {
+    host[num_groups + 1 + g] = acc;
+    acc += (offsets[g + 1] - offsets[g]) * (offsets[g + 1] - offsets[g]);
+  }
+  int2* tiles_host = reinterpret_cast<int2*>(host.data() + 2 * num_groups + 1);
+  ktf::tc_within_tiles(offsets, num_groups, tiles_host);
+  const size_t table_bytes = host.size() * sizeof(long long);
+  const size_t rows_at = (table_bytes + 255) & ~(size_t)255;
+  TcOperands o;
+  int rc = tc_operands(p, u, n, u, n, nullptr, rows_at + (size_t)n * sizeof(ktf::WithinRow), st, &o, /*enrolled_rows=*/true);
+  if (rc != KTF_OK) return rc;
+  long long* table = reinterpret_cast<long long*>(o.extra);
+  ktf::WithinRow* rows = reinterpret_cast<ktf::WithinRow*>(o.extra + rows_at);
+  KTF_CUDA(cudaMemcpyAsync(table, host.data(), table_bytes, cudaMemcpyHostToDevice, st));
+  within_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(table, table + num_groups + 1, num_groups, n, rows);
+  KTF_LAUNCH_OK();
+  const ktf::TcWithin w{reinterpret_cast<const int2*>(table + 2 * num_groups + 1), num_tiles, rows};
+  ktf::TcScore g = o.gemm(0, n, n, o.Ai, o.Bj, scores, 0);
+  g.within = &w;
+  return ktf::tc_gemm_score(g, st);
+}
+
 // Argument checks of the k-best entry points `fn`, one order for all: k (1 .. k_max, named k_max_name), the handle,
 // float32 / sm_100, n_enroll; n_test <= 0 is then a no-op, and the pointers are checked last.  Scores when they pass.
 int score_topk_checked(const char* fn, int k_max, const char* k_max_name, const ktf_plda* p, const void* u_test,
@@ -1032,6 +1085,25 @@ int ktf_topk_merge_large(const float* scores_in_dev, const int64_t* index_in_dev
                 "ktf_topk_merge_large: null argument");
   return topk_select(ListRows{scores_in_dev, (const long long*)index_in_dev, n_rows, k_in}, n_rows,
                      (long long)num_lists * k_in, k, scores_dev, (long long*)index_dev, (cudaStream_t)stream);
+}
+
+int ktf_plda_score_within(const ktf_plda* p, const void* u_dev, const int64_t* offsets_host, int32_t num_groups,
+                          float* scores_dev, void* stream) {
+  KTF_CHECK_ARG(p, "ktf_plda_score_within: null handle");
+  KTF_CHECK_ARG(p->use_tc, "ktf_plda_score_within needs a float32 PLDA handle on an sm_100 device");
+  KTF_CHECK_ARG(num_groups >= 0, "ktf_plda_score_within: num_groups = %d, must be >= 0", num_groups);
+  if (num_groups == 0) return KTF_OK;
+  KTF_CHECK_ARG(offsets_host, "ktf_plda_score_within: null offsets");
+  KTF_CHECK_ARG(offsets_host[0] >= 0, "ktf_plda_score_within: offsets[0] = %lld, must be >= 0",
+                (long long)offsets_host[0]);
+  for (int32_t g = 0; g < num_groups; ++g)
+    KTF_CHECK_ARG(offsets_host[g + 1] >= offsets_host[g], "ktf_plda_score_within: group %d has a negative length", g);
+  KTF_CHECK_ARG(offsets_host[num_groups] - offsets_host[0] < (1LL << 31),
+                "ktf_plda_score_within: more than 2^31 - 1 rows");
+  if (offsets_host[num_groups] == offsets_host[0]) return KTF_OK;
+  KTF_CHECK_ARG(u_dev && scores_dev, "ktf_plda_score_within: null argument");
+  return score_within_tc(p, (const float*)u_dev + offsets_host[0] * p->dim, offsets_host, num_groups, scores_dev,
+                         (cudaStream_t)stream);
 }
 
 int ktf_plda_score(const ktf_plda* p, const void* u_test_dev, int64_t n_test, const void* u_enroll_dev,

@@ -53,7 +53,25 @@ struct TcScore {
   int k;
   float* part_score;
   long long* part_index;
+  // - within-group rows (raw value, value (acc + row_add[i]) + col_add[j]; non-null `within`, m == n, C fp32): only the
+  //   tiles of TcWithin::tiles are computed, and entry (i, j) is stored, at C[rows[i].dst + j], only when
+  //   rows[i].lo <= j < rows[i].hi.
+  const struct TcWithin* within;
+};
+// Row i of a within-group score: its group is columns [lo, hi), and its entries go to dst + column.
+struct WithinRow {
+  long long dst;
+  int lo, hi;
+};
+struct TcWithin {
+  const int2* tiles;         // (row block of 256 rows, n-tile of 256 columns), from tc_within_tiles
+  long long num_tiles;
+  const WithinRow* rows;     // (m)
 };
 int tc_gemm_score(const TcScore& s, cudaStream_t st);
 int tc_topk_lists(long long m, long long n, long long K);
+// The tiles a within-group score computes for groups [offsets[g], offsets[g + 1]) of the rows (relative to offsets[0]):
+// every 256-row block with the n-tiles that cover the groups its rows belong to.  Returns their number and writes them
+// to `tiles` when it is not null.
+long long tc_within_tiles(const int64_t* offsets, int num_groups, int2* tiles);
 }  // namespace ktf

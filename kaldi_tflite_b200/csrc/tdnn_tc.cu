@@ -67,18 +67,23 @@ enum { kModeTopk8 = 3, kModeTopk16 = 4, kModeTopk32 = 5 };
 enum { kModeNormTopk8 = 6, kModeNormTopk16 = 7, kModeNormTopk32 = 8 };
 // Pair kernel, the AS-norm rows of kModeNorm rounded once to bf16 and stored as kModeBf16 stores its rows.
 enum { kModeNormBf16 = 9 };
-constexpr int kNumModes = 10;
-//                                   Bf16 F32 Norm Tk8 Tk16 Tk32 NTk8 NTk16 NTk32 NBf16
-constexpr int kModeTopkCap[kNumModes] = {0, 0, 0, 8, 16, 32, 8, 16, 32, 0};   // top-k list capacity, 0 = rows stored
-constexpr bool kModeIsNorm[kNumModes] = {0, 0, 1, 0, 0, 0, 1, 1, 1, 1};      // AS-norm value (kEpiNorm)
-constexpr bool kModeIsBf16[kNumModes] = {1, 0, 0, 0, 0, 0, 0, 0, 0, 1};      // rows stored as bf16
+// Pair kernel, within-group scores (PLDA diarization): the tiles of TcArgs::within_tiles only, fp32 values
+// (acc + row addend) + column addend, each row stored at the columns of its own group into that group's packed matrix
+// (TcArgs::within_rows, store_chunk_within).
+enum { kModeWithin = 10 };
+constexpr int kNumModes = 11;
+//                                   Bf16 F32 Norm Tk8 Tk16 Tk32 NTk8 NTk16 NTk32 NBf16 Within
+constexpr int kModeTopkCap[kNumModes] = {0, 0, 0, 8, 16, 32, 8, 16, 32, 0, 0};   // top-k list capacity, 0 = rows stored
+constexpr bool kModeIsNorm[kNumModes] = {0, 0, 1, 0, 0, 0, 1, 1, 1, 1, 0};      // AS-norm value (kEpiNorm)
+constexpr bool kModeIsBf16[kNumModes] = {1, 0, 0, 0, 0, 0, 0, 0, 0, 1, 0};      // rows stored as bf16
 // TcArgs::row_best is tested at run time (only tc_gemm_score's raw fp32 rows pass it).  The AS-norm modes after kModeTopk32
 // compile the test out: in kModeNormBf16 at 16 epilogue warps the dead path costs 8 bytes of spills.
-constexpr bool kModeRowBest[kNumModes] = {1, 1, 1, 1, 1, 1, 0, 0, 0, 0};
+constexpr bool kModeRowBest[kNumModes] = {1, 1, 1, 1, 1, 1, 0, 0, 0, 0, 0};
 constexpr int topk_cap(int mode) { return kModeTopkCap[mode]; }
 constexpr bool mode_norm(int mode) { return kModeIsNorm[mode]; }
 constexpr bool mode_bf16(int mode) { return kModeIsBf16[mode]; }
 constexpr bool mode_row_best(int mode) { return kModeRowBest[mode]; }
+constexpr bool mode_within(int mode) { return mode == kModeWithin; }
 
 // rowmap flags
 constexpr int kRowStore = 1, kRowFirst = 2, kRowLast = 4;
@@ -131,6 +136,11 @@ struct TcArgs {
   int topk_unit_tiles;
   float* topk_score;
   long long* topk_index;
+  // pair kernel, kModeWithin: the clusters share out the tiles within_tiles[0 .. within_num_tiles) (row block, n-tile);
+  // row i goes to out + within_rows[i].dst + column for the columns [lo, hi) of its group
+  const int2* within_tiles;
+  long long within_num_tiles;
+  const ktf::WithinRow* within_rows;
 };
 
 __device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
@@ -427,6 +437,30 @@ __device__ __forceinline__ void store_chunk_ragged(const unsigned (&r)[32], cons
           else *reinterpret_cast<float*>(dst + h * ld_bytes) = v;
         }
       }
+    }
+    __syncwarp();
+  }
+}
+
+// kModeWithin chunk store: the values (acc + row addend) + column addend of a 32 x 32 chunk, staged as in
+// store_chunk_ragged (16 columns per pass), then every row's entries in its own group's column range [lo, hi) go to
+// out + dst + column -- the group's packed matrix, whose row pitch is the group size, so no box or tensor map fits it.
+// A warp store writes 16 consecutive floats of two rows.
+__device__ __forceinline__ void store_chunk_within(const unsigned (&r)[32], const float* vb, float radd, unsigned char* stg,
+                                                   int lane, const ktf::WithinRow& w, int col0, float* out) {
+  constexpr int kCols = 16;
+#pragma unroll
+  for (int pass = 0; pass < 32 / kCols; ++pass) {
+    float* mine = reinterpret_cast<float*>(stg + lane * kStgPitch);
+#pragma unroll
+    for (int i = 0; i < kCols; ++i) mine[i] = (__uint_as_float(r[pass * kCols + i]) + radd) + vb[pass * kCols + i];
+    __syncwarp();
+#pragma unroll 1
+    for (int k = lane; k < 32 * kCols; k += 32) {
+      const int rr = k / kCols, col = col0 + pass * kCols + k % kCols;
+      const long long dst = __shfl_sync(0xffffffffu, w.dst, rr);
+      const int lo = __shfl_sync(0xffffffffu, w.lo, rr), hi = __shfl_sync(0xffffffffu, w.hi, rr);
+      if (col >= lo && col < hi) out[dst + col] = *reinterpret_cast<const float*>(stg + rr * kStgPitch + (k % kCols) * 4);
     }
     __syncwarp();
   }
@@ -783,6 +817,7 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   constexpr int kCap = topk_cap(MODE);
   constexpr bool kTopk = kCap > 0;
   constexpr bool kNorm = mode_norm(MODE);
+  constexpr bool kWithin = mode_within(MODE);
   constexpr int kTopkVecs = topk_vecs(MODE);
   using TCfg = TopkCfg<EW, kTopk ? kCap : 8, kTopkVecs>;
   constexpr int kPairStages = kTopk ? TCfg::kStages : Cfg::kStages;
@@ -820,13 +855,18 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   const long long topk_units = kTopk ? m_tiles * (((long long)n_tiles + unit_tiles - 1) / unit_tiles) : 0;
   const long long topk_mine = cluster_id < topk_units ? (topk_units - 1 - cluster_id) / num_clusters + 1 : 0;
   const long long t_begin = kTopk ? 0 : cluster_id;                                    // this cluster's tiles
-  const long long t_end = kTopk ? topk_mine * unit_tiles : total_tiles, t_step = kTopk ? 1 : num_clusters;
+  const long long t_end = kTopk ? topk_mine * unit_tiles : kWithin ? a.within_num_tiles : total_tiles;
+  const long long t_step = kTopk ? 1 : num_clusters;
   auto topk_unit = [&](long long tile_) { return (unsigned)cluster_id + ((unsigned)tile_ / unit_tiles) * (unsigned)num_clusters; };
   auto coords = [&](long long tile_, long long& mt_, int& nt_) {
     if constexpr (kTopk) {
       const unsigned u = topk_unit(tile_), s = u / (unsigned)m_tiles;
       mt_ = u - s * (unsigned)m_tiles;
       nt_ = (int)(s * unit_tiles + (unsigned)tile_ % unit_tiles);
+    } else if constexpr (kWithin) {
+      const int2 t = a.within_tiles[tile_];
+      mt_ = t.x;
+      nt_ = t.y;
     } else {
       tile_coords(tile_, m_tiles, n_tiles, a.reverse, a.group_m, mt_, nt_);
     }
@@ -986,6 +1026,10 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     };
     int nx_flags = 0;
     float nx_radd = 0.0f, nx_rh = 0.0f, nx_rmu = 0.0f;   // (rh / rmu: Norm mode's 0.5 / sigma_t and mu_t)
+    ktf::WithinRow nx_wrow{0, 0, 0};                     // (kModeWithin: the row's group, see TcArgs::within_rows)
+    auto load_within_row = [&](long long row_) {
+      return row_ < m_rows ? a.within_rows[row_] : ktf::WithinRow{0, 0, 0};
+    };
     auto load_row_meta = [&](long long row_, int& f_, float& ra_, float& rh_, float& rmu_) {
       f_ = 0;
       ra_ = 0.0f;
@@ -1038,7 +1082,11 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       // the stall samples); request the next tile's now
       int flags = nx_flags;
       float radd = nx_radd, rh = nx_rh, rmu = nx_rmu;
+      ktf::WithinRow wrow = nx_wrow;
       if (it == 0) load_row_meta(row, flags, radd, rh, rmu);
+      if constexpr (kWithin) {
+        if (it == 0) wrow = load_within_row(row);
+      }
       {
         const long long next = tile + t_step;
         if (next < t_end) {
@@ -1047,6 +1095,7 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
           coords(next, mt2, nt2);
           if (nt2 != nt && pre_nt != nt2) prefetch_vec(nt2);
           load_row_meta(mt2 * BM2 + (long long)rank * BM + quarter * 32 + lane, nx_flags, nx_radd, nx_rh, nx_rmu);
+          if constexpr (kWithin) nx_wrow = load_within_row(mt2 * BM2 + (long long)rank * BM + quarter * 32 + lane);
         }
       }
       mbar_wait(&tfull_bar[acc], acc_phase);
@@ -1120,6 +1169,13 @@ tdnn_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
             }
           }
           __syncwarp();                          // converged again before the next .sync.aligned TMEM load / wait
+          if (kRB == 1 && c + 1 < kPChunks) tmem_ld32_issue(taddr0 + (unsigned)((c + 1) * 32), r[0]);
+          continue;
+        }
+        if constexpr (kWithin) {
+          // (warp-uniform: chunks that no row of the warp keeps are skipped)
+          if (col0 < n_cols && __any_sync(0xffffffffu, wrow.lo < col0 + 32 && col0 < wrow.hi))
+            store_chunk_within(r[c % kRB], wv + c * 32, radd, stg2, lane, wrow, col0, static_cast<float*>(a.out));
           if (kRB == 1 && c + 1 < kPChunks) tmem_ld32_issue(taddr0 + (unsigned)((c + 1) * 32), r[0]);
           continue;
         }
@@ -1841,7 +1897,7 @@ int launch_gemm_pair_ew(const CUtensorMap& tmA, const CUtensorMap& tmB_half, con
   if (!mode_norm(MODE) && args.row_add != nullptr && (args.scale != nullptr || args.offset != nullptr)) return KTF_EINVAL;
   CUtensorMap tmC = tmA;
   args.tma_store = 0;
-  if (args.out != nullptr) {
+  if (args.out != nullptr && !mode_within(MODE)) {
     const int es = mode_bf16(MODE) ? 2 : 4;
     if (encode_map_out(&tmC, args.out, es, (unsigned long long)args.n_rows, (unsigned long long)args.m_rows,
                        (unsigned long long)args.out_ld))
@@ -1855,6 +1911,8 @@ int launch_gemm_pair_ew(const CUtensorMap& tmA, const CUtensorMap& tmB_half, con
   if (topk_cap(MODE))   // work units, not tiles, are what the clusters share out
     tiles = ((args.m_rows + 2 * BM - 1) / (2 * BM)) *
             (((args.n_rows + BN - 1) / BN + args.topk_unit_tiles - 1) / args.topk_unit_tiles);
+  if (mode_within(MODE)) tiles = args.within_num_tiles;
+  if (tiles <= 0) return KTF_OK;
   static int dbg = -1;
   if (dbg < 0) {
     const char* e = getenv("KTF_TC_DEBUG");
@@ -2136,9 +2194,12 @@ TopkPlan topk_plan(long long m, long long n, long long K) {
 }
 
 // The pair-kernel mode of a score: from its value (raw or AS-norm), its output (rows, row_best or top-k), the list
-// capacity k needs and the row format.  -1: no mode computes it (AS-norm with row_best, k outside 1..32).
+// capacity k needs and the row format.  -1: no mode computes it (AS-norm with row_best, k outside 1..32, a within-group
+// score with anything but raw fp32 rows of a square matrix).
 int score_mode(const ktf::TcScore& s) {
   const bool norm = s.col_half_inv != nullptr;
+  if (s.within != nullptr)
+    return norm || s.row_best != nullptr || s.part_score != nullptr || s.c_bf16 || s.m != s.n ? -1 : kModeWithin;
   if (s.part_score != nullptr) {
     if (s.k < 1 || s.k > 32) return -1;
     const int cap = s.k <= 8 ? 0 : s.k <= 16 ? 1 : 2;
@@ -2157,6 +2218,22 @@ int launch_score(int ew, const CUtensorMap& tmA, const CUtensorMap& tmBh, const 
 
 namespace ktf {
 
+long long tc_within_tiles(const int64_t* offsets, int num_groups, int2* tiles) {
+  const long long base = offsets[0], n = offsets[num_groups] - base;
+  long long count = 0;
+  int g = 0;
+  for (long long r0 = 0; r0 < n; r0 += 2 * BM) {
+    const long long r1 = std::min(r0 + 2 * BM, n) - 1;                 // the block's last row
+    while (offsets[g + 1] - base <= r0) ++g;                           // (empty groups hold no row)
+    int g1 = g;
+    while (offsets[g1 + 1] - base <= r1) ++g1;
+    const long long c0 = offsets[g] - base, c1 = offsets[g1 + 1] - base;
+    for (long long t = c0 / BN; t < (c1 + BN - 1) / BN; ++t, ++count)
+      if (tiles != nullptr) tiles[count] = make_int2((int)(r0 / (2 * BM)), (int)t);
+  }
+  return count;
+}
+
 int tc_topk_lists(long long m, long long n, long long K) {
   if (m <= 0 || n <= 0) return 0;
   const TopkPlan pl = topk_plan(m, n, K);
@@ -2170,7 +2247,8 @@ int tc_gemm_score(const TcScore& s, cudaStream_t st) {
   if (topk && (s.m <= 0 || s.n <= 0)) return KTF_OK;
   const int mode = score_mode(s);
   if (mode < 0) {
-    ktf::set_error("tc_gemm_score: no pair-kernel mode for this score (AS-norm with row_best, or k = %d outside 1..32)",
+    ktf::set_error("tc_gemm_score: no pair-kernel mode for this score (AS-norm with row_best, k = %d outside 1..32, or "
+                   "a within-group score that is not raw fp32 rows of a square matrix)",
                    s.k);
     return KTF_EINVAL;
   }
@@ -2193,7 +2271,13 @@ int tc_gemm_score(const TcScore& s, cudaStream_t st) {
   args.scale = s.col_half_inv;
   args.offset = s.col_mean;
   int ew;
-  if (topk) {
+  if (s.within != nullptr) {
+    ew = pair_epi_warps(args.kblocks_per_tap);
+    args.out = s.C;
+    args.within_tiles = s.within->tiles;
+    args.within_num_tiles = s.within->num_tiles;
+    args.within_rows = s.within->rows;
+  } else if (topk) {
     const TopkPlan pl = topk_plan(s.m, s.n, s.K);
     ew = pl.ew;
     args.topk_k = s.k;
@@ -2222,6 +2306,7 @@ int tc_gemm_score(const TcScore& s, cudaStream_t st) {
     case kModeNormTopk16: return launch_score<kModeNormTopk16>(ew, tmA, tmBh, args, st);
     case kModeNormTopk32: return launch_score<kModeNormTopk32>(ew, tmA, tmBh, args, st);
     case kModeNormBf16: return launch_score<kModeNormBf16>(ew, tmA, tmBh, args, st);
+    case kModeWithin: return launch_score<kModeWithin>(ew, tmA, tmBh, args, st);
   }
   return KTF_EINVAL;
 }

@@ -270,6 +270,29 @@ class PLDA(Layer):
                                  N.KTF_PLDA_TOPK_LARGE_MAX, u_test, u_enroll, k, (u_cohort, top_n, test_stats,
                                                                                   enroll_stats), num_examples)
 
+    def withinScores(self, u, lengths):
+        """Within-recording scores for diarization (Kaldi's ivector-plda-scoring-dense without its PCA): recording r is
+        the next `lengths[r]` rows of the transformed vectors `u` (float32 CUDA, from `transformVector`), and its
+        (n_r, n_r) float32 matrix S_r[i, j] = LLR(enrolled u_i | test u_j), each entry bit-equal to
+        `logLikelihoodRatio(u_r)[j, i]`.  Returns one view per recording into a single buffer that packs the matrices
+        one after another (the layout `diarization.agglomerative_cluster` takes without a copy); one score launch for
+        the whole batch.  float32 layers only."""
+        self._need_float32("withinScores")
+        lengths = [int(n) for n in lengths]
+        if any(n < 0 for n in lengths):
+            raise ValueError("lengths must be >= 0")
+        offsets = np.concatenate(([0], np.cumsum(lengths, dtype=np.int64))).astype(np.int64)
+        if u.dtype != torch.float32 or u.dim() != 2 or u.shape[1] != self.dim or not u.is_contiguous():
+            raise ValueError(f"u must be a contiguous float32 (n, {self.dim}) tensor")
+        if int(offsets[-1]) != u.shape[0]:
+            raise ValueError(f"lengths sum to {int(offsets[-1])}, u has {u.shape[0]} rows")
+        sizes = [n * n for n in lengths]
+        buf = torch.empty((sum(sizes),), device=u.device, dtype=torch.float32)
+        N.check(N.lib().ktf_plda_score_within(self.handle, T.ptr(u), T.host_ptr(offsets), len(lengths), T.ptr(buf),
+                                              T.stream_ptr()))
+        starts = np.concatenate(([0], np.cumsum(sizes)))
+        return [buf[int(a):int(a) + n * n].view(n, n) for a, n in zip(starts[:-1], lengths)]
+
     def call(self, inputs):
         x = T.as_device(inputs)
         self._maybe_build(x.shape)
